@@ -7,7 +7,10 @@ recurrent stack -- encoder 2 layers x T=9 + decoder horizon 3 x 2 layers = 24 ce
 reference's STCGNN.forward/backward minus MGP_Gen and out_proj -- the hot path this repo replaces.
 One "step" = forward + backward of one batch of B windows per GPU; a sample = one [T,N,C] window.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl b200|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl b200|reference] [--dump-outputs DIR]
+
+`--dump-outputs DIR` also writes what the last timed step computed (loss, stack output, every gradient) as
+DIR/<name>.npy, so that two builds can be compared output for output.
 
 Prints ONE JSON line (rank 0).  `value` = device-resident throughput; `e2e` = the same through the
 public module API with host (pinned) inputs copied in and the loss read back every step;
@@ -31,7 +34,9 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark writes nothing into the tree it runs from
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 SF = dict(N=100, C=5, h=16, Din=1, Ks=2, Kc=2, layers=2, T=9, horizon=3, grid=(10, 10))
@@ -58,7 +63,13 @@ def parse():
                         "(default batch 4 per GPU; no CPU arm)")
     p.add_argument("--cuda-graph", action="store_true",
                    help="capture the whole fwd+bwd step once and replay it (stc_gnn_b200.GraphedStep; N=1 only)")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR",
+                   help="write the last timed step's loss, stack output (a fixed sample of it above 4 M elements) and "
+                        "gradients as DIR/<name>.npy")
+    args = p.parse_args()
+    if args.steps < 1:
+        p.error("--steps must be at least 1")
+    return args
 
 
 def measured_traffic(kernel):
@@ -104,6 +115,28 @@ def synthetic_inputs(B, seed, device="cpu", pin=False):
 def loss_fn(out, y):
     """Stand-in for out_proj + loss: mean over the hidden axis, squared error against the target."""
     return (out.mean(dim=-1) - y).square().mean()
+
+
+DUMP_SAMPLE = 4 << 20      # elements kept of an output larger than this (16 MB of fp32)
+DUMP_LIMIT = 64 << 20      # bytes written by --dump-outputs in all
+
+
+def dump_outputs(path, arrays):
+    """Write {name: tensor} as path/<name>.npy in float32.  A tensor of more than DUMP_SAMPLE elements is replaced by
+    the elements at DUMP_SAMPLE positions drawn (with a fixed seed, sorted) from its flattened index range: the same
+    positions on every run with the same arguments."""
+    os.makedirs(path, exist_ok=True)
+    total = 0
+    for name, t in arrays.items():
+        t = t.detach()
+        if t.numel() > DUMP_SAMPLE:
+            idx = torch.randint(t.numel(), (DUMP_SAMPLE,), generator=torch.Generator().manual_seed(0)).sort().values
+            t = t.reshape(-1)[idx.to(t.device)]
+        a = t.float().cpu().numpy()
+        total += a.nbytes
+        if total > DUMP_LIMIT:
+            raise SystemExit(f"--dump-outputs: more than {DUMP_LIMIT} bytes")
+        np.save(os.path.join(path, f"{name}.npy"), a)
 
 
 # ------------------------------------------------------------------------------------------------
@@ -412,11 +445,19 @@ def run_b200(args):
         if bucket is not None:
             bucket.allreduce()
 
+    last = {}   # --dump-outputs: the latest step's output and loss (under --cuda-graph, the graph's static tensors)
+
+    def step_loss(X, y):
+        out = stack(Gs, Gc, X)
+        loss = loss_fn(out, y)
+        if args.dump_outputs:   # detached: a kept autograd graph would keep the leaves' AccumulateGrad nodes alive
+            last.update(out=out.detach(), loss=loss.detach())
+        return loss
+
     def step(X, y):
         for p in leaves:
             p.grad = None
-        out = stack(Gs, Gc, X)
-        loss = loss_fn(out, y)
+        loss = step_loss(X, y)
         loss.backward()
         allreduce_grads()
         return loss
@@ -456,8 +497,7 @@ def run_b200(args):
         l0 = _lib.LAUNCHES
         step(X_res, y_res)
         per_step_launches = _lib.LAUNCHES - l0
-        graphed = S.GraphedStep(lambda X, y: loss_fn(stack(Gs, Gc, X), y), [X_res, y_res], leaves,
-                                warmup=max(args.warmup, 3))
+        graphed = S.GraphedStep(step_loss, [X_res, y_res], leaves, warmup=max(args.warmup, 3))
         run_resident = lambda: graphed.replay(X_res, y_res)
     else:
         run_resident = lambda: step(X_res, y_res)
@@ -468,6 +508,11 @@ def run_b200(args):
     ms_total = timed(run_resident, args.steps)
     launches = (per_step_launches * args.steps) if graphed else (_lib.LAUNCHES - l0)
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:
+        grads = {f"grad.{n}": p.grad for n, p in stack.named_parameters() if p.grad is not None}   # unused cells: none
+        if WL is SF:
+            grads.update({"grad.Gs": Gs.grad, "grad.Gc": Gc.grad})
+        dump_outputs(args.dump_outputs, {"loss": last["loss"], "out": last["out"], **grads})
     ms_step = ms_total / args.steps
     value = B * world / (ms_step / 1e3)
 

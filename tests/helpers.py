@@ -72,11 +72,11 @@ def oracle_cell_with_grads(t, cfg, dtype=torch.float64):
 
 
 def find_reference():
-    """Directory holding the UNMODIFIED reference's framework/*.py, or None.  Probe order: $STC_REF_DIR,
-    /root/reference/framework (the build container), baseline/_ref/framework (staged by tools/stage_reference.sh; the
-    only one that can exist on the GPU box).  Tests that need the live reference skip when this returns None."""
+    """Directory holding the UNMODIFIED reference's framework/*.py, or None.  The reference is not part of this
+    repository: point $STC_REF_DIR at a checkout's framework/ directory, or stage one under baseline/_ref
+    (tools/stage_reference.sh).  Tests that need the live reference skip when this returns None."""
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    for cand in (os.environ.get("STC_REF_DIR"), "/root/reference/framework", os.path.join(root, "baseline", "_ref", "framework")):
+    for cand in (os.environ.get("STC_REF_DIR"), os.path.join(root, "baseline", "_ref", "framework")):
         if cand and os.path.isfile(os.path.join(cand, "STC_GNN.py")):
             return cand
     return None

@@ -11,9 +11,10 @@ import torch
 
 import stc_gnn_b200 as S
 from stc_gnn_b200 import _lib
+from tests.helpers import GOLDEN, find_reference
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF_DIR = os.environ.get("STC_REF_DIR", "/root/reference/framework")
+REF_DIR = find_reference()
 
 
 def header_functions():
@@ -98,7 +99,27 @@ def test_product_package_never_imports_the_oracle():
                 assert "oracle" not in text, f"{f} mentions the oracle"
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_DIR), reason="reference tree not present (GPU box)")
+def test_seeded_init_matches_reference_fixture():
+    """The reference's encoder + decoder built in fp64 under torch.manual_seed(5) at the config 5 shapes: the sum of
+    |W| over every cell (rounded to fp32) that tests/golden/stack_longc.npz stores.  A seeded RecurrentStack draws the
+    same weights only when its cells take the reference's construction order, init and shapes."""
+    import numpy as np
+    z = np.load(os.path.join(GOLDEN, "stack_longc.npz"))
+    B, T, N, C, Din, h, Ks, Kc, layers, horizon = (int(v) for v in z["meta"])
+    prev = torch.get_default_dtype()
+    torch.set_default_dtype(torch.float64)
+    try:
+        torch.manual_seed(int(z["weight_seed"]))
+        stack = S.RecurrentStack(N, C, Ks, Kc, Din, h, layers, horizon)
+    finally:
+        torch.set_default_dtype(prev)
+    sd = stack.state_dict()
+    assert all(float(v.abs().sum()) == 0.0 for k, v in sd.items() if k.endswith(".b"))
+    wsum = sum(float(v.float().double().abs().sum()) for k, v in sd.items() if k.endswith(".W"))
+    assert abs(wsum - float(z["weight_checksum"])) < 1e-12 * wsum, (wsum, float(z["weight_checksum"]))
+
+
+@pytest.mark.skipif(REF_DIR is None, reason="needs the live reference (set STC_REF_DIR)")
 def test_seeded_init_and_checkpoint_compat_with_live_reference():
     sys.dont_write_bytecode = True
     if REF_DIR not in sys.path:

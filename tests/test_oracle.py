@@ -1,16 +1,16 @@
 """CPU tests: the oracle (oracle/stc_oracle.py) against the golden vectors generated from the real
 reference (tests/golden/make_golden.py), against its own analytic backward, and -- when the reference
 tree is present (build container only) -- against the live reference."""
-import os
 import sys
 
 import pytest
 import torch
 
 from oracle import stc_oracle as O
-from tests.helpers import CELL_CASES, GRAD_KEYS, load_cell, load_pred, load_stack, oracle_cell_with_grads, random_case
+from tests.helpers import (CELL_CASES, GRAD_KEYS, find_reference, load_cell, load_pred, load_stack, oracle_cell_with_grads,
+                           random_case)
 
-REF_DIR = os.environ.get("STC_REF_DIR", "/root/reference/framework")
+REF_DIR = find_reference()
 
 
 def test_golden_files_present():
@@ -116,7 +116,7 @@ def test_grid_adjacency_matches_shipped_shape():
     assert sorted(set(A.sum(1).tolist())) == [3.0, 5.0, 8.0]
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_DIR), reason="reference tree not present (GPU box)")
+@pytest.mark.skipif(REF_DIR is None, reason="needs the live reference (set STC_REF_DIR)")
 @pytest.mark.parametrize("Ks,Kc,act", [(2, 2, None), (3, 2, "relu"), (4, 3, None)])
 def test_oracle_matches_live_reference(Ks, Kc, act):
     sys.dont_write_bytecode = True
