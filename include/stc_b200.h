@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define STC_ABI_VERSION 1
+#define STC_ABI_VERSION 2
 
 typedef enum {
   STC_OK = 0,
@@ -61,7 +61,10 @@ typedef struct {
  *   dense: vals = Gs row-major [N][N]  (vals[n*N+m] = Gs[n,m]); the other fields are ignored.
  *   CSR  : (rowptr, col, vals) is Gs in CSR (row n lists the m with Gs[n,m] != 0, used by backward),
  *          (t_rowptr, t_col, t_vals) is Gs^T in CSR (row m lists the n, used by forward).
- *          Column indices are int32; nnz < 2^31. */
+ *          Column indices are int32; nnz < 2^31.
+ *          The edge values may be learned: stc_cell_bwd then returns their gradient in Gs-CSR order (the order of
+ *          `vals`, [nnz]) through its dGs argument; the sparsity pattern itself is fixed.  An edge stored with the
+ *          value 0 is still an edge and gets a gradient. */
 typedef struct {
   int32_t kind;
   int64_t nnz;
@@ -117,7 +120,8 @@ int stc_cell_fwd_stage(const StcDims* d, int32_t stage, const float* gc,
  *   d_xt      [B][N][C][Din] contiguous, or NULL when Xt needs no gradient
  *   d_h_prev  [B][N][C][h]
  *   dWg,dbg,dWc,dbc  same shapes as the parameters (dbg/dbc NULL when has_bias == 0)
- *   dGs       [N][N] dense or NULL (must be NULL for a CSR support: constants by construction)
+ *   dGs       dense support: [N][N];  CSR support: [nnz], the gradient w.r.t. the edge values `vals` (Gs-CSR
+ *             order), computed inside the adjoint hops (stc_support_apply_edge_grad);  NULL: no support gradient
  *   dGc       [C][C] or NULL
  *   accumulate_params != 0: parameter/support gradients are ADDED to the buffers' contents
  *   (lets a time loop accumulate dW over steps); == 0: they are overwritten.
@@ -138,7 +142,8 @@ int stc_cell_bwd(const StcDims* d, const StcSupport* gs, const float* gc,
  *   dyx_terms_out [Ks-1][B][N][C][Din]: stc_cell_bwd_x writes the adjoints of those terms there and does NOT fold them:
  *                 no Xt-side adjoint hop and no Xt-side dGs contribution is launched; d_xt (if given) holds the term-0
  *                 part only.  The caller folds all timesteps at once (dGs += sum_t X_t (x) dY_1,t via
- *                 stc_support_outer, dXt += Gs dY_1 via stc_support_apply).  Both pointers go together. */
+ *                 stc_support_outer, dXt += Gs dY_1 via stc_support_apply; for a CSR support with learned edge values
+ *                 stc_support_apply_edge_grad does both).  Both pointers go together. */
 int stc_cell_fwd_x(const StcDims* d, const StcSupport* gs, const float* gc,
                    const float* xt, int64_t xt_batch_stride, const float* h_prev,
                    const float* Wg, const float* bg, const float* Wc, const float* bc,
@@ -154,6 +159,15 @@ int stc_cell_bwd_x(const StcDims* d, const StcSupport* gs, const float* gc,
  * Gs [N][N] with A = X ([B][N][width], batch stride in elements) and Bm = dL/dY ([B][N][width] contiguous). */
 int stc_support_outer(int32_t N, int32_t B, int32_t width, const float* a, int64_t a_batch_stride, const float* b,
                       float coef, float* dGs, void* stream);
+/* The same gradient for a CSR support, sampled at its edges and fused into the adjoint hop (CSR only):
+ *   y = alpha * Gs x + beta * z                                    (exactly what stc_support_apply, transpose = 0, writes)
+ *   dvals[e] += coef * sum_{b,j} a[b][row(e)][j] * x[b][col(e)][j] (e walks Gs's CSR: rowptr / col / vals order)
+ * x, z, y as in stc_support_apply; a [B][N][width] with its own batch stride (elements); dvals [nnz] is only added
+ * to.  It is what stc_cell_bwd runs for every adjoint hop when it is handed dGs for a CSR support. */
+int stc_support_apply_edge_grad(const StcSupport* gs, int32_t N, int32_t B, int32_t width,
+                                const float* x, int64_t x_batch_stride, const float* z, int64_t z_batch_stride,
+                                float* y, float alpha, float beta, const float* a, int64_t a_batch_stride, float coef,
+                                float* dvals, void* stream);
 
 /* ---- the backward split the same way (gradients through a row-partitioned graph) ----
  * Order: stage STC_STAGE_CANDI first, then STC_STAGE_GATES (the reverse of the forward).
@@ -167,7 +181,8 @@ int stc_support_outer(int32_t N, int32_t B, int32_t width, const float* a, int64
  *      finishes dGc,
  *   4. the caller folds STC_SCRATCH_DYX into d_xt and STC_SCRATCH_DYH into d_h_prev the same way.
  * Rows whose d_h_out and STC_SCRATCH_DYR term-0 entries are zero contribute nothing to any parameter gradient (that
- * is how the halo rows of an extended node set are kept out of dW).  A constant (CSR) support has no dGs.      */
+ * is how the halo rows of an extended node set are kept out of dW).  This split path has no dGs: a row-partitioned
+ * support is constant.                                                                                          */
 enum { STC_SCRATCH_DYR = 0, STC_SCRATCH_DYX, STC_SCRATCH_DYH, STC_SCRATCH_REGIONS };
 int stc_cell_bwd_scratch_layout(const StcDims* d, int64_t* offsets_floats, int32_t n_offsets);
 int stc_cell_bwd_stage(const StcDims* d, int32_t stage, const float* gc,

@@ -73,12 +73,13 @@ def _ptr(t):
 
 
 class _CellFunction(torch.autograd.Function):
-    """One cell step. Inputs that may need gradients: Gs (dense only), Gc, Xt, H, Wg, bg, Wc, bc, and -- when the
+    """One cell step. Inputs that may need gradients: Gs (dense only), Gc, Xt, H, Wg, bg, Wc, bc, -- when the
     caller hoisted the Xt-side spatial terms out of the time loop (stack.py) -- those terms `Yx` [Ks-1,B,N,C,Din], whose
-    gradient is returned un-folded."""
+    gradient is returned un-folded, and `Ev`, the edge values [nnz] of a learnable CsrSupport Gs (the support object
+    itself is not a tensor autograd can see; Ev is its `vals`)."""
 
     @staticmethod
-    def forward(ctx, Gs, Gc, Xt, H, Wg, bg, Wc, bc, Yx, cfg):
+    def forward(ctx, Gs, Gc, Xt, H, Wg, bg, Wc, bc, Yx, Ev, cfg):
         lib = _lib.load()
         Ks, Kc, act = cfg
         B, N, C, Din = Xt.shape
@@ -100,9 +101,13 @@ class _CellFunction(torch.autograd.Function):
             raise RuntimeError("gates.b and candi.b must both be present or both absent")
         csr = isinstance(Gs, CsrSupport)
         if csr:
-            gs_struct, gs_keep = Gs.struct(), Gs
             if Gs.N != N:
                 raise RuntimeError(f"CSR support has {Gs.N} nodes, Xt has {N}")
+            if Ev is not None and Ev is not Gs.vals:
+                raise RuntimeError("edge values passed to the cell must be the CsrSupport's own `vals`")
+            if Gs.learnable:   # the values may have changed since the last step (optimizer update, new with_values)
+                Gs.sync_t_vals()
+            gs_struct = Gs.struct()
         else:
             if not Gs.is_cuda or Gs.dtype != torch.float32 or Gs.shape != (N, N):
                 raise RuntimeError(f"Gs must be a float32 CUDA [N,N] tensor or a CsrSupport, got {tuple(Gs.shape)} {Gs.dtype}")
@@ -144,11 +149,12 @@ class _CellFunction(torch.autograd.Function):
         # leaves whose gradient the backward adds into `.grad` directly (index = position among forward's inputs)
         ctx.sinks = {}
         if INPLACE_LEAF_GRADS:
-            for i, t in ((0, None if csr else Gs), (1, Gc), (4, Wg), (5, bg), (6, Wc), (7, bc)):
+            for i, t in ((0, None if csr else Gs), (1, Gc), (4, Wg), (5, bg), (6, Wc), (7, bc), (9, Ev)):
                 if t is not None and ctx.needs_input_grad[i] and t.is_leaf and t.is_contiguous():
                     ctx.sinks[i] = t
+        ctx.has_ev = Ev is not None
         ctx.save_for_backward(*( [] if csr else [gs_keep] ), Gc_c, Xt_c, H_c, Wg_c, Wc_c, saved,
-                              *([Yx_c] if Yx_c is not None else []))
+                              *([Yx_c] if Yx_c is not None else []), *([Ev] if Ev is not None else []))
         return Hn
 
     @staticmethod
@@ -158,6 +164,8 @@ class _CellFunction(torch.autograd.Function):
         Ks, Kc, act = ctx.cfg
         B, N, C, Din, h = ctx.dims_tuple
         sv = list(ctx.saved_tensors)
+        if ctx.has_ev:
+            sv.pop()   # saved only so that autograd refuses a backward after an in-place change of the values
         Yx = sv.pop() if ctx.hoisted else None
         if ctx.csr:
             Gs = ctx.gs_obj
@@ -166,7 +174,7 @@ class _CellFunction(torch.autograd.Function):
         else:
             Gs, Gc, Xt, H, Wg, Wc, saved = sv
             gs_struct = dense_struct(Gs)
-        need = ctx.needs_input_grad  # Gs, Gc, Xt, H, Wg, bg, Wc, bc, Yx, cfg
+        need = ctx.needs_input_grad  # Gs, Gc, Xt, H, Wg, bg, Wc, bc, Yx, Ev, cfg
         dev = dHn.device
         dHn = dHn.contiguous()
         L, P = Din + h, Ks * Kc
@@ -178,7 +186,7 @@ class _CellFunction(torch.autograd.Function):
         dXt = new(B, N, C, Din) if need[2] else None
         dH = new(B, N, C, h)
         dYx = torch.empty_like(Yx) if ctx.hoisted else None
-        returned = [None] * 10
+        returned = [None] * 11
 
         def target(i, shape, wanted=True):
             """Buffer the kernels ADD input i's gradient into: the leaf's own `.grad` (created zeroed on first use in a
@@ -197,7 +205,8 @@ class _CellFunction(torch.autograd.Function):
 
         dWg, dWc = target(4, (P * L, 2 * h)), target(6, (P * L, h))
         dbg, dbc = target(5, (2 * h,), ctx.has_bias), target(7, (h,), ctx.has_bias)
-        dGs = target(0, (N, N), need[0] and not ctx.csr)
+        # a CSR support's gradient is that of its edge values: [nnz] in Gs-CSR order
+        dGs = target(9, (Gs.nnz,), need[9]) if ctx.csr else target(0, (N, N), need[0])
         dGc = target(1, (C, C), need[1])
         returned[2], returned[3], returned[8] = dXt, dH, dYx
         if B == 0:  # empty batch: every parameter gradient is zero (the targets are zeroed or untouched), nothing to launch
@@ -216,7 +225,7 @@ class _CellFunction(torch.autograd.Function):
             status = lib.stc_cell_bwd(*common, stream)
         _lib.check(status, "stc_cell_bwd")
         _lib.note_launches()
-        for i in (0, 1, 4, 5, 6, 7, 8):    # inputs that need no gradient get none, whatever was computed for them
+        for i in (0, 1, 4, 5, 6, 7, 8, 9):    # inputs that need no gradient get none, whatever was computed for them
             if not need[i]:
                 returned[i] = None
         return tuple(returned)
@@ -224,7 +233,13 @@ class _CellFunction(torch.autograd.Function):
 
 def stc_cell_forward(Gs, Gc, Xt, Ht_1, Wg, bg, Wc, bc, Ks: int, Kc: int, activation=None) -> torch.Tensor:
     """Functional form of the cell: H' = STC_Cell(Gs, Gc, Xt, Ht_1) with explicit weights (differentiable)."""
-    return _CellFunction.apply(Gs, Gc, Xt, Ht_1, Wg, bg, Wc, bc, None, (int(Ks), int(Kc), _activation_code(activation)))
+    return _CellFunction.apply(Gs, Gc, Xt, Ht_1, Wg, bg, Wc, bc, None, _edge_values(Gs),
+                               (int(Ks), int(Kc), _activation_code(activation)))
+
+
+def _edge_values(Gs):
+    """The edge values of a learnable CsrSupport (a tensor input of the cell, so autograd routes their gradient)."""
+    return Gs.vals if isinstance(Gs, CsrSupport) and Gs.learnable else None
 
 
 class STC_Cell(nn.Module):
@@ -265,7 +280,7 @@ class STC_Cell(nn.Module):
                                             getattr(self.candi, "b", None), self.Ks, self.Kc, _ACT_NAMES[self._act],
                                             reduce_params=getattr(Gs, "reduce_per_cell", True))
         return _CellFunction.apply(Gs, Gc, Xt, Ht_1, self.gates.W, getattr(self.gates, "b", None), self.candi.W,
-                                   getattr(self.candi, "b", None), _Yx, (self.Ks, self.Kc, self._act))
+                                   getattr(self.candi, "b", None), _Yx, _edge_values(Gs), (self.Ks, self.Kc, self._act))
 
 
 _CSR_CACHE = {}
@@ -277,8 +292,9 @@ def _csr_cache(G: torch.Tensor) -> CsrSupport:
     The entry keeps the keyed tensor alive: while it is cached its buffers cannot be freed and handed to a
     different sparse tensor at the same address, so a hit always means "this very tensor, unmodified"."""
     if G.requires_grad:
-        raise RuntimeError("STC_Cell (B200): a sparse Gs is a constant support and gets no gradient; detach it or "
-                           "pass a dense [N,N] tensor when dGs is needed")
+        raise RuntimeError("STC_Cell (B200): a torch sparse Gs is a constant support and gets no gradient; for learned "
+                           "edge weights on a fixed pattern pass CsrSupport(rowptr, col, vals_requiring_grad, N) "
+                           "(or a dense [N,N] tensor when the whole dGs is needed)")
     if G.layout == torch.sparse_csr:
         vals, idx = G.values(), G.col_indices()
     else:

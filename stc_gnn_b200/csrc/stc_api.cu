@@ -325,7 +325,7 @@ int stc_timing_collect(double* ms, int64_t* launches, double* bytes, int32_t n_k
 const char* stc_kernel_kind_name(int32_t kind) {
   static const char* names[KK_COUNT] = {"support_dense", "support_csr", "support_outer", "cheby_small",
                                         "conv_fwd",      "conv_bwd_dx", "conv_bwd_dw", "tc_conv_fwd", "tc_conv_bwd_dx", "tc_conv_bwd_dw",
-                                        "tc_support", "tc_gemm_test", "tc_outer", "tc_support_big"};
+                                        "tc_support", "tc_gemm_test", "tc_outer", "tc_support_big", "support_csr_grad"};
   return (kind >= 0 && kind < KK_COUNT) ? names[kind] : "?";
 }
 
@@ -618,6 +618,8 @@ int stc_cell_fwd_stage(const StcDims* dp, int32_t stage, const float* gc, const 
 
 // reverse of the feature-side recurrence Y_k = 2 A^T Y_{k-1} - Y_{k-2} (Y_1 = A^T Y_0) for one operand:
 //   ybar[k-1] += (k>=2 ? 2 : 1) * Gs * ybar[k];  ybar[k-2] -= ybar[k];  dGs += coef * Y_{k-1} (x) ybar[k]
+// For a CSR support dGs is the [nnz] gradient of its edge values, and that product is only needed at the edges: the
+// adjoint hop already gathers every ybar[k][b,m,:] it needs, so the hop computes it (launch_support_csr_edge_grad).
 static int adjoint_chain(const StcDims& d, const StcSupport& gs, int width, const float* y0, int64_t y0_bs,
                          const float* yk /* terms k>=1, contiguous */, float* ybar0, float* ybark /* k>=1 */,
                          float* dGs, cudaStream_t st, Lanes* lanes = nullptr, int outer_lane = 1) {
@@ -627,6 +629,15 @@ static int adjoint_chain(const StcDims& d, const StcSupport& gs, int width, cons
     const float coef = k >= 2 ? 2.f : 1.f;
     float* yb_k = ybark + (size_t)(k - 1) * Rw;
     float* yb_km1 = k == 1 ? ybar0 : ybark + (size_t)(k - 2) * Rw;
+    float* axpy = nullptr;
+    if (k >= 2) axpy = k == 2 ? ybar0 : ybark + (size_t)(k - 3) * Rw;
+    if (dGs && gs.kind == STC_SUPPORT_CSR) {
+      const float* yprev = k == 1 ? y0 : yk + (size_t)(k - 2) * Rw;
+      const int64_t yprev_bs = k == 1 ? y0_bs : nbs;
+      STC_TRY(launch_support_csr_edge_grad(gs, d.N, d.B, width, yb_k, nbs, yb_km1, nbs, yb_km1, coef, 1.f, axpy, -1.f,
+                                           yprev, yprev_bs, coef, dGs, st));
+      continue;
+    }
     if (dGs) {
       const float* yprev = k == 1 ? y0 : yk + (size_t)(k - 2) * Rw;
       const int64_t yprev_bs = k == 1 ? y0_bs : nbs;
@@ -639,8 +650,6 @@ static int adjoint_chain(const StcDims& d, const StcSupport& gs, int width, cons
       }
       STC_TRY(launch_support_outer(d.N, d.B, width, yprev, yprev_bs, yb_k, coef, dGs, so));
     }
-    float* axpy = nullptr;
-    if (k >= 2) axpy = k == 2 ? ybar0 : ybark + (size_t)(k - 3) * Rw;
     STC_TRY(launch_support_apply(gs, d.N, d.B, width, false, yb_k, nbs, yb_km1, nbs, yb_km1, coef, 1.f, axpy, -1.f,
                                  st));
   }
@@ -694,7 +703,9 @@ static int check_bwd_args(const StcDims* dp, const float* gc, const float* xt, c
 }
 
 // zero the parameter / support gradients unless the caller accumulates over a time loop; zero the dT_k(Gc) partials
-static int bwd_begin(const BwdCtx& b, float* dWg, float* dbg, float* dWc, float* dbc, float* dGs, int accumulate_params) {
+// (dGs holds dGs_floats: N*N for a dense support, nnz for a CSR support)
+static int bwd_begin(const BwdCtx& b, float* dWg, float* dbg, float* dWc, float* dbc, float* dGs, size_t dGs_floats,
+                     int accumulate_params) {
   const StcDims& d = b.d;
   const int L = d.Din + d.h, P = d.Ks * d.Kc;
   if (!accumulate_params) {
@@ -704,7 +715,7 @@ static int bwd_begin(const BwdCtx& b, float* dWg, float* dbg, float* dWc, float*
       STC_CUDA_OK(cudaMemsetAsync(dbg, 0, sizeof(float) * 2 * d.h, b.st));
       STC_CUDA_OK(cudaMemsetAsync(dbc, 0, sizeof(float) * d.h, b.st));
     }
-    if (dGs) STC_CUDA_OK(cudaMemsetAsync(dGs, 0, sizeof(float) * d.N * d.N, b.st));
+    if (dGs && dGs_floats) STC_CUDA_OK(cudaMemsetAsync(dGs, 0, sizeof(float) * dGs_floats, b.st));
     if (b.dGc) STC_CUDA_OK(cudaMemsetAsync(b.dGc, 0, sizeof(float) * d.C * d.C, b.st));
   }
   if (d.B > 0 && b.want_dGc()) STC_CUDA_OK(cudaMemsetAsync(b.sc + b.w.dQ, 0, sizeof(float) * d.Kc * d.C * d.C, b.st));
@@ -794,8 +805,8 @@ static int cell_bwd_impl(const StcDims* dp, const StcSupport* gs, const float* g
     set_error("%s: NULL argument", who);
     return STC_ERR_BAD_ARG;
   }
-  if (dGs && gs->kind != STC_SUPPORT_DENSE) {
-    set_error("%s: dGs is only defined for a dense support", who);
+  if (dGs && gs->kind == STC_SUPPORT_CSR && (!gs->rowptr || !gs->col || !gs->vals || gs->nnz < 0)) {
+    set_error("%s: the edge-value gradient of a CSR support needs its rowptr/col/vals and nnz", who);
     return STC_ERR_BAD_ARG;
   }
   if (d.Ks > 1 && ((yx_terms != nullptr) != (dyx_terms_out != nullptr))) {
@@ -814,7 +825,8 @@ static int cell_bwd_impl(const StcDims* dp, const StcSupport* gs, const float* g
     b.yx_pre = yx_terms;
     b.dyx_out = dyx_terms_out;
   }
-  STC_TRY(bwd_begin(b, dWg, dbg, dWc, dbc, dGs, accumulate_params));
+  const size_t dGs_floats = gs->kind == STC_SUPPORT_CSR ? (size_t)gs->nnz : (size_t)d.N * d.N;
+  STC_TRY(bwd_begin(b, dWg, dbg, dWc, dbc, dGs, dGs_floats, accumulate_params));
   if (d.B == 0) return STC_OK;
   const size_t Rh = w.R * d.h;
   const int CD = d.C * d.Din, CH = d.C * d.h;
@@ -872,6 +884,24 @@ int stc_support_outer(int32_t N, int32_t B, int32_t width, const float* a, int64
   return launch_support_outer(N, B, width, a, a_batch_stride, b, coef, dGs, (cudaStream_t)stream);
 }
 
+int stc_support_apply_edge_grad(const StcSupport* gs, int32_t N, int32_t B, int32_t width, const float* x,
+                                int64_t x_batch_stride, const float* z, int64_t z_batch_stride, float* y, float alpha,
+                                float beta, const float* a, int64_t a_batch_stride, float coef, float* dvals,
+                                void* stream) {
+  reset_launch_count();
+  if (!gs || !x || !y || !a || !dvals) {
+    set_error("stc_support_apply_edge_grad: NULL argument");
+    return STC_ERR_BAD_ARG;
+  }
+  if (gs->kind != STC_SUPPORT_CSR) {
+    set_error("stc_support_apply_edge_grad: CSR supports only (a dense support's gradient is stc_support_outer)");
+    return STC_ERR_UNSUPPORTED;
+  }
+  STC_TRY(check_arch());
+  return launch_support_csr_edge_grad(*gs, N, B, width, x, x_batch_stride, z, z_batch_stride, y, alpha, beta, nullptr,
+                                      0.f, a, a_batch_stride, coef, dvals, (cudaStream_t)stream);
+}
+
 int stc_cell_bwd_scratch_layout(const StcDims* dp, int64_t* offsets, int32_t n_offsets) {
   STC_TRY(check_dims(dp));
   if (!offsets || n_offsets < STC_SCRATCH_REGIONS) {
@@ -906,7 +936,7 @@ int stc_cell_bwd_stage(const StcDims* dp, int32_t stage, const float* gc, const 
   const BwdCtx b{d, w, gc, xt, xt_batch_stride, h_prev, d_h_out, d_xt, d_h_prev, dGc,
                  const_cast<float*>((const float*)savedv), (float*)scratchv, (cudaStream_t)stream};
   if (stage == STC_STAGE_CANDI) {   // the first backward stage: also clears the gradients it and the gates stage add into
-    STC_TRY(bwd_begin(b, dWg, dbg, dWc, dbc, nullptr, accumulate_params));
+    STC_TRY(bwd_begin(b, dWg, dbg, dWc, dbc, nullptr, 0, accumulate_params));
     if (d.B == 0) return STC_OK;
     return bwd_candi(b, Wc, dWc, dbc);
   }

@@ -42,7 +42,8 @@ void reset_launch_count();
 // ---- optional per-kernel timing (stc_timing_* in the ABI) ---------------------------------------
 enum KernelKind {
   KK_SUPPORT_DENSE = 0, KK_SUPPORT_CSR, KK_SUPPORT_OUTER, KK_CHEBY_SMALL, KK_CONV_FWD, KK_CONV_BWD_DX,
-  KK_CONV_BWD_DW, KK_TC_CONV_FWD, KK_TC_CONV_BWD_DX, KK_TC_CONV_BWD_DW, KK_TC_SUPPORT, KK_TC_GEMM_TEST, KK_TC_OUTER, KK_TC_SUPPORT_BIG, KK_COUNT
+  KK_CONV_BWD_DW, KK_TC_CONV_FWD, KK_TC_CONV_BWD_DX, KK_TC_CONV_BWD_DW, KK_TC_SUPPORT, KK_TC_GEMM_TEST, KK_TC_OUTER, KK_TC_SUPPORT_BIG,
+  KK_SUPPORT_CSR_GRAD, KK_COUNT
 };
 struct ScopedKernelTimer {  // declare right before a launch; the destructor records the stop event
   ScopedKernelTimer(int kind, cudaStream_t st, double alg_bytes);
@@ -110,6 +111,13 @@ int try_launch_support_tc_big(const float* G, int N, int B, int width, bool tran
                               bool* handled);
 int try_launch_outer_tc(int N, int B, int width, const float* a, int64_t a_bs, const float* bmat, float coef, float* dG,
                         cudaStream_t st, bool* handled);
+
+// adjoint hop y = alpha * Gs x + beta * z (+ the Chebyshev axpy) of a CSR support with the edge-value gradient fused in:
+// dvals[e = (n,m)] += coef * sum_{b,j} a[b,n,j] * x[b,m,j]  (dvals in the order of gs.rowptr / gs.col / gs.vals)
+int launch_support_csr_edge_grad(const StcSupport& gs, int N, int B, int width, const float* x, int64_t x_bs,
+                                 const float* z, int64_t z_bs, float* y, float alpha, float beta, float* axpy_out,
+                                 float axpy_coef, const float* a, int64_t a_bs, float coef, float* dvals,
+                                 cudaStream_t st);
 
 int launch_support_outer(int N, int B, int width, const float* a, int64_t a_bs, const float* bmat, float coef,
                          float* dG, cudaStream_t st);

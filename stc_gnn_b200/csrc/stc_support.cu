@@ -2,7 +2,9 @@
 //
 //  support_dense_kernel  Y = alpha * A X + beta * Z with A = Gs^T (forward, 'bncl,nm->bmcl',
 //                        /root/reference/framework/STC_GNN.py:37) or A = Gs (adjoint, used by backward).
-//  support_csr_kernel    same operator for a CSR support (one warp per (batch, node) row slab).
+//  support_csr_kernel    same operator for a CSR support (one warp per (batch, node) row slab).  GRAD = true: the
+//                        adjoint hop with the gradient of the edge values fused in (learnable CSR supports),
+//                        dvals[e = (n,m)] += coef * sum_{b,j} A[b,n,j] * X[b,m,j]; Y is computed exactly as without it.
 //  support_outer_kernel  dGs[n',m] += coef * sum_{b,j} A[b,n',j] * Bm[b,m,j]  (gradient of the spatial
 //                        mode product w.r.t. the support; reference gets it from autograd of :37).
 //  cheby_small_*         matrix-space Chebyshev terms of the small C x C categorical support and their
@@ -119,12 +121,24 @@ axpy_rows_kernel(float* __restrict__ out, const float* __restrict__ x, long long
 // ------------------------------------------------------------------------------------------------
 // CSR support: one warp per (b, m) output row slab; lanes sweep the contiguous `width` axis
 // ------------------------------------------------------------------------------------------------
-template <int VEC>
+// Edge-value gradient fused into the hop (GRAD): the warp keeps its own row's slab chunk A[b,n,j0..] in registers; every
+// gathered neighbour slab X[b,m,:] is dotted with it, warp-reduced and added to dvals[e] with one atomic per
+// (b, column chunk, edge).  That costs one extra read of the row's own slab instead of a second gather of the
+// neighbours (a separate sampled dense x dense product).  The hop's accumulators are untouched by it.
+struct CsrEdgeGrad {
+  const float* a;   // [B][N][W], batch stride a_bs (elements)
+  long long a_bs;
+  float coef;
+  float* dvals;     // [nnz], in the order of the walked CSR (rowptr / col)
+};
+
+template <int VEC, bool GRAD>
 __global__ void __launch_bounds__(256)
 support_csr_kernel(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ col,
                    const float* __restrict__ vals, int N, long long rows_total, const float* __restrict__ X,
                    long long x_bs, const float* Z, long long z_bs, float* Y, int W, float alpha, float beta,
-                   float* axpy_out, float axpy_coef, const int32_t* __restrict__ row_list, int n_list) {
+                   float* axpy_out, float axpy_coef, const int32_t* __restrict__ row_list, int n_list,
+                   CsrEdgeGrad eg) {
   // row_list != nullptr: only the n_list output nodes it names are computed (rows_total = B * n_list); the other
   // rows of Y are not touched (the row-partitioned path computes interior rows while the halo exchange is in flight)
   constexpr int U = 4;  // independent accumulators per lane per pass
@@ -144,9 +158,28 @@ support_csr_kernel(const int32_t* __restrict__ rowptr, const int32_t* __restrict
       for (int u = 0; u < U; ++u)
 #pragma unroll
         for (int v = 0; v < VEC; ++v) acc[u][v] = 0.f;
+      float ar[GRAD ? U : 1][VEC];   // this row's own slab chunk (GRAD only)
+      if (GRAD) {
+        const float* arow = eg.a + b * eg.a_bs + (long long)m * W;
+#pragma unroll
+        for (int u = 0; u < (GRAD ? U : 1); ++u) {
+          int j = j0 + (u * 32 + lane) * VEC;
+#pragma unroll
+          for (int v = 0; v < VEC; ++v) ar[u][v] = 0.f;
+          if (j < W) {
+            if (VEC == 4) {
+              float4 t = *reinterpret_cast<const float4*>(arow + j);
+              ar[u][0] = t.x; ar[u][1 % VEC] = t.y; ar[u][2 % VEC] = t.z; ar[u][3 % VEC] = t.w;
+            } else {
+              ar[u][0] = arow[j];
+            }
+          }
+        }
+      }
       for (int e = e0; e < e1; ++e) {
         const float g = vals[e];
         const float* xr = xb + (long long)col[e] * W;
+        float dot = 0.f;
 #pragma unroll
         for (int u = 0; u < U; ++u) {
           int j = j0 + (u * 32 + lane) * VEC;
@@ -157,10 +190,24 @@ support_csr_kernel(const int32_t* __restrict__ rowptr, const int32_t* __restrict
               acc[u][1 % VEC] = fmaf(g, x.y, acc[u][1 % VEC]);
               acc[u][2 % VEC] = fmaf(g, x.z, acc[u][2 % VEC]);
               acc[u][3 % VEC] = fmaf(g, x.w, acc[u][3 % VEC]);
+              if (GRAD) {
+                const int ug = GRAD ? u : 0;
+                dot = fmaf(ar[ug][0], x.x, dot);
+                dot = fmaf(ar[ug][1 % VEC], x.y, dot);
+                dot = fmaf(ar[ug][2 % VEC], x.z, dot);
+                dot = fmaf(ar[ug][3 % VEC], x.w, dot);
+              }
             } else {
-              acc[u][0] = fmaf(g, xr[j], acc[u][0]);
+              const float x = xr[j];
+              acc[u][0] = fmaf(g, x, acc[u][0]);
+              if (GRAD) dot = fmaf(ar[GRAD ? u : 0][0], x, dot);
             }
           }
+        }
+        if (GRAD) {
+#pragma unroll
+          for (int o = 16; o > 0; o >>= 1) dot += __shfl_xor_sync(0xffffffffu, dot, o);
+          if (lane == 0) atomicAdd(eg.dvals + e, eg.coef * dot);
         }
       }
 #pragma unroll
@@ -192,6 +239,40 @@ support_csr_kernel(const int32_t* __restrict__ rowptr, const int32_t* __restrict
 }
 
 static bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
+
+// one CSR hop (rp, ci, va walk the rows of the operator applied); eg.dvals != nullptr selects the edge-gradient variant
+static int launch_csr(const int32_t* rp, const int32_t* ci, const float* va, long long nnz, int N, int B, int width,
+                      const float* x, int64_t x_bs, const float* z, int64_t z_bs, float* y, float alpha, float beta,
+                      float* axpy_out, float axpy_coef, const int32_t* row_list, int n_list, const CsrEdgeGrad& eg,
+                      cudaStream_t st) {
+  const bool grad = eg.dvals != nullptr;
+  long long rows_total = (long long)B * (row_list ? n_list : N);
+  bool vec = (width % 4 == 0) && (x_bs % 4 == 0) && (z == nullptr || z_bs % 4 == 0) && aligned16(x) &&
+             aligned16(y) && (z == nullptr || aligned16(z)) && (axpy_out == nullptr || aligned16(axpy_out)) &&
+             (!grad || (eg.a_bs % 4 == 0 && aligned16(eg.a)));
+  int warps_per_block = 8;
+  long long want = (rows_total + warps_per_block - 1) / warps_per_block;
+  int grid = (int)(want < (long long)device_sm_count() * 16 ? want : (long long)device_sm_count() * 16);
+  if (grid < 1) grid = 1;
+  // compulsory traffic of the hop; the edge-gradient variant also reads the row's own slab of A and updates dvals
+  const double hop = 4.0 * rows_total * width * (2 + (beta != 0.f ? 1 : 0) + (axpy_out ? 2 : 0)) + 8.0 * nnz + 4.0 * (N + 1);
+  ScopedKernelTimer _t(grad ? KK_SUPPORT_CSR_GRAD : KK_SUPPORT_CSR, st, grad ? hop + 4.0 * rows_total * width + 4.0 * nnz : hop);
+  const dim3 blk(warps_per_block * 32);
+#define STC_CSR_LAUNCH(V, G)                                                                                        \
+  support_csr_kernel<V, G><<<grid, blk, 0, st>>>(rp, ci, va, N, rows_total, x, x_bs, z, z_bs, y, width, alpha, beta, \
+                                                 axpy_out, axpy_coef, row_list, n_list, eg)
+  if (grad) {
+    if (vec) STC_CSR_LAUNCH(4, true);
+    else STC_CSR_LAUNCH(1, true);
+    STC_LAUNCH_OK("support_csr_kernel<grad>");
+  } else {
+    if (vec) STC_CSR_LAUNCH(4, false);
+    else STC_CSR_LAUNCH(1, false);
+    STC_LAUNCH_OK("support_csr_kernel");
+  }
+#undef STC_CSR_LAUNCH
+  return STC_OK;
+}
 
 int launch_support_apply(const StcSupport& gs, int N, int B, int width, bool transpose, const float* x,
                          int64_t x_bs, const float* z, int64_t z_bs, float* y, float alpha, float beta,
@@ -262,23 +343,29 @@ int launch_support_apply(const StcSupport& gs, int N, int B, int width, bool tra
     set_error("CSR support needs both Gs and Gs^T (rowptr/col/vals and t_rowptr/t_col/t_vals)");
     return STC_ERR_BAD_ARG;
   }
-  long long rows_total = (long long)B * (row_list ? n_list : N);
-  bool vec = (width % 4 == 0) && (x_bs % 4 == 0) && (z == nullptr || z_bs % 4 == 0) && aligned16(x) &&
-             aligned16(y) && (z == nullptr || aligned16(z)) && (axpy_out == nullptr || aligned16(axpy_out));
-  int warps_per_block = 8;
-  long long want = (rows_total + warps_per_block - 1) / warps_per_block;
-  int grid = (int)(want < (long long)device_sm_count() * 16 ? want : (long long)device_sm_count() * 16);
-  if (grid < 1) grid = 1;
-  ScopedKernelTimer _t(KK_SUPPORT_CSR, st,
-                       4.0 * rows_total * width * (2 + (beta != 0.f ? 1 : 0) + (axpy_out ? 2 : 0)) + 8.0 * gs.nnz + 4.0 * (N + 1));
-  if (vec)
-    support_csr_kernel<4><<<grid, warps_per_block * 32, 0, st>>>(rp, ci, va, N, rows_total, x, x_bs, z, z_bs, y,
-                                                                  width, alpha, beta, axpy_out, axpy_coef, row_list, n_list);
-  else
-    support_csr_kernel<1><<<grid, warps_per_block * 32, 0, st>>>(rp, ci, va, N, rows_total, x, x_bs, z, z_bs, y,
-                                                                  width, alpha, beta, axpy_out, axpy_coef, row_list, n_list);
-  STC_LAUNCH_OK("support_csr_kernel");
-  return STC_OK;
+  return launch_csr(rp, ci, va, gs.nnz, N, B, width, x, x_bs, z, z_bs, y, alpha, beta, axpy_out, axpy_coef, row_list,
+                    n_list, CsrEdgeGrad{nullptr, 0, 0.f, nullptr}, st);
+}
+
+int launch_support_csr_edge_grad(const StcSupport& gs, int N, int B, int width, const float* x, int64_t x_bs,
+                                 const float* z, int64_t z_bs, float* y, float alpha, float beta, float* axpy_out,
+                                 float axpy_coef, const float* a, int64_t a_bs, float coef, float* dvals,
+                                 cudaStream_t st) {
+  if (B <= 0 || N <= 0 || width <= 0) return STC_OK;
+  if (gs.kind != STC_SUPPORT_CSR || !gs.rowptr || !gs.col || !gs.vals) {
+    set_error("support edge gradient: needs a CSR support with rowptr/col/vals");
+    return STC_ERR_BAD_ARG;
+  }
+  if (!a || !dvals) {
+    set_error("support edge gradient: NULL a or dvals");
+    return STC_ERR_BAD_ARG;
+  }
+  if (beta != 0.f && z == nullptr) {
+    set_error("support_apply: beta != 0 needs z");
+    return STC_ERR_BAD_ARG;
+  }
+  return launch_csr(gs.rowptr, gs.col, gs.vals, gs.nnz, N, B, width, x, x_bs, z, z_bs, y, alpha, beta, axpy_out,
+                    axpy_coef, nullptr, 0, CsrEdgeGrad{a, (long long)a_bs, coef, dvals}, st);
 }
 
 // ------------------------------------------------------------------------------------------------
