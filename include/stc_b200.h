@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define STC_ABI_VERSION 2
+#define STC_ABI_VERSION 3
 
 typedef enum {
   STC_OK = 0,
@@ -168,6 +168,14 @@ int stc_support_apply_edge_grad(const StcSupport* gs, int32_t N, int32_t B, int3
                                 const float* x, int64_t x_batch_stride, const float* z, int64_t z_batch_stride,
                                 float* y, float alpha, float beta, const float* a, int64_t a_batch_stride, float coef,
                                 float* dvals, void* stream);
+/* The same fused hop restricted to the rows n listed in rows[n_rows] (int32, device), like stc_support_apply_rows:
+ * only those rows of y are written (the others are not touched), only the edges of those rows get a gradient, and a
+ * is read at those rows only.  The row-partitioned path (stc_gnn_b200/halo.py) runs it on the interior rows while the
+ * halo exchange is in flight, then on the boundary rows, when the partitioned support's edge values are learned. */
+int stc_support_apply_rows_edge_grad(const StcSupport* gs, int32_t N, int32_t B, int32_t width,
+                                     const float* x, int64_t x_batch_stride, const float* z, int64_t z_batch_stride,
+                                     float* y, float alpha, float beta, const float* a, int64_t a_batch_stride,
+                                     float coef, float* dvals, const int32_t* rows, int32_t n_rows, void* stream);
 
 /* ---- the backward split the same way (gradients through a row-partitioned graph) ----
  * Order: stage STC_STAGE_CANDI first, then STC_STAGE_GATES (the reverse of the forward).
@@ -181,8 +189,9 @@ int stc_support_apply_edge_grad(const StcSupport* gs, int32_t N, int32_t B, int3
  *      finishes dGc,
  *   4. the caller folds STC_SCRATCH_DYX into d_xt and STC_SCRATCH_DYH into d_h_prev the same way.
  * Rows whose d_h_out and STC_SCRATCH_DYR term-0 entries are zero contribute nothing to any parameter gradient (that
- * is how the halo rows of an extended node set are kept out of dW).  This split path has no dGs: a row-partitioned
- * support is constant.                                                                                          */
+ * is how the halo rows of an extended node set are kept out of dW).  The stages take no dGs: when the support's edge
+ * values are learned, the caller forms their gradient inside its adjoint hops (steps 2 and 4) with
+ * stc_support_apply_edge_grad / stc_support_apply_rows_edge_grad, A = the matching forward terms of `saved`.      */
 enum { STC_SCRATCH_DYR = 0, STC_SCRATCH_DYX, STC_SCRATCH_DYH, STC_SCRATCH_REGIONS };
 int stc_cell_bwd_scratch_layout(const StcDims* d, int64_t* offsets_floats, int32_t n_offsets);
 int stc_cell_bwd_stage(const StcDims* d, int32_t stage, const float* gc,

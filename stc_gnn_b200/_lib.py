@@ -10,7 +10,7 @@ from ctypes import POINTER, Structure, c_char_p, c_float, c_int, c_int32, c_int6
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "libstc_b200.so")
 
-ABI_VERSION = 2
+ABI_VERSION = 3
 ACT_NONE, ACT_RELU = 0, 1
 SUPPORT_DENSE, SUPPORT_CSR = 0, 1
 
@@ -23,6 +23,7 @@ EXPORTED = (
     "stc_cell_bwd_scratch_layout", "stc_cell_bwd_stage",
     "stc_support_apply_rows", "stc_halo_pack", "stc_halo_unpack", "stc_concurrency_set",
     "stc_cell_fwd_x", "stc_cell_bwd_x", "stc_support_outer", "stc_support_apply_edge_grad",
+    "stc_support_apply_rows_edge_grad",
 )
 STAGE_GATES, STAGE_CANDI = 0, 1
 SAVED_REGIONS = ("u", "r", "c", "Yr", "Yx", "Yh", "Q", "Pg", "Pc")
@@ -70,6 +71,9 @@ def load(build_if_missing: bool = True):
     lib.stc_support_apply_edge_grad.argtypes = [POINTER(StcSupport), c_int32, c_int32, c_int32, c_void_p, c_int64,
                                                 c_void_p, c_int64, c_void_p, c_float, c_float, c_void_p, c_int64,
                                                 c_float, c_void_p, c_void_p]
+    lib.stc_support_apply_rows_edge_grad.restype = c_int
+    lib.stc_support_apply_rows_edge_grad.argtypes = lib.stc_support_apply_edge_grad.argtypes[:-1] + [c_void_p, c_int32,
+                                                                                                    c_void_p]
     lib.stc_cell_saved_layout.restype = c_int
     lib.stc_cell_saved_layout.argtypes = [POINTER(StcDims), POINTER(c_int64), c_int32]
     lib.stc_cell_fwd_stage.restype = c_int

@@ -902,6 +902,28 @@ int stc_support_apply_edge_grad(const StcSupport* gs, int32_t N, int32_t B, int3
                                       0.f, a, a_batch_stride, coef, dvals, (cudaStream_t)stream);
 }
 
+int stc_support_apply_rows_edge_grad(const StcSupport* gs, int32_t N, int32_t B, int32_t width, const float* x,
+                                     int64_t x_batch_stride, const float* z, int64_t z_batch_stride, float* y,
+                                     float alpha, float beta, const float* a, int64_t a_batch_stride, float coef,
+                                     float* dvals, const int32_t* rows, int32_t n_rows, void* stream) {
+  reset_launch_count();
+  if (!gs || !x || !y || !a || !dvals || !rows) {
+    set_error("stc_support_apply_rows_edge_grad: NULL argument");
+    return STC_ERR_BAD_ARG;
+  }
+  if (gs->kind != STC_SUPPORT_CSR) {
+    set_error("stc_support_apply_rows_edge_grad: CSR supports only");
+    return STC_ERR_UNSUPPORTED;
+  }
+  if (n_rows < 0 || n_rows > N) {
+    set_error("stc_support_apply_rows_edge_grad: n_rows %d outside [0, N = %d]", n_rows, N);
+    return STC_ERR_BAD_ARG;
+  }
+  STC_TRY(check_arch());
+  return launch_support_csr_edge_grad(*gs, N, B, width, x, x_batch_stride, z, z_batch_stride, y, alpha, beta, nullptr,
+                                      0.f, a, a_batch_stride, coef, dvals, (cudaStream_t)stream, rows, n_rows);
+}
+
 int stc_cell_bwd_scratch_layout(const StcDims* dp, int64_t* offsets, int32_t n_offsets) {
   STC_TRY(check_dims(dp));
   if (!offsets || n_offsets < STC_SCRATCH_REGIONS) {

@@ -113,11 +113,12 @@ int try_launch_outer_tc(int N, int B, int width, const float* a, int64_t a_bs, c
                         cudaStream_t st, bool* handled);
 
 // adjoint hop y = alpha * Gs x + beta * z (+ the Chebyshev axpy) of a CSR support with the edge-value gradient fused in:
-// dvals[e = (n,m)] += coef * sum_{b,j} a[b,n,j] * x[b,m,j]  (dvals in the order of gs.rowptr / gs.col / gs.vals)
+// dvals[e = (n,m)] += coef * sum_{b,j} a[b,n,j] * x[b,m,j]  (dvals in the order of gs.rowptr / gs.col / gs.vals).
+// row_list != nullptr: only the n_list rows n it names are computed, and only their edges get a gradient.
 int launch_support_csr_edge_grad(const StcSupport& gs, int N, int B, int width, const float* x, int64_t x_bs,
                                  const float* z, int64_t z_bs, float* y, float alpha, float beta, float* axpy_out,
                                  float axpy_coef, const float* a, int64_t a_bs, float coef, float* dvals,
-                                 cudaStream_t st);
+                                 cudaStream_t st, const int32_t* row_list = nullptr, int n_list = 0);
 
 int launch_support_outer(int N, int B, int width, const float* a, int64_t a_bs, const float* bmat, float coef,
                          float* dG, cudaStream_t st);

@@ -140,7 +140,8 @@ support_csr_kernel(const int32_t* __restrict__ rowptr, const int32_t* __restrict
                    float* axpy_out, float axpy_coef, const int32_t* __restrict__ row_list, int n_list,
                    CsrEdgeGrad eg) {
   // row_list != nullptr: only the n_list output nodes it names are computed (rows_total = B * n_list); the other
-  // rows of Y are not touched (the row-partitioned path computes interior rows while the halo exchange is in flight)
+  // rows of Y are not touched (the row-partitioned path computes interior rows while the halo exchange is in flight);
+  // with GRAD only the edges of the listed rows get a gradient, and A is read at the listed rows only
   constexpr int U = 4;  // independent accumulators per lane per pass
   const int lane = threadIdx.x & 31;
   const long long warp0 = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
@@ -350,8 +351,9 @@ int launch_support_apply(const StcSupport& gs, int N, int B, int width, bool tra
 int launch_support_csr_edge_grad(const StcSupport& gs, int N, int B, int width, const float* x, int64_t x_bs,
                                  const float* z, int64_t z_bs, float* y, float alpha, float beta, float* axpy_out,
                                  float axpy_coef, const float* a, int64_t a_bs, float coef, float* dvals,
-                                 cudaStream_t st) {
+                                 cudaStream_t st, const int32_t* row_list, int n_list) {
   if (B <= 0 || N <= 0 || width <= 0) return STC_OK;
+  if (row_list && n_list <= 0) return STC_OK;
   if (gs.kind != STC_SUPPORT_CSR || !gs.rowptr || !gs.col || !gs.vals) {
     set_error("support edge gradient: needs a CSR support with rowptr/col/vals");
     return STC_ERR_BAD_ARG;
@@ -365,7 +367,7 @@ int launch_support_csr_edge_grad(const StcSupport& gs, int N, int B, int width, 
     return STC_ERR_BAD_ARG;
   }
   return launch_csr(gs.rowptr, gs.col, gs.vals, gs.nnz, N, B, width, x, x_bs, z, z_bs, y, alpha, beta, axpy_out,
-                    axpy_coef, nullptr, 0, CsrEdgeGrad{a, (long long)a_bs, coef, dvals}, st);
+                    axpy_coef, row_list, n_list, CsrEdgeGrad{a, (long long)a_bs, coef, dvals}, st);
 }
 
 // ------------------------------------------------------------------------------------------------

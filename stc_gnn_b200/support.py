@@ -163,11 +163,12 @@ def support_apply(Gs, X: torch.Tensor, transpose: bool = True, alpha: float = 1.
 
 def support_apply_edge_grad(Gs: CsrSupport, X: torch.Tensor, A: torch.Tensor, dvals: torch.Tensor, coef: float = 1.0,
                             alpha: float = 1.0, beta: float = 0.0, Z: torch.Tensor = None,
-                            out: torch.Tensor = None) -> torch.Tensor:
+                            out: torch.Tensor = None, rows: torch.Tensor = None) -> torch.Tensor:
     """The adjoint hop Y = alpha * Gs X + beta * Z of a CSR support with the gradient of its edge values fused in:
     dvals[e = (n, m)] += coef * sum_{b,...} A[b,n,...] * X[b,m,...]  (dvals [nnz] float32, Gs-CSR order; only added
     to).  Y is what support_apply(Gs, X, transpose=False, ...) returns.  A ([B,N,...] like X) may be a batch-strided
-    view whose per-sample slab is contiguous.  CUDA only."""
+    view whose per-sample slab is contiguous.  `rows` (int32 CUDA tensor; needs `out`): compute just those output
+    nodes n, leave every other row of `out` untouched, and add the gradient of those rows' edges only.  CUDA only."""
     lib = _lib.load()
     if not isinstance(Gs, CsrSupport):
         raise RuntimeError("support_apply_edge_grad: CSR supports only (a dense support's gradient is stc_support_outer)")
@@ -187,9 +188,16 @@ def support_apply_edge_grad(Gs: CsrSupport, X: torch.Tensor, A: torch.Tensor, dv
     if Y.shape != Xc.shape or not Y.is_contiguous():
         raise RuntimeError("support_apply_edge_grad: `out` must be a contiguous tensor of X's shape")
     zc = Z.contiguous() if Z is not None else None
-    status = lib.stc_support_apply_edge_grad(Gs.struct(), N, B, width, Xc.data_ptr(), N * width,
-                                             zc.data_ptr() if zc is not None else None, N * width, Y.data_ptr(),
-                                             float(alpha), float(beta), Ac.data_ptr(), a_bs, float(coef),
-                                             dvals.data_ptr(), torch.cuda.current_stream().cuda_stream)
-    _lib.check(status, "stc_support_apply_edge_grad")
+    common = (Gs.struct(), N, B, width, Xc.data_ptr(), N * width, zc.data_ptr() if zc is not None else None, N * width,
+              Y.data_ptr(), float(alpha), float(beta), Ac.data_ptr(), a_bs, float(coef), dvals.data_ptr())
+    stream = torch.cuda.current_stream().cuda_stream
+    if rows is not None:
+        if rows.dtype != torch.int32 or not rows.is_cuda or not rows.is_contiguous():
+            raise RuntimeError("support_apply_edge_grad: `rows` must be a contiguous int32 CUDA tensor")
+        if out is None:
+            raise RuntimeError("support_apply_edge_grad: `rows` needs `out` (the other rows keep their contents)")
+        _lib.check(lib.stc_support_apply_rows_edge_grad(*common, rows.data_ptr(), rows.numel(), stream),
+                   "stc_support_apply_rows_edge_grad")
+        return Y
+    _lib.check(lib.stc_support_apply_edge_grad(*common, stream), "stc_support_apply_edge_grad")
     return Y

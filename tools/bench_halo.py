@@ -10,9 +10,20 @@ the adjoint hops with their own halo exchanges; the parameter gradients are all-
 partitioned result (outputs and every gradient) against the unpartitioned cell run on the same GPU -> `parity_ok`.
 
 Strong scaling: the global problem is fixed, each rank owns N / world nodes.  Time = max over ranks (CUDA events,
-barrier on both sides).  Rank 0 prints one JSON line."""
+barrier on both sides).  Rank 0 prints one JSON line.
+
+`--train --learned`: the same training step with learnable edge values (an `nn.Parameter` [nnz] behind the
+partitioned support, its gradient formed inside the adjoint hops) and with the constant support, in one process,
+alternating ROUNDS times; both reduce their gradients once per step in a flat bucket (the learnable one also holds
+the [nnz] edge gradient).  It runs the partitioned path at every world size, world 1 included, and reports
+median / min / max ms of each, their ratio, nnz, the bucket sizes, and the device's name, power limit and maximum SM
+clock.  At world > 1, `parity_ok` also covers the edge gradient against the unpartitioned learnable cell.
+`--gloo`: every rank on cuda:0, exchanging over gloo -- a full-size parity check of the partitioned path on a
+machine with one GPU; its times measure ranks sharing one GPU, not scaling."""
 import json
 import os
+import statistics
+import subprocess
 import sys
 
 import torch
@@ -33,6 +44,107 @@ def violations(got, ref, atol_scale):
     return int((err > 1e-4 * ref.abs() + atol_scale * scale).sum()), float(err.max() / scale)
 
 
+def learned_main(B, world, rank, dev):
+    """--train --learned: learnable vs constant partitioned training step (see the module docstring)."""
+    N, C, F, Ks, Kc, ROUNDS, iters = 65536, 8, 64, 4, 2, 7, 10
+    rp, ci, va = knn_csr(N, 8)
+    torch.manual_seed(0)
+    cell = S.STC_Cell(N, C, Ks, Kc, F, F).to(dev)
+    params = list(cell.parameters())
+    Gc = (torch.rand(C, C, generator=torch.Generator().manual_seed(1)) / C).to(dev).requires_grad_(True)
+    g = torch.Generator().manual_seed(100)
+    Xg = torch.randn(B, N, C, F, generator=g)
+    Hg = torch.randn(B, N, C, F, generator=g) * 0.5
+    dHg = torch.randn(B, N, C, F, generator=g)
+    # non-uniform values, identical on every rank (one seed)
+    vals = torch.nn.Parameter((va * (0.5 + torch.rand(va.numel(), generator=torch.Generator().manual_seed(7)))).to(dev))
+    const = PartitionedSupport(rp, ci, vals.detach().cpu(), N, rank, world)
+    learned = const.with_values(vals)
+    lo, n = const.start, const.nloc
+    blk = lambda t: t[:, lo:lo + n].contiguous().to(dev)
+    X, H, dHn = blk(Xg).requires_grad_(True), blk(Hg).requires_grad_(True), blk(dHg)
+    buckets = {"constant": S.dp.GradBucket(params + [Gc]), "learnable": S.dp.GradBucket(params + [Gc, vals])}
+    sups = {"constant": const, "learnable": learned}
+
+    def step(which):
+        def run():
+            for t in (X, H, vals, Gc, *params):
+                t.grad = None
+            out = partitioned_cell_forward(sups[which], Gc, X, H, cell.gates.W, cell.gates.b, cell.candi.W,
+                                           cell.candi.b, Ks, Kc, reduce_params=False)
+            out.backward(dHn)
+            buckets[which].allreduce()       # ONE gradient all-reduce per step (a no-op at world 1)
+            return out
+        return run
+
+    variants = {k: step(k) for k in sups}
+    parity = None
+    if world > 1:
+        # this rank's block of the partitioned result == the unpartitioned learnable cell on the same GPU
+        out_p = variants["learnable"]().detach().clone()
+        got = [out_p, X.grad.clone(), H.grad.clone()] + [t.grad.clone() for t in params + [Gc, vals]]
+        full = S.CsrSupport(rp.to(dev), ci.to(dev), vals, N)
+        Xf, Hf = Xg.to(dev).requires_grad_(True), Hg.to(dev).requires_grad_(True)
+        for t in params + [Gc, vals]:
+            t.grad = None
+        out_f = cell(Gs=full, Gc=Gc, Xt=Xf, Ht_1=Hf)
+        out_f.backward(dHg.to(dev))
+        want = [out_f.detach()[:, lo:lo + n], Xf.grad[:, lo:lo + n], Hf.grad[:, lo:lo + n]] + \
+               [t.grad.clone() for t in params + [Gc, vals]]
+        names = ["H'", "dXt", "dH", "dWg", "dbg", "dWc", "dbc", "dGc", "dvals"]
+        worst, nbad = {}, 0
+        for nm, a_, b_ in zip(names, got, want):
+            # reduced gradients sum B*N*C = 1 M rows (dvals: B*C*F = 1,024 products per edge) in another order
+            nb, w = violations(a_, b_, 1e-5 if nm in ("H'", "dXt", "dH") else 3e-5)
+            worst[nm] = w
+            nbad += nb
+        flag = torch.tensor([float(nbad)], device=dev)
+        dist.all_reduce(flag)
+        parity = {"parity_ok": float(flag.item()) == 0.0, "worst_err_over_mean_ref_rank0": worst}
+        del Xf, Hf, out_f, want, got, full
+        torch.cuda.empty_cache()
+
+    for fn in variants.values():
+        for _ in range(3):
+            fn()
+    torch.cuda.synchronize()
+    samples = {k: [] for k in variants}
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    for _ in range(ROUNDS):
+        for k, fn in variants.items():
+            if world > 1:
+                dist.barrier()
+            e0.record()
+            for _ in range(iters):
+                fn()
+            e1.record()
+            torch.cuda.synchronize()
+            samples[k].append(e0.elapsed_time(e1) / iters)
+    if world > 1:                            # time of a round = the slowest rank's
+        for k in samples:
+            t = torch.tensor(samples[k], device=dev)
+            dist.all_reduce(t, op=dist.ReduceOp.MAX)
+            samples[k] = t.tolist()
+    if rank == 0:
+        try:
+            smi = subprocess.run(["nvidia-smi", "--query-gpu=power.limit,clocks.max.sm", "--format=csv,noheader"],
+                                 capture_output=True, text=True, timeout=30).stdout.strip().splitlines()[0]
+        except Exception as e:  # the measurement still stands, but says that the limit is unknown
+            smi = f"unavailable: {e!r}"
+        summ = lambda v: {"median": statistics.median(v), "min": min(v), "max": max(v)}
+        backend = dist.get_backend() if world > 1 else None
+        rec = {"kind": "config4_cell_step_partitioned_learned", "n_gpus": 1 if backend in (None, "gloo") else world,
+               "n_ranks": world, "backend": backend, "device": torch.cuda.get_device_name(dev),
+               "power_limit_and_max_sm_clock": smi, "N": N, "C": C, "F": F, "Ks": Ks, "Kc": Kc, "B": B, "nnz": learned.nnz,
+               "local_rows": n, "fwd_halo_rows": const.fwd.nhalo, "rounds": ROUNDS, "steps_per_round": iters,
+               "constant_ms": summ(samples["constant"]), "learnable_ms": summ(samples["learnable"]),
+               "ratio_learnable_over_constant": statistics.median(samples["learnable"]) / statistics.median(samples["constant"]),
+               "bucket_floats_constant": buckets["constant"].numel, "bucket_floats_learnable": buckets["learnable"].numel}
+        if parity:
+            rec.update(parity)
+        print(json.dumps(rec), flush=True)
+
+
 def main():
     train = "--train" in sys.argv
     per_cell = "--reduce-per-cell" in sys.argv
@@ -40,12 +152,24 @@ def main():
     B = int(pos[0]) if pos else 2
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
-    local = int(os.environ.get("LOCAL_RANK", "0"))
+    gloo = "--gloo" in sys.argv
+    local = 0 if gloo else int(os.environ.get("LOCAL_RANK", "0"))
     torch.cuda.set_device(local)
     dev = torch.device("cuda", local)
     if world > 1:
-        dist.init_process_group("nccl", device_id=dev)
+        if gloo:
+            dist.init_process_group("gloo")
+        else:
+            dist.init_process_group("nccl", device_id=dev)
     _lib.load()
+    if "--learned" in sys.argv:
+        if not train:
+            raise SystemExit("--learned measures the training step: pass --train as well")
+        learned_main(B, world, rank, dev)
+        if world > 1:
+            dist.barrier()
+            dist.destroy_process_group()
+        return
     N, C, F, Ks, Kc = 65536, 8, 64, 4, 2
     rp, ci, va = knn_csr(N, 8)
     torch.manual_seed(0)
