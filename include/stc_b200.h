@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define STC_ABI_VERSION 3
+#define STC_ABI_VERSION 4
 
 typedef enum {
   STC_OK = 0,
@@ -176,6 +176,23 @@ int stc_support_apply_rows_edge_grad(const StcSupport* gs, int32_t N, int32_t B,
                                      const float* x, int64_t x_batch_stride, const float* z, int64_t z_batch_stride,
                                      float* y, float alpha, float beta, const float* a, int64_t a_batch_stride,
                                      float coef, float* dvals, const int32_t* rows, int32_t n_rows, void* stream);
+
+/* ---- graph generator on a fixed CSR pattern (the sparse form of MGP_Gen's spatial half, STC_GNN.py:227-233) ----
+ * gs is a CSR support whose rowptr / col give the pattern; its vals (and the Gs^T fields) are ignored.
+ * u, v [N][width] row-major (node-major: width = B*T*hg, the generator's tanh(alpha X Wu), tanh(alpha X Wv)).
+ * stc_pair_scores_csr:  scores[e] = <u[n], v[m]> - <v[n], u[m]>  for every stored edge e = (n, m), in Gs-CSR order
+ *                       (M[n,m] - M[m,n] of the dense generator at the stored edges; a self-loop scores exactly 0).
+ * stc_edge_softmax_fwd: p[e] = exp(relu(scores[e]) - max) / sum over the stored edges e' of row n of
+ *                       exp(relu(scores[e']) - max); entries off the pattern take no part; an empty row writes nothing.
+ * stc_edge_softmax_bwd: dscores[e] = [scores[e] > 0] * p[e] * (dp[e] - sum_{e' in row n} p[e'] dp[e']).
+ * All three are deterministic (no atomics: a second call gives bitwise the same output).  The gradient of the scores
+ * needs no export: with D = the pattern carrying dscores, du = (D - D^T) v and dv = (D^T - D) u, two
+ * stc_support_apply hops each (transpose = 0 walks D, transpose = 1 walks D^T). */
+int stc_pair_scores_csr(const StcSupport* gs, int32_t N, int64_t width, const float* u, const float* v,
+                        float* scores, void* stream);
+int stc_edge_softmax_fwd(const StcSupport* gs, int32_t N, const float* scores, float* p, void* stream);
+int stc_edge_softmax_bwd(const StcSupport* gs, int32_t N, const float* scores, const float* p, const float* dp,
+                         float* dscores, void* stream);
 
 /* ---- the backward split the same way (gradients through a row-partitioned graph) ----
  * Order: stage STC_STAGE_CANDI first, then STC_STAGE_GATES (the reverse of the forward).

@@ -6,6 +6,8 @@ Public surface:
   CsrSupport          sparse spatial support: fixed pattern, constant or learnable edge values
   support_apply       the spatial mode product on its own
   support_apply_edge_grad  the adjoint CSR hop with the edge-value gradient fused in
+  SparseGraphGenerator  the reference's spatial graph generator on a fixed CSR pattern (returns a learnable CsrSupport)
+  pair_softmax_csr    its differentiable core: row softmax of relu(<U_n,V_m> - <V_n,U_m>) over the stored edges
   install / run_main  rebind STC_GNN.STC_Cell so Model_Trainer.py / Main.py run unchanged
   dp                  batch data-parallel gradient bucket (one flat all-reduce per step)
   halo                row-partitioned CSR support with per-hop halo exchange
@@ -16,4 +18,5 @@ from .support import CsrSupport, support_apply, support_apply_edge_grad  # noqa:
 from .install import install, run_main  # noqa: F401
 from .stack import RecurrentStack  # noqa: F401
 from .graph import GraphedStep  # noqa: F401
+from .sparse_mgp import SparseGraphGenerator, pair_softmax_csr  # noqa: F401
 from . import dp, halo, mgp  # noqa: F401

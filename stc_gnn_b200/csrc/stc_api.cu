@@ -325,7 +325,8 @@ int stc_timing_collect(double* ms, int64_t* launches, double* bytes, int32_t n_k
 const char* stc_kernel_kind_name(int32_t kind) {
   static const char* names[KK_COUNT] = {"support_dense", "support_csr", "support_outer", "cheby_small",
                                         "conv_fwd",      "conv_bwd_dx", "conv_bwd_dw", "tc_conv_fwd", "tc_conv_bwd_dx", "tc_conv_bwd_dw",
-                                        "tc_support", "tc_gemm_test", "tc_outer", "tc_support_big", "support_csr_grad"};
+                                        "tc_support", "tc_gemm_test", "tc_outer", "tc_support_big", "support_csr_grad",
+                                        "pair_scores_csr", "edge_softmax"};
   return (kind >= 0 && kind < KK_COUNT) ? names[kind] : "?";
 }
 
@@ -922,6 +923,65 @@ int stc_support_apply_rows_edge_grad(const StcSupport* gs, int32_t N, int32_t B,
   STC_TRY(check_arch());
   return launch_support_csr_edge_grad(*gs, N, B, width, x, x_batch_stride, z, z_batch_stride, y, alpha, beta, nullptr,
                                       0.f, a, a_batch_stride, coef, dvals, (cudaStream_t)stream, rows, n_rows);
+}
+
+static int check_pattern(const StcSupport* gs, int32_t N, const char* who) {
+  if (!gs) {
+    set_error("%s: NULL pattern", who);
+    return STC_ERR_BAD_ARG;
+  }
+  if (gs->kind != STC_SUPPORT_CSR) {
+    set_error("%s: the pattern must be a CSR support (kind %d)", who, gs->kind);
+    return STC_ERR_UNSUPPORTED;
+  }
+  if (!gs->rowptr || !gs->col || gs->nnz < 0) {
+    set_error("%s: the pattern needs rowptr / col and nnz >= 0", who);
+    return STC_ERR_BAD_ARG;
+  }
+  if (N <= 0) {
+    set_error("%s: N = %d must be positive", who, N);
+    return STC_ERR_BAD_ARG;
+  }
+  return STC_OK;
+}
+
+int stc_pair_scores_csr(const StcSupport* gs, int32_t N, int64_t width, const float* u, const float* v, float* scores,
+                        void* stream) {
+  reset_launch_count();
+  STC_TRY(check_pattern(gs, N, "stc_pair_scores_csr"));
+  if (!u || !v || !scores) {
+    set_error("stc_pair_scores_csr: NULL argument");
+    return STC_ERR_BAD_ARG;
+  }
+  if (width <= 0) {
+    set_error("stc_pair_scores_csr: width = %lld must be positive", (long long)width);
+    return STC_ERR_BAD_ARG;
+  }
+  STC_TRY(check_arch());
+  return launch_pair_scores_csr(gs->rowptr, gs->col, gs->nnz, N, width, u, v, scores, (cudaStream_t)stream);
+}
+
+int stc_edge_softmax_fwd(const StcSupport* gs, int32_t N, const float* scores, float* p, void* stream) {
+  reset_launch_count();
+  STC_TRY(check_pattern(gs, N, "stc_edge_softmax_fwd"));
+  if (!scores || !p) {
+    set_error("stc_edge_softmax_fwd: NULL argument");
+    return STC_ERR_BAD_ARG;
+  }
+  STC_TRY(check_arch());
+  return launch_edge_softmax(false, gs->rowptr, gs->nnz, N, scores, nullptr, nullptr, p, (cudaStream_t)stream);
+}
+
+int stc_edge_softmax_bwd(const StcSupport* gs, int32_t N, const float* scores, const float* p, const float* dp,
+                         float* dscores, void* stream) {
+  reset_launch_count();
+  STC_TRY(check_pattern(gs, N, "stc_edge_softmax_bwd"));
+  if (!scores || !p || !dp || !dscores) {
+    set_error("stc_edge_softmax_bwd: NULL argument");
+    return STC_ERR_BAD_ARG;
+  }
+  STC_TRY(check_arch());
+  return launch_edge_softmax(true, gs->rowptr, gs->nnz, N, scores, p, dp, dscores, (cudaStream_t)stream);
 }
 
 int stc_cell_bwd_scratch_layout(const StcDims* dp, int64_t* offsets, int32_t n_offsets) {

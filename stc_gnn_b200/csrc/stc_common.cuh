@@ -43,7 +43,7 @@ void reset_launch_count();
 enum KernelKind {
   KK_SUPPORT_DENSE = 0, KK_SUPPORT_CSR, KK_SUPPORT_OUTER, KK_CHEBY_SMALL, KK_CONV_FWD, KK_CONV_BWD_DX,
   KK_CONV_BWD_DW, KK_TC_CONV_FWD, KK_TC_CONV_BWD_DX, KK_TC_CONV_BWD_DW, KK_TC_SUPPORT, KK_TC_GEMM_TEST, KK_TC_OUTER, KK_TC_SUPPORT_BIG,
-  KK_SUPPORT_CSR_GRAD, KK_COUNT
+  KK_SUPPORT_CSR_GRAD, KK_PAIR_SCORES_CSR, KK_EDGE_SOFTMAX, KK_COUNT
 };
 struct ScopedKernelTimer {  // declare right before a launch; the destructor records the stop event
   ScopedKernelTimer(int kind, cudaStream_t st, double alg_bytes);
@@ -122,6 +122,13 @@ int launch_support_csr_edge_grad(const StcSupport& gs, int N, int B, int width, 
 
 int launch_support_outer(int N, int B, int width, const float* a, int64_t a_bs, const float* bmat, float coef,
                          float* dG, cudaStream_t st);
+
+// graph generator on a fixed CSR pattern (stc_pair_graph.cu): scores S[e = (n,m)] = <U_n,V_m> - <V_n,U_m> and the
+// softmax of relu(S) over each row's stored edges (bwd: dS from S, P, dP into `out`)
+int launch_pair_scores_csr(const int32_t* rowptr, const int32_t* col, long long nnz, int N, long long width,
+                           const float* u, const float* v, float* scores, cudaStream_t st);
+int launch_edge_softmax(bool bwd, const int32_t* rowptr, long long nnz, int N, const float* s, const float* p,
+                        const float* dp, float* out, cudaStream_t st);
 
 int launch_cheby_small(const float* G, int C, int K, float* Q, cudaStream_t st);
 int launch_cheby_small_bwd(const float* G, const float* Q, float* dQ, int C, int K, float* dG, cudaStream_t st);
