@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define STC_ABI_VERSION 4
+#define STC_ABI_VERSION 5
 
 typedef enum {
   STC_OK = 0,
@@ -190,6 +190,14 @@ int stc_support_apply_rows_edge_grad(const StcSupport* gs, int32_t N, int32_t B,
  * stc_support_apply hops each (transpose = 0 walks D, transpose = 1 walks D^T). */
 int stc_pair_scores_csr(const StcSupport* gs, int32_t N, int64_t width, const float* u, const float* v,
                         float* scores, void* stream);
+/* stc_pair_scores_csr restricted to the rows n listed in rows[n_rows] (int32, device): only the scores of those rows'
+ * edges are written (every other entry of `scores` is not touched), each bitwise what stc_pair_scores_csr writes for
+ * it.  u and v rows are ld >= width floats apart (u[n] = u + n * ld), so U and V may be the two halves of one
+ * [N][2 * width] buffer.  Rejects ld < width; n_rows == 0 launches nothing.  The row-partitioned generator
+ * (stc_gnn_b200/sparse_mgp.py) scores the rows of its local operator whose neighbours are all local while the halo
+ * exchange of [U | V] is in flight, then the others. */
+int stc_pair_scores_csr_rows(const StcSupport* gs, int32_t N, int64_t width, int64_t ld, const float* u, const float* v,
+                             float* scores, const int32_t* rows, int32_t n_rows, void* stream);
 int stc_edge_softmax_fwd(const StcSupport* gs, int32_t N, const float* scores, float* p, void* stream);
 int stc_edge_softmax_bwd(const StcSupport* gs, int32_t N, const float* scores, const float* p, const float* dp,
                          float* dscores, void* stream);

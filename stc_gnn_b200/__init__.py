@@ -18,5 +18,5 @@ from .support import CsrSupport, support_apply, support_apply_edge_grad  # noqa:
 from .install import install, run_main  # noqa: F401
 from .stack import RecurrentStack  # noqa: F401
 from .graph import GraphedStep  # noqa: F401
-from .sparse_mgp import SparseGraphGenerator, pair_softmax_csr  # noqa: F401
+from .sparse_mgp import SparseGraphGenerator, pair_softmax_csr, pair_softmax_partitioned  # noqa: F401
 from . import dp, halo, mgp  # noqa: F401

@@ -961,6 +961,32 @@ int stc_pair_scores_csr(const StcSupport* gs, int32_t N, int64_t width, const fl
   return launch_pair_scores_csr(gs->rowptr, gs->col, gs->nnz, N, width, u, v, scores, (cudaStream_t)stream);
 }
 
+int stc_pair_scores_csr_rows(const StcSupport* gs, int32_t N, int64_t width, int64_t ld, const float* u, const float* v,
+                             float* scores, const int32_t* rows, int32_t n_rows, void* stream) {
+  reset_launch_count();
+  STC_TRY(check_pattern(gs, N, "stc_pair_scores_csr_rows"));
+  if (!u || !v || !scores || !rows) {
+    set_error("stc_pair_scores_csr_rows: NULL argument");
+    return STC_ERR_BAD_ARG;
+  }
+  if (width <= 0) {
+    set_error("stc_pair_scores_csr_rows: width = %lld must be positive", (long long)width);
+    return STC_ERR_BAD_ARG;
+  }
+  if (ld < width) {
+    set_error("stc_pair_scores_csr_rows: row stride ld = %lld is smaller than width = %lld", (long long)ld,
+              (long long)width);
+    return STC_ERR_BAD_ARG;
+  }
+  if (n_rows < 0 || n_rows > N) {
+    set_error("stc_pair_scores_csr_rows: n_rows %d outside [0, N = %d]", n_rows, N);
+    return STC_ERR_BAD_ARG;
+  }
+  STC_TRY(check_arch());
+  return launch_pair_scores_csr_rows(gs->rowptr, gs->col, gs->nnz, N, width, ld, u, v, scores, rows, n_rows,
+                                     (cudaStream_t)stream);
+}
+
 int stc_edge_softmax_fwd(const StcSupport* gs, int32_t N, const float* scores, float* p, void* stream) {
   reset_launch_count();
   STC_TRY(check_pattern(gs, N, "stc_edge_softmax_fwd"));

@@ -127,6 +127,10 @@ int launch_support_outer(int N, int B, int width, const float* a, int64_t a_bs, 
 // softmax of relu(S) over each row's stored edges (bwd: dS from S, P, dP into `out`)
 int launch_pair_scores_csr(const int32_t* rowptr, const int32_t* col, long long nnz, int N, long long width,
                            const float* u, const float* v, float* scores, cudaStream_t st);
+// the same restricted to the rows listed in rows[n_rows] (the others are not written); u, v rows are ld >= width apart
+int launch_pair_scores_csr_rows(const int32_t* rowptr, const int32_t* col, long long nnz, int N, long long width,
+                                long long ld, const float* u, const float* v, float* scores, const int32_t* rows,
+                                int n_rows, cudaStream_t st);
 int launch_edge_softmax(bool bwd, const int32_t* rowptr, long long nnz, int N, const float* s, const float* p,
                         const float* dp, float* out, cudaStream_t st);
 

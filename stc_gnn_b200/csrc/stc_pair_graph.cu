@@ -31,18 +31,25 @@ static int csr_warp_grid(long long rows, int warps_per_block) {
 constexpr int PS_U = 4;   // float(4)s per lane and operand in one column chunk
 constexpr int PS_E = 4;   // edges of one group (8 spills at VEC = 4; the grid and kNN patterns store 8-10 edges a row)
 
-template <int VEC>
+//
+// ROWS: only the n_rows rows listed in `rows` are scored (the other entries of `scores` are not touched), and U / V
+// have the row stride ld >= W, so that U and V can share one extended buffer [U | V] (the row-partitioned generator,
+// stc_gnn_b200/sparse_mgp.py).  A listed row's arithmetic is the plain kernel's, so its scores are bitwise the same.
+template <int VEC, bool ROWS>
 __global__ void __launch_bounds__(256)
 pair_scores_csr_kernel(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ col, int N, long long W,
-                       const float* __restrict__ U, const float* __restrict__ V, float* __restrict__ scores) {
+                       const float* __restrict__ U, const float* __restrict__ V, float* __restrict__ scores,
+                       long long ld, const int32_t* __restrict__ rows, int n_rows) {
   constexpr long long CHUNK = 32LL * VEC * PS_U;
+  const long long LD = ROWS ? ld : W;
   const int lane = threadIdx.x & 31;
   const long long warp0 = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const long long nwarps = ((long long)gridDim.x * blockDim.x) >> 5;
-  for (long long n = warp0; n < N; n += nwarps) {
+  for (long long i = warp0; i < (ROWS ? n_rows : N); i += nwarps) {
+    const long long n = ROWS ? rows[i] : i;
     const int e0 = rowptr[n], e1 = rowptr[n + 1];
-    const float* un = U + n * W;
-    const float* vn = V + n * W;
+    const float* un = U + n * LD;
+    const float* vn = V + n * LD;
     for (int g0 = e0; g0 < e1; g0 += PS_E) {
       const int cnt = min(PS_E, e1 - g0);
       int nb[PS_E];
@@ -72,8 +79,8 @@ pair_scores_csr_kernel(const int32_t* __restrict__ rowptr, const int32_t* __rest
 #pragma unroll
         for (int k = 0; k < PS_E; ++k) {
           if (k >= cnt) break;
-          const float* um = U + nb[k] * W;
-          const float* vm = V + nb[k] * W;
+          const float* um = U + nb[k] * LD;
+          const float* vm = V + nb[k] * LD;
 #pragma unroll
           for (int u = 0; u < PS_U; ++u) {
             const long long j = j0 + (long long)(u * 32 + lane) * VEC;
@@ -113,9 +120,26 @@ int launch_pair_scores_csr(const int32_t* rowptr, const int32_t* col, long long 
   // are L2 hits of rows other warps have just read.
   ScopedKernelTimer _t(KK_PAIR_SCORES_CSR, st,
                        4.0 * 2 * N * width + 4.0 * 2 * width * nnz + 8.0 * nnz + 4.0 * (N + 1) + 4.0 * nnz);
-  if (vec) pair_scores_csr_kernel<4><<<grid, 256, 0, st>>>(rowptr, col, N, width, u, v, scores);
-  else pair_scores_csr_kernel<1><<<grid, 256, 0, st>>>(rowptr, col, N, width, u, v, scores);
+  if (vec) pair_scores_csr_kernel<4, false><<<grid, 256, 0, st>>>(rowptr, col, N, width, u, v, scores, width, nullptr, 0);
+  else pair_scores_csr_kernel<1, false><<<grid, 256, 0, st>>>(rowptr, col, N, width, u, v, scores, width, nullptr, 0);
   STC_LAUNCH_OK("pair_scores_csr_kernel");
+  return STC_OK;
+}
+
+int launch_pair_scores_csr_rows(const int32_t* rowptr, const int32_t* col, long long nnz, int N, long long width,
+                                long long ld, const float* u, const float* v, float* scores, const int32_t* rows,
+                                int n_rows, cudaStream_t st) {
+  if (n_rows <= 0) return STC_OK;
+  const bool vec = (width % 4 == 0) && (ld % 4 == 0) && aligned16(u) && aligned16(v);
+  const int grid = csr_warp_grid(n_rows, 8);
+  // the plain kernel's count for the listed rows; their edge count is not known on the host, so it is taken at the
+  // pattern's mean degree (nnz / N edges a row), plus the row list itself
+  const double er = (double)nnz * n_rows / N;
+  ScopedKernelTimer _t(KK_PAIR_SCORES_CSR, st,
+                       4.0 * 2 * n_rows * width + 4.0 * 2 * width * er + 4.0 * er + 8.0 * n_rows + 4.0 * er + 4.0 * n_rows);
+  if (vec) pair_scores_csr_kernel<4, true><<<grid, 256, 0, st>>>(rowptr, col, N, width, u, v, scores, ld, rows, n_rows);
+  else pair_scores_csr_kernel<1, true><<<grid, 256, 0, st>>>(rowptr, col, N, width, u, v, scores, ld, rows, n_rows);
+  STC_LAUNCH_OK("pair_scores_csr_kernel<rows>");
   return STC_OK;
 }
 

@@ -154,7 +154,10 @@ class ValueMaps:
       bwd (operator Gs): rows = this rank's nodes n, edges in global Gs-CSR order.  Its values are the slice
           vals[edge_lo:edge_hi] and its edge gradient is the same slice of the global [nnz] gradient.
       fwd (operator Gs^T): rows = this rank's nodes m, edges sorted by (m, global n) as in `CsrSupport.t_perm`; edge i
-          is global edge fwd_ids[i], so its values are vals[fwd_ids]."""
+          is global edge fwd_ids[i], so its values are vals[fwd_ids].
+    Gather layout of an [nnz] vector whose slices [edge_lo:edge_hi] live on their ranks (`gather_edges`): every rank's
+    slice is padded to `edge_pad` floats, so rank r's slice lands at [r * edge_pad, r * edge_pad + hi_r - lo_r) of the
+    all-gathered buffer; `edge_bounds[r]` = (lo_r, hi_r)."""
     edge_lo: int
     edge_hi: int
     bwd_rowptr: torch.Tensor
@@ -162,6 +165,14 @@ class ValueMaps:
     fwd_rowptr: torch.Tensor
     fwd_col: torch.Tensor
     fwd_ids: torch.Tensor
+    edge_bounds: List[tuple]
+    edge_pad: int
+
+    def padded_index(self, ids: torch.Tensor) -> torch.Tensor:
+        """Positions in the padded all-gather buffer of the global edges `ids` (host, integer arithmetic)."""
+        lo = torch.tensor([b[0] for b in self.edge_bounds], dtype=torch.long)
+        owner = torch.bucketize(ids, lo[1:], right=True)
+        return owner * self.edge_pad + (ids - lo[owner])
 
 
 def _csr_operator(rowptr: torch.Tensor, col: torch.Tensor, vals: torch.Tensor, n: int):
@@ -256,9 +267,12 @@ class PartitionedSupport:
             ids = mine[torch.sort((col[mine] - s) * N + row[mine], stable=True).indices]
             f_rowptr = torch.zeros(nloc + 1, dtype=torch.long)
             f_rowptr[1:] = torch.cumsum(torch.bincount(col[ids] - s, minlength=nloc), 0)
+            bounds = [(int(rowptr[a]), int(rowptr[b])) for a, b in (shard_bounds(N, r, self.world)
+                                                                    for r in range(self.world))]
             m = self._dev["maps"] = ValueMaps(edge_lo=lo, edge_hi=hi, bwd_rowptr=pad(rowptr[s:e + 1] - lo),
                                               bwd_col=ext(col[lo:hi]), fwd_rowptr=pad(f_rowptr), fwd_col=ext(row[ids]),
-                                              fwd_ids=ids)
+                                              fwd_ids=ids, edge_bounds=bounds,
+                                              edge_pad=max(b - a for a, b in bounds))
         return m
 
     def sync_values(self, device) -> None:
@@ -272,19 +286,32 @@ class PartitionedSupport:
         return X.narrow(node_dim, self.start, self.nloc)
 
     # -- device form of the local operators (square, padded with empty rows so the square C-ABI kernel applies) --
+    def _operator_structure(self, direction: str, device):
+        """(rowptr, col, forward map or None) of the local operator of `direction` (see ValueMaps), on the device."""
+        skey = ("learned", direction, str(device))
+        st = self._dev.get(skey)
+        if st is None:
+            m = self.maps()
+            rp, c = (m.fwd_rowptr, m.fwd_col) if direction == "fwd" else (m.bwd_rowptr, m.bwd_col)
+            ids = m.fwd_ids.to(device) if direction == "fwd" else None
+            st = self._dev[skey] = (rp.to(torch.int32).to(device), c.to(torch.int32).to(device), ids)
+        return st
+
+    def local_operator(self, direction: str, vals: torch.Tensor):
+        """The local operator of `direction` (see ValueMaps) carrying `vals` (float32, on the device: 'bwd' the
+        [edge_hi - edge_lo] edges of this rank's rows in Gs-CSR order, 'fwd' the edges fwd_ids), as a CsrSupport that
+        is applied with transpose=False over the extended node set.  Only the pattern is read when it is handed to the
+        generator's kernels."""
+        rp, c, _ = self._operator_structure(direction, vals.device)
+        return _csr_operator(rp, c, vals, self.fwd.next)
+
     def _learned_operator(self, direction: str, device):
         """(local operator bound to `vals`, forward map on the device or None)."""
         key = (direction, str(device))
         hit = self._ops.get(key)
         if hit is None:
-            skey = ("learned", direction, str(device))
-            st = self._dev.get(skey)
             m = self.maps()
-            if st is None:
-                rp, c = (m.fwd_rowptr, m.fwd_col) if direction == "fwd" else (m.bwd_rowptr, m.bwd_col)
-                ids = m.fwd_ids.to(device) if direction == "fwd" else None
-                st = self._dev[skey] = (rp.to(torch.int32).to(device), c.to(torch.int32).to(device), ids)
-            rp, c, ids = st
+            rp, c, ids = self._operator_structure(direction, device)
             v = self.vals.detach()
             if not v.is_cuda or v.dtype != torch.float32 or not v.is_contiguous() or v.device != torch.device(device):
                 raise RuntimeError(f"PartitionedSupport: learnable values must be a contiguous float32 tensor on {device}, "
@@ -383,19 +410,17 @@ class PartitionedSupport:
         boundary rows into a persistent send buffer, one NCCL all-to-all of packed rows, `stc_halo_unpack` into the halo
         rows -- while the main stream already computes the INTERIOR output rows (those whose neighbours are all local,
         `stc_support_apply_rows`); the main stream then waits for the exchange and computes the boundary rows.  No
-        tensor is copied, sliced or allocated per hop.
+        tensor is copied, sliced or allocated per hop (`_overlapped`).
 
         Edge-gradient form (learnable support, direction 'bwd'): `dvals` is this rank's slice
         [edge_lo:edge_hi] of the global [nnz] gradient, and both launches also add
         dvals[e = (n, m)] += coef * sum A_ext[:, n] * X_ext[:, m]  (A_ext [B, nloc + nhalo, ...] the forward term the hop's
         adjoint belongs to; read at the local rows only).  A learnable forward hop reads the values `sync_values` last
         gathered."""
-        from . import _lib
         from .support import support_apply, support_apply_edge_grad
         plan = self.fwd if direction == "fwd" else self.bwd
         B = X_ext.shape[0]
         X3 = X_ext.view(B, plan.next, -1)
-        W = X3.shape[-1]
         out3 = out_ext.view(B, plan.next, -1)
         Z3 = None if Z_ext is None else Z_ext.view(B, plan.next, -1)
         sup = self.device_support(direction, X_ext.device)
@@ -408,14 +433,28 @@ class PartitionedSupport:
         else:
             tr = self.transposed(direction)
             hop = lambda rows=None: support_apply(sup, X3, transpose=tr, alpha=alpha, beta=beta, Z=Z3, out=out3, rows=rows)
+        self._overlapped(direction, X3, hop)
+
+    def _overlapped(self, direction: str, X3: torch.Tensor, launch: Callable[[Optional[torch.Tensor]], None]) -> None:
+        """The exchange-overlap skeleton of every computation on an extended tensor X3 [B, nloc + nhalo, W] whose output
+        rows read their neighbours' rows of X3 through the local operator of `direction`.
+
+        The halo rows of X3 are refreshed in place ON A SIDE STREAM -- `stc_halo_pack` of the boundary rows into a
+        persistent send buffer, one all-to-all of packed rows, `stc_halo_unpack` into the halo rows -- while the main
+        stream runs `launch(interior rows)` (the rows whose neighbours are all local); the main stream then waits for
+        the exchange and runs `launch(boundary rows)` (the rows reading a halo row, and the halo rows).  The row lists
+        are int32 device tensors.  At world 1 it is `launch(None)`: every row, nothing exchanged."""
+        from . import _lib
+        plan = self.fwd if direction == "fwd" else self.bwd
         if plan.world == 1:
-            hop()
+            launch(None)
             return
+        B, _, W = X3.shape
         lib = _lib.load()
-        st = self._device_state(direction, X_ext.device)
-        send, recv = self._buffers(st, plan, B * W, X_ext.device)
+        st = self._device_state(direction, X3.device)
+        send, recv = self._buffers(st, plan, B * W, X3.device)
         main, side = torch.cuda.current_stream(), st["side"]
-        st["ready"].record(main)                     # X_ext's local rows are final once the main stream gets here
+        st["ready"].record(main)                     # X3's local rows are final once the main stream gets here
         with torch.cuda.stream(side):
             side.wait_event(st["ready"])
             _lib.check(lib.stc_halo_pack(X3.data_ptr(), plan.next * W, W, B, st["send_idx"].data_ptr(), st["nsend"],
@@ -426,9 +465,9 @@ class PartitionedSupport:
                                            side.cuda_stream), "stc_halo_unpack")
             st["done"].record(side)
         if st["interior"].numel():
-            hop(st["interior"])
+            launch(st["interior"])
         main.wait_event(st["done"])
-        hop(st["boundary"])
+        launch(st["boundary"])
 
     def spatial_terms(self, X_local: torch.Tensor, Ks: int, apply_fn=None) -> List[torch.Tensor]:
         """Feature-side Chebyshev terms Y_0..Y_{Ks-1} of this rank's block (Y_1 = Gs^T Y_0, Y_k = 2 Gs^T Y_{k-1} - Y_{k-2};
@@ -465,6 +504,50 @@ def adjoint_chain_ext(ps: PartitionedSupport, ybar: List[torch.Tensor], hop: Opt
         if k >= 2:
             ybar[k - 2][:, :n].sub_(ybar[k][:, :n])
     return ybar[0]
+
+
+def gather_edges_padded(ps: PartitionedSupport, x_loc: torch.Tensor, async_op: bool = False):
+    """All-gather of every rank's slice x_loc [edge_hi - edge_lo] of an [nnz] edge vector (Gs-CSR order) into the padded
+    buffer [world * edge_pad] of `ValueMaps` (one collective: NCCL needs equal chunks, so each slice is padded to the
+    largest).  Returns (buffer, work handle or None); the padding entries are zeros.  World > 1 only."""
+    m = ps.maps()
+    send = x_loc.new_zeros(m.edge_pad)
+    send[:x_loc.numel()] = x_loc
+    out = x_loc.new_empty(ps.world * m.edge_pad)
+    work = dist.all_gather_into_tensor(out, send, group=ps.group, async_op=async_op)
+    return out, work
+
+
+def unpad_edges(ps: PartitionedSupport, buf: torch.Tensor) -> torch.Tensor:
+    """The [nnz] vector (Gs-CSR order) of a padded all-gather buffer."""
+    m = ps.maps()
+    return torch.cat([buf.narrow(0, r * m.edge_pad, hi - lo) for r, (lo, hi) in enumerate(m.edge_bounds)])
+
+
+class _GatherEdges(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, x_loc, ps):
+        m = ps.maps()
+        ctx.lo, ctx.n = m.edge_lo, m.edge_hi - m.edge_lo
+        return unpad_edges(ps, gather_edges_padded(ps, x_loc.detach().contiguous())[0])
+
+    @staticmethod
+    def backward(ctx, dfull):
+        return dfull.narrow(0, ctx.lo, ctx.n), None
+
+
+def gather_edges(ps: PartitionedSupport, x_loc: torch.Tensor) -> torch.Tensor:
+    """The full [nnz] edge vector (Gs-CSR order, the same bytes on every rank) from every rank's slice
+    x_loc = full[edge_lo:edge_hi], in one all-gather (`gather_edges_padded`); x_loc itself at world 1.
+
+    Differentiable, with NO communication in the backward: the gradient of x_loc is the slice [edge_lo:edge_hi] of the
+    gradient arriving at the full vector, which must therefore be exact on this rank's edges.  A partitioned cell
+    guarantees that for the learnable support it returns: with `reduce_per_cell` the [nnz] gradient is all-reduced,
+    without it this rank's partial gradient is non-zero only in its own slice and complete there (a rank's adjoint
+    hops form the gradient of the edges of its own rows, and of no other)."""
+    if ps.world == 1:
+        return x_loc
+    return _GatherEdges.apply(x_loc, ps)
 
 
 class _PartitionedCell(torch.autograd.Function):

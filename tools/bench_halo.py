@@ -18,6 +18,12 @@ alternating ROUNDS times; both reduce their gradients once per step in a flat bu
 the [nnz] edge gradient).  It runs the partitioned path at every world size, world 1 included, and reports
 median / min / max ms of each, their ratio, nnz, the bucket sizes, and the device's name, power limit and maximum SM
 clock.  At world > 1, `parity_ok` also covers the edge gradient against the unpartitioned learnable cell.
+`--train --generated`: the config 4 step with the spatial support generated from the input window on the kNN pattern
+(`SparseGraphGenerator` on the partitioned pattern, X_seq [B, T = 12, N, C], hg = 16) in front of the partitioned cell,
+against the learnable partitioned step on fixed values, alternating as `--learned` does; also the generator's own
+forward + backward per rank.  At world > 1, `parity_ok` covers P, the Wu / Wv / X_seq gradients and the cell outputs
+against the unpartitioned generator + cell on the same GPU, and over NCCL the replicated form (X_seq all-gathered, the
+whole generator on every rank, its [nnz] gradient all-reduced) is timed as well.
 `--gloo`: every rank on cuda:0, exchanging over gloo -- a full-size parity check of the partitioned path on a
 machine with one GPU; its times measure ranks sharing one GPU, not scaling."""
 import json
@@ -145,6 +151,161 @@ def learned_main(B, world, rank, dev):
         print(json.dumps(rec), flush=True)
 
 
+def _device_record(dev):
+    try:
+        smi = subprocess.run(["nvidia-smi", "--query-gpu=power.limit,clocks.max.sm", "--format=csv,noheader"],
+                             capture_output=True, text=True, timeout=30).stdout.strip().splitlines()[0]
+    except Exception as e:  # the measurement still stands, but says that the limit is unknown
+        smi = f"unavailable: {e!r}"
+    return {"device": torch.cuda.get_device_name(dev), "power_limit_and_max_sm_clock": smi}
+
+
+def _alternate(variants, world, rounds, iters):
+    """{name: [ms per step of each round]}, the variants alternating, a round's time the slowest rank's."""
+    for fn in variants.values():
+        for _ in range(3):
+            fn()
+    torch.cuda.synchronize()
+    samples = {k: [] for k in variants}
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    for _ in range(rounds):
+        for k, fn in variants.items():
+            if world > 1:
+                dist.barrier()
+            e0.record()
+            for _ in range(iters):
+                fn()
+            e1.record()
+            torch.cuda.synchronize()
+            samples[k].append(e0.elapsed_time(e1) / iters)
+    if world > 1:
+        for k in samples:
+            t = torch.tensor(samples[k], device=torch.cuda.current_device())
+            dist.all_reduce(t, op=dist.ReduceOp.MAX)
+            samples[k] = t.tolist()
+    return samples
+
+
+def generated_main(B, world, rank, dev):
+    """--train --generated: generator + partitioned step vs the learnable partitioned step (see the module docstring)."""
+    N, C, F, Ks, Kc, T, hg, ROUNDS, iters = 65536, 8, 64, 4, 2, 12, 16, 7, 10
+    rp, ci, va = knn_csr(N, 8)
+    torch.manual_seed(0)
+    cell = S.STC_Cell(N, C, Ks, Kc, F, F).to(dev)
+    gen = S.SparseGraphGenerator(C, hg).to(dev)
+    params, gparams = list(cell.parameters()), list(gen.parameters())
+    Gc = (torch.rand(C, C, generator=torch.Generator().manual_seed(1)) / C).to(dev).requires_grad_(True)
+    g = torch.Generator().manual_seed(100)
+    Xg = torch.randn(B, N, C, F, generator=g)
+    Hg = torch.randn(B, N, C, F, generator=g) * 0.5
+    dHg = torch.randn(B, N, C, F, generator=g)
+    Xsg = torch.randn(B, T, N, C, generator=g)
+    vals = torch.nn.Parameter((va * (0.5 + torch.rand(va.numel(), generator=torch.Generator().manual_seed(7)))).to(dev))
+    const = PartitionedSupport(rp, ci, vals.detach().cpu(), N, rank, world)
+    const.reduce_per_cell = False            # every gradient goes through one bucket per step
+    learned = const.with_values(vals)
+    lo, n = const.start, const.nloc
+    blk = lambda t, d=1: t.narrow(d, lo, n).contiguous().to(dev)
+    X, H, dHn = blk(Xg).requires_grad_(True), blk(Hg).requires_grad_(True), blk(dHg)
+    Xs = blk(Xsg, 2).requires_grad_(True)
+    wP = torch.randn(learned.nnz, generator=torch.Generator().manual_seed(5)).to(dev)
+    buckets = {"learnable": S.dp.GradBucket(params + [Gc, vals]), "generated": S.dp.GradBucket(params + [Gc] + gparams)}
+    cell_args = lambda: (Gc, X, H, cell.gates.W, cell.gates.b, cell.candi.W, cell.candi.b, Ks, Kc)
+    # one-rank groups: the unpartitioned generator runs without batch-DP collectives
+    singles = [dist.new_group([r]) for r in range(world)] if world > 1 else [None]
+
+    def clear():
+        for t in (X, H, Xs, vals, Gc, *params, *gparams):
+            t.grad = None
+
+    def learnable_step():
+        clear()
+        out = partitioned_cell_forward(learned, *cell_args(), reduce_params=False)
+        out.backward(dHn)
+        buckets["learnable"].allreduce()
+        return out
+
+    def generated_step():
+        clear()
+        sup = gen(Xs, const)
+        out = partitioned_cell_forward(sup, *cell_args(), reduce_params=False)
+        out.backward(dHn)
+        buckets["generated"].allreduce()
+        return out, sup
+
+    def generator_only():
+        clear()
+        (gen(Xs, const).vals * wP).sum().backward()
+
+    variants = {"learnable": learnable_step, "generated": lambda: generated_step()[0]}
+    if world > 1 and dist.get_backend() == "nccl":
+        # the replicated form: every rank gathers the whole window and runs the whole generator; the [nnz] gradient
+        # arriving at P must then be all-reduced (mgp.reduce_grad) before the generator's backward
+        cs = S.CsrSupport(rp.to(dev), ci.to(dev), va.to(dev), N)
+        rep_bucket = S.dp.GradBucket(params + [Gc])
+
+        def replicated_step():
+            clear()
+            parts = [torch.empty_like(Xs) for _ in range(world)]
+            dist.all_gather(parts, Xs.detach())
+            Xfull = torch.cat(parts, dim=2)
+            P = S.mgp.reduce_grad(gen(Xfull, cs, group=singles[rank]).vals)
+            out = partitioned_cell_forward(const.with_values(P), *cell_args(), reduce_params=False)
+            out.backward(dHn)
+            rep_bucket.allreduce()
+            return out
+        variants["replicated"] = replicated_step
+
+    parity = None
+    if world > 1:
+        out_p, sup = generated_step()
+        got = [sup.vals.detach().clone(), out_p.detach().clone(), X.grad.clone(), H.grad.clone(), Xs.grad.clone()] + \
+              [t.grad.clone() for t in gparams + params + [Gc]]
+        clear()
+        full = S.CsrSupport(rp.to(dev), ci.to(dev), va.to(dev), N)
+        Xf, Hf, Xsf = (t.to(dev).requires_grad_(True) for t in (Xg, Hg, Xsg))
+        gsup = gen(Xsf, full, group=singles[rank])
+        out_f = cell(Gs=gsup, Gc=Gc, Xt=Xf, Ht_1=Hf)
+        out_f.backward(dHg.to(dev))
+        want = [gsup.vals.detach(), out_f.detach()[:, lo:lo + n], Xf.grad[:, lo:lo + n], Hf.grad[:, lo:lo + n],
+                Xsf.grad[:, :, lo:lo + n]] + [t.grad.clone() for t in gparams + params + [Gc]]
+        names = ["P", "H'", "dXt", "dH", "dX_seq", "dWu", "dWv", "dWg", "dbg", "dWc", "dbc", "dGc"]
+        floors = {"P": 1e-5, "H'": 1e-5, "dXt": 1e-5, "dH": 1e-5, "dX_seq": 1e-5, "dWu": 5e-5, "dWv": 5e-5}
+        worst, nbad = {}, 0
+        m = const.maps()
+        for nm, a_, b_ in zip(names, got, want):
+            if nm == "P":            # this rank's rows, and the whole vector every rank holds
+                nb, worst["P_own_rows"] = violations(a_[m.edge_lo:m.edge_hi], b_[m.edge_lo:m.edge_hi], 1e-5)
+                nbad += nb
+            nb, worst[nm] = violations(a_, b_, floors.get(nm, 3e-5))
+            nbad += nb
+        flag = torch.tensor([float(nbad)], device=dev)
+        dist.all_reduce(flag)
+        parity = {"parity_ok": float(flag.item()) == 0.0, "worst_err_over_mean_ref_rank0": worst}
+        del Xf, Hf, Xsf, gsup, out_f, want, got, full, sup, out_p
+        clear()
+        torch.cuda.empty_cache()
+
+    gen_only = _alternate({"generator": generator_only}, world, 3, iters)["generator"]
+    samples = _alternate(variants, world, ROUNDS, iters)
+    if rank == 0:
+        summ = lambda v: {"median": statistics.median(v), "min": min(v), "max": max(v)}
+        backend = dist.get_backend() if world > 1 else None
+        rec = {"kind": "config4_cell_step_partitioned_generated", "n_gpus": 1 if backend in (None, "gloo") else world,
+               "n_ranks": world, "backend": backend, **_device_record(dev), "N": N, "C": C, "F": F, "Ks": Ks,
+               "Kc": Kc, "B": B, "T": T, "hg": hg, "nnz": learned.nnz, "local_rows": n,
+               "fwd_halo_rows": const.fwd.nhalo, "rounds": ROUNDS, "steps_per_round": iters,
+               "generator_fwd_bwd_ms": summ(gen_only)}
+        rec.update({f"{k}_step_ms": summ(v) for k, v in samples.items()})
+        med = {k: statistics.median(v) for k, v in samples.items()}
+        rec["ratio_generated_over_learnable"] = med["generated"] / med["learnable"]
+        if "replicated" in med:
+            rec["ratio_generated_over_replicated"] = med["generated"] / med["replicated"]
+        if parity:
+            rec.update(parity)
+        print(json.dumps(rec), flush=True)
+
+
 def main():
     train = "--train" in sys.argv
     per_cell = "--reduce-per-cell" in sys.argv
@@ -162,6 +323,14 @@ def main():
         else:
             dist.init_process_group("nccl", device_id=dev)
     _lib.load()
+    if "--generated" in sys.argv:
+        if not train:
+            raise SystemExit("--generated measures the training step: pass --train as well")
+        generated_main(B, world, rank, dev)
+        if world > 1:
+            dist.barrier()
+            dist.destroy_process_group()
+        return
     if "--learned" in sys.argv:
         if not train:
             raise SystemExit("--learned measures the training step: pass --train as well")
