@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define STC_ABI_VERSION 5
+#define STC_ABI_VERSION 6
 
 typedef enum {
   STC_OK = 0,
@@ -201,6 +201,21 @@ int stc_pair_scores_csr_rows(const StcSupport* gs, int32_t N, int64_t width, int
 int stc_edge_softmax_fwd(const StcSupport* gs, int32_t N, const float* scores, float* p, void* stream);
 int stc_edge_softmax_bwd(const StcSupport* gs, int32_t N, const float* scores, const float* p, const float* dp,
                          float* dscores, void* stream);
+
+/* Top-k pair scores of the graph generator over ALL candidate columns (no pattern):
+ *   S[n][m] = <u[n], v[m]> - <v[n], u[m]>  (3xTF32, S[n][n] = 0 exactly), u, v [N][width] row-major, width % 4 == 0,
+ *   u, v and ws 16-byte aligned.
+ *   cols[n][0..k)  the k columns of row n with the largest S (ties: smaller column), ascending;  scores [N][k] the
+ *   matching S values (may be NULL).  A NaN score (NaN or inf in u / v) ranks, and is reported, as -inf; cols always
+ *   holds k distinct columns in [0, N).  1 <= k <= min(N, 32); k > 32 returns STC_ERR_UNSUPPORTED.  Deterministic: the
+ *   output is bitwise the same on every call.  Nothing of size N^2 is formed: each row's best columns are kept on chip
+ *   while the column tiles stream.  ws: at least stc_pair_topk_workspace_bytes(N, width, k) bytes of scratch (0 for
+ *   arguments stc_pair_topk would reject).  The size depends on the SM count of the current device: query it with the
+ *   device current on which stc_pair_topk will run.  The sparse generator (stc_gnn_b200/sparse_mgp.py topk_pattern) builds its
+ *   k-regular pattern from cols. */
+size_t stc_pair_topk_workspace_bytes(int32_t N, int64_t width, int32_t k);
+int stc_pair_topk(int32_t N, int64_t width, const float* u, const float* v, int32_t k,
+                  int32_t* cols, float* scores, void* ws, size_t ws_bytes, void* stream);
 
 /* ---- the backward split the same way (gradients through a row-partitioned graph) ----
  * Order: stage STC_STAGE_CANDI first, then STC_STAGE_GATES (the reverse of the forward).

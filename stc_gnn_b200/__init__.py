@@ -8,6 +8,7 @@ Public surface:
   support_apply_edge_grad  the adjoint CSR hop with the edge-value gradient fused in
   SparseGraphGenerator  the reference's spatial graph generator on a fixed CSR pattern (returns a learnable CsrSupport)
   pair_softmax_csr    its differentiable core: row softmax of relu(<U_n,V_m> - <V_n,U_m>) over the stored edges
+  pair_topk / topk_pattern  the k best columns of every row over all N (the generator's k= mode chooses its pattern)
   install / run_main  rebind STC_GNN.STC_Cell so Model_Trainer.py / Main.py run unchanged
   dp                  batch data-parallel gradient bucket (one flat all-reduce per step)
   halo                row-partitioned CSR support with per-hop halo exchange
@@ -18,5 +19,6 @@ from .support import CsrSupport, support_apply, support_apply_edge_grad  # noqa:
 from .install import install, run_main  # noqa: F401
 from .stack import RecurrentStack  # noqa: F401
 from .graph import GraphedStep  # noqa: F401
-from .sparse_mgp import SparseGraphGenerator, pair_softmax_csr, pair_softmax_partitioned  # noqa: F401
+from .sparse_mgp import (SparseGraphGenerator, pair_softmax_csr, pair_softmax_partitioned, pair_topk,  # noqa: F401
+                         topk_pattern)
 from . import dp, halo, mgp  # noqa: F401

@@ -10,7 +10,7 @@ from ctypes import POINTER, Structure, c_char_p, c_float, c_int, c_int32, c_int6
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "libstc_b200.so")
 
-ABI_VERSION = 5
+ABI_VERSION = 6
 ACT_NONE, ACT_RELU = 0, 1
 SUPPORT_DENSE, SUPPORT_CSR = 0, 1
 
@@ -24,7 +24,7 @@ EXPORTED = (
     "stc_support_apply_rows", "stc_halo_pack", "stc_halo_unpack", "stc_concurrency_set",
     "stc_cell_fwd_x", "stc_cell_bwd_x", "stc_support_outer", "stc_support_apply_edge_grad",
     "stc_support_apply_rows_edge_grad", "stc_pair_scores_csr", "stc_edge_softmax_fwd", "stc_edge_softmax_bwd",
-    "stc_pair_scores_csr_rows",
+    "stc_pair_scores_csr_rows", "stc_pair_topk_workspace_bytes", "stc_pair_topk",
 )
 STAGE_GATES, STAGE_CANDI = 0, 1
 SAVED_REGIONS = ("u", "r", "c", "Yr", "Yx", "Yh", "Q", "Pg", "Pc")
@@ -80,6 +80,11 @@ def load(build_if_missing: bool = True):
     lib.stc_pair_scores_csr_rows.restype = c_int
     lib.stc_pair_scores_csr_rows.argtypes = [POINTER(StcSupport), c_int32, c_int64, c_int64, c_void_p, c_void_p,
                                              c_void_p, c_void_p, c_int32, c_void_p]
+    lib.stc_pair_topk_workspace_bytes.restype = c_size_t
+    lib.stc_pair_topk_workspace_bytes.argtypes = [c_int32, c_int64, c_int32]
+    lib.stc_pair_topk.restype = c_int
+    lib.stc_pair_topk.argtypes = [c_int32, c_int64, c_void_p, c_void_p, c_int32, c_void_p, c_void_p, c_void_p, c_size_t,
+                                  c_void_p]
     lib.stc_edge_softmax_fwd.restype = c_int
     lib.stc_edge_softmax_fwd.argtypes = [POINTER(StcSupport), c_int32, c_void_p, c_void_p, c_void_p]
     lib.stc_edge_softmax_bwd.restype = c_int

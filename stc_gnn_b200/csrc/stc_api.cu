@@ -326,7 +326,7 @@ const char* stc_kernel_kind_name(int32_t kind) {
   static const char* names[KK_COUNT] = {"support_dense", "support_csr", "support_outer", "cheby_small",
                                         "conv_fwd",      "conv_bwd_dx", "conv_bwd_dw", "tc_conv_fwd", "tc_conv_bwd_dx", "tc_conv_bwd_dw",
                                         "tc_support", "tc_gemm_test", "tc_outer", "tc_support_big", "support_csr_grad",
-                                        "pair_scores_csr", "edge_softmax"};
+                                        "pair_scores_csr", "edge_softmax", "pair_topk"};
   return (kind >= 0 && kind < KK_COUNT) ? names[kind] : "?";
 }
 
@@ -1008,6 +1008,49 @@ int stc_edge_softmax_bwd(const StcSupport* gs, int32_t N, const float* scores, c
   }
   STC_TRY(check_arch());
   return launch_edge_softmax(true, gs->rowptr, gs->nnz, N, scores, p, dp, dscores, (cudaStream_t)stream);
+}
+
+static int check_topk_shape(int32_t N, int64_t width, int32_t k, const char* who) {
+  if (N <= 0 || width <= 0 || width % 4 != 0 || width > (1 << 28)) {
+    set_error("%s: N = %d must be positive and width = %lld a positive multiple of 4 (at most 2^28)", who, N,
+              (long long)width);
+    return STC_ERR_BAD_ARG;
+  }
+  if (k > 32) {
+    set_error("%s: k = %d: at most 32 columns a row are kept on chip", who, k);
+    return STC_ERR_UNSUPPORTED;
+  }
+  if (k < 1 || k > N) {
+    set_error("%s: k = %d outside [1, N = %d]", who, k, N);
+    return STC_ERR_BAD_ARG;
+  }
+  return STC_OK;
+}
+
+size_t stc_pair_topk_workspace_bytes(int32_t N, int64_t width, int32_t k) {
+  if (check_topk_shape(N, width, k, "stc_pair_topk_workspace_bytes") != STC_OK) return 0;
+  return pair_topk_ws_bytes(N, k);
+}
+
+int stc_pair_topk(int32_t N, int64_t width, const float* u, const float* v, int32_t k, int32_t* cols, float* scores,
+                  void* ws, size_t ws_bytes, void* stream) {
+  reset_launch_count();
+  STC_TRY(check_topk_shape(N, width, k, "stc_pair_topk"));
+  if (!u || !v || !cols || !ws) {
+    set_error("stc_pair_topk: NULL argument");
+    return STC_ERR_BAD_ARG;
+  }
+  if ((reinterpret_cast<uintptr_t>(u) | reinterpret_cast<uintptr_t>(v) | reinterpret_cast<uintptr_t>(ws)) & 15) {
+    set_error("stc_pair_topk: u, v and ws must be 16-byte aligned");
+    return STC_ERR_BAD_ARG;
+  }
+  STC_TRY(check_arch());
+  const size_t need = pair_topk_ws_bytes(N, k);
+  if (ws_bytes < need) {
+    set_error("stc_pair_topk: workspace of %zu bytes, %zu needed", ws_bytes, need);
+    return STC_ERR_WORKSPACE;
+  }
+  return launch_pair_topk(N, (int)width, u, v, k, cols, scores, ws, (cudaStream_t)stream);
 }
 
 int stc_cell_bwd_scratch_layout(const StcDims* dp, int64_t* offsets, int32_t n_offsets) {

@@ -331,13 +331,6 @@ struct TcOuterPlan {
   uint32_t imgA, imgB, off_lo, off_bar, smem_bytes;
 };
 
-__device__ __forceinline__ void cp_async16(uint32_t smem_dst, const void* gsrc) {
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(smem_dst), "l"(gsrc) : "memory");
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-template <int N>
-__device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
-
 // Round-2 structure (profiles/r3l_outer_support_ncu.txt): with 16-byte loads into registers two atoms ahead the
 // compiler's register reuse serialised every fetch behind the previous one (long-scoreboard stalls on address
 // arithmetic, 0.27-0.35 of HBM whatever the MMA count).  Now the operand chunks travel global -> shared with cp.async

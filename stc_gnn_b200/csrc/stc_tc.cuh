@@ -268,6 +268,14 @@ __device__ __forceinline__ void mbar_arrive_expect_tx(uint64_t* bar, uint32_t by
   asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
 }
 
+// ---- cp.async global -> shared (16 bytes, L2 only), completion tracked per thread in commit groups -----------
+__device__ __forceinline__ void cp_async16(uint32_t smem_dst, const void* gsrc) {
+  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(smem_dst), "l"(gsrc) : "memory");
+}
+__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
+template <int N>
+__device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
+
 // ---- vector reduction into global memory ----------------------------------------------------------------
 // red.global.add.v4.f32 (sm_90+): one L2 atomic transaction for four consecutive floats.  The end-of-kernel
 // accumulations (dW, dGs: every CTA adds its partial sums into the same few thousand addresses) are bound by the

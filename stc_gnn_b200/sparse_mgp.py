@@ -24,6 +24,24 @@ same overlap skeleton as a partitioned hop (stc_pair_scores_csr_rows scores the 
 rank's slice P[edge_lo:edge_hi] is all-gathered into the full [nnz] P.  The backward needs no reduction of dP (the
 gradient arriving at P is exact on the rank's rows) and one all-gather of dS for the transpose term
 (`pair_softmax_partitioned`).  At world 1 it is bitwise the unpartitioned generator.
+
+The pattern may also be chosen from the scores themselves (`gen(X_seq, k=k)`, `topk_pattern`): with
+S[n, m] = <U_n, V_m> - <V_n, U_m> for EVERY m (m = n included, whose score is exactly 0),
+
+    selection  row n stores the k columns with the largest S[n, m]; equal scores go to the smaller column; columns are
+               stored in ascending order, every row has exactly k edges (1 <= k <= min(N, 32)), rowptr = k * arange(N+1)
+    values     exactly those of the fixed-pattern generator on the selected pattern: stc_pair_scores_csr recomputes the
+               scores in fp32 and stc_edge_softmax_fwd takes the softmax of their relu over the k stored edges, so
+               gen(X_seq, k=k) is bitwise gen(X_seq, pattern=<the selected pattern>), and with k = N it is the
+               reference's dense Ps
+    gradient   flows through the values only: the selection is piecewise constant in U, V and gets no gradient, as in
+               any top-k graph learner
+
+The selection is the CUDA kernel stc_pair_topk: all N^2 scores as 128 x 128 tiles of one 3xTF32 tensor-core GEMM
+[U | V] [V | -U]^T, each row's k best kept on chip, so memory stays O(N k) where the score matrix alone would take
+4 N^2 bytes (17 GB at N = 65,536).  Its output is a pure function of (U, V, k): bitwise the same on every call.  A
+score within the 3xTF32 rounding (about 1e-6 relative) of a row's k-th score may be ranked differently from an fp64
+evaluation.
 """
 from __future__ import annotations
 
@@ -33,6 +51,8 @@ from torch import nn
 from . import _lib, halo, mgp
 from .halo import PartitionedSupport
 from .support import CsrSupport, support_apply
+
+TOPK_MAX = 32   # stc_pair_topk keeps at most this many columns a row on chip
 
 
 def _check_pattern(pattern, N: int, who: str) -> None:
@@ -234,6 +254,52 @@ def pair_softmax_partitioned(U_loc: torch.Tensor, V_loc: torch.Tensor, ps: Parti
     return halo.gather_edges(ps, P_loc)
 
 
+def _check_topk_args(N: int, k, who: str) -> None:
+    if isinstance(k, bool) or not isinstance(k, int):
+        raise RuntimeError(f"{who}: k must be an int, got {type(k).__name__}")
+    if k < 1 or k > TOPK_MAX or k > N:
+        raise RuntimeError(f"{who}: k = {k} outside [1, min(N = {N}, {TOPK_MAX})]")
+
+
+def pair_topk(U: torch.Tensor, V: torch.Tensor, k: int, scores: bool = False):
+    """cols [N, k] int32: the k columns m of each row n with the largest S[n, m] = <U_n, V_m> - <V_n, U_m> over all N
+    candidates (S[n, n] = 0; ties to the smaller column), ascending in each row (stc_pair_topk).  With `scores`, also
+    the matching S values [N, k] (float32, 3xTF32).  U, V: [N, width] float32 CUDA; a width that is not a multiple of 4
+    is padded with zero columns, which add nothing to any score.  A NaN score (NaN or inf in U / V) ranks, and is
+    reported, as -inf, so every row still gets k distinct columns in [0, N).  Not differentiable: the result is an
+    index set."""
+    for name, t in (("U", U), ("V", V)):
+        if t.dtype != torch.float32 or t.dim() != 2:
+            raise RuntimeError(f"pair_topk: {name} must be a [N, width] float32 CUDA tensor, got {tuple(t.shape)} "
+                               f"{t.dtype}")
+    if U.shape != V.shape or U.device != V.device:
+        raise RuntimeError(f"pair_topk: U {tuple(U.shape)} on {U.device} and V {tuple(V.shape)} on {V.device} must match")
+    N, width = U.shape
+    _check_topk_args(N, k, "pair_topk")
+    if not U.is_cuda:
+        raise RuntimeError(f"pair_topk: U, V live on {U.device} (there is no CPU path)")
+    if width == 0:
+        raise RuntimeError("pair_topk: width must be positive")
+    pad = -width % 4
+    U, V = (torch.nn.functional.pad(t.detach(), (0, pad)) if pad else t.detach().contiguous() for t in (U, V))
+    U, V = (t if t.data_ptr() % 16 == 0 else t.clone() for t in (U, V))
+    lib = _lib.load()
+    cols = torch.empty(N, k, dtype=torch.int32, device=U.device)
+    sc = torch.empty(N, k, dtype=torch.float32, device=U.device) if scores else None
+    ws_bytes = lib.stc_pair_topk_workspace_bytes(N, width + pad, k)
+    ws = torch.empty(ws_bytes, dtype=torch.uint8, device=U.device)
+    _lib.check(lib.stc_pair_topk(N, width + pad, U.data_ptr(), V.data_ptr(), k, cols.data_ptr(),
+                                 sc.data_ptr() if scores else None, ws.data_ptr(), ws_bytes,
+                                 torch.cuda.current_stream().cuda_stream), "stc_pair_topk")
+    return (cols, sc) if scores else cols
+
+
+def topk_pattern(U: torch.Tensor, V: torch.Tensor, k: int) -> CsrSupport:
+    """The k-regular pattern `pair_topk` selects, as a `CsrSupport` with zero values and its Gs^T permutation, built on
+    the device with no host synchronisation."""
+    return CsrSupport._k_regular(pair_topk(U, V, k))
+
+
 class SparseGraphGenerator(nn.Module):
     """The spatial half of the reference's `MGP_Gen` on a fixed CSR pattern: forward(X_seq, pattern) returns the
     pattern carrying the generated edge values, a `CsrSupport` the cell learns through.
@@ -251,7 +317,7 @@ class SparseGraphGenerator(nn.Module):
         for p in self.params_S.values():
             nn.init.xavier_normal_(p)
 
-    def forward(self, X_seq: torch.Tensor, pattern, group=None, average: bool = False):
+    def forward(self, X_seq: torch.Tensor, pattern=None, group=None, average: bool = False, k: int = None):
         """X_seq [B, T, N, C] float32 CUDA -> `pattern.with_values(P)`.  Under torch.no_grad() the values do not require
         grad and the cell treats the support as constant.  `group` / `average`: batch data-parallel, as in
         `pair_softmax_csr` (X_seq is this rank's shard).
@@ -262,22 +328,43 @@ class SparseGraphGenerator(nn.Module):
         are replicated and their gradients are partial sums over the rank's nodes: with `pattern.reduce_per_cell`
         (default) the backward all-reduces them, so `.grad` is the full gradient on every rank; without it the partial
         sums are left for the caller's `dp.GradBucket`, as for the cell.  The gradient of X_seq is exact, with no
-        communication.  Batch data-parallelism (`group`, `average`) cannot be combined with the row partition."""
+        communication.  Batch data-parallelism (`group`, `average`) cannot be combined with the row partition.
+
+        `k` instead of `pattern`: the pattern is chosen from the scores, the k largest of every row over all N columns
+        (`topk_pattern` on U, V detached; module docstring), and P is formed on it as on a fixed pattern.  The result is
+        a k-regular `CsrSupport`.  Not combinable with a row-partitioned graph or with batch data-parallelism."""
         Wu, Wv = self.params_S["Wu"], self.params_S["Wv"]
         partitioned = isinstance(pattern, PartitionedSupport)
+        if k is not None:
+            if partitioned:
+                raise RuntimeError("SparseGraphGenerator: k= selects the pattern on one device; a row-partitioned "
+                                   "pattern cannot be combined with it")
+            if group is not None or average:
+                raise RuntimeError("SparseGraphGenerator: k= cannot be combined with batch data-parallelism "
+                                   "(group= / average=): every rank would select from its own shard's scores")
+        both = "SparseGraphGenerator: give exactly one of `pattern` (a fixed pattern) and `k` (select the k best " \
+               "columns of every row)"
+        if pattern is not None and k is not None:
+            raise RuntimeError(both)
         if partitioned and (group is not None or average):
             raise RuntimeError("SparseGraphGenerator: batch data-parallelism (group= / average=) cannot be combined "
                                "with a row-partitioned pattern")
         if not X_seq.is_cuda or X_seq.dtype != torch.float32 or X_seq.dim() != 4:
             raise RuntimeError(f"SparseGraphGenerator: X_seq must be a [B, T, N, C] float32 CUDA tensor (there is no "
                                f"CPU path), got {tuple(X_seq.shape)} {X_seq.dtype} on {X_seq.device}")
+        if pattern is None and k is None:
+            raise RuntimeError(both)
         B, T, N, C = X_seq.shape
-        _check_pattern(pattern, N, "SparseGraphGenerator")
+        if k is not None:
+            _check_topk_args(N, k, "SparseGraphGenerator")
+        else:
+            _check_pattern(pattern, N, "SparseGraphGenerator")
         if C != Wu.shape[0]:
             raise RuntimeError(f"SparseGraphGenerator: X_seq has {C} categories, params_S.Wu expects {Wu.shape[0]}")
-        if X_seq.device != Wu.device or (not partitioned and pattern.device != Wu.device):
-            raise RuntimeError(f"SparseGraphGenerator: X_seq ({X_seq.device}), the pattern ({pattern.device}) and the "
-                               f"parameters ({Wu.device}) must share a device")
+        if X_seq.device != Wu.device or (pattern is not None and not partitioned and pattern.device != Wu.device):
+            where = "" if pattern is None else f", the pattern ({pattern.device})"
+            raise RuntimeError(f"SparseGraphGenerator: X_seq ({X_seq.device}){where} and the parameters ({Wu.device}) "
+                               f"must share a device")
         if partitioned and pattern.reduce_per_cell and pattern.world > 1:
             Wu, Wv = mgp.reduce_grad(Wu, pattern.group), mgp.reduce_grad(Wv, pattern.group)
         Xn = X_seq.permute(2, 0, 1, 3).reshape(N, B * T, C)       # node-major copy of the small input
@@ -285,4 +372,6 @@ class SparseGraphGenerator(nn.Module):
         V = torch.tanh(self.alpha * (Xn @ Wv)).reshape(N, -1)
         if partitioned:
             return pattern.with_values(pair_softmax_partitioned(U, V, pattern))
+        if k is not None:
+            pattern = topk_pattern(U.detach(), V.detach(), k)
         return pattern.with_values(pair_softmax_csr(U, V, pattern, group, average))

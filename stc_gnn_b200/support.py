@@ -86,6 +86,20 @@ class CsrSupport:
         return out
 
     @classmethod
+    def _k_regular(cls, cols: torch.Tensor) -> "CsrSupport":
+        """The pattern whose row n stores the k columns cols[n] ([N, k] int32, ascending in each row), with constant
+        zero values, built without a host synchronisation (`k_regular_structure`); `with_values` puts values on it."""
+        N, k = cols.shape
+        rowptr, col, t_rowptr, t_col, t_perm = k_regular_structure(cols)
+        out = cls.__new__(cls)
+        out.N, out.rowptr, out.col, out.nnz, out.device = N, rowptr, col, N * k, cols.device
+        out.vals = torch.zeros(N * k, dtype=torch.float32, device=cols.device)
+        out._t_struct = (t_rowptr, t_col, t_perm)
+        out.t_rowptr, out.t_col, out.t_perm = out._t_struct
+        out.t_vals = torch.zeros(N * k, dtype=torch.float32, device=cols.device)
+        return out
+
+    @classmethod
     def from_dense(cls, G: torch.Tensor) -> "CsrSupport":
         s = G.detach().to_sparse_csr()
         return cls(s.crow_indices(), s.col_indices(), s.values(), G.shape[0])
@@ -105,6 +119,24 @@ class CsrSupport:
         s.vals, s.rowptr, s.col = self.vals.data_ptr(), self.rowptr.data_ptr(), self.col.data_ptr()
         s.t_vals, s.t_rowptr, s.t_col = self.t_vals.data_ptr(), self.t_rowptr.data_ptr(), self.t_col.data_ptr()
         return s
+
+
+def k_regular_structure(cols: torch.Tensor):
+    """(rowptr, col, t_rowptr, t_col, t_perm) of the pattern storing cols[n] ([N, k] integer, ascending in each row) in
+    row n: what `CsrSupport._transpose_structure` gives for the same (rowptr, col), in integer arithmetic on cols'
+    device, with no host synchronisation (every size is N or N * k, known on the host).  The keys col * N + row are
+    distinct, so the sort needs no stability; the Gs^T row counts come from index_add_ rather than a bincount."""
+    N, k = cols.shape
+    dev = cols.device
+    col = cols.to(torch.int32).reshape(-1).contiguous()
+    rowptr = (torch.arange(N + 1, device=dev, dtype=torch.int64) * k).to(torch.int32)
+    row = torch.arange(N, device=dev, dtype=torch.int64)[:, None].expand(N, k).reshape(-1)
+    colL = col.to(torch.int64)
+    t_perm = torch.sort(colL * N + row).indices.contiguous()
+    counts = torch.zeros(N, dtype=torch.int64, device=dev).index_add_(0, colL, torch.ones_like(colL))
+    t_rowptr = torch.zeros(N + 1, dtype=torch.int64, device=dev)
+    t_rowptr[1:] = torch.cumsum(counts, 0)
+    return rowptr, col, t_rowptr.to(torch.int32).contiguous(), row[t_perm].to(torch.int32).contiguous(), t_perm
 
 
 def dense_struct(G: torch.Tensor) -> _lib.StcSupport:
