@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define STC_ABI_VERSION 6
+#define STC_ABI_VERSION 7
 
 typedef enum {
   STC_OK = 0,
@@ -134,27 +134,37 @@ int stc_cell_bwd(const StcDims* d, const StcSupport* gs, const float* gc,
                  int32_t accumulate_params, const void* saved, size_t saved_bytes,
                  void* scratch, size_t scratch_bytes, void* stream);
 
-/* ---- the Xt-side spatial terms hoisted out of the time loop (SURVEY 8f row f1) ----
- * In the encoder's first layer Xt does not depend on the recurrence (STC_GNN.py:107-118), so its spatial terms for ALL
- * timesteps can be produced by one batched stc_support_apply and handed in:
- *   yx_terms      [Ks-1][B][N][C][Din] contiguous = Y_1 .. Y_{Ks-1} of this step's Xt (NULL: computed inside, as
- *                 stc_cell_fwd / stc_cell_bwd do); the forward then launches no Xt-side hop.
- *   dyx_terms_out [Ks-1][B][N][C][Din]: stc_cell_bwd_x writes the adjoints of those terms there and does NOT fold them:
- *                 no Xt-side adjoint hop and no Xt-side dGs contribution is launched; d_xt (if given) holds the term-0
- *                 part only.  The caller folds all timesteps at once (dGs += sum_t X_t (x) dY_1,t via
- *                 stc_support_outer, dXt += Gs dY_1 via stc_support_apply; for a CSR support with learned edge values
- *                 stc_support_apply_edge_grad does both).  Both pointers go together. */
+/* ---- spatial terms computed once for two readers (SURVEY 8f row f1; stc_gnn_b200/stack.py) ----
+ * The encoder's first layer produces the Xt-side terms of ALL timesteps with one batched stc_support_apply
+ * (STC_GNN.py:107-118: Xt does not depend on the recurrence), and every hidden state of the recurrent stack is read by
+ * two cells, one as Xt and one as H, whose terms Y_k = T_k(Gs^T) Y_0 are the same bytes.  Per side (Xt, H):
+ *   y?_terms      [Ks-1][B][N][C][Din or h] contiguous = Y_1 .. Y_{Ks-1} of that side's input (NULL: computed inside, as
+ *                 stc_cell_fwd / stc_cell_bwd do); the forward then launches no hop for that side, and the backward
+ *                 reads the same terms (they must be unchanged).
+ *   dy?_terms_out [Ks-1][B][N][C][Din or h] (with y?_terms): stc_cell_bwd_x writes the adjoints of the supplied terms
+ *                 there and does NOT fold them: no adjoint hop and no dGs contribution is launched for that side, and
+ *                 d_xt / d_h_prev holds the term-0 part only.  The caller folds them: the _XSideTerms path with
+ *                 stc_support_outer / stc_support_apply (stc_support_apply_edge_grad for learned CSR values), the cell
+ *                 that produced shared terms through its own dy?_fold.  NULL: the adjoints are dropped (an input whose
+ *                 terms are known and needs no gradient, e.g. a zero initial state).
+ *   dy?_fold      [Ks-1][B][N][C][Din or h] (without y?_terms): adjoints of this call's OWN terms of that side, from
+ *                 another reader of them.  They are added to the adjoints the convolutions produce (in the dx
+ *                 epilogue) before that side's adjoint chain runs, so one hop and one dGs product serve both readers.
+ * The stc_cell_saved_layout regions Yx / Yh of a call that computed them hold that side's terms. */
 int stc_cell_fwd_x(const StcDims* d, const StcSupport* gs, const float* gc,
                    const float* xt, int64_t xt_batch_stride, const float* h_prev,
                    const float* Wg, const float* bg, const float* Wc, const float* bc,
-                   float* h_out, void* saved, size_t saved_bytes, const float* yx_terms, void* stream);
+                   float* h_out, void* saved, size_t saved_bytes, const float* yx_terms, const float* yh_terms,
+                   void* stream);
 int stc_cell_bwd_x(const StcDims* d, const StcSupport* gs, const float* gc,
                    const float* xt, int64_t xt_batch_stride, const float* h_prev,
                    const float* Wg, const float* Wc, const float* d_h_out,
                    float* d_xt, float* d_h_prev,
                    float* dWg, float* dbg, float* dWc, float* dbc, float* dGs, float* dGc,
                    int32_t accumulate_params, const void* saved, size_t saved_bytes,
-                   void* scratch, size_t scratch_bytes, const float* yx_terms, float* dyx_terms_out, void* stream);
+                   void* scratch, size_t scratch_bytes, const float* yx_terms, float* dyx_terms_out,
+                   const float* dyx_fold, const float* yh_terms, float* dyh_terms_out, const float* dyh_fold,
+                   void* stream);
 /* dGs[n][m] += coef * sum_{b,j} A[b][n][j] * Bm[b][m][j]  -- the gradient of the mode product Y = Gs^T X w.r.t. a dense
  * Gs [N][N] with A = X ([B][N][width], batch stride in elements) and Bm = dL/dY ([B][N][width] contiguous). */
 int stc_support_outer(int32_t N, int32_t B, int32_t width, const float* a, int64_t a_batch_stride, const float* b,

@@ -10,7 +10,7 @@ from ctypes import POINTER, Structure, c_char_p, c_float, c_int, c_int32, c_int6
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "libstc_b200.so")
 
-ABI_VERSION = 6
+ABI_VERSION = 7
 ACT_NONE, ACT_RELU = 0, 1
 SUPPORT_DENSE, SUPPORT_CSR = 0, 1
 
@@ -65,7 +65,7 @@ def load(build_if_missing: bool = True):
     lib.stc_cell_fwd.argtypes = [POINTER(StcDims), POINTER(StcSupport), c_void_p, c_void_p, c_int64, c_void_p,
                                  c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]
     lib.stc_cell_fwd_x.restype = c_int
-    lib.stc_cell_fwd_x.argtypes = lib.stc_cell_fwd.argtypes[:-1] + [c_void_p, c_void_p]
+    lib.stc_cell_fwd_x.argtypes = lib.stc_cell_fwd.argtypes[:-1] + [c_void_p, c_void_p, c_void_p]
     lib.stc_support_outer.restype = c_int
     lib.stc_support_outer.argtypes = [c_int32, c_int32, c_int32, c_void_p, c_int64, c_void_p, c_float, c_void_p, c_void_p]
     lib.stc_support_apply_edge_grad.restype = c_int
@@ -100,7 +100,7 @@ def load(build_if_missing: bool = True):
                                  c_void_p, c_void_p, c_void_p, c_int32, c_void_p, c_size_t, c_void_p, c_size_t,
                                  c_void_p]
     lib.stc_cell_bwd_x.restype = c_int
-    lib.stc_cell_bwd_x.argtypes = lib.stc_cell_bwd.argtypes[:-1] + [c_void_p, c_void_p, c_void_p]
+    lib.stc_cell_bwd_x.argtypes = lib.stc_cell_bwd.argtypes[:-1] + [c_void_p] * 7
     lib.stc_cell_bwd_scratch_layout.restype = c_int
     lib.stc_cell_bwd_scratch_layout.argtypes = [POINTER(StcDims), POINTER(c_int64), c_int32]
     lib.stc_cell_bwd_stage.restype = c_int

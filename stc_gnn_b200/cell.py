@@ -72,14 +72,38 @@ def _ptr(t):
     return t.data_ptr() if t is not None else None
 
 
+_SAVED_OFFSETS = {}
+
+
+def _terms_view(saved, dims, key, side, shape):
+    """The spatial terms [Ks-1,B,N,C,w] a cell call computed for one side: a view of its `saved` buffer."""
+    offs = _SAVED_OFFSETS.get(key)
+    if offs is None:
+        if len(_SAVED_OFFSETS) > 256:
+            _SAVED_OFFSETS.clear()
+        offs = _SAVED_OFFSETS[key] = _lib.saved_layout(dims)
+    n = 1
+    for s_ in shape:
+        n *= s_
+    return saved[offs["Yx" if side == "x" else "Yh"]:][:n].view(shape)
+
+
 class _CellFunction(torch.autograd.Function):
-    """One cell step. Inputs that may need gradients: Gs (dense only), Gc, Xt, H, Wg, bg, Wc, bc, -- when the
-    caller hoisted the Xt-side spatial terms out of the time loop (stack.py) -- those terms `Yx` [Ks-1,B,N,C,Din], whose
-    gradient is returned un-folded, and `Ev`, the edge values [nnz] of a learnable CsrSupport Gs (the support object
-    itself is not a tensor autograd can see; Ev is its `vals`)."""
+    """One cell step. Inputs that may need gradients: Gs (dense only), Gc, Xt, H, Wg, bg, Wc, bc, `Ev`, the edge values
+    [nnz] of a learnable CsrSupport Gs (the support object itself is not a tensor autograd can see; Ev is its `vals`),
+    and caller-supplied spatial terms of either side (stack.py): `Yx` [Ks-1,B,N,C,Din] of Xt and `Yh` [Ks-1,B,N,C,h] of
+    H.  No hop runs for a supplied side, and the gradient of its terms is returned un-folded.
+
+    `share` = (give, yx_shared):
+      give       sides ("x", "h") whose computed terms are also returned (views of `saved`), after H' in that order; the
+                 gradient arriving at them (from the cell that took them) is folded in before this cell's own adjoint
+                 chain of that side, so one hop and one dGs product serve both readers.
+      yx_shared  the supplied `Yx` came from another cell that folds their adjoint into the chain of Xt itself: then
+                 Xt's own gradient is its direct term only.  Without it (the _XSideTerms path, which folds only into
+                 dGs) Xt may not need a gradient."""
 
     @staticmethod
-    def forward(ctx, Gs, Gc, Xt, H, Wg, bg, Wc, bc, Yx, Ev, cfg):
+    def forward(ctx, Gs, Gc, Xt, H, Wg, bg, Wc, bc, Yx, Ev, cfg, Yh=None, share=None):
         lib = _lib.load()
         Ks, Kc, act = cfg
         B, N, C, Din = Xt.shape
@@ -124,25 +148,33 @@ class _CellFunction(torch.autograd.Function):
         saved = torch.empty(_buffer_floats(lib, dims, ctx.size_key)[0], dtype=torch.float32, device=Xt.device)
         Hn = torch.empty((B, N, C, h), dtype=torch.float32, device=Xt.device)
         stream = torch.cuda.current_stream().cuda_stream
-        Yx_c = None
-        if Yx is not None and Ks > 1:
-            if Yx.shape != (Ks - 1, B, N, C, Din) or not Yx.is_cuda or Yx.dtype != torch.float32:
-                raise RuntimeError(f"hoisted Xt-side terms must be a float32 CUDA tensor of shape {(Ks - 1, B, N, C, Din)}, "
-                                   f"got {tuple(Yx.shape)}")
-            Yx_c = Yx.contiguous()
+        give, yx_shared = share if share is not None else ((), False)
+
+        def supplied(Y, w, what):
+            if Y is None or Ks <= 1:
+                return None
+            if Y.shape != (Ks - 1, B, N, C, w) or not Y.is_cuda or Y.dtype != torch.float32:
+                raise RuntimeError(f"supplied {what} terms must be a float32 CUDA tensor of shape {(Ks - 1, B, N, C, w)}, "
+                                   f"got {tuple(Y.shape)}")
+            return Y.contiguous()
+
+        Yx_c, Yh_c = supplied(Yx, Din, "Xt-side"), supplied(Yh, h, "H-side")
+        for side in give:
+            if side not in ("x", "h") or Ks <= 1 or (Yx_c if side == "x" else Yh_c) is not None:
+                raise RuntimeError(f"a cell can only give terms of a side it computes itself (give={give!r}, Ks={Ks})")
         if B == 0:
             status = 0
-        elif Yx_c is not None:
+        elif Yx_c is not None or Yh_c is not None:
             status = lib.stc_cell_fwd_x(dims, gs_struct, Gc_c.data_ptr(), Xt_c.data_ptr(), xbs, H_c.data_ptr(),
                                         Wg_c.data_ptr(), _ptr(bg_c), Wc_c.data_ptr(), _ptr(bc_c), Hn.data_ptr(),
-                                        saved.data_ptr(), saved.numel() * 4, Yx_c.data_ptr(), stream)
+                                        saved.data_ptr(), saved.numel() * 4, _ptr(Yx_c), _ptr(Yh_c), stream)
         else:
             status = lib.stc_cell_fwd(dims, gs_struct, Gc_c.data_ptr(), Xt_c.data_ptr(), xbs, H_c.data_ptr(),
                                       Wg_c.data_ptr(), _ptr(bg_c), Wc_c.data_ptr(), _ptr(bc_c), Hn.data_ptr(),
                                       saved.data_ptr(), saved.numel() * 4, stream)
         _lib.check(status, "stc_cell_fwd")
         _lib.note_launches()
-        ctx.hoisted = Yx_c is not None
+        ctx.hoisted, ctx.h_given, ctx.yx_shared, ctx.give = Yx_c is not None, Yh_c is not None, bool(yx_shared), tuple(give)
         ctx.cfg, ctx.dims_tuple, ctx.xbs, ctx.csr = cfg, (B, N, C, Din, h), xbs, csr
         ctx.gs_obj = Gs if csr else None
         ctx.has_bias = bg is not None
@@ -154,18 +186,24 @@ class _CellFunction(torch.autograd.Function):
                     ctx.sinks[i] = t
         ctx.has_ev = Ev is not None
         ctx.save_for_backward(*( [] if csr else [gs_keep] ), Gc_c, Xt_c, H_c, Wg_c, Wc_c, saved,
-                              *([Yx_c] if Yx_c is not None else []), *([Ev] if Ev is not None else []))
-        return Hn
+                              *([Yx_c] if Yx_c is not None else []), *([Yh_c] if Yh_c is not None else []),
+                              *([Ev] if Ev is not None else []))
+        if not give:
+            return Hn
+        ctx.set_materialize_grads(False)   # no gradient for given terms: nothing to fold (rather than a zero tensor)
+        return (Hn,) + tuple(_terms_view(saved, dims, ctx.size_key, side, (Ks - 1, B, N, C, Din if side == "x" else h))
+                             for side in give)
 
     @staticmethod
     @torch.autograd.function.once_differentiable
-    def backward(ctx, dHn):
+    def backward(ctx, dHn, *dGiven):
         lib = _lib.load()
         Ks, Kc, act = ctx.cfg
         B, N, C, Din, h = ctx.dims_tuple
         sv = list(ctx.saved_tensors)
         if ctx.has_ev:
             sv.pop()   # saved only so that autograd refuses a backward after an in-place change of the values
+        Yh = sv.pop() if ctx.h_given else None
         Yx = sv.pop() if ctx.hoisted else None
         if ctx.csr:
             Gs = ctx.gs_obj
@@ -174,19 +212,22 @@ class _CellFunction(torch.autograd.Function):
         else:
             Gs, Gc, Xt, H, Wg, Wc, saved = sv
             gs_struct = dense_struct(Gs)
-        need = ctx.needs_input_grad  # Gs, Gc, Xt, H, Wg, bg, Wc, bc, Yx, Ev, cfg
-        dev = dHn.device
-        dHn = dHn.contiguous()
+        n_in = len(ctx.needs_input_grad)   # Yh and share are optional trailing inputs
+        need = tuple(ctx.needs_input_grad) + (False,) * (13 - n_in)  # Gs, Gc, Xt, H, Wg, bg, Wc, bc, Yx, Ev, cfg, Yh, share
+        dev = H.device
+        dHn = dHn.contiguous() if dHn is not None else torch.zeros(B, N, C, h, dtype=torch.float32, device=dev)
         L, P = Din + h, Ks * Kc
         dims = _dims(B, N, C, Din, h, Ks, Kc, act, ctx.has_bias)
         new = lambda *shape: torch.empty(shape, dtype=torch.float32, device=dev)
-        if ctx.hoisted and need[2]:
+        if ctx.hoisted and need[2] and not ctx.yx_shared:
             raise RuntimeError("hoisted Xt-side terms: the gradient w.r.t. Xt is folded by the caller (stack.py hoists only "
                                "when the input sequence needs no gradient)")
         dXt = new(B, N, C, Din) if need[2] else None
         dH = new(B, N, C, h)
-        dYx = torch.empty_like(Yx) if ctx.hoisted else None
-        returned = [None] * 11
+        dYx = torch.empty_like(Yx) if ctx.hoisted and need[8] else None
+        dYh = torch.empty_like(Yh) if ctx.h_given and need[11] else None
+        fold = {side: g.contiguous() for side, g in zip(ctx.give, dGiven) if g is not None and B > 0}
+        returned = [None] * 13
 
         def target(i, shape, wanted=True):
             """Buffer the kernels ADD input i's gradient into: the leaf's own `.grad` (created zeroed on first use in a
@@ -208,27 +249,29 @@ class _CellFunction(torch.autograd.Function):
         # a CSR support's gradient is that of its edge values: [nnz] in Gs-CSR order
         dGs = target(9, (Gs.nnz,), need[9]) if ctx.csr else target(0, (N, N), need[0])
         dGc = target(1, (C, C), need[1])
-        returned[2], returned[3], returned[8] = dXt, dH, dYx
+        returned[2], returned[3], returned[8], returned[11] = dXt, dH, dYx, dYh
         if B == 0:  # empty batch: every parameter gradient is zero (the targets are zeroed or untouched), nothing to launch
-            if dYx is not None:
-                dYx.zero_()
-            return tuple(returned)
+            for t in (dYx, dYh):
+                if t is not None:
+                    t.zero_()
+            return tuple(returned[:n_in])
         scratch = torch.empty(_buffer_floats(lib, dims, ctx.size_key)[1], dtype=torch.float32, device=dev)
         common = (dims, gs_struct, Gc.data_ptr(), Xt.data_ptr(), ctx.xbs, H.data_ptr(), Wg.data_ptr(),
                   Wc.data_ptr(), dHn.data_ptr(), _ptr(dXt), dH.data_ptr(), dWg.data_ptr(), _ptr(dbg),
                   dWc.data_ptr(), _ptr(dbc), _ptr(dGs), _ptr(dGc), 1, saved.data_ptr(),
                   saved.numel() * 4, scratch.data_ptr(), scratch.numel() * 4)
         stream = torch.cuda.current_stream().cuda_stream
-        if ctx.hoisted:
-            status = lib.stc_cell_bwd_x(*common, Yx.data_ptr(), dYx.data_ptr(), stream)
+        if ctx.hoisted or ctx.h_given or fold:
+            fx, fh = fold.get("x"), fold.get("h")
+            status = lib.stc_cell_bwd_x(*common, _ptr(Yx), _ptr(dYx), _ptr(fx), _ptr(Yh), _ptr(dYh), _ptr(fh), stream)
         else:
             status = lib.stc_cell_bwd(*common, stream)
         _lib.check(status, "stc_cell_bwd")
         _lib.note_launches()
-        for i in (0, 1, 4, 5, 6, 7, 8, 9):    # inputs that need no gradient get none, whatever was computed for them
+        for i in (0, 1, 4, 5, 6, 7, 8, 9, 11):    # inputs that need no gradient get none, whatever was computed for them
             if not need[i]:
                 returned[i] = None
-        return tuple(returned)
+        return tuple(returned[:n_in])
 
 
 def stc_cell_forward(Gs, Gc, Xt, Ht_1, Wg, bg, Wc, bc, Ks: int, Kc: int, activation=None) -> torch.Tensor:
@@ -265,6 +308,13 @@ class STC_Cell(nn.Module):
     def init_hidden(self, batch_size: int):
         weight = next(self.parameters()).data
         return weight.new_zeros(batch_size, self.num_nodes, self.num_categories, self.hidden_dim)
+
+    def _shared_step(self, Gs, Gc, Xt, Ht_1, Yx=None, Yh=None, give=(), yx_shared=False):
+        """One step of RecurrentStack with spatial terms shared between the two cells that read a hidden state
+        (dense or CSR Gs): see _CellFunction.  Returns H' or, with `give`, (H', the terms of each side given)."""
+        return _CellFunction.apply(Gs, Gc, Xt, Ht_1, self.gates.W, getattr(self.gates, "b", None), self.candi.W,
+                                   getattr(self.candi, "b", None), Yx, _edge_values(Gs), (self.Ks, self.Kc, self._act),
+                                   Yh, (give, yx_shared))
 
     def forward(self, Gs, Gc: torch.Tensor, Xt: torch.Tensor, Ht_1: torch.Tensor, _Yx: torch.Tensor = None):
         """`_Yx` (not part of the reference's signature): the spatial terms of Xt, [Ks-1,B,N,C,Din], when the caller

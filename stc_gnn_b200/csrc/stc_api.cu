@@ -435,6 +435,7 @@ struct FwdCtx {
   cudaStream_t st;
   Lanes* lanes = nullptr;   // set by stc_cell_fwd: the Xt-side terms and the Gc terms may run beside the H-side terms
   const float* yx_pre = nullptr;   // caller-supplied spatial terms of Xt ([Ks-1][B][N][C][Din]): skip the Xt-side hops
+  const float* yh_pre = nullptr;   // caller-supplied spatial terms of H ([Ks-1][B][N][C][h]): skip the H-side hops
 };
 
 // spatial Chebyshev terms of Xt and H:  Y_1 = Gs^T Y_0,  Y_k = 2 Gs^T Y_{k-1} - Y_{k-2}
@@ -447,7 +448,7 @@ static int fwd_terms_xh(const FwdCtx& f) {
   const long long nbs_h = (long long)d.N * CH;
   // the two recurrences are independent of each other: Xt's on side stream 0 (when lanes are active), H's on the caller's
   cudaStream_t sx = f.st;
-  if (f.lanes && f.lanes->active() && d.Ks > 1 && !f.yx_pre) {
+  if (f.lanes && f.lanes->active() && d.Ks > 1 && !f.yx_pre && !f.yh_pre) {
     STC_TRY(f.lanes->fork(0));
     sx = f.lanes->stream(0);
   }
@@ -460,7 +461,7 @@ static int fwd_terms_xh(const FwdCtx& f) {
     STC_TRY(launch_support_apply(*f.gs, d.N, d.B, CD, true, xin, xin_bs, xz, xz_bs, ws + w.Yx + (size_t)(k - 1) * Rx,
                                  alpha, beta, nullptr, 0.f, sx));
   }
-  for (int k = 1; k < d.Ks; ++k) {
+  for (int k = 1; k < d.Ks && !f.yh_pre; ++k) {
     const float alpha = k == 1 ? 1.f : 2.f, beta = k == 1 ? 0.f : -1.f;
     const float* hin = k == 1 ? f.h_prev : ws + w.Yh + (size_t)(k - 2) * Rh;
     const float* hz = k == 1 ? nullptr : (k == 2 ? f.h_prev : ws + w.Yh + (size_t)(k - 3) * Rh);
@@ -480,7 +481,7 @@ static int fwd_gates(const FwdCtx& f, const float* Wg, const float* bg) {
   ConvArgs a = base_args(d, f.xt, f.xt_bs, Wg, ws + w.Q, ws, w, 0);
   if (f.yx_pre) a.yx = f.yx_pre;
   a.h0 = f.h_prev;
-  a.yh = ws + w.Yh;
+  a.yh = f.yh_pre ? f.yh_pre : ws + w.Yh;
   a.bias = d.has_bias ? bg : nullptr;
   a.Hprev = f.h_prev;
   a.u = ws + w.u;
@@ -551,8 +552,8 @@ static int check_fwd_args(const StcDims* dp, const float* gc, const float* xt, c
 
 static int cell_fwd_impl(const StcDims* dp, const StcSupport* gs, const float* gc, const float* xt,
                          int64_t xt_batch_stride, const float* h_prev, const float* Wg, const float* bg, const float* Wc,
-                         const float* bc, float* h_out, void* wsv, size_t ws_bytes, const float* yx_terms, void* stream,
-                         const char* who) {
+                         const float* bc, float* h_out, void* wsv, size_t ws_bytes, const float* yx_terms,
+                         const float* yh_terms, void* stream, const char* who) {
   reset_launch_count();
   STC_TRY(check_fwd_args(dp, gc, xt, h_prev, Wg, bg, Wc, bc, h_out, wsv, ws_bytes, who));
   if (!gs) {
@@ -567,6 +568,7 @@ static int cell_fwd_impl(const StcDims* dp, const StcSupport* gs, const float* g
   FwdCtx f{d, w, gs, gc, xt, xt_batch_stride, h_prev, (float*)wsv, (cudaStream_t)stream};
   f.lanes = &lanes;
   f.yx_pre = d.Ks > 1 ? yx_terms : nullptr;
+  f.yh_pre = d.Ks > 1 ? yh_terms : nullptr;
   STC_TRY(fwd_terms_xh(f));
   STC_TRY(fwd_gates(f, Wg, bg));
   STC_TRY(fwd_terms_rh(f));
@@ -577,15 +579,16 @@ static int cell_fwd_impl(const StcDims* dp, const StcSupport* gs, const float* g
 int stc_cell_fwd(const StcDims* dp, const StcSupport* gs, const float* gc, const float* xt,
                  int64_t xt_batch_stride, const float* h_prev, const float* Wg, const float* bg, const float* Wc,
                  const float* bc, float* h_out, void* wsv, size_t ws_bytes, void* stream) {  // wsv = `saved`
-  return cell_fwd_impl(dp, gs, gc, xt, xt_batch_stride, h_prev, Wg, bg, Wc, bc, h_out, wsv, ws_bytes, nullptr, stream,
-                       "stc_cell_fwd");
+  return cell_fwd_impl(dp, gs, gc, xt, xt_batch_stride, h_prev, Wg, bg, Wc, bc, h_out, wsv, ws_bytes, nullptr, nullptr,
+                       stream, "stc_cell_fwd");
 }
 
 int stc_cell_fwd_x(const StcDims* dp, const StcSupport* gs, const float* gc, const float* xt,
                    int64_t xt_batch_stride, const float* h_prev, const float* Wg, const float* bg, const float* Wc,
-                   const float* bc, float* h_out, void* wsv, size_t ws_bytes, const float* yx_terms, void* stream) {
-  return cell_fwd_impl(dp, gs, gc, xt, xt_batch_stride, h_prev, Wg, bg, Wc, bc, h_out, wsv, ws_bytes, yx_terms, stream,
-                       "stc_cell_fwd_x");
+                   const float* bc, float* h_out, void* wsv, size_t ws_bytes, const float* yx_terms,
+                   const float* yh_terms, void* stream) {
+  return cell_fwd_impl(dp, gs, gc, xt, xt_batch_stride, h_prev, Wg, bg, Wc, bc, h_out, wsv, ws_bytes, yx_terms, yh_terms,
+                       stream, "stc_cell_fwd_x");
 }
 
 int stc_cell_saved_layout(const StcDims* dp, int64_t* offsets, int32_t n_offsets) {
@@ -676,6 +679,10 @@ struct BwdCtx {
   Lanes* lanes = nullptr;   // set by stc_cell_bwd: dW runs beside the adjoint hops on side stream 0
   const float* yx_pre = nullptr;   // caller-supplied spatial terms of Xt (as in forward)
   float* dyx_out = nullptr;        // caller's buffer for the x-part adjoints of terms k >= 1 (the caller folds them)
+  const float* yh_pre = nullptr;   // the same for H
+  float* dyh_out = nullptr;
+  const float* dyx_fold = nullptr; // adjoints of this call's own Xt-side terms k >= 1 from another reader: folded in
+  const float* dyh_fold = nullptr; //   the dx epilogue before the adjoint chain of that side
   bool want_dGc() const { return dGc != nullptr && d.Kc > 1; }
   float* dYx0() const { return d_xt ? d_xt : sc + w.dYx0; }
 };
@@ -750,6 +757,7 @@ static int bwd_candi(const BwdCtx& b, const float* Wc, float* dWc, float* dbc) {
   a.dYx0 = b.dYx0();
   a.dYx = b.dyx_out ? b.dyx_out : b.sc + w.dYx;
   a.accum_x = 0;
+  a.dYx_add = b.dyx_fold;
   a.dYh0 = b.sc + w.dYr;
   a.dYh = b.sc + w.dYr + Rh;
   a.dQ = b.want_dGc() ? b.sc + w.dQ : nullptr;
@@ -767,7 +775,7 @@ static int bwd_gates(const BwdCtx& b, const float* Wg, float* dWg, float* dbg) {
   ConvArgs a = base_args(d, b.xt, b.xt_bs, Wg, b.sv + w.Q, b.sv, w, 0);
   if (b.yx_pre) a.yx = b.yx_pre;
   a.h0 = b.h_prev;
-  a.yh = b.sv + w.Yh;
+  a.yh = b.yh_pre ? b.yh_pre : b.sv + w.Yh;
   a.Hprev = b.h_prev;
   a.u = b.sv + w.u;
   a.r = b.sv + w.r;
@@ -780,7 +788,8 @@ static int bwd_gates(const BwdCtx& b, const float* Wg, float* dWg, float* dbg) {
   a.dYx = b.dyx_out ? b.dyx_out : b.sc + w.dYx;
   a.accum_x = 1;
   a.dYh0 = b.d_h_prev;
-  a.dYh = b.sc + w.dYh;
+  a.dYh = b.dyh_out ? b.dyh_out : b.sc + w.dYh;
+  a.dYh_add = b.dyh_fold;
   a.dQ = b.want_dGc() ? b.sc + w.dQ : nullptr;
   a.dW = dWg;
   a.Psave = b.sv + w.Pg;
@@ -796,8 +805,9 @@ static int cell_bwd_impl(const StcDims* dp, const StcSupport* gs, const float* g
                          int64_t xt_batch_stride, const float* h_prev, const float* Wg, const float* Wc,
                          const float* d_h_out, float* d_xt, float* d_h_prev, float* dWg, float* dbg, float* dWc, float* dbc,
                          float* dGs, float* dGc, int32_t accumulate_params, const void* savedv, size_t saved_bytes,
-                         void* scratchv, size_t scratch_bytes, const float* yx_terms, float* dyx_terms_out, void* stream,
-                         const char* who) {
+                         void* scratchv, size_t scratch_bytes, const float* yx_terms, float* dyx_terms_out,
+                         const float* dyx_fold, const float* yh_terms, float* dyh_terms_out, const float* dyh_fold,
+                         void* stream, const char* who) {
   reset_launch_count();
   STC_TRY(check_bwd_args(dp, gc, xt, h_prev, Wg, Wc, d_h_out, d_h_prev, dWg, dbg, dWc, dbc, savedv, saved_bytes, scratchv,
                          scratch_bytes, who));
@@ -810,8 +820,8 @@ static int cell_bwd_impl(const StcDims* dp, const StcSupport* gs, const float* g
     set_error("%s: the edge-value gradient of a CSR support needs its rowptr/col/vals and nnz", who);
     return STC_ERR_BAD_ARG;
   }
-  if (d.Ks > 1 && ((yx_terms != nullptr) != (dyx_terms_out != nullptr))) {
-    set_error("%s: yx_terms and dyx_terms_out go together (the caller that supplied the Xt-side terms folds their adjoints)", who);
+  if ((yx_terms && dyx_fold) || (yh_terms && dyh_fold)) {
+    set_error("%s: a side either takes supplied terms or folds an adjoint into its own terms, not both", who);
     return STC_ERR_BAD_ARG;
   }
   const WsLayout w = make_layout(d);
@@ -822,9 +832,18 @@ static int cell_bwd_impl(const StcDims* dp, const StcSupport* gs, const float* g
            const_cast<float*>((const float*)savedv), (float*)scratchv, st};
   b.lanes = &lanes;
   const bool hoisted = d.Ks > 1 && yx_terms != nullptr;
+  const bool h_given = d.Ks > 1 && yh_terms != nullptr;
   if (hoisted) {
     b.yx_pre = yx_terms;
     b.dyx_out = dyx_terms_out;
+  }
+  if (h_given) {
+    b.yh_pre = yh_terms;
+    b.dyh_out = dyh_terms_out;
+  }
+  if (d.Ks > 1) {
+    b.dyx_fold = dyx_fold;
+    b.dyh_fold = dyh_fold;
   }
   const size_t dGs_floats = gs->kind == STC_SUPPORT_CSR ? (size_t)gs->nnz : (size_t)d.N * d.N;
   STC_TRY(bwd_begin(b, dWg, dbg, dWc, dbc, dGs, dGs_floats, accumulate_params));
@@ -850,7 +869,8 @@ static int cell_bwd_impl(const StcDims* dp, const StcSupport* gs, const float* g
     }
     STC_TRY(adjoint_chain(d, *gs, CD, xt, xt_batch_stride, b.sv + w.Yx, b.dYx0(), b.sc + w.dYx, dGs, sx, &lanes, 1));
   }
-  STC_TRY(adjoint_chain(d, *gs, CH, h_prev, (int64_t)d.N * CH, b.sv + w.Yh, d_h_prev, b.sc + w.dYh, dGs, st, &lanes, 1));
+  if (!h_given)   // (given: the h-part adjoints of terms k >= 1 sit in dyh_terms_out, or are dropped when it is NULL)
+    STC_TRY(adjoint_chain(d, *gs, CH, h_prev, (int64_t)d.N * CH, b.sv + w.Yh, d_h_prev, b.sc + w.dYh, dGs, st, &lanes, 1));
   return lanes.join_all();
 }
 
@@ -860,18 +880,19 @@ int stc_cell_bwd(const StcDims* dp, const StcSupport* gs, const float* gc, const
                  float* dGs, float* dGc, int32_t accumulate_params, const void* savedv, size_t saved_bytes,
                  void* scratchv, size_t scratch_bytes, void* stream) {
   return cell_bwd_impl(dp, gs, gc, xt, xt_batch_stride, h_prev, Wg, Wc, d_h_out, d_xt, d_h_prev, dWg, dbg, dWc, dbc, dGs, dGc,
-                       accumulate_params, savedv, saved_bytes, scratchv, scratch_bytes, nullptr, nullptr, stream,
-                       "stc_cell_bwd");
+                       accumulate_params, savedv, saved_bytes, scratchv, scratch_bytes, nullptr, nullptr, nullptr, nullptr,
+                       nullptr, nullptr, stream, "stc_cell_bwd");
 }
 
 int stc_cell_bwd_x(const StcDims* dp, const StcSupport* gs, const float* gc, const float* xt,
                    int64_t xt_batch_stride, const float* h_prev, const float* Wg, const float* Wc,
                    const float* d_h_out, float* d_xt, float* d_h_prev, float* dWg, float* dbg, float* dWc, float* dbc,
                    float* dGs, float* dGc, int32_t accumulate_params, const void* savedv, size_t saved_bytes,
-                   void* scratchv, size_t scratch_bytes, const float* yx_terms, float* dyx_terms_out, void* stream) {
+                   void* scratchv, size_t scratch_bytes, const float* yx_terms, float* dyx_terms_out,
+                   const float* dyx_fold, const float* yh_terms, float* dyh_terms_out, const float* dyh_fold, void* stream) {
   return cell_bwd_impl(dp, gs, gc, xt, xt_batch_stride, h_prev, Wg, Wc, d_h_out, d_xt, d_h_prev, dWg, dbg, dWc, dbc, dGs, dGc,
-                       accumulate_params, savedv, saved_bytes, scratchv, scratch_bytes, yx_terms, dyx_terms_out, stream,
-                       "stc_cell_bwd_x");
+                       accumulate_params, savedv, saved_bytes, scratchv, scratch_bytes, yx_terms, dyx_terms_out, dyx_fold,
+                       yh_terms, dyh_terms_out, dyh_fold, stream, "stc_cell_bwd_x");
 }
 
 int stc_support_outer(int32_t N, int32_t B, int32_t width, const float* a, int64_t a_batch_stride, const float* b,

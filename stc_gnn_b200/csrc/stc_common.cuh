@@ -175,7 +175,12 @@ struct ConvArgs {
   int accum_x;         // add into dYx* instead of overwrite (gates phase after candidate phase)
   float* dYh0;         // k = 0 h-part adjoint destination (d_h_prev for gates, d(rH) for candidate)
   float* dYh;          // k >= 1
-  float* dQ;           // [Kc][C][C] atomically accumulated, or null
+  // adjoints another cell folds into this one's terms k >= 1 (the cell that hopped a shared hidden state once for both
+  // of its readers, stack.py): the x-part starts from dYx_add (candidate phase, accum_x == 0), the h-part written by the
+  // gates phase adds dYh_add; null = nothing to fold
+  const float* dYx_add;   // [Ks-1][R][Din]
+  const float* dYh_add;   // [Ks-1][R][h]
+  float* dQ;          // [Kc][C][C] atomically accumulated, or null
   float* dW;           // atomically accumulated
   // tuning switches (STC_OPT environment bit mask, default all on) and the optional phase trace (stc_debug_trace_set)
   int opt;

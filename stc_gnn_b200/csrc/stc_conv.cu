@@ -315,19 +315,23 @@ conv_bwd_dx_kernel(const ConvArgs a, const ConvTile t, const int DP) {
       float* dx = (k == 0) ? a.dYx0 : a.dYx + (size_t)(k - 1) * R * Din;
       if (dx) {
         dx += row0 * Din;
+        // prior contents: the other convolution's x-part (accum_x), else a folded adjoint of the term (k >= 1)
+        const float* xprior = a.accum_x ? dx
+                              : (k >= 1 && a.dYx_add) ? a.dYx_add + (size_t)(k - 1) * R * Din + row0 * Din : nullptr;
         for (int idx = threadIdx.x; idx < rows_valid * Din; idx += blockDim.x) {
           int row = idx / Din, l = idx - row * Din;
           float v = DY[row * LP + l];
-          dx[idx] = a.accum_x ? dx[idx] + v : v;
+          dx[idx] = xprior ? xprior[idx] + v : v;
         }
       }
       float* dh = (k == 0) ? a.dYh0 : a.dYh + (size_t)(k - 1) * R * h;
       dh += row0 * h;
-      const bool add_direct = (k == 0 && a.phase == 0);
+      const float* hprior = (k == 0 && a.phase == 0) ? dh   // direct terms of dH
+                            : (k >= 1 && a.dYh_add) ? a.dYh_add + (size_t)(k - 1) * R * h + row0 * h : nullptr;
       for (int idx = threadIdx.x; idx < rows_valid * h; idx += blockDim.x) {
         int row = idx / h, l = idx - row * h;
         float v = DY[row * LP + Din + l];
-        dh[idx] = add_direct ? dh[idx] + v : v;
+        dh[idx] = hprior ? hprior[idx] + v : v;
       }
     }
   }

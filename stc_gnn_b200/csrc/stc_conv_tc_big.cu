@@ -792,11 +792,17 @@ tc_conv_bwd_dx_big_kernel(const ConvArgs a, const BigDxPlan p, const uint8_t* __
               const float4* src = reinterpret_cast<const float4*>(a.dYh0 + gr * h + c0);
               prev[gi][0] = src[0];
               prev[gi][1] = src[1];
+            } else if (k >= 1 && a.dYh_add != nullptr) {   // adjoint another cell folds into this term
+              const float4* src = reinterpret_cast<const float4*>(a.dYh_add + (size_t)(k - 1) * R * h + gr * h + c0);
+              prev[gi][0] = src[0];
+              prev[gi][1] = src[1];
             }
           } else {
             const int xi = c0 - h;
-            if (xi < Din && xvec && a.accum_x) {
-              const float* src = (k == 0 ? a.dYx0 : a.dYx + (size_t)(k - 1) * R * Din) + gr * Din + xi;
+            const float* xsrc = a.accum_x ? (k == 0 ? a.dYx0 : a.dYx + (size_t)(k - 1) * R * Din)
+                                : (k >= 1 && a.dYx_add != nullptr) ? a.dYx_add + (size_t)(k - 1) * R * Din : nullptr;
+            if (xi < Din && xvec && xsrc != nullptr) {
+              const float* src = xsrc + gr * Din + xi;
               prev[gi][0] = *reinterpret_cast<const float4*>(src);
               if (xi + 4 < Din) prev[gi][1] = *reinterpret_cast<const float4*>(src + 4);
             }
@@ -895,9 +901,12 @@ tc_conv_bwd_dx_big_kernel(const ConvArgs a, const BigDxPlan p, const uint8_t* __
             reinterpret_cast<float4*>(dst)[0] = make_float4(v[0] + p0.x, v[1] + p0.y, v[2] + p0.z, v[3] + p0.w);
             if (xi + 4 < Din) reinterpret_cast<float4*>(dst)[1] = make_float4(v[4] + p1.x, v[5] + p1.y, v[6] + p1.z, v[7] + p1.w);
           } else {
+            const float* prior = a.accum_x ? dst
+                                 : (k >= 1 && a.dYx_add != nullptr) ? a.dYx_add + (size_t)(k - 1) * R * Din + gr * Din + xi
+                                                                     : nullptr;
 #pragma unroll
             for (int i = 0; i < 8; ++i)
-              if (xi + i < Din) dst[i] = a.accum_x ? dst[i] + v[i] : v[i];
+              if (xi + i < Din) dst[i] = prior ? prior[i] + v[i] : v[i];
           }
         }
       }
@@ -937,7 +946,7 @@ int try_launch_conv_bwd_dx_big(const ConvArgs& a, cudaStream_t st, bool* handled
   *handled = false;
   if (a.Wimg == nullptr || !big_dx_shape_ok(a) || (a.opt & OPT_WIDE_DX_FFMA)) return STC_OK;
   if (!aligned16g(a.dHn) || !aligned16g(a.u) || !aligned16g(a.c) || !aligned16g(a.Hprev) || !aligned16g(a.dpre) ||
-      !aligned16g(a.dYh0) || !aligned16g(a.dYh) || !aligned16g(a.Psave) || (a.dpre_ld % 4) != 0 ||
+      !aligned16g(a.dYh0) || !aligned16g(a.dYh) || !aligned16g(a.dYh_add) || !aligned16g(a.Psave) || (a.dpre_ld % 4) != 0 ||
       (a.phase == 0 && (!aligned16g(a.r) || !aligned16g(a.drH))) || ((reinterpret_cast<uintptr_t>(a.Wimg) & 127) != 0)) {
     set_error("tcgen05 wide-state backward needs 16-byte aligned gradient / workspace tensors");
     return STC_ERR_BAD_ARG;
@@ -949,7 +958,7 @@ int try_launch_conv_bwd_dx_big(const ConvArgs& a, cudaStream_t st, bool* handled
   p.KBLp = (p.KBL + 15) & ~15;
   p.nkc = 2 * a.Hout / 32;
   p.DP = a.Hout + 4;
-  p.x_vec = (a.Din % 4 == 0) && aligned16g(a.dYx0) && aligned16g(a.dYx);
+  p.x_vec = (a.Din % 4 == 0) && aligned16g(a.dYx0) && aligned16g(a.dYx) && aligned16g(a.dYx_add);
   const long long total_nodes = (long long)a.B * a.N;
   p.ntiles = ceil_div(total_nodes, p.npt);
   p.stage_bytes = (uint32_t)(2 * p.KBLp * ATOM_ROW_BYTES);

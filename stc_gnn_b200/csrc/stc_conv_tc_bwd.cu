@@ -96,13 +96,18 @@ __device__ __forceinline__ void dx_prefetch_tile(const ConvArgs& a, const TcDxPl
     l2_prefetch(a.drH + row0 * a.h, hb);
   }
   if (want_dQ) l2_prefetch(a.Psave + row0 * p.PW, (uint32_t)(nv * a.C * p.PW * 4));
+  const long long R = total_nodes * a.C;
   if (a.accum_x && p.x_vec) {
     const uint32_t xb = (uint32_t)(nv * a.C * a.Din * 4);
-    const long long R = total_nodes * a.C;
     if (a.dYx0) l2_prefetch(a.dYx0 + row0 * a.Din, xb);
     if (a.dYx)
       for (int k = 1; k < a.Ks; ++k) l2_prefetch(a.dYx + (size_t)(k - 1) * R * a.Din + row0 * a.Din, xb);
+  } else if (a.dYx_add && p.x_vec) {
+    const uint32_t xb = (uint32_t)(nv * a.C * a.Din * 4);
+    for (int k = 1; k < a.Ks; ++k) l2_prefetch(a.dYx_add + (size_t)(k - 1) * R * a.Din + row0 * a.Din, xb);
   }
+  if (a.dYh_add)
+    for (int k = 1; k < a.Ks; ++k) l2_prefetch(a.dYh_add + (size_t)(k - 1) * R * a.h + row0 * a.h, hb);
 }
 
 // FAST: contiguous-column epilogue of the common shape (Ks = 2, h = 16, Din <= 16, one main accumulator)
@@ -411,12 +416,13 @@ tc_conv_bwd_dx_kernel(const ConvArgs a, const TcDxPlan p) {
     STC_TRACE(3);
     // x-part adjoint this pass adds to (the other convolution's contribution): requested now, consumed in the epilogue --
     // the read-modify-write latency travels under the MMAs and the dQ pass instead of sitting at the end of every tile
+    // (or, for term 1, the adjoint another cell folds into it)
     float4 xprev[4];
 #pragma unroll
     for (int i = 0; i < 4; ++i) xprev[i] = make_float4(0.f, 0.f, 0.f, 0.f);
     if constexpr (FAST) {
-      if (a.accum_x && p.x_vec && erow < rows_valid) {
-        const float* dbase_pf = (half == 0 ? a.dYx0 : a.dYx);
+      if (p.x_vec && erow < rows_valid) {
+        const float* dbase_pf = a.accum_x ? (half == 0 ? a.dYx0 : a.dYx) : (half == 0 ? nullptr : a.dYx_add);
         if (dbase_pf != nullptr) {
           const float* src = dbase_pf + (row0 + erow) * Din;
 #pragma unroll
@@ -509,6 +515,14 @@ tc_conv_bwd_dx_kernel(const ConvArgs a, const TcDxPlan p) {
               v[i] += d.x; v[i + 1] += d.y; v[i + 2] += d.z; v[i + 3] += d.w;
             }
           }
+          if (k == 1 && a.dYh_add != nullptr) {   // the folded adjoint of term 1 (pulled into L2 one tile ahead)
+            const float4* ap = reinterpret_cast<const float4*>(a.dYh_add + gr * 16);
+#pragma unroll
+            for (int i = 0; i < 4; ++i) {
+              const float4 q = ap[i];
+              v[4 * i] += q.x; v[4 * i + 1] += q.y; v[4 * i + 2] += q.z; v[4 * i + 3] += q.w;
+            }
+          }
           float* dst = (k == 0 ? a.dYh0 : a.dYh) + gr * 16;
 #pragma unroll
           for (int i = 0; i < 16; i += 4) *reinterpret_cast<float4*>(dst + i) = make_float4(v[i], v[i + 1], v[i + 2], v[i + 3]);
@@ -541,7 +555,7 @@ tc_conv_bwd_dx_kernel(const ConvArgs a, const TcDxPlan p) {
                                  __uint_as_float(sm[4 * i + 1]) + __uint_as_float(mn[4 * i + 1]),
                                  __uint_as_float(sm[4 * i + 2]) + __uint_as_float(mn[4 * i + 2]),
                                  __uint_as_float(sm[4 * i + 3]) + __uint_as_float(mn[4 * i + 3]));
-            if (a.accum_x) {
+            if (a.accum_x || (k == 1 && a.dYx_add != nullptr)) {
 #pragma unroll
               for (int i = 0; i < 4; ++i)
                 if (4 * i < Din) { o[i].x += xprev[i].x; o[i].y += xprev[i].y; o[i].z += xprev[i].z; o[i].w += xprev[i].w; }
@@ -550,11 +564,12 @@ tc_conv_bwd_dx_kernel(const ConvArgs a, const TcDxPlan p) {
             for (int i = 0; i < 4; ++i)
               if (4 * i < Din) *reinterpret_cast<float4*>(dst + 4 * i) = o[i];
           } else {
+            const float* prior = a.accum_x ? dst : (k == 1 && a.dYx_add != nullptr) ? a.dYx_add + gr * Din : nullptr;
 #pragma unroll
             for (int i = 0; i < 16; ++i)
               if (i < Din) {
                 const float vi = __uint_as_float(sm[i]) + __uint_as_float(mn[i]);
-                dst[i] = a.accum_x ? dst[i] + vi : vi;
+                dst[i] = prior ? prior[i] + vi : vi;
               }
           }
         }
@@ -589,6 +604,12 @@ tc_conv_bwd_dx_kernel(const ConvArgs a, const TcDxPlan p) {
 #pragma unroll
             for (int i = 0; i < 8; ++i) v[i] += dp[i];
           }
+          if (k >= 1 && a.dYh_add != nullptr) {
+            const float4* ap = reinterpret_cast<const float4*>(a.dYh_add + (size_t)(k - 1) * R * h + gr * h + kb);
+            const float4 p0 = ap[0], p1 = ap[1];
+            v[0] += p0.x; v[1] += p0.y; v[2] += p0.z; v[3] += p0.w;
+            v[4] += p1.x; v[5] += p1.y; v[6] += p1.z; v[7] += p1.w;
+          }
           reinterpret_cast<float4*>(dst)[0] = make_float4(v[0], v[1], v[2], v[3]);
           reinterpret_cast<float4*>(dst)[1] = make_float4(v[4], v[5], v[6], v[7]);
         } else {
@@ -596,10 +617,13 @@ tc_conv_bwd_dx_kernel(const ConvArgs a, const TcDxPlan p) {
           float* dbase = (k == 0 ? a.dYx0 : a.dYx + (size_t)(k - 1) * R * Din);
           if (dbase == nullptr) continue;
           float* dst = dbase + gr * Din + xi;
+          const float* prior = a.accum_x ? dst
+                               : (k >= 1 && a.dYx_add != nullptr) ? a.dYx_add + (size_t)(k - 1) * R * Din + gr * Din + xi
+                                                                   : nullptr;
           if (p.x_vec && xi + 8 <= Din) {   // both 16-byte halves in flight at once (the accumulate is a read-modify-write)
             float4 o0 = make_float4(v[0], v[1], v[2], v[3]), o1 = make_float4(v[4], v[5], v[6], v[7]);
-            if (a.accum_x) {
-              const float4 p0 = reinterpret_cast<const float4*>(dst)[0], p1 = reinterpret_cast<const float4*>(dst)[1];
+            if (prior != nullptr) {
+              const float4 p0 = reinterpret_cast<const float4*>(prior)[0], p1 = reinterpret_cast<const float4*>(prior)[1];
               o0.x += p0.x; o0.y += p0.y; o0.z += p0.z; o0.w += p0.w;
               o1.x += p1.x; o1.y += p1.y; o1.z += p1.z; o1.w += p1.w;
             }
@@ -608,7 +632,7 @@ tc_conv_bwd_dx_kernel(const ConvArgs a, const TcDxPlan p) {
           } else {
 #pragma unroll
             for (int i = 0; i < 8; ++i)
-              if (xi + i < Din) dst[i] = a.accum_x ? dst[i] + v[i] : v[i];
+              if (xi + i < Din) dst[i] = prior ? prior[i] + v[i] : v[i];
           }
         }
       }
@@ -669,7 +693,8 @@ int try_launch_conv_bwd_dx_tc(const ConvArgs& a, cudaStream_t st, bool* handled)
   *handled = false;
   if (!conv_tc_eligible(a)) return STC_OK;
   if (!aligned16b(a.dHn) || !aligned16b(a.u) || !aligned16b(a.c) || !aligned16b(a.Hprev) || !aligned16b(a.dpre) ||
-      !aligned16b(a.dYh0) || !aligned16b(a.dYh) || !aligned16b(a.Psave) || (a.phase == 0 && (!aligned16b(a.r) || !aligned16b(a.drH)))) {
+      !aligned16b(a.dYh0) || !aligned16b(a.dYh) || !aligned16b(a.dYh_add) || !aligned16b(a.Psave) ||
+      (a.phase == 0 && (!aligned16b(a.r) || !aligned16b(a.drH)))) {
     set_error("tcgen05 backward needs 16-byte aligned gradient / workspace tensors");
     return STC_ERR_BAD_ARG;
   }
@@ -687,7 +712,7 @@ int try_launch_conv_bwd_dx_tc(const ConvArgs& a, cudaStream_t st, bool* handled)
   while (p.tmem_cols < (p.nmain + 1) * p.Npad) p.tmem_cols *= 2;
   p.DP = a.Hout + 4;
   p.PW = (a.Kc - 1) * a.Hout;
-  p.x_vec = (a.Din % 4 == 0) && aligned16b(a.dYx0) && aligned16b(a.dYx);
+  p.x_vec = (a.Din % 4 == 0) && aligned16b(a.dYx0) && aligned16b(a.dYx) && aligned16b(a.dYx_add);
   const long long total_nodes = (long long)a.B * a.N;
   p.ntiles = ceil_div(total_nodes, p.npt);
   const size_t atomB = (size_t)p.Npad * ATOM_ROW_BYTES;
