@@ -514,6 +514,17 @@ tc_outer_kernel(const float* __restrict__ A, long long a_bs, const float* __rest
             store_split4(hb + p.imgA, lbp + p.imgA, soff[i], *reinterpret_cast<const float4*>(hb + p.imgA + soff[i]));
           }
         }
+      } else if (j < ((W + 7) & ~7)) {
+        // W % 8 == 4: the last K-step of the sample's last atom reads 4 columns past W.  Nothing was copied there, so the
+        // stage still holds a column of an earlier atom (any CTA with more than one sample): zero it in both images.
+        uint8_t* hb = Hring + (size_t)(seq % TO_SH) * hsz;
+        uint8_t* lbp = Lring + (size_t)(seq % TO_SL) * hsz;
+        const float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
+#pragma unroll
+        for (int i = 0; i < 4; ++i) {
+          if (r0 + 32 * i < rowsA) store_split4(hb, lbp, soff[i], z);
+          if (r0 + 32 * i < rowsB) store_split4(hb + p.imgA, lbp + p.imgA, soff[i], z);
+        }
       }
       fence_async_smem();
       __syncwarp();
