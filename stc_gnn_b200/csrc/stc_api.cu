@@ -326,7 +326,7 @@ const char* stc_kernel_kind_name(int32_t kind) {
   static const char* names[KK_COUNT] = {"support_dense", "support_csr", "support_outer", "cheby_small",
                                         "conv_fwd",      "conv_bwd_dx", "conv_bwd_dw", "tc_conv_fwd", "tc_conv_bwd_dx", "tc_conv_bwd_dw",
                                         "tc_support", "tc_gemm_test", "tc_outer", "tc_support_big", "support_csr_grad",
-                                        "pair_scores_csr", "edge_softmax", "pair_topk"};
+                                        "pair_scores_csr", "edge_softmax", "pair_topk", "tc_support_adj"};
   return (kind >= 0 && kind < KK_COUNT) ? names[kind] : "?";
 }
 
@@ -645,6 +645,14 @@ static int adjoint_chain(const StcDims& d, const StcSupport& gs, int width, cons
     if (dGs) {
       const float* yprev = k == 1 ? y0 : yk + (size_t)(k - 2) * Rw;
       const int64_t yprev_bs = k == 1 ? y0_bs : nbs;
+      // One pass over ybar[k] for both of its readers (dense N <= 112).  Not when the lanes are active: there the outer
+      // product runs beside the hops, off the critical path that fusing would lengthen.
+      if (gs.kind == STC_SUPPORT_DENSE && gs.vals && !(lanes && lanes->active())) {
+        bool handled = false;
+        STC_TRY(try_launch_support_adj_tc(gs.vals, d.N, d.B, width, yb_k, nbs, yb_km1, axpy, yprev, yprev_bs, coef, dGs,
+                                          st, &handled));
+        if (handled) continue;
+      }
       // the outer product only READS ybar[k] (final once the previous hop on `st` is queued) and Y[k-1]; nothing later in
       // the chain writes either, so it runs beside the hops on the outer lane and is joined at the end of the call
       cudaStream_t so = st;

@@ -43,7 +43,7 @@ void reset_launch_count();
 enum KernelKind {
   KK_SUPPORT_DENSE = 0, KK_SUPPORT_CSR, KK_SUPPORT_OUTER, KK_CHEBY_SMALL, KK_CONV_FWD, KK_CONV_BWD_DX,
   KK_CONV_BWD_DW, KK_TC_CONV_FWD, KK_TC_CONV_BWD_DX, KK_TC_CONV_BWD_DW, KK_TC_SUPPORT, KK_TC_GEMM_TEST, KK_TC_OUTER, KK_TC_SUPPORT_BIG,
-  KK_SUPPORT_CSR_GRAD, KK_PAIR_SCORES_CSR, KK_EDGE_SOFTMAX, KK_PAIR_TOPK, KK_COUNT
+  KK_SUPPORT_CSR_GRAD, KK_PAIR_SCORES_CSR, KK_EDGE_SOFTMAX, KK_PAIR_TOPK, KK_TC_SUPPORT_ADJ, KK_COUNT
 };
 struct ScopedKernelTimer {  // declare right before a launch; the destructor records the stop event
   ScopedKernelTimer(int kind, cudaStream_t st, double alg_bytes);
@@ -111,6 +111,13 @@ int try_launch_support_tc_big(const float* G, int N, int B, int width, bool tran
                               bool* handled);
 int try_launch_outer_tc(int N, int B, int width, const float* a, int64_t a_bs, const float* bmat, float coef, float* dG,
                         cudaStream_t st, bool* handled);
+// one adjoint step of a dense support with N <= 112 in one kernel (rows of ybar are N * width floats apart):
+//   axpy_out -= x (when not NULL, its own pass first);  ybar += coef * Gs x;  dG += coef * a (x) x
+int try_launch_support_adj_tc(const float* G, int N, int B, int width, const float* x, int64_t x_bs, float* ybar,
+                              float* axpy_out, const float* a, int64_t a_bs, float coef, float* dG, cudaStream_t st,
+                              bool* handled);
+// out[b] += coef * x[b] over B slabs of N * width floats (out contiguous; 16-byte aligned, width % 4 == 0)
+int launch_axpy_rows(float* out, const float* x, int64_t x_bs, float coef, int N, int B, int width, cudaStream_t st);
 
 // adjoint hop y = alpha * Gs x + beta * z (+ the Chebyshev axpy) of a CSR support with the edge-value gradient fused in:
 // dvals[e = (n,m)] += coef * sum_{b,j} a[b,n,j] * x[b,m,j]  (dvals in the order of gs.rowptr / gs.col / gs.vals).

@@ -118,6 +118,14 @@ axpy_rows_kernel(float* __restrict__ out, const float* __restrict__ x, long long
   }
 }
 
+int launch_axpy_rows(float* out, const float* x, int64_t x_bs, float coef, int N, int B, int width, cudaStream_t st) {
+  const long long per_b4 = (long long)N * width / 4, total4 = per_b4 * B;
+  const int blocks = (int)std::min<long long>((total4 + 255) / 256, (long long)device_sm_count() * 16);
+  axpy_rows_kernel<<<blocks, 256, 0, st>>>(out, x, x_bs, coef, per_b4, total4);
+  STC_LAUNCH_OK("axpy_rows_kernel");
+  return STC_OK;
+}
+
 // ------------------------------------------------------------------------------------------------
 // CSR support: one warp per (b, m) output row slab; lanes sweep the contiguous `width` axis
 // ------------------------------------------------------------------------------------------------
@@ -301,12 +309,7 @@ int launch_support_apply(const StcSupport& gs, int N, int B, int width, bool tra
                             (reinterpret_cast<uintptr_t>(x) & 15) == 0 && (reinterpret_cast<uintptr_t>(axpy_out) & 15) == 0;
     if (axpy_out == nullptr || axpy_split) {
       bool handled = false;
-      if (axpy_split) {
-        const long long per_b4 = (long long)N * width / 4, total4 = per_b4 * B;
-        const int blocks = (int)std::min<long long>((total4 + 255) / 256, (long long)device_sm_count() * 16);
-        axpy_rows_kernel<<<blocks, 256, 0, st>>>(axpy_out, x, x_bs, axpy_coef, per_b4, total4);
-        STC_LAUNCH_OK("axpy_rows_kernel");
-      }
+      if (axpy_split) STC_TRY(launch_axpy_rows(axpy_out, x, x_bs, axpy_coef, N, B, width, st));
       STC_TRY(try_launch_support_tc(gs.vals, N, B, width, transpose, x, x_bs, z, z_bs, y, alpha, beta, st, &handled));
       if (handled) return STC_OK;
       STC_TRY(try_launch_support_tc_big(gs.vals, N, B, width, transpose, x, x_bs, z, z_bs, y, alpha, beta, st, &handled));

@@ -613,4 +613,367 @@ int try_launch_outer_tc(int N, int B, int width, const float* a, int64_t a_bs, c
   return STC_OK;
 }
 
+// ------------------------------------------------------------------------------------------------
+//  tc_support_adj_kernel   one step k of the Chebyshev adjoint of a dense support (N <= 112), both products that read
+//                          ybar_k in one pass over it:
+//      Yb[b,m,:]  = coef * sum_n Gs[m,n] X[b,n,:] + Yb[b,m,:]       (tc_support_kernel with A = Gs, beta = 1)
+//      dGs[n][m] += coef * sum_{b,j} A[b,n,j] X[b,m,j]              (tc_outer_kernel, one-tile form)
+//  with X = ybar_k, Yb = ybar_{k-1}, A = Y_{k-1}.  The pair reads X twice and splits it twice; here the producers load
+//  each 32-feature chunk of one sample (one SW128 atom) once, split it once and write it twice: MN-major
+//  (SWIZZLE_128B_BASE32B, the B operand of the hop) and K-major SW128 (the B operand of the outer product; the tensor
+//  core takes BASE32B only for MN-major tf32 operands, so the two images cannot share bytes).
+//  The hop is bitwise the one of tc_support_kernel: the same K order, pass order and epilogue expression (an MMA result
+//  does not depend on the N width of the tile).  dGs only re-associates: one [main | cross] slot drained into fp32
+//  registers every TA_DRAIN chunks (64 K-steps per chain, the bound of profiles/r1_tc_precision.txt).
+//  Warps: 0 issues the MMAs, 1-8 load / split / stage the chunks and drain the dGs slot, 9-12 run the hop epilogue
+//  through the staging tile of tc_support_kernel.  The CTAs split the samples, as in tc_outer_kernel.
+// ------------------------------------------------------------------------------------------------
+constexpr int TA_PROD_WARPS = 8, TA_EPI_WARPS = 4;
+constexpr int TA_THREADS = 32 * (1 + TA_PROD_WARPS + TA_EPI_WARPS);
+constexpr int TA_STAGES = 2;
+constexpr int TA_DRAIN = 16;              // chunks per dGs chain: 16 x 4 = 64 K-steps per accumulator
+constexpr int TA_OLD = ATOM_K + 4;        // row stride (floats) of the output staging tile
+constexpr int TA_MAX_N = 112;
+
+struct TcAdjPlan {
+  int N, Kp, Npad, W, B, atoms_per_sample;
+  uint32_t col_hop, col_g;                // TMEM columns of the hop accumulators and of the support
+  uint32_t imgA, imgBk, imgX, stage_bytes, off_o, off_bar, smem_bytes;
+};
+
+__global__ void __launch_bounds__(TA_THREADS, 1)
+tc_support_adj_kernel(const float* __restrict__ G, const float* __restrict__ X, long long x_bs, float* Yb,
+                      const float* __restrict__ A, long long a_bs, float coef, float* dG, const TcAdjPlan p) {
+  extern __shared__ __align__(1024) uint8_t smem[];
+  if ((smem_u32(smem) & 1023u) != 0u) __trap();
+  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+  const int N = p.N, Kp = p.Kp, W = p.W, aps = p.atoms_per_sample;
+  // one stage: [A hi | A lo | X K-major hi | lo | X MN-major hi | lo]
+  const uint32_t off_bk = 2 * p.imgA, off_xm = off_bk + 2 * p.imgBk;
+  uint64_t* full = reinterpret_cast<uint64_t*>(smem + p.off_bar);   // [TA_STAGES] producers -> MMA
+  uint64_t* empty = full + TA_STAGES;                                // [TA_STAGES] MMA (hop + outer) -> producers
+  uint64_t* hopfull = empty + TA_STAGES;                             // MMA -> epilogue
+  uint64_t* hopempty = hopfull + 1;                                  // epilogue -> MMA
+  uint64_t* drained = hopempty + 1;                                  // producers have read the dGs slot
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(drained + 1);
+  if (tid == 0) {
+    for (int i = 0; i < TA_STAGES; ++i) {
+      mbar_init(&full[i], TA_PROD_WARPS);
+      mbar_init(&empty[i], 1);
+    }
+    mbar_init(hopfull, 1);
+    mbar_init(hopempty, TA_EPI_WARPS);
+    mbar_init(drained, TA_PROD_WARPS);
+    mbar_fence_init();
+  }
+  if (warp == 0) tmem_alloc(tmem_slot, 512);
+  // rows past N of every image are never written by the producers: zero them once
+  for (uint32_t i = tid * 16u; i < TA_STAGES * p.stage_bytes; i += TA_THREADS * 16u)
+    *reinterpret_cast<float4*>(smem + i) = make_float4(0.f, 0.f, 0.f, 0.f);
+  fence_async_smem();
+  fence_before_sync();
+  __syncthreads();
+  fence_after_sync();
+  const uint32_t tmem_base = *tmem_slot;
+  {  // the support in TMEM as in tc_support_kernel: lane m, column k -> Gs[m][k]; hi at col_g, lo Kp columns later
+    const uint32_t tG = tmem_base + p.col_g;
+    if (warp < 12) {
+      const int q = warp & 3, part = warp >> 2;
+      const int m = q * 32 + lane;
+      const uint32_t tl = tG + ((uint32_t)(q * 32) << 16);
+      for (int k0 = part * 8; k0 < Kp; k0 += 24) {
+        float hi[8], lo[8];
+#pragma unroll
+        for (int i = 0; i < 8; ++i) {
+          const int k = k0 + i;
+          split_tf32((k < N && m < N) ? G[(size_t)m * N + k] : 0.f, hi[i], lo[i]);
+        }
+        tmem_st8(tl + (uint32_t)k0, hi);
+        tmem_st8(tl + (uint32_t)(Kp + k0), lo);
+      }
+      tmem_st_wait();
+    }
+  }
+  fence_before_sync();
+  __syncthreads();
+  fence_after_sync();
+  const int nsamples = (p.B - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x;
+  const int nchunks = nsamples * aps;
+  // chunk c of this CTA: sample blockIdx.x + (c / aps) * gridDim.x, features [32 (c % aps), +32) (never past a sample)
+  auto chunk_sample = [&](int c) { return (long long)blockIdx.x + (long long)(c / aps) * gridDim.x; };
+  auto chunk_col = [&](int c) { return (c % aps) * ATOM_K; };
+
+  if (uniform_warp_index() == 0) {
+    // =========================== MMA issuer ===========================
+    const uint32_t tmem_base = uniform_u32(*tmem_slot);
+    if (elect_one_sync()) {
+      const uint32_t idesc_hop2 = make_idesc_tf32_atmem_bmn(128, 2 * ATOM_K), idesc_hop = make_idesc_tf32_atmem_bmn(128, ATOM_K);
+      const uint32_t idesc_outer = make_idesc_tf32(128, p.Npad);
+      const uint32_t tG = tmem_base + p.col_g, d_hop = tmem_base + p.col_hop;
+      const uint32_t d_main = tmem_base, d_cross = tmem_base + (uint32_t)p.Npad;
+      uint32_t drain_parity = 0;
+      for (int c = 0; c < nchunks; ++c) {
+        const int st = c % TA_STAGES;
+        mbar_wait(&full[st], (uint32_t)(c / TA_STAGES) & 1u);   // the producers staged this chunk
+        mbar_wait(hopempty, ((uint32_t)c & 1u) ^ 1u);             // the epilogue read the previous hop result
+        fence_after_sync();
+        const uint32_t s0 = smem_u32(smem + (size_t)st * p.stage_bytes);
+        // hop: the MMA sequence of tc_support_kernel on a 32-column tile ([X_hi | X_lo] are one column-block apart)
+        const uint64_t xh0 = make_smem_desc_mn32(s0 + off_xm, p.imgX, MN32_GROUP_BYTES);
+#pragma unroll 1
+        for (int ks = 0; ks < Kp / 8; ++ks) {
+          const uint64_t o = (uint64_t)(ks * ((2 * MN32_GROUP_BYTES) >> 4));
+          const uint32_t gh = tG + (uint32_t)(ks * 8), gl = gh + (uint32_t)Kp;
+          mma_tf32_atmem(d_hop, gh, xh0 + o, idesc_hop2, ks > 0 ? 1u : 0u);   // [main | cross] (+)= G_hi x [X_hi | X_lo]
+          mma_tf32_atmem(d_hop + ATOM_K, gl, xh0 + o, idesc_hop, 1u);         // cross += G_lo x X_hi
+        }
+        mma_commit(hopfull);
+        // outer product: the MMA sequence of tc_outer_kernel into the one [main | cross] slot
+        const int in_set = c % TA_DRAIN;
+        if (c > 0 && in_set == 0) {   // a new chain: the producers must have drained the slot
+          mbar_wait(drained, drain_parity);
+          drain_parity ^= 1u;
+          fence_after_sync();
+        }
+        const int kleft = W - chunk_col(c);
+        const int ksteps = kleft >= ATOM_K ? 4 : (kleft + 7) / 8;
+        const uint32_t a_hi = s0, a_lo = s0 + p.imgA, b_hi = s0 + off_bk, b_lo = b_hi + p.imgBk;
+        for (int ks = 0; ks < ksteps; ++ks) {
+          const uint32_t o = ks * 32;
+          const uint64_t ah = make_smem_desc_sw128(a_hi + o), al = make_smem_desc_sw128(a_lo + o);
+          const uint64_t bh = make_smem_desc_sw128(b_hi + o), bl = make_smem_desc_sw128(b_lo + o);
+          const uint32_t accf = (in_set == 0 && ks == 0) ? 0u : 1u;
+          mma_tf32(d_cross, al, bh, idesc_outer, accf);
+          mma_tf32(d_cross, ah, bl, idesc_outer, 1u);
+          mma_tf32(d_main, ah, bh, idesc_outer, accf);
+        }
+        mma_commit(&empty[st]);   // both products have read the stage
+      }
+    }
+  } else if (warp <= TA_PROD_WARPS) {
+    // =========================== producers / dGs drain ===========================
+    const int pt = tid - 32;
+    const int q = pt & 7, r0 = pt >> 3;   // 16-byte chunk q of rows r0 + 32 i
+    uint32_t kofs[4], mofs[4];
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+      kofs[i] = atom_chunk_offset(r0 + 32 * i, q);
+      mofs[i] = mn32_chunk_offset(r0 + 32 * i, q);
+    }
+    float4 rx[4], ra[4];
+    // columns past W are loaded as zeros, so that no image keeps a column of an earlier chunk
+    auto fetch = [&](int c, float4 (&x)[4], float4 (&a)[4]) {
+      const int j = chunk_col(c) + 4 * q;
+      const bool ok = c < nchunks && j < W;
+      const long long b = ok ? chunk_sample(c) : 0;
+      const float* xs = X + b * x_bs + j;
+      const float* as = A + b * a_bs + j;
+#pragma unroll
+      for (int i = 0; i < 4; ++i) {
+        const int r = r0 + 32 * i;
+        const bool v = ok && r < N;
+        x[i] = v ? __ldg(reinterpret_cast<const float4*>(xs + (long long)r * W)) : make_float4(0.f, 0.f, 0.f, 0.f);
+        a[i] = v ? __ldg(reinterpret_cast<const float4*>(as + (long long)r * W)) : make_float4(0.f, 0.f, 0.f, 0.f);
+      }
+    };
+    auto stage = [&](int c, const float4 (&x)[4], const float4 (&a)[4]) {
+      const int st = c % TA_STAGES;
+      mbar_wait(&empty[st], ((uint32_t)(c / TA_STAGES) & 1u) ^ 1u);   // both products of chunk c - TA_STAGES are done
+      uint8_t* s0 = smem + (size_t)st * p.stage_bytes;
+#pragma unroll
+      for (int i = 0; i < 4; ++i) {
+        if (r0 + 32 * i < N) {
+          float4 h, l;
+          split_tf32(x[i].x, h.x, l.x);
+          split_tf32(x[i].y, h.y, l.y);
+          split_tf32(x[i].z, h.z, l.z);
+          split_tf32(x[i].w, h.w, l.w);
+          *reinterpret_cast<float4*>(s0 + off_bk + kofs[i]) = h;
+          *reinterpret_cast<float4*>(s0 + off_bk + p.imgBk + kofs[i]) = l;
+          *reinterpret_cast<float4*>(s0 + off_xm + mofs[i]) = h;
+          *reinterpret_cast<float4*>(s0 + off_xm + p.imgX + mofs[i]) = l;
+          store_split4(s0, s0 + p.imgA, kofs[i], a[i]);
+        }
+      }
+      fence_async_smem();
+      __syncwarp();
+      if (lane == 0) mbar_arrive(&full[st]);
+    };
+    // dGs slot: thread (sub-partition sp, half) owns row 32 sp + lane and Npad / 2 columns
+    const int sp = warp & 3, half = (warp - 1) >> 2;
+    const int nrow = sp * 32 + lane;
+    const uint32_t tl = tmem_base + ((uint32_t)(sp * 32) << 16);
+    const int ncols_half = p.Npad >> 1, col0 = half * ncols_half;
+    float acc[7][8];   // Npad <= 112 -> at most 56 columns per thread
+#pragma unroll
+    for (int i = 0; i < 7; ++i)
+#pragma unroll
+      for (int j = 0; j < 8; ++j) acc[i][j] = 0.f;
+    auto drain = [&](int c) {   // chunk c closes a chain
+      mbar_wait(&empty[c % TA_STAGES], (uint32_t)(c / TA_STAGES) & 1u);
+      fence_after_sync();
+#pragma unroll
+      for (int ch = 0; ch < 7; ++ch) {
+        if (ch * 8 < ncols_half) {
+          float v[8], t[8];
+          tmem_ld8(tl + (uint32_t)(p.Npad + col0 + ch * 8), v);
+          tmem_ld8(tl + (uint32_t)(col0 + ch * 8), t);
+#pragma unroll
+          for (int i = 0; i < 8; ++i) acc[ch][i] += v[i] + t[i];
+        }
+      }
+      fence_before_sync();
+      __syncwarp();
+      if (lane == 0) mbar_arrive(drained);
+    };
+    // One chunk in registers (two would not fit beside the dGs partials: 13 warps get 128 registers a thread): the next
+    // chunk's loads are issued as soon as this one is staged and fly during the stage wait and the drains.  A chain is
+    // drained once the first chunk of the next one is staged, so that its hop runs meanwhile.
+    fetch(0, rx, ra);
+    for (int c = 0; c < nchunks; ++c) {
+      stage(c, rx, ra);
+      fetch(c + 1, rx, ra);
+      if (c > 0 && c % TA_DRAIN == 0) drain(c - 1);
+    }
+    drain(nchunks - 1);
+
+    if (nrow < N) {
+      const bool v4 = (N & 3) == 0 && (reinterpret_cast<uintptr_t>(dG) & 15) == 0;
+#pragma unroll
+      for (int ch = 0; ch < 7; ++ch) {
+        if (ch * 8 < ncols_half) {
+#pragma unroll
+          for (int i = 0; i < 8; i += 4) {
+            const int m = col0 + ch * 8 + i;
+            float* dst = &dG[(size_t)nrow * N + m];
+            if (v4 && m + 3 < N) {
+              red_add_v4(dst, coef * acc[ch][i], coef * acc[ch][i + 1], coef * acc[ch][i + 2], coef * acc[ch][i + 3]);
+            } else {
+#pragma unroll
+              for (int e = 0; e < 4; ++e)
+                if (m + e < N) atomicAdd(dst + e, coef * acc[ch][i + e]);
+            }
+          }
+        }
+      }
+    }
+  } else {
+    // =========================== hop epilogue: TMEM -> staging tile -> coalesced rows ===========================
+    const int sp = warp & 3;
+    const int m = sp * 32 + lane;
+    const bool live = m < N;
+    const uint32_t tl = tmem_base + p.col_hop + ((uint32_t)(sp * 32) << 16);
+    float* Obuf = reinterpret_cast<float*>(smem + p.off_o);
+    const int et = tid - 32 * (1 + TA_PROD_WARPS);   // 0..127
+    const int ch = et & 7, er0 = et >> 3;            // global side: 16-byte chunk `ch` of rows er0 + 16 i
+    const long long nw = (long long)N * W;
+    float4 zreg[8];                                  // Yb travels one chunk ahead in registers (N <= 128)
+    auto fetch_z = [&](int c) {
+      const int j = chunk_col(c) + 4 * ch;
+      const bool ok = c < nchunks && j < W;
+      const float* zsrc = Yb + (ok ? chunk_sample(c) : 0) * nw + j;
+#pragma unroll
+      for (int i = 0; i < 8; ++i) {
+        const int r = er0 + 16 * i;
+        zreg[i] = (ok && r < N) ? *reinterpret_cast<const float4*>(zsrc + (long long)r * W) : make_float4(0.f, 0.f, 0.f, 0.f);
+      }
+    };
+    fetch_z(0);
+    for (int c = 0; c < nchunks; ++c) {
+      const int jc = chunk_col(c) + 4 * ch;
+      const long long bc = chunk_sample(c);
+#pragma unroll
+      for (int i = 0; i < 8; ++i) {
+        const int r = er0 + 16 * i;
+        if (r < N) *reinterpret_cast<float4*>(Obuf + r * TA_OLD + 4 * ch) = zreg[i];
+      }
+      asm volatile("bar.sync 1, 128;" ::: "memory");
+      fetch_z(c + 1);
+      mbar_wait(hopfull, (uint32_t)c & 1u);
+      fence_after_sync();
+      float* orow = Obuf + m * TA_OLD;
+#pragma unroll
+      for (int hh = 0; hh < ATOM_K / 16; ++hh) {
+        uint32_t vm[16], vs[16];
+        tmem_ld16_async(tl + (uint32_t)(hh * 16), vm);
+        tmem_ld16_async(tl + (uint32_t)(ATOM_K + hh * 16), vs);
+        tmem_ld_wait();
+        tmem_ld_pin16(vm);
+        tmem_ld_pin16(vs);
+        if (live) {
+#pragma unroll
+          for (int g = 0; g < 4; ++g) {
+            // tc_support_kernel's o = alpha * (main + cross); o = fmaf(beta, z, o) with beta = 1 (kept uncontracted)
+            float4* slot = reinterpret_cast<float4*>(orow + hh * 16 + 4 * g);
+            const float4 z = *slot;
+            float4 o;
+            o.x = __fadd_rn(coef * (__uint_as_float(vm[4 * g + 0]) + __uint_as_float(vs[4 * g + 0])), z.x);
+            o.y = __fadd_rn(coef * (__uint_as_float(vm[4 * g + 1]) + __uint_as_float(vs[4 * g + 1])), z.y);
+            o.z = __fadd_rn(coef * (__uint_as_float(vm[4 * g + 2]) + __uint_as_float(vs[4 * g + 2])), z.z);
+            o.w = __fadd_rn(coef * (__uint_as_float(vm[4 * g + 3]) + __uint_as_float(vs[4 * g + 3])), z.w);
+            *slot = o;
+          }
+        }
+      }
+      fence_before_sync();
+      __syncwarp();
+      if (lane == 0) mbar_arrive(hopempty);   // the accumulators are free again while the chunk is still being stored
+      asm volatile("bar.sync 1, 128;" ::: "memory");
+      if (jc < W) {
+        float* ydst = Yb + bc * nw + jc;
+#pragma unroll 4
+        for (int r = er0; r < N; r += 16)
+          *reinterpret_cast<float4*>(ydst + (long long)r * W) = *reinterpret_cast<const float4*>(Obuf + r * TA_OLD + 4 * ch);
+      }
+      asm volatile("bar.sync 1, 128;" ::: "memory");   // the staging tile is rewritten by the next chunk
+    }
+  }
+  __syncthreads();
+  if (warp == 0) tmem_dealloc(tmem_base, 512);
+}
+
+int try_launch_support_adj_tc(const float* G, int N, int B, int width, const float* x, int64_t x_bs, float* ybar,
+                              float* axpy_out, const float* a, int64_t a_bs, float coef, float* dG, cudaStream_t st,
+                              bool* handled) {
+  *handled = false;
+  if (tc_support_disabled() || B <= 0) return STC_OK;
+  if (N < 8 || N > TA_MAX_N || width % 4 != 0 || x_bs % 4 != 0 || a_bs % 4 != 0) return STC_OK;
+  if (!aligned16s(x) || !aligned16s(ybar) || !aligned16s(a) || (axpy_out && !aligned16s(axpy_out))) return STC_OK;
+  TcAdjPlan p;
+  p.N = N;
+  p.Kp = (N + 7) & ~7;
+  p.Npad = (N + 15) & ~15;
+  p.W = width;
+  p.B = B;
+  p.atoms_per_sample = (width + ATOM_K - 1) / ATOM_K;
+  // TMEM (512 columns): dGs [main | cross] 2 Npad, then the hop's [main | cross] 2 x 32, then the support hi | lo 2 Kp.
+  // N = 100: 224 + 64 + 208 = 496;  N = 112: 224 + 64 + 224 = 512.  No room for a second hop accumulator (tc_support_kernel
+  // has two): the hop of chunk c + 1 waits until the epilogue has read chunk c out of TMEM.
+  p.col_hop = 2 * (uint32_t)p.Npad;
+  p.col_g = p.col_hop + 2 * ATOM_K;
+  if (p.col_g + 2 * (uint32_t)p.Kp > 512) return STC_OK;
+  p.imgA = 128 * ATOM_ROW_BYTES;                                            // M = 128 rows of Y_{k-1}
+  p.imgBk = (uint32_t)round_up((size_t)p.Npad * ATOM_ROW_BYTES, 1024);    // Npad rows of ybar_k
+  p.imgX = (uint32_t)p.Kp * ATOM_ROW_BYTES;                                 // Kp K-rows of one 32-column block
+  p.stage_bytes = 2 * (p.imgA + p.imgBk + p.imgX);
+  // shared memory at N = 112: 2 stages x (32 + 28 + 28 KB) + the 18 KB staging tile = 194 KB
+  size_t o = (size_t)TA_STAGES * p.stage_bytes;
+  p.off_o = (uint32_t)o;
+  o += (size_t)128 * TA_OLD * sizeof(float);
+  p.off_bar = (uint32_t)o;
+  o += 8 * (2 * TA_STAGES + 3) + 16;
+  p.smem_bytes = (uint32_t)o;
+  if (p.smem_bytes > 227 * 1024) return STC_OK;
+  STC_TRY(set_smem(tc_support_adj_kernel, p.smem_bytes));
+  // the Chebyshev axpy ybar[k-2] -= ybar[k] of terms k >= 2 stays its own pass, ahead of the kernel (as in the pair)
+  if (axpy_out) STC_TRY(launch_axpy_rows(axpy_out, x, x_bs, -1.f, N, B, width, st));
+  int grid = device_sm_count();
+  if (grid > B) grid = B;
+  ScopedKernelTimer _t(KK_TC_SUPPORT_ADJ, st, 4.0 * B * N * width * 4 + 4.0 * N * N);
+  tc_support_adj_kernel<<<grid, TA_THREADS, p.smem_bytes, st>>>(G, x, x_bs, ybar, a, a_bs, coef, dG, p);
+  STC_LAUNCH_OK("tc_support_adj_kernel");
+  *handled = true;
+  return STC_OK;
+}
+
 }  // namespace stc
