@@ -227,6 +227,19 @@ size_t stc_pair_topk_workspace_bytes(int32_t N, int64_t width, int32_t k);
 int stc_pair_topk(int32_t N, int64_t width, const float* u, const float* v, int32_t k,
                   int32_t* cols, float* scores, void* ws, size_t ws_bytes, void* stream);
 
+/* stc_pair_topk for the query rows [row0, row0 + n_rows) only, scored against all N columns: cols / scores are
+ * [n_rows][k] (global column ids), row i holding row row0 + i of the full selection, bitwise (the K-chain order and the
+ * column tiling do not depend on the rows selected; the segment merge is a total order on (score, column)).  u, v are
+ * the full [N][width] operands.  0 <= row0, row0 + n_rows <= N; row0 need not be a multiple of 128.  n_rows == 0
+ * launches nothing and reads no other argument.  The segment count comes from the number of 128-row blocks, so a block
+ * of N / 8 rows still fills the device.  ws: at least stc_pair_topk_rows_workspace_bytes(N, width, n_rows, k) bytes
+ * (sized for n_rows; 0 for n_rows == 0 and for arguments stc_pair_topk_rows would reject), queried on the device it
+ * runs on.  Every argument check returns before a launch.  The row-partitioned generator (stc_gnn_b200/sparse_mgp.py)
+ * selects each rank's own rows with it. */
+size_t stc_pair_topk_rows_workspace_bytes(int32_t N, int64_t width, int32_t n_rows, int32_t k);
+int stc_pair_topk_rows(int32_t N, int64_t width, const float* u, const float* v, int32_t row0, int32_t n_rows,
+                       int32_t k, int32_t* cols, float* scores, void* ws, size_t ws_bytes, void* stream);
+
 /* ---- the backward split the same way (gradients through a row-partitioned graph) ----
  * Order: stage STC_STAGE_CANDI first, then STC_STAGE_GATES (the reverse of the forward).
  *   1. STC_STAGE_CANDI: clears the parameter and Gc gradients unless accumulate_params, runs the candidate-conv adjoint.  Leaves

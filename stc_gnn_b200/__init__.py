@@ -11,7 +11,8 @@ Public surface:
   pair_topk / topk_pattern  the k best columns of every row over all N (the generator's k= mode chooses its pattern)
   install / run_main  rebind STC_GNN.STC_Cell so Model_Trainer.py / Main.py run unchanged
   dp                  batch data-parallel gradient bucket (one flat all-reduce per step)
-  halo                row-partitioned CSR support with per-hop halo exchange
+  halo                row-partitioned CSR support with per-hop halo exchange (RowPartition: the generator's k= mode
+                      on the row-partitioned graph, each rank selecting its own rows)
   GraphedStep         CUDA-graph capture/replay of one forward+backward step (launch-bound small batches)
 """
 from .cell import STC_Cell, GraphConvParams, stc_cell_forward  # noqa: F401

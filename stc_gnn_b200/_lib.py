@@ -25,6 +25,7 @@ EXPORTED = (
     "stc_cell_fwd_x", "stc_cell_bwd_x", "stc_support_outer", "stc_support_apply_edge_grad",
     "stc_support_apply_rows_edge_grad", "stc_pair_scores_csr", "stc_edge_softmax_fwd", "stc_edge_softmax_bwd",
     "stc_pair_scores_csr_rows", "stc_pair_topk_workspace_bytes", "stc_pair_topk",
+    "stc_pair_topk_rows_workspace_bytes", "stc_pair_topk_rows",
 )
 STAGE_GATES, STAGE_CANDI = 0, 1
 SAVED_REGIONS = ("u", "r", "c", "Yr", "Yx", "Yh", "Q", "Pg", "Pc")
@@ -85,6 +86,11 @@ def load(build_if_missing: bool = True):
     lib.stc_pair_topk.restype = c_int
     lib.stc_pair_topk.argtypes = [c_int32, c_int64, c_void_p, c_void_p, c_int32, c_void_p, c_void_p, c_void_p, c_size_t,
                                   c_void_p]
+    lib.stc_pair_topk_rows_workspace_bytes.restype = c_size_t
+    lib.stc_pair_topk_rows_workspace_bytes.argtypes = [c_int32, c_int64, c_int32, c_int32]
+    lib.stc_pair_topk_rows.restype = c_int
+    lib.stc_pair_topk_rows.argtypes = [c_int32, c_int64, c_void_p, c_void_p, c_int32, c_int32, c_int32, c_void_p,
+                                       c_void_p, c_void_p, c_size_t, c_void_p]
     lib.stc_edge_softmax_fwd.restype = c_int
     lib.stc_edge_softmax_fwd.argtypes = [POINTER(StcSupport), c_int32, c_void_p, c_void_p, c_void_p]
     lib.stc_edge_softmax_bwd.restype = c_int

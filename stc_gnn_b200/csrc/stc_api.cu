@@ -326,7 +326,7 @@ const char* stc_kernel_kind_name(int32_t kind) {
   static const char* names[KK_COUNT] = {"support_dense", "support_csr", "support_outer", "cheby_small",
                                         "conv_fwd",      "conv_bwd_dx", "conv_bwd_dw", "tc_conv_fwd", "tc_conv_bwd_dx", "tc_conv_bwd_dw",
                                         "tc_support", "tc_gemm_test", "tc_outer", "tc_support_big", "support_csr_grad",
-                                        "pair_scores_csr", "edge_softmax", "pair_topk", "tc_support_adj"};
+                                        "pair_scores_csr", "edge_softmax", "pair_topk", "tc_support_adj", "pair_topk_rows"};
   return (kind >= 0 && kind < KK_COUNT) ? names[kind] : "?";
 }
 
@@ -1058,7 +1058,13 @@ static int check_topk_shape(int32_t N, int64_t width, int32_t k, const char* who
 
 size_t stc_pair_topk_workspace_bytes(int32_t N, int64_t width, int32_t k) {
   if (check_topk_shape(N, width, k, "stc_pair_topk_workspace_bytes") != STC_OK) return 0;
-  return pair_topk_ws_bytes(N, k);
+  return pair_topk_ws_bytes(N, N, k);
+}
+
+size_t stc_pair_topk_rows_workspace_bytes(int32_t N, int64_t width, int32_t n_rows, int32_t k) {
+  if (check_topk_shape(N, width, k, "stc_pair_topk_rows_workspace_bytes") != STC_OK || n_rows < 0 || n_rows > N)
+    return 0;
+  return pair_topk_ws_bytes(N, n_rows, k);
 }
 
 int stc_pair_topk(int32_t N, int64_t width, const float* u, const float* v, int32_t k, int32_t* cols, float* scores,
@@ -1074,12 +1080,38 @@ int stc_pair_topk(int32_t N, int64_t width, const float* u, const float* v, int3
     return STC_ERR_BAD_ARG;
   }
   STC_TRY(check_arch());
-  const size_t need = pair_topk_ws_bytes(N, k);
+  const size_t need = pair_topk_ws_bytes(N, N, k);
   if (ws_bytes < need) {
     set_error("stc_pair_topk: workspace of %zu bytes, %zu needed", ws_bytes, need);
     return STC_ERR_WORKSPACE;
   }
-  return launch_pair_topk(N, (int)width, u, v, k, cols, scores, ws, (cudaStream_t)stream);
+  return launch_pair_topk(N, (int)width, u, v, 0, N, k, cols, scores, ws, (cudaStream_t)stream);
+}
+
+int stc_pair_topk_rows(int32_t N, int64_t width, const float* u, const float* v, int32_t row0, int32_t n_rows,
+                       int32_t k, int32_t* cols, float* scores, void* ws, size_t ws_bytes, void* stream) {
+  reset_launch_count();
+  STC_TRY(check_topk_shape(N, width, k, "stc_pair_topk_rows"));
+  if (row0 < 0 || n_rows < 0 || (int64_t)row0 + n_rows > N) {
+    set_error("stc_pair_topk_rows: rows [%d, %d + %d) outside [0, N = %d)", row0, row0, n_rows, N);
+    return STC_ERR_BAD_ARG;
+  }
+  if (n_rows == 0) return STC_OK;
+  if (!u || !v || !cols || !ws) {
+    set_error("stc_pair_topk_rows: NULL argument");
+    return STC_ERR_BAD_ARG;
+  }
+  if ((reinterpret_cast<uintptr_t>(u) | reinterpret_cast<uintptr_t>(v) | reinterpret_cast<uintptr_t>(ws)) & 15) {
+    set_error("stc_pair_topk_rows: u, v and ws must be 16-byte aligned");
+    return STC_ERR_BAD_ARG;
+  }
+  STC_TRY(check_arch());
+  const size_t need = pair_topk_ws_bytes(N, n_rows, k);
+  if (ws_bytes < need) {
+    set_error("stc_pair_topk_rows: workspace of %zu bytes, %zu needed", ws_bytes, need);
+    return STC_ERR_WORKSPACE;
+  }
+  return launch_pair_topk(N, (int)width, u, v, row0, n_rows, k, cols, scores, ws, (cudaStream_t)stream);
 }
 
 int stc_cell_bwd_scratch_layout(const StcDims* dp, int64_t* offsets, int32_t n_offsets) {

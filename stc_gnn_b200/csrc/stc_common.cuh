@@ -43,7 +43,7 @@ void reset_launch_count();
 enum KernelKind {
   KK_SUPPORT_DENSE = 0, KK_SUPPORT_CSR, KK_SUPPORT_OUTER, KK_CHEBY_SMALL, KK_CONV_FWD, KK_CONV_BWD_DX,
   KK_CONV_BWD_DW, KK_TC_CONV_FWD, KK_TC_CONV_BWD_DX, KK_TC_CONV_BWD_DW, KK_TC_SUPPORT, KK_TC_GEMM_TEST, KK_TC_OUTER, KK_TC_SUPPORT_BIG,
-  KK_SUPPORT_CSR_GRAD, KK_PAIR_SCORES_CSR, KK_EDGE_SOFTMAX, KK_PAIR_TOPK, KK_TC_SUPPORT_ADJ, KK_COUNT
+  KK_SUPPORT_CSR_GRAD, KK_PAIR_SCORES_CSR, KK_EDGE_SOFTMAX, KK_PAIR_TOPK, KK_TC_SUPPORT_ADJ, KK_PAIR_TOPK_ROWS, KK_COUNT
 };
 struct ScopedKernelTimer {  // declare right before a launch; the destructor records the stop event
   ScopedKernelTimer(int kind, cudaStream_t st, double alg_bytes);
@@ -140,11 +140,12 @@ int launch_pair_scores_csr_rows(const int32_t* rowptr, const int32_t* col, long 
                                 int n_rows, cudaStream_t st);
 int launch_edge_softmax(bool bwd, const int32_t* rowptr, long long nnz, int N, const float* s, const float* p,
                         const float* dp, float* out, cudaStream_t st);
-// top-k pair scores over all columns (stc_pair_topk.cu); arguments checked by the caller (1 <= k <= min(N, 32),
-// width % 4 == 0, u / v 16-byte aligned, ws of pair_topk_ws_bytes)
-size_t pair_topk_ws_bytes(int N, int k);
-int launch_pair_topk(int N, int width, const float* u, const float* v, int k, int32_t* cols, float* scores, void* ws,
-                     cudaStream_t st);
+// top-k pair scores of the rows [row0, row0 + n_rows) over all N columns (stc_pair_topk.cu); arguments checked by the
+// caller (1 <= k <= min(N, 32), width % 4 == 0, 0 <= row0, row0 + n_rows <= N, u / v 16-byte aligned, ws of
+// pair_topk_ws_bytes); n_rows == 0 launches nothing and needs no workspace
+size_t pair_topk_ws_bytes(int N, int n_rows, int k);
+int launch_pair_topk(int N, int width, const float* u, const float* v, int row0, int n_rows, int k, int32_t* cols,
+                     float* scores, void* ws, cudaStream_t st);
 
 int launch_cheby_small(const float* G, int C, int K, float* Q, cudaStream_t st);
 int launch_cheby_small_bwd(const float* G, const float* Q, float* dQ, int C, int K, float* dG, cudaStream_t st);

@@ -1,5 +1,7 @@
 // Top-k pair scores of the graph generator over ALL candidate columns: the pattern-choosing step of the sparse MGP_Gen
-// (stc_gnn_b200/sparse_mgp.py topk_pattern).  Nothing of size N^2 ever reaches HBM.
+// (stc_gnn_b200/sparse_mgp.py topk_pattern).  Nothing of size N^2 ever reaches HBM.  The query rows may be a block
+// [row0, row0 + n_rows) of the N nodes (a rank of the row-partitioned generator selects its own rows only); the column
+// tiles always start at column 0, so each row's K chains, tiles and result are those of the full selection.
 //
 //  tc_pair_topk_kernel      S[n][m] = <U_n, V_m> - <V_n, U_m> = [U | V]_n . [V | -U]_m: one 3xTF32 GEMM with K = 2W over
 //      128 x 128 tiles.  A CTA owns the 128 query rows of block blockIdx.x and sweeps the column tiles of segment
@@ -46,6 +48,7 @@ constexpr uint32_t TK_SMEM = TK_OFF_BAR + 8 * (2 * TK_SH + 1) + 16;
 
 struct TopkPlan {
   int N, W, k;
+  int row0, n_rows;    // the query rows [row0, row0 + n_rows); the columns are always all N
   int aph;             // K-atoms per half (ceil(W / 32)); a tile takes 2 aph atoms
   int ntiles, tiles_per_seg;
 };
@@ -100,7 +103,7 @@ tc_pair_topk_kernel(const float* __restrict__ U, const float* __restrict__ V, fl
   fence_after_sync();
   const int warp_u = uniform_warp_index();
   const uint32_t tmem_base = uniform_u32(*tmem_slot);
-  const int n0 = (int)blockIdx.x * TK_TILE, rowsA = min(TK_TILE, N - n0);
+  const int n0 = p.row0 + (int)blockIdx.x * TK_TILE, rowsA = min(TK_TILE, p.row0 + p.n_rows - n0);
   const int t0 = (int)blockIdx.y * p.tiles_per_seg, t1 = min(p.ntiles, t0 + p.tiles_per_seg);
   const long long natoms = (long long)(t1 - t0) * apt;
 
@@ -277,7 +280,7 @@ tc_pair_topk_kernel(const float* __restrict__ U, const float* __restrict__ V, fl
     cp_async_wait<0>();
 
     if (half == 0 && nrow < rowsA) {   // the last tile's barrier has passed: the list is complete
-      const size_t o = ((size_t)blockIdx.y * N + n0 + nrow) * k;
+      const size_t o = ((size_t)blockIdx.y * p.n_rows + (n0 - p.row0) + nrow) * k;
       for (int i = 0; i < k; ++i) {
         ws_s[o + i] = ls[i];
         ws_c[o + i] = lc[i];
@@ -290,12 +293,12 @@ tc_pair_topk_kernel(const float* __restrict__ U, const float* __restrict__ V, fl
 }
 
 __global__ void __launch_bounds__(128)
-pair_topk_merge_kernel(const float* __restrict__ ws_s, const int* __restrict__ ws_c, int N, int nseg, int k,
+pair_topk_merge_kernel(const float* __restrict__ ws_s, const int* __restrict__ ws_c, int n_rows, int nseg, int k,
                        int32_t* __restrict__ cols, float* __restrict__ scores) {
   __shared__ float Ms[128 * TK_LD];
   __shared__ int Mc[128 * TK_LD];
   const int n = (int)(blockIdx.x * blockDim.x + threadIdx.x);
-  if (n >= N) return;
+  if (n >= n_rows) return;
   float* ls = Ms + threadIdx.x * TK_LD;
   int* lc = Mc + threadIdx.x * TK_LD;
   for (int i = 0; i < k; ++i) {   // segment 0's list is sorted already
@@ -303,7 +306,7 @@ pair_topk_merge_kernel(const float* __restrict__ ws_s, const int* __restrict__ w
     lc[i] = ws_c[(size_t)n * k + i];
   }
   for (int sg = 1; sg < nseg; ++sg) {
-    const size_t o = ((size_t)sg * N + n) * k;
+    const size_t o = ((size_t)sg * n_rows + n) * k;
     for (int i = 0; i < k; ++i) {
       const float s = ws_s[o + i];
       const int c = ws_c[o + i];
@@ -323,14 +326,17 @@ pair_topk_merge_kernel(const float* __restrict__ ws_s, const int* __restrict__ w
 
 namespace {
 struct TopkGeom {
-  int ntiles, tiles_per_seg, nseg;
+  int rblocks, ntiles, tiles_per_seg, nseg;
 };
 // Row blocks alone fill the device when there are at least twice as many as SMs (config 4: 512); otherwise the column
-// range is split into segments until the grid does (config 3, N = 4,096: 32 row blocks x 8 segments of 4 tiles).
-TopkGeom topk_geom(int N) {
+// range is split into segments until the grid does (config 3, N = 4,096: 32 row blocks x 8 segments of 4 tiles; config
+// 4 with a rank's n_rows = N / 8: 64 row blocks x 5 segments).  Only the row blocks count: a rank selecting a block of
+// rows still sweeps all ceil(N / 128) column tiles.
+TopkGeom topk_geom(int N, int n_rows) {
   TopkGeom g;
+  g.rblocks = ceil_div(n_rows, TK_TILE);
   g.ntiles = ceil_div(N, TK_TILE);
-  int nseg = ceil_div(2 * device_sm_count(), g.ntiles);
+  int nseg = ceil_div(2 * device_sm_count(), g.rblocks);
   if (nseg < 1) nseg = 1;
   if (nseg > g.ntiles) nseg = g.ntiles;
   g.tiles_per_seg = ceil_div(g.ntiles, nseg);
@@ -339,29 +345,35 @@ TopkGeom topk_geom(int N) {
 }
 }  // namespace
 
-size_t pair_topk_ws_bytes(int N, int k) {
-  return (size_t)topk_geom(N).nseg * N * k * (sizeof(float) + sizeof(int));
+size_t pair_topk_ws_bytes(int N, int n_rows, int k) {
+  if (n_rows == 0) return 0;
+  return (size_t)topk_geom(N, n_rows).nseg * n_rows * k * (sizeof(float) + sizeof(int));
 }
 
-int launch_pair_topk(int N, int width, const float* u, const float* v, int k, int32_t* cols, float* scores, void* ws,
-                     cudaStream_t st) {
-  const TopkGeom g = topk_geom(N);
+int launch_pair_topk(int N, int width, const float* u, const float* v, int row0, int n_rows, int k, int32_t* cols,
+                     float* scores, void* ws, cudaStream_t st) {
+  if (n_rows == 0) return STC_OK;
+  const TopkGeom g = topk_geom(N, n_rows);
   float* ws_s = static_cast<float*>(ws);
-  int* ws_c = reinterpret_cast<int*>(ws_s + (size_t)g.nseg * N * k);
+  int* ws_c = reinterpret_cast<int*>(ws_s + (size_t)g.nseg * n_rows * k);
   TopkPlan p;
   p.N = N;
   p.W = width;
   p.k = k;
+  p.row0 = row0;
+  p.n_rows = n_rows;
   p.aph = ceil_div(width, ATOM_K);
   p.ntiles = g.ntiles;
   p.tiles_per_seg = g.tiles_per_seg;
   STC_TRY(set_smem(tc_pair_topk_kernel, TK_SMEM));
-  // compulsory HBM traffic: U and V read once (8 N W) and the [N][k] columns and scores written (8 N k); the A rows
-  // re-read for every tile and the workspace lists stay in L2 at the shapes the benchmark runs
-  ScopedKernelTimer _t(KK_PAIR_TOPK, st, 8.0 * N * width + 8.0 * N * k);
-  tc_pair_topk_kernel<<<dim3(g.ntiles, g.nseg), TK_THREADS, TK_SMEM, st>>>(u, v, ws_s, ws_c, p);
+  // compulsory HBM traffic: U and V read once (8 N W: every column row is a B operand; the block's A rows are among
+  // them) and the [n_rows][k] columns and scores written (8 n_rows k); the A rows re-read for every tile and the
+  // workspace lists stay in L2 at the shapes the benchmark runs
+  const bool full = row0 == 0 && n_rows == N;
+  ScopedKernelTimer _t(full ? KK_PAIR_TOPK : KK_PAIR_TOPK_ROWS, st, 8.0 * N * width + 8.0 * n_rows * k);
+  tc_pair_topk_kernel<<<dim3(g.rblocks, g.nseg), TK_THREADS, TK_SMEM, st>>>(u, v, ws_s, ws_c, p);
   STC_LAUNCH_OK("tc_pair_topk_kernel");
-  pair_topk_merge_kernel<<<ceil_div(N, 128), 128, 0, st>>>(ws_s, ws_c, N, g.nseg, k, cols, scores);
+  pair_topk_merge_kernel<<<ceil_div(n_rows, 128), 128, 0, st>>>(ws_s, ws_c, n_rows, g.nseg, k, cols, scores);
   STC_LAUNCH_OK("pair_topk_merge_kernel");
   return STC_OK;
 }

@@ -169,10 +169,12 @@ class ValueMaps:
     edge_pad: int
 
     def padded_index(self, ids: torch.Tensor) -> torch.Tensor:
-        """Positions in the padded all-gather buffer of the global edges `ids` (host, integer arithmetic)."""
-        lo = torch.tensor([b[0] for b in self.edge_bounds], dtype=torch.long)
-        owner = torch.bucketize(ids, lo[1:], right=True)
-        return owner * self.edge_pad + (ids - lo[owner])
+        """Positions in the padded all-gather buffer of the global edges `ids` (integer arithmetic on ids' device, no
+        host copy)."""
+        out = ids.clone()
+        for r, (lo, hi) in enumerate(self.edge_bounds):
+            out = torch.where((ids >= lo) & (ids < hi), ids + (r * self.edge_pad - lo), out)
+        return out
 
 
 def _csr_operator(rowptr: torch.Tensor, col: torch.Tensor, vals: torch.Tensor, n: int):
@@ -222,6 +224,7 @@ class PartitionedSupport:
         self.reduce_per_cell = True
         self._dev = {}       # structure on the device (shared with `with_values` copies)
         self._ops = {}       # learnable: the local operators bound to this object's `vals`
+        self._streams = {}   # side streams and events of the exchange overlap (a RowPartition shares its own)
 
     @classmethod
     def from_dense(cls, G: torch.Tensor, rank: int, world: int, group=None) -> "PartitionedSupport":
@@ -232,6 +235,15 @@ class PartitionedSupport:
     def from_csr_support(cls, cs, rank: int, world: int, group=None) -> "PartitionedSupport":
         """The partition of a `CsrSupport`; a learnable one shares its `vals` (the same tensor, not a copy)."""
         return cls(cs.rowptr, cs.col, cs.vals, cs.N, rank, world, group)
+
+    @classmethod
+    def k_regular(cls, cols: torch.Tensor, rank: int, world: int, group=None) -> "PartitionedSupport":
+        """The partition of the k-regular pattern whose row n stores the columns cols[n] ([N, k] integer, ascending in
+        each row, identical on every rank), with constant zero values: field for field what
+        `PartitionedSupport(k * arange(N + 1), cols.flatten(), zeros, N, rank, world, group)` builds (plans, `maps()`
+        and the exchange state), computed in integer torch ops on cols' device (CPU or CUDA) with one device-to-host
+        copy of a few counts.  `RowPartition.support` is the same with the partition's persistent state."""
+        return RowPartition(cols.shape[0], rank, world, group).support(cols)
 
     @property
     def learnable(self) -> bool:
@@ -387,9 +399,17 @@ class PartitionedSupport:
             st = self._dev[key] = {
                 "send_idx": send.to(torch.int32).to(device), "nsend": int(send.numel()),
                 "interior": interior.to(torch.int32).to(device), "boundary": boundary.to(torch.int32).to(device),
-                "buffers": {}, "side": torch.cuda.Stream(device=device), "ready": torch.cuda.Event(), "done": torch.cuda.Event(),
+                "buffers": {},
             }
         return st
+
+    def _stream_state(self, direction: str, device):
+        """(side stream, ready event, done event) of the exchange overlap of `direction`, created once per partition."""
+        key = (direction, str(device))
+        ss = self._streams.get(key)
+        if ss is None:
+            ss = self._streams[key] = (torch.cuda.Stream(device=device), torch.cuda.Event(), torch.cuda.Event())
+        return ss
 
     def _buffers(self, st, plan, slab: int, device):
         buf = st["buffers"].get(slab)
@@ -453,20 +473,21 @@ class PartitionedSupport:
         lib = _lib.load()
         st = self._device_state(direction, X3.device)
         send, recv = self._buffers(st, plan, B * W, X3.device)
-        main, side = torch.cuda.current_stream(), st["side"]
-        st["ready"].record(main)                     # X3's local rows are final once the main stream gets here
+        side, ready, done = self._stream_state(direction, X3.device)
+        main = torch.cuda.current_stream()
+        ready.record(main)                           # X3's local rows are final once the main stream gets here
         with torch.cuda.stream(side):
-            side.wait_event(st["ready"])
+            side.wait_event(ready)
             _lib.check(lib.stc_halo_pack(X3.data_ptr(), plan.next * W, W, B, st["send_idx"].data_ptr(), st["nsend"],
                                          send.data_ptr(), side.cuda_stream), "stc_halo_pack")
             dist.all_to_all_single(recv, send, output_split_sizes=plan.recv_counts, input_split_sizes=plan.send_counts,
                                    group=self.group)
             _lib.check(lib.stc_halo_unpack(recv.data_ptr(), W, B, plan.nloc, plan.nhalo, X3.data_ptr(), plan.next * W,
                                            side.cuda_stream), "stc_halo_unpack")
-            st["done"].record(side)
+            done.record(side)
         if st["interior"].numel():
             launch(st["interior"])
-        main.wait_event(st["done"])
+        main.wait_event(done)
         launch(st["boundary"])
 
     def spatial_terms(self, X_local: torch.Tensor, Ks: int, apply_fn=None) -> List[torch.Tensor]:
@@ -479,6 +500,124 @@ class PartitionedSupport:
             else:
                 terms.append(self.apply(terms[k - 1], "fwd", alpha=2.0, beta=-1.0, Z_local=terms[k - 2], apply_fn=apply_fn))
         return terms
+
+
+def _positions(mask: torch.Tensor, count: int) -> torch.Tensor:
+    """The indices of the True entries of a 1-D mask, ascending; `count` (known on the host) of them.  A stable sort of
+    the inverted mask instead of `nonzero`, which would synchronise with the device."""
+    return torch.sort((~mask).to(torch.int8), stable=True).indices[:count]
+
+
+class RowPartition:
+    """The row partition of an N-node graph over `world` ranks (rank r owns the nodes `dp.shard_bounds(N, r, world)`)
+    without a fixed pattern: the generator selects a new pattern on every forward (`SparseGraphGenerator(...)(X_seq,
+    k=k, partition=...)`) and `support(cols)` partitions it on the device.  The state that outlives a pattern lives
+    here: the side streams and events of the exchange overlap, and `reduce_per_cell` (copied onto every support; see
+    `PartitionedSupport`)."""
+
+    def __init__(self, num_nodes: int, rank: int, world: int, group: Optional[dist.ProcessGroup] = None):
+        self.N, self.rank, self.world, self.group = int(num_nodes), rank, world, group
+        self.start, stop = shard_bounds(self.N, rank, world)
+        self.nloc = stop - self.start
+        self.reduce_per_cell = True
+        self._streams = {}
+
+    def gather_rows(self, x_loc: torch.Tensor) -> torch.Tensor:
+        """[N, ...] from every rank's node block x_loc [nloc, ...] (one all-gather; the blocks are padded to the largest,
+        ceil(N / world) rows, and compacted); x_loc itself at world 1.  Every rank must call it."""
+        if self.world == 1:
+            return x_loc
+        big = shard_bounds(self.N, 0, self.world)[1]
+        send = x_loc.new_zeros((big,) + tuple(x_loc.shape[1:]))
+        send[:self.nloc] = x_loc
+        out = x_loc.new_empty((self.world * big,) + tuple(x_loc.shape[1:]))
+        dist.all_gather_into_tensor(out, send, group=self.group)
+        return torch.cat([out.narrow(0, r * big, e - s) for r, (s, e) in
+                          enumerate(shard_bounds(self.N, r, self.world) for r in range(self.world))])
+
+    def support(self, cols: torch.Tensor) -> PartitionedSupport:
+        """`PartitionedSupport.k_regular(cols, rank, world, group)` sharing this partition's streams and events.
+
+        Every rank derives what each peer needs from the replicated selection (as `build_plan` does from the replicated
+        graph), in integer torch ops on cols' device.  The halo of rank p is the set of nodes outside block p that a row
+        of p reads or that reads a row of p (the symmetric halo); it is held as a [world, N] membership table, from which
+        the halo lists, the send lists, the extended column numbering and the per-peer counts follow by cumulative
+        sums.  The Gs^T side comes from `support.k_regular_structure`.  One device-to-host copy carries the sizes the
+        host needs (nhalo, the per-peer send and receive counts, the interior counts of both directions, the range of
+        this rank's columns in Gs^T order)."""
+        from .support import k_regular_structure
+        N, k = cols.shape
+        if N != self.N:
+            raise RuntimeError(f"RowPartition: the selection has {N} rows, the partition {self.N} nodes")
+        dev, L = cols.device, torch.long
+        rank, world, s, nloc = self.rank, self.world, self.start, self.nloc
+        e = s + nloc
+        rowptr, col32, t_rowptr, t_col, t_perm = k_regular_structure(cols)
+        col, nnz = col32.to(L), N * k
+        row = torch.arange(N, device=dev, dtype=L)[:, None].expand(N, k).reshape(-1)
+        base, extra = divmod(N, world)
+        p = torch.arange(world + 1, device=dev, dtype=L)
+        starts = p * base + p.clamp(max=extra)                     # shard_bounds of every rank, then N
+        owner = lambda x: torch.bucketize(x, starts[1:], right=True)
+        ro, co = owner(row), owner(col)
+        cross = (ro != co).to(L)
+        member = torch.zeros(world * N, dtype=L, device=dev)
+        member.index_add_(0, ro * N + col, cross).index_add_(0, co * N + row, cross)
+        member = (member > 0).view(world, N)                       # member[p, x]: x is in the halo of rank p
+        mine = member[rank]
+        csum = torch.zeros(N + 1, dtype=L, device=dev)
+        csum[1:] = torch.cumsum(mine, 0)
+        recv = csum[starts[1:]] - csum[starts[:-1]]
+        sendm = member[:, s:e]                                     # what each peer needs of this rank's nodes
+        send = sendm.sum(1)
+        ids = torch.arange(N, device=dev, dtype=L)
+        ext = torch.where((ids >= s) & (ids < e), ids - s, nloc + csum[1:] - 1)   # extended numbering of halo + local
+        own = co.view(N, k)[s:e] != rank
+        has_b = own.any(1)                                         # adjoint rows reading a halo column
+        has_f = torch.zeros(nloc, dtype=L, device=dev)
+        if nloc:
+            into = ((co == rank) & (ro != rank)).to(L)
+            has_f.index_add_(0, torch.where(co == rank, col - s, 0), into)
+        has_f = has_f > 0                                          # forward rows reading a halo column
+        info = torch.cat([csum[N:], recv, send, (~has_f).sum().view(1), (~has_b).sum().view(1),
+                          t_rowptr[s:s + 1].to(L), t_rowptr[e:e + 1].to(L)]).cpu().tolist()   # the one host copy
+        nhalo, recv_counts, send_counts = info[0], info[1:1 + world], info[1 + world:1 + 2 * world]
+        nint_f, nint_b, f0, f1 = info[1 + 2 * world:]
+        halo_global = _positions(mine, nhalo)
+        send_cat = _positions(sendm.reshape(-1), sum(send_counts)) % max(nloc, 1)
+        send_idx = list(torch.split(send_cat, send_counts))
+        lo, hi = k * s, k * e
+        fwd_ids = t_perm[f0:f1]                                    # this rank's columns, Gs^T order = (m, global n)
+        f_edges = torch.sort(fwd_ids).values                       # the same edges in Gs-CSR order
+        zeros = lambda n: torch.zeros(n, dtype=torch.float32, device=dev)
+
+        def plan(op_row, op_col):
+            return HaloPlan(rank=rank, world=world, start=s, nloc=nloc, nhalo=nhalo, send_idx=send_idx,
+                            recv_counts=recv_counts, halo_global=halo_global, op_row=op_row, op_col=op_col,
+                            op_val=zeros(op_row.numel()))
+
+        ps = PartitionedSupport.__new__(PartitionedSupport)
+        ps.N, ps.rank, ps.world, ps.group = N, rank, world, self.group
+        ps._rowptr, ps._col, ps.nnz, ps.vals = rowptr.to(L), col, nnz, None
+        ps.fwd = plan(col[f_edges] - s, ext[row[f_edges]])
+        ps.bwd = plan(row[lo:hi] - s, ext[col[lo:hi]])
+        ps.start, ps.nloc = s, nloc
+        ps.reduce_per_cell = self.reduce_per_cell
+        ps._ops, ps._streams = {}, self._streams
+        nxt = nloc + nhalo
+        pad = lambda rp: torch.cat([rp, rp[-1:].expand(nhalo)])
+        bounds = [(k * a, k * b) for a, b in (shard_bounds(N, r, world) for r in range(world))]
+        maps = ValueMaps(edge_lo=lo, edge_hi=hi, bwd_rowptr=pad(rowptr[s:e + 1].to(L) - lo), bwd_col=ps.bwd.op_col,
+                         fwd_rowptr=pad(t_rowptr[s:e + 1].to(L) - f0), fwd_col=ext[t_col[f0:f1].to(L)], fwd_ids=fwd_ids,
+                         edge_bounds=bounds, edge_pad=max(b - a for a, b in bounds))
+        ps._dev = {"maps": maps}
+        halo_rows = torch.arange(nloc, nxt, device=dev, dtype=L)
+        for direction, has, nint in (("fwd", has_f, nint_f), ("bwd", has_b, nint_b)):
+            ps._dev[("xchg", direction, str(dev))] = {
+                "send_idx": send_cat.to(torch.int32), "nsend": int(send_cat.numel()),
+                "interior": _positions(~has, nint).to(torch.int32),
+                "boundary": torch.cat([_positions(has, nloc - nint), halo_rows]).to(torch.int32), "buffers": {}}
+        return ps
 
 
 def adjoint_chain_ext(ps: PartitionedSupport, ybar: List[torch.Tensor], hop: Optional[Callable] = None,

@@ -42,6 +42,14 @@ The selection is the CUDA kernel stc_pair_topk: all N^2 scores as 128 x 128 tile
 4 N^2 bytes (17 GB at N = 65,536).  Its output is a pure function of (U, V, k): bitwise the same on every call.  A
 score within the 3xTF32 rounding (about 1e-6 relative) of a row's k-th score may be ranked differently from an fp64
 evaluation.
+
+The selection also runs on the row-partitioned graph (`gen(X_seq_block, k=k, partition=halo.RowPartition(N, rank,
+world))`): every rank all-gathers U, V of all N nodes (detached; [N, width] each), selects its own rows over all N
+columns (`pair_topk(..., rows=(start, nloc))`, stc_pair_topk_rows: each row bitwise that row of the full selection),
+all-gathers the [N, k] selection and partitions it on the device (`RowPartition.support`, one small device-to-host
+copy), then forms P exactly as on a fixed partitioned pattern.  Scores of unrelated nodes pick neighbours anywhere in
+the graph, so the halo of a selected pattern can approach every remote node: each hop then moves close to an
+all-gather.
 """
 from __future__ import annotations
 
@@ -261,13 +269,16 @@ def _check_topk_args(N: int, k, who: str) -> None:
         raise RuntimeError(f"{who}: k = {k} outside [1, min(N = {N}, {TOPK_MAX})]")
 
 
-def pair_topk(U: torch.Tensor, V: torch.Tensor, k: int, scores: bool = False):
+def pair_topk(U: torch.Tensor, V: torch.Tensor, k: int, scores: bool = False, rows=None):
     """cols [N, k] int32: the k columns m of each row n with the largest S[n, m] = <U_n, V_m> - <V_n, U_m> over all N
     candidates (S[n, n] = 0; ties to the smaller column), ascending in each row (stc_pair_topk).  With `scores`, also
     the matching S values [N, k] (float32, 3xTF32).  U, V: [N, width] float32 CUDA; a width that is not a multiple of 4
     is padded with zero columns, which add nothing to any score.  A NaN score (NaN or inf in U / V) ranks, and is
     reported, as -inf, so every row still gets k distinct columns in [0, N).  Not differentiable: the result is an
-    index set."""
+    index set.
+
+    `rows=(row0, n_rows)`: only the rows [row0, row0 + n_rows), still scored against all N columns
+    (stc_pair_topk_rows); the result is [n_rows, k] and bitwise those rows of the full selection."""
     for name, t in (("U", U), ("V", V)):
         if t.dtype != torch.float32 or t.dim() != 2:
             raise RuntimeError(f"pair_topk: {name} must be a [N, width] float32 CUDA tensor, got {tuple(t.shape)} "
@@ -276,6 +287,9 @@ def pair_topk(U: torch.Tensor, V: torch.Tensor, k: int, scores: bool = False):
         raise RuntimeError(f"pair_topk: U {tuple(U.shape)} on {U.device} and V {tuple(V.shape)} on {V.device} must match")
     N, width = U.shape
     _check_topk_args(N, k, "pair_topk")
+    row0, n_rows = (0, N) if rows is None else (int(rows[0]), int(rows[1]))
+    if row0 < 0 or n_rows < 0 or row0 + n_rows > N:
+        raise RuntimeError(f"pair_topk: rows [{row0}, {row0} + {n_rows}) outside [0, N = {N})")
     if not U.is_cuda:
         raise RuntimeError(f"pair_topk: U, V live on {U.device} (there is no CPU path)")
     if width == 0:
@@ -284,13 +298,20 @@ def pair_topk(U: torch.Tensor, V: torch.Tensor, k: int, scores: bool = False):
     U, V = (torch.nn.functional.pad(t.detach(), (0, pad)) if pad else t.detach().contiguous() for t in (U, V))
     U, V = (t if t.data_ptr() % 16 == 0 else t.clone() for t in (U, V))
     lib = _lib.load()
-    cols = torch.empty(N, k, dtype=torch.int32, device=U.device)
-    sc = torch.empty(N, k, dtype=torch.float32, device=U.device) if scores else None
-    ws_bytes = lib.stc_pair_topk_workspace_bytes(N, width + pad, k)
-    ws = torch.empty(ws_bytes, dtype=torch.uint8, device=U.device)
-    _lib.check(lib.stc_pair_topk(N, width + pad, U.data_ptr(), V.data_ptr(), k, cols.data_ptr(),
-                                 sc.data_ptr() if scores else None, ws.data_ptr(), ws_bytes,
-                                 torch.cuda.current_stream().cuda_stream), "stc_pair_topk")
+    cols = torch.empty(n_rows, k, dtype=torch.int32, device=U.device)
+    sc = torch.empty(n_rows, k, dtype=torch.float32, device=U.device) if scores else None
+    stream = torch.cuda.current_stream().cuda_stream
+    if rows is None:
+        ws_bytes = lib.stc_pair_topk_workspace_bytes(N, width + pad, k)
+        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=U.device)
+        _lib.check(lib.stc_pair_topk(N, width + pad, U.data_ptr(), V.data_ptr(), k, cols.data_ptr(),
+                                     sc.data_ptr() if scores else None, ws.data_ptr(), ws_bytes, stream), "stc_pair_topk")
+    elif n_rows:
+        ws_bytes = lib.stc_pair_topk_rows_workspace_bytes(N, width + pad, n_rows, k)
+        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=U.device)
+        _lib.check(lib.stc_pair_topk_rows(N, width + pad, U.data_ptr(), V.data_ptr(), row0, n_rows, k, cols.data_ptr(),
+                                          sc.data_ptr() if scores else None, ws.data_ptr(), ws_bytes, stream),
+                   "stc_pair_topk_rows")
     return (cols, sc) if scores else cols
 
 
@@ -317,7 +338,8 @@ class SparseGraphGenerator(nn.Module):
         for p in self.params_S.values():
             nn.init.xavier_normal_(p)
 
-    def forward(self, X_seq: torch.Tensor, pattern=None, group=None, average: bool = False, k: int = None):
+    def forward(self, X_seq: torch.Tensor, pattern=None, group=None, average: bool = False, k: int = None,
+                partition: halo.RowPartition = None):
         """X_seq [B, T, N, C] float32 CUDA -> `pattern.with_values(P)`.  Under torch.no_grad() the values do not require
         grad and the cell treats the support as constant.  `group` / `average`: batch data-parallel, as in
         `pair_softmax_csr` (X_seq is this rank's shard).
@@ -332,9 +354,26 @@ class SparseGraphGenerator(nn.Module):
 
         `k` instead of `pattern`: the pattern is chosen from the scores, the k largest of every row over all N columns
         (`topk_pattern` on U, V detached; module docstring), and P is formed on it as on a fixed pattern.  The result is
-        a k-regular `CsrSupport`.  Not combinable with a row-partitioned graph or with batch data-parallelism."""
+        a k-regular `CsrSupport`.  Not combinable with batch data-parallelism, nor with a fixed `PartitionedSupport`.
+
+        `k` with `partition` (a `halo.RowPartition`): the same selection on the row-partitioned graph.  X_seq is this
+        rank's node block [B, T, nloc, C]; U, V of every node are all-gathered (detached), the rank selects its own rows
+        (`pair_topk(..., rows=(start, nloc))`), the [N, k] selection is all-gathered and partitioned on the device
+        (`partition.support`), and P is formed on it exactly as on a fixed partitioned pattern (gradients, the Wu / Wv
+        reduction by `partition.reduce_per_cell`, the no-grad path).  The result is a `PartitionedSupport`; every rank
+        runs the forward and the backward."""
         Wu, Wv = self.params_S["Wu"], self.params_S["Wv"]
         partitioned = isinstance(pattern, PartitionedSupport)
+        if partition is not None:
+            if not isinstance(partition, halo.RowPartition):
+                raise RuntimeError(f"SparseGraphGenerator: partition must be a halo.RowPartition, got "
+                                   f"{type(partition).__name__}")
+            if k is None or pattern is not None:
+                raise RuntimeError("SparseGraphGenerator: partition= selects the pattern on the row-partitioned graph: "
+                                   "give k=, and no pattern")
+            if group is not None or average:
+                raise RuntimeError("SparseGraphGenerator: batch data-parallelism (group= / average=) cannot be combined "
+                                   "with a row partition")
         if k is not None:
             if partitioned:
                 raise RuntimeError("SparseGraphGenerator: k= selects the pattern on one device; a row-partitioned "
@@ -355,7 +394,12 @@ class SparseGraphGenerator(nn.Module):
         if pattern is None and k is None:
             raise RuntimeError(both)
         B, T, N, C = X_seq.shape
-        if k is not None:
+        if partition is not None:
+            if N != partition.nloc:
+                raise RuntimeError(f"SparseGraphGenerator: this rank's block of the partition has {partition.nloc} "
+                                   f"nodes, the input {N}")
+            _check_topk_args(partition.N, k, "SparseGraphGenerator")
+        elif k is not None:
             _check_topk_args(N, k, "SparseGraphGenerator")
         else:
             _check_pattern(pattern, N, "SparseGraphGenerator")
@@ -365,11 +409,18 @@ class SparseGraphGenerator(nn.Module):
             where = "" if pattern is None else f", the pattern ({pattern.device})"
             raise RuntimeError(f"SparseGraphGenerator: X_seq ({X_seq.device}){where} and the parameters ({Wu.device}) "
                                f"must share a device")
-        if partitioned and pattern.reduce_per_cell and pattern.world > 1:
-            Wu, Wv = mgp.reduce_grad(Wu, pattern.group), mgp.reduce_grad(Wv, pattern.group)
+        rows_split = pattern if partitioned else partition
+        if rows_split is not None and rows_split.reduce_per_cell and rows_split.world > 1:
+            Wu, Wv = mgp.reduce_grad(Wu, rows_split.group), mgp.reduce_grad(Wv, rows_split.group)
         Xn = X_seq.permute(2, 0, 1, 3).reshape(N, B * T, C)       # node-major copy of the small input
         U = torch.tanh(self.alpha * (Xn @ Wu)).reshape(N, -1)      # [N, B*T*hg], contiguous
         V = torch.tanh(self.alpha * (Xn @ Wv)).reshape(N, -1)
+        if partition is not None:
+            W = U.shape[1]
+            UV = partition.gather_rows(torch.cat([U.detach(), V.detach()], 1))   # [N, 2W]: every node's U, V
+            sel = pair_topk(UV[:, :W], UV[:, W:], k, rows=(partition.start, partition.nloc))
+            pattern = partition.support(partition.gather_rows(sel))
+            partitioned = True
         if partitioned:
             return pattern.with_values(pair_softmax_partitioned(U, V, pattern))
         if k is not None:

@@ -24,6 +24,13 @@ against the learnable partitioned step on fixed values, alternating as `--learne
 forward + backward per rank.  At world > 1, `parity_ok` covers P, the Wu / Wv / X_seq gradients and the cell outputs
 against the unpartitioned generator + cell on the same GPU, and over NCCL the replicated form (X_seq all-gathered, the
 whole generator on every rank, its [nnz] gradient all-reduced) is timed as well.
+`--train --generated --k 16`: the same step with the pattern selected from the scores on the row partition
+(`SparseGraphGenerator(...)(X_seq, k=16, partition=RowPartition(...))`: U, V all-gathered, each rank selecting its own
+rows, the selection all-gathered and partitioned on the device) against `--generated` on the kNN pattern, alternating;
+also, per rank and max over ranks, the phases of the selection (all-gather of U, V; the row-block selection; all-gather
+of the [nloc, k] selection; the plan build) and the halo rows of both plans of the selected pattern.  `parity_ok`
+(every world size, world 1 included) covers the selection, P, the cell outputs and every gradient against the
+unpartitioned generator (`topk_pattern` on the whole U, V, i.e. `gen(X_seq, k=16)`) + cell on the same GPU.
 `--gloo`: every rank on cuda:0, exchanging over gloo -- a full-size parity check of the partitioned path on a
 machine with one GPU; its times measure ranks sharing one GPU, not scaling."""
 import json
@@ -39,7 +46,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 import stc_gnn_b200 as S  # noqa: E402
 from stc_gnn_b200 import _lib  # noqa: E402
-from stc_gnn_b200.halo import PartitionedSupport, partitioned_cell_forward  # noqa: E402
+from stc_gnn_b200.halo import PartitionedSupport, RowPartition, partitioned_cell_forward  # noqa: E402
 from stc_gnn_b200.synth import knn_csr  # noqa: E402
 
 
@@ -306,10 +313,120 @@ def generated_main(B, world, rank, dev):
         print(json.dumps(rec), flush=True)
 
 
+def selected_main(B, world, rank, dev, k):
+    """--train --generated --k K: the step on the selected pattern vs the step on the kNN pattern (module docstring)."""
+    N, C, F, Ks, Kc, T, hg, ROUNDS, iters = 65536, 8, 64, 4, 2, 12, 16, 5, 5
+    rp, ci, va = knn_csr(N, 8)
+    torch.manual_seed(0)
+    cell = S.STC_Cell(N, C, Ks, Kc, F, F).to(dev)
+    gen = S.SparseGraphGenerator(C, hg).to(dev)
+    params, gparams = list(cell.parameters()), list(gen.parameters())
+    Gc = (torch.rand(C, C, generator=torch.Generator().manual_seed(1)) / C).to(dev).requires_grad_(True)
+    g = torch.Generator().manual_seed(100)
+    Xg = torch.randn(B, N, C, F, generator=g)
+    Hg = torch.randn(B, N, C, F, generator=g) * 0.5
+    dHg = torch.randn(B, N, C, F, generator=g)
+    Xsg = torch.randn(B, T, N, C, generator=g)
+    knn = PartitionedSupport(rp, ci, va, N, rank, world)
+    knn.reduce_per_cell = False
+    part = RowPartition(N, rank, world)
+    part.reduce_per_cell = False             # every gradient goes through one bucket per step
+    lo, n = part.start, part.nloc
+    blk = lambda t, d=1: t.narrow(d, lo, n).contiguous().to(dev)
+    X, H, dHn = blk(Xg).requires_grad_(True), blk(Hg).requires_grad_(True), blk(dHg)
+    Xs = blk(Xsg, 2).requires_grad_(True)
+    bucket = S.dp.GradBucket(params + [Gc] + gparams)
+    cell_args = lambda: (Gc, X, H, cell.gates.W, cell.gates.b, cell.candi.W, cell.candi.b, Ks, Kc)
+    singles = [dist.new_group([r]) for r in range(world)] if world > 1 else [None]
+
+    def clear():
+        for t in (X, H, Xs, Gc, *params, *gparams):
+            t.grad = None
+
+    def step(selected):
+        clear()
+        sup = gen(Xs, k=k, partition=part) if selected else gen(Xs, knn)
+        out = partitioned_cell_forward(sup, *cell_args(), reduce_params=False)
+        out.backward(dHn)
+        bucket.allreduce()
+        return out, sup
+
+    # the selection's phases on their own
+    with torch.no_grad():
+        Xn = Xs.permute(2, 0, 1, 3).reshape(n, B * T, C)
+        UVl = torch.cat([torch.tanh(gen.alpha * (Xn @ gen.params_S[w])).reshape(n, -1) for w in ("Wu", "Wv")], 1)
+    W = UVl.shape[1] // 2
+    UV = part.gather_rows(UVl)
+    Ug, Vg = UV[:, :W].contiguous(), UV[:, W:].contiguous()
+    sel = S.pair_topk(Ug, Vg, k, rows=(lo, n))
+    cols = part.gather_rows(sel)
+    phases = _alternate({"allgather_uv": lambda: part.gather_rows(UVl),
+                         "select_rows": lambda: S.pair_topk(Ug, Vg, k, rows=(lo, n)),
+                         "allgather_selection": lambda: part.gather_rows(sel),
+                         "plan_build": lambda: part.support(cols)}, world, 3, iters)
+
+    out_p, sup = step(True)
+    got = [sup._col.view(N, k).to(torch.int32), sup.vals.detach().clone(), out_p.detach().clone(), X.grad.clone(),
+           H.grad.clone(), Xs.grad.clone()] + [t.grad.clone() for t in gparams + params + [Gc]]
+    halo = {"fwd_halo_rows": sup.fwd.nhalo, "bwd_halo_rows": sup.bwd.nhalo,
+            "halo_fraction_of_remote_nodes": sup.fwd.nhalo / max(1, N - n), "knn_fwd_halo_rows": knn.fwd.nhalo}
+    if world == 1:   # what rank 0 of a wider split of the same selection would exchange per hop
+        sel_cols = sup._col.view(N, k)
+        halo["rank0_halo_rows_at_world"] = {
+            w: {"selected": RowPartition(N, 0, w).support(sel_cols).fwd.nhalo,
+                "remote_nodes": N - RowPartition(N, 0, w).nloc,
+                "knn": PartitionedSupport(rp, ci, va, N, 0, w).fwd.nhalo} for w in (2, 4, 8)}
+    del out_p, sup
+    clear()
+    Xf, Hf, Xsf = (t.to(dev).requires_grad_(True) for t in (Xg, Hg, Xsg))
+    with torch.no_grad():
+        Xn = Xsf.permute(2, 0, 1, 3).reshape(N, B * T, C)
+        Uf, Vf = (torch.tanh(gen.alpha * (Xn @ gen.params_S[w])).reshape(N, -1) for w in ("Wu", "Wv"))
+    pattern = S.topk_pattern(Uf, Vf, k)     # gen(Xsf, k=k) without the batch-DP collectives of a process group
+    gsup = gen(Xsf, pattern, group=singles[rank])
+    out_f = cell(Gs=gsup, Gc=Gc, Xt=Xf, Ht_1=Hf)
+    out_f.backward(dHg.to(dev))
+    want = [pattern.col.view(N, k), gsup.vals.detach(), out_f.detach()[:, lo:lo + n], Xf.grad[:, lo:lo + n],
+            Hf.grad[:, lo:lo + n], Xsf.grad[:, :, lo:lo + n]] + [t.grad.clone() for t in gparams + params + [Gc]]
+    names = ["selection", "P", "H'", "dXt", "dH", "dX_seq", "dWu", "dWv", "dWg", "dbg", "dWc", "dbc", "dGc"]
+    floors = {"P": 1e-5, "H'": 1e-5, "dXt": 1e-5, "dH": 1e-5, "dX_seq": 1e-5, "dWu": 5e-5, "dWv": 5e-5}
+    worst, nbad = {}, 0
+    rows_differing = int((got[0] != want[0]).any(1).sum())
+    nbad += rows_differing
+    for nm, a_, b_ in zip(names[1:], got[1:], want[1:]):
+        nb, worst[nm] = violations(a_, b_, floors.get(nm, 3e-5))
+        nbad += nb
+    if world > 1:
+        flag = torch.tensor([float(nbad)], device=dev)
+        dist.all_reduce(flag)
+        nbad = float(flag.item())
+    parity = {"parity_ok": nbad == 0, "selection_rows_differing_rank0": rows_differing,
+              "worst_err_over_mean_ref_rank0": worst}
+    del Xf, Hf, Xsf, gsup, out_f, want, got, pattern
+    clear()
+    torch.cuda.empty_cache()
+
+    samples = _alternate({"selected": lambda: step(True)[0], "knn_generated": lambda: step(False)[0]}, world, ROUNDS,
+                         iters)
+    if rank == 0:
+        summ = lambda v: {"median": statistics.median(v), "min": min(v), "max": max(v)}
+        backend = dist.get_backend() if world > 1 else None
+        rec = {"kind": "config4_cell_step_partitioned_selected", "n_gpus": 1 if backend in (None, "gloo") else world,
+               "n_ranks": world, "backend": backend, **_device_record(dev), "N": N, "C": C, "F": F, "Ks": Ks,
+               "Kc": Kc, "B": B, "T": T, "hg": hg, "k": k, "local_rows": n, **halo,
+               "selection_phases_ms_max_over_ranks": {p: summ(v) for p, v in phases.items()},
+               "rounds": ROUNDS, "steps_per_round": iters}
+        rec.update({f"{nm}_step_ms": summ(v) for nm, v in samples.items()})
+        rec["ratio_selected_over_knn_generated"] = statistics.median(samples["selected"]) / \
+            statistics.median(samples["knn_generated"])
+        rec.update(parity)
+        print(json.dumps(rec), flush=True)
+
+
 def main():
     train = "--train" in sys.argv
     per_cell = "--reduce-per-cell" in sys.argv
-    pos = [a for a in sys.argv[1:] if not a.startswith("--")]
+    pos = [a for i, a in enumerate(sys.argv[1:], 1) if not a.startswith("--") and sys.argv[i - 1] != "--k"]
     B = int(pos[0]) if pos else 2
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
@@ -326,7 +443,10 @@ def main():
     if "--generated" in sys.argv:
         if not train:
             raise SystemExit("--generated measures the training step: pass --train as well")
-        generated_main(B, world, rank, dev)
+        if "--k" in sys.argv:
+            selected_main(B, world, rank, dev, int(sys.argv[sys.argv.index("--k") + 1]))
+        else:
+            generated_main(B, world, rank, dev)
         if world > 1:
             dist.barrier()
             dist.destroy_process_group()

@@ -4,7 +4,7 @@
   config3  grid N = 4096, B = 8, T = 12, C = 16
   config4  kNN N = 65,536, B = 2, T = 12, C = 8
 
-  python tools/bench_topk_graph.py [config3] [config4] > out.jsonl
+  python tools/bench_topk_graph.py [config3] [config4] [rows] > out.jsonl
 
 For hg in {16, 64} (width W = B*T*hg) and k = 16 each line reports:
   - the selection kernel (CUDA events around many calls after a warm-up): ms, useful TFLOP/s from 2 N^2 (2W) (the 3xTF32
@@ -14,6 +14,9 @@ For hg in {16, 64} (width W = B*T*hg) and k = 16 each line reports:
     default, the precision this project holds to) and with TF32 matmuls, each with its peak memory; the TF32 form's
     count of rows whose selected set differs from the kernel's, and the fp32 form's;
   - the generator's forward + backward with k = 16 against the same on the fixed pattern (grid / kNN).
+`rows` (config 4, W = 384, k = 16): the selection of one rank's row block, n_rows = N / world for world 2, 4, 8
+(`pair_topk(..., rows=)`, stc_pair_topk_rows), timed alternating with the full selection, with the segment count the
+kernel chose for the block and whether the block is bitwise those rows of the full selection.
 The first line names the device, its power limit and maximum SM clock.
 """
 import json
@@ -145,6 +148,26 @@ def bench(which, hg):
     emit(**out)
 
 
+def bench_rows():
+    N, W = 65536, 384
+    U, V = (torch.tanh(torch.randn(N, W, generator=torch.Generator().manual_seed(s))).to(DEV) for s in (1, 2))
+    lib = _lib.load()
+    blocks = {w: (N // w, N // w) for w in (2, 4, 8)}     # rank 1's rows of an even split
+    variants = {"full": lambda: S.pair_topk(U, V, K)}
+    variants.update({f"world{w}": (lambda b=b: S.pair_topk(U, V, K, rows=b)) for w, b in blocks.items()})
+    t = alternate(variants, 3)
+    full = S.pair_topk(U, V, K)
+    full_ms = statistics.median(t["full"])
+    for w, (r0, n) in blocks.items():
+        ws = lib.stc_pair_topk_rows_workspace_bytes(N, W, n, K)
+        ms = statistics.median(t[f"world{w}"])
+        emit(kind="pair_topk_rows", config="config4", N=N, W=W, k=K, world=w, row0=r0, n_rows=n,
+             segments=ws // (8 * n * K), row_blocks=-(-n // 128), kernel_ms=summary(t[f"world{w}"]),
+             full_selection_ms=summary(t["full"]), fraction_of_full=ms / full_ms, ideal_fraction=n / N,
+             workspace_bytes=ws, full_workspace_bytes=lib.stc_pair_topk_workspace_bytes(N, W, K),
+             bitwise_full_rows=bool(torch.equal(S.pair_topk(U, V, K, rows=(r0, n)), full[r0:r0 + n])))
+
+
 def main():
     if not torch.cuda.is_available():
         raise SystemExit("bench_topk_graph.py needs a CUDA device")
@@ -156,6 +179,9 @@ def main():
         smi = f"unavailable: {e!r}"
     emit(kind="device", name=torch.cuda.get_device_name(0), nvidia_smi=smi)
     for which in sys.argv[1:] or ["config3", "config4"]:
+        if which == "rows":
+            bench_rows()
+            continue
         if which not in CONFIGS:
             raise SystemExit(f"unknown config {which!r} (use {', '.join(CONFIGS)})")
         for hg in (16, 64):
