@@ -169,6 +169,13 @@ int stc_cell_bwd_x(const StcDims* d, const StcSupport* gs, const float* gc,
  * Gs [N][N] with A = X ([B][N][width], batch stride in elements) and Bm = dL/dY ([B][N][width] contiguous). */
 int stc_support_outer(int32_t N, int32_t B, int32_t width, const float* a, int64_t a_batch_stride, const float* b,
                       float coef, float* dGs, void* stream);
+/* stc_support_outer with a workspace for the deterministic mode's partial slots (stc_deterministic_set): ws holds at
+ * least stc_support_outer_workspace_bytes(N, B, width) bytes, 16-byte aligned (NULL when that is 0).  The size is 0
+ * while the mode is off and depends on the SM count of the current device; query it on the device that runs the
+ * product.  In deterministic mode the plain stc_support_outer returns STC_ERR_UNSUPPORTED. */
+size_t stc_support_outer_workspace_bytes(int32_t N, int32_t B, int32_t width);
+int stc_support_outer_ws(int32_t N, int32_t B, int32_t width, const float* a, int64_t a_batch_stride, const float* b,
+                         float coef, float* dGs, void* ws, size_t ws_bytes, void* stream);
 /* The same gradient for a CSR support, sampled at its edges and fused into the adjoint hop (CSR only):
  *   y = alpha * Gs x + beta * z                                    (exactly what stc_support_apply, transpose = 0, writes)
  *   dvals[e] += coef * sum_{b,j} a[b][row(e)][j] * x[b][col(e)][j] (e walks Gs's CSR: rowptr / col / vals order)
@@ -256,6 +263,10 @@ int stc_pair_topk_rows(int32_t N, int64_t width, const float* u, const float* v,
  * values are learned, the caller forms their gradient inside its adjoint hops (steps 2 and 4) with
  * stc_support_apply_edge_grad / stc_support_apply_rows_edge_grad, A = the matching forward terms of `saved`.      */
 enum { STC_SCRATCH_DYR = 0, STC_SCRATCH_DYX, STC_SCRATCH_DYH, STC_SCRATCH_REGIONS };
+/* Offset of the deterministic-mode partial slots (stc_deterministic_set): written to offsets[STC_SCRATCH_DET] when
+ * n_offsets > STC_SCRATCH_DET.  They run from there to the end of `scratch`, after every other region (with the mode
+ * off the offset equals stc_cell_bwd_scratch_bytes / 4: no slots). */
+enum { STC_SCRATCH_DET = STC_SCRATCH_REGIONS };
 int stc_cell_bwd_scratch_layout(const StcDims* d, int64_t* offsets_floats, int32_t n_offsets);
 int stc_cell_bwd_stage(const StcDims* d, int32_t stage, const float* gc,
                        const float* xt, int64_t xt_batch_stride, const float* h_prev,
@@ -298,6 +309,17 @@ int stc_tf32x3_gemm(const float* a, const float* b, float* d, int32_t M, int32_t
  * before the call returns; by default only for problems too small to fill the device.  mode: -1 = by problem size
  * (default; the STC_CONCURRENCY environment variable sets the initial value), 0 = always one stream, 1 = always fork. */
 int stc_concurrency_set(int32_t mode);
+
+/* Deterministic mode (process-wide; off by default).  on = 1: every gradient that several CTAs add to -- dW and the
+ * bias gradients, dGc, a dense dGs, a CSR support's edge-value gradient -- is summed in a fixed order instead of with
+ * float atomics: per-CTA partials go to slots of `scratch` (stc_cell_bwd_scratch_bytes grows while the mode is on) and one
+ * reduction kernel per gradient adds them in slot order; the CSR edge gradient has exactly one writer per edge.  Then
+ * the same call with the same inputs, configuration and device gives bitwise the same outputs and gradients.
+ * Not promised: equality with the default mode, across stc_concurrency_set modes, or across devices with different SM
+ * counts.  Every backward path has a fixed-order form: the tensor-core, wide-state and general (FFMA) convolution
+ * kernels, the dense and CSR support gradients.  The forward, `saved`
+ * and stc_cell_saved_bytes do not depend on the mode.  on other than 0 / 1: STC_ERR_BAD_ARG. */
+int stc_deterministic_set(int32_t on);
 
 /* Number of kernel launches the last stc_cell_fwd / stc_cell_bwd on this thread issued
  * (bench.py reports gpu_launches from these). */

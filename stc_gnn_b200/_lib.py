@@ -26,6 +26,7 @@ EXPORTED = (
     "stc_support_apply_rows_edge_grad", "stc_pair_scores_csr", "stc_edge_softmax_fwd", "stc_edge_softmax_bwd",
     "stc_pair_scores_csr_rows", "stc_pair_topk_workspace_bytes", "stc_pair_topk",
     "stc_pair_topk_rows_workspace_bytes", "stc_pair_topk_rows",
+    "stc_deterministic_set", "stc_support_outer_workspace_bytes", "stc_support_outer_ws",
 )
 STAGE_GATES, STAGE_CANDI = 0, 1
 SAVED_REGIONS = ("u", "r", "c", "Yr", "Yx", "Yh", "Q", "Pg", "Pc")
@@ -69,6 +70,12 @@ def load(build_if_missing: bool = True):
     lib.stc_cell_fwd_x.argtypes = lib.stc_cell_fwd.argtypes[:-1] + [c_void_p, c_void_p, c_void_p]
     lib.stc_support_outer.restype = c_int
     lib.stc_support_outer.argtypes = [c_int32, c_int32, c_int32, c_void_p, c_int64, c_void_p, c_float, c_void_p, c_void_p]
+    lib.stc_support_outer_workspace_bytes.restype = c_size_t
+    lib.stc_support_outer_workspace_bytes.argtypes = [c_int32, c_int32, c_int32]
+    lib.stc_support_outer_ws.restype = c_int
+    lib.stc_support_outer_ws.argtypes = lib.stc_support_outer.argtypes[:-1] + [c_void_p, c_size_t, c_void_p]
+    lib.stc_deterministic_set.restype = c_int
+    lib.stc_deterministic_set.argtypes = [c_int32]
     lib.stc_support_apply_edge_grad.restype = c_int
     lib.stc_support_apply_edge_grad.argtypes = [POINTER(StcSupport), c_int32, c_int32, c_int32, c_void_p, c_int64,
                                                 c_void_p, c_int64, c_void_p, c_float, c_float, c_void_p, c_int64,
@@ -179,6 +186,22 @@ def note_launches() -> None:
 def set_concurrency(mode: int) -> None:
     """-1: fork independent kernels of a cell call onto side streams only for small problems (default); 0: never; 1: always."""
     check(load().stc_concurrency_set(int(mode)), "stc_concurrency_set")
+
+
+_DET_SENT = 0   # the library starts with the mode off
+
+
+def sync_deterministic() -> bool:
+    """Give the library's deterministic mode (fixed-order gradient reductions, stc_deterministic_set) the value of
+    torch.are_deterministic_algorithms_enabled(); the ctypes call is made only when that value changed since the last
+    call.  Returns the mode."""
+    global _DET_SENT
+    import torch
+    on = 1 if torch.are_deterministic_algorithms_enabled() else 0
+    if on != _DET_SENT:
+        check(load().stc_deterministic_set(on), "stc_deterministic_set")
+        _DET_SENT = on
+    return bool(on)
 
 
 def timing_enable(on: bool) -> None:

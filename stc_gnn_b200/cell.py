@@ -58,8 +58,10 @@ _SIZES = {}
 
 
 def _buffer_floats(lib, dims: _lib.StcDims, key):
-    """(saved, scratch) buffer sizes in floats of a cell call, cached per shape: at the reference's batch size a training
-    step is bound by host-side call overhead (48 cell calls), so the two size queries are not repeated."""
+    """(saved, scratch) buffer sizes in floats of a cell call, cached per shape and deterministic mode (the scratch holds
+    the partial slots while it is on): at the reference's batch size a training step is bound by host-side call
+    overhead (48 cell calls), so the two size queries are not repeated."""
+    key = key + (_lib.sync_deterministic(),)
     hit = _SIZES.get(key)
     if hit is None:
         if len(_SIZES) > 256:

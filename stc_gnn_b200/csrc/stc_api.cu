@@ -5,6 +5,7 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include <algorithm>
 #include <atomic>
 #include <mutex>
 #include <vector>
@@ -206,6 +207,11 @@ struct Lanes {
   }
 };
 
+static std::atomic<int> g_det{0};
+bool det_mode() { return g_det.load(std::memory_order_relaxed) != 0; }
+// every dW / dx kernel with a fixed-order form runs at most two CTAs per SM
+int det_conv_slots() { return 2 * device_sm_count(); }
+
 WsLayout make_layout(const StcDims& d) {
   WsLayout w;
   const size_t A = 64;  // 256-byte alignment of every region
@@ -247,6 +253,30 @@ WsLayout make_layout(const StcDims& d) {
     const size_t ig = w.Wimg_c > w.Wimg_g ? conv_big_dx_img_floats(d.C, d.Din, d.h, d.Ks, d.Kc, 2 * d.h) : 0;
     const size_t ic = w.saved_total > w.Wimg_c ? conv_big_dx_img_floats(d.C, d.Din, d.h, d.Ks, d.Kc, d.h) : 0;
     w.Wimg_dx = take(ig > ic ? ig : ic);
+  }
+  {  // deterministic mode: partial slots of the cross-CTA reductions (after every region of the default layout)
+    const bool det = det_mode();
+    const size_t P = (size_t)d.Ks * d.Kc, L = (size_t)d.Din + d.h, S = det ? (size_t)det_conv_slots() : 0;
+    size_t dw = S * P * L * 2 * d.h, dx = S * (2 * (size_t)d.h + (size_t)(d.Kc - 1) * d.C * d.C);
+    if (det) {   // the general (FFMA) kernels: one slot per CTA (dx) / per row chunk and row group (dW)
+      ConvArgs t;
+      memset(&t, 0, sizeof(t));
+      t.B = d.B; t.N = d.N; t.C = d.C; t.Din = d.Din; t.h = d.h; t.Ks = d.Ks; t.Kc = d.Kc;
+      for (int hout : {2 * d.h, d.h}) {
+        t.Hout = hout;
+        dw = std::max(dw, conv_dw_general_det_floats(t));
+        dx = std::max(dx, conv_dx_general_det_floats(t));
+      }
+    }
+    w.det_dw = take(dw);
+    w.det_dx = take(dx);
+    long long g = 0;
+    if (det)
+      for (int width : {d.C * d.Din, d.C * d.h}) {
+        const long long f = support_outer_det_floats(d.N, d.B, width);
+        if (f > g) g = f;
+      }
+    w.det_dgs = take((size_t)g);
   }
   w.scratch_total = o;
   return w;
@@ -326,7 +356,8 @@ const char* stc_kernel_kind_name(int32_t kind) {
   static const char* names[KK_COUNT] = {"support_dense", "support_csr", "support_outer", "cheby_small",
                                         "conv_fwd",      "conv_bwd_dx", "conv_bwd_dw", "tc_conv_fwd", "tc_conv_bwd_dx", "tc_conv_bwd_dw",
                                         "tc_support", "tc_gemm_test", "tc_outer", "tc_support_big", "support_csr_grad",
-                                        "pair_scores_csr", "edge_softmax", "pair_topk", "tc_support_adj", "pair_topk_rows"};
+                                        "pair_scores_csr", "edge_softmax", "pair_topk", "tc_support_adj", "pair_topk_rows",
+                                        "det_reduce"};
   return (kind >= 0 && kind < KK_COUNT) ? names[kind] : "?";
 }
 
@@ -343,6 +374,15 @@ int stc_concurrency_set(int32_t mode) {
     return STC_ERR_BAD_ARG;
   }
   g_concurrency.store(mode, std::memory_order_relaxed);
+  return STC_OK;
+}
+
+int stc_deterministic_set(int32_t on) {
+  if (on != 0 && on != 1) {
+    set_error("stc_deterministic_set: %d (use 0 = atomics, 1 = fixed-order reductions)", on);
+    return STC_ERR_BAD_ARG;
+  }
+  g_det.store(on, std::memory_order_relaxed);
   return STC_OK;
 }
 
@@ -626,7 +666,8 @@ int stc_cell_fwd_stage(const StcDims* dp, int32_t stage, const float* gc, const 
 // adjoint hop already gathers every ybar[k][b,m,:] it needs, so the hop computes it (launch_support_csr_edge_grad).
 static int adjoint_chain(const StcDims& d, const StcSupport& gs, int width, const float* y0, int64_t y0_bs,
                          const float* yk /* terms k>=1, contiguous */, float* ybar0, float* ybark /* k>=1 */,
-                         float* dGs, cudaStream_t st, Lanes* lanes = nullptr, int outer_lane = 1) {
+                         float* dGs, cudaStream_t st, Lanes* lanes = nullptr, int outer_lane = 1,
+                         float* det_dgs = nullptr) {
   const size_t Rw = (size_t)d.B * d.N * width;
   const int64_t nbs = (int64_t)d.N * width;
   for (int k = d.Ks - 1; k >= 1; --k) {
@@ -660,7 +701,7 @@ static int adjoint_chain(const StcDims& d, const StcSupport& gs, int width, cons
         STC_TRY(lanes->fork_from(st, outer_lane));
         so = lanes->stream(outer_lane);
       }
-      STC_TRY(launch_support_outer(d.N, d.B, width, yprev, yprev_bs, yb_k, coef, dGs, so));
+      STC_TRY(launch_support_outer(d.N, d.B, width, yprev, yprev_bs, yb_k, coef, dGs, so, det_dgs));
     }
     STC_TRY(launch_support_apply(gs, d.N, d.B, width, false, yb_k, nbs, yb_km1, nbs, yb_km1, coef, 1.f, axpy, -1.f,
                                  st));
@@ -739,7 +780,10 @@ static int bwd_begin(const BwdCtx& b, float* dWg, float* dbg, float* dWc, float*
 }
 
 // dW = Y_k^T [Ds | Dm_c] needs only what dx just wrote (dpre) and forward's saved terms: side stream 0 when lanes are active
-static int launch_dw_beside(const BwdCtx& b, const ConvArgs& a) {
+// (deterministic mode: dx and dW each reduce through their own slot region, so the two may run side by side)
+static int launch_dw_beside(const BwdCtx& b, const ConvArgs& dx_args) {
+  ConvArgs a = dx_args;
+  if (det_mode()) a.det_ws = b.sc + b.w.det_dw;
   if (b.lanes && b.lanes->active()) {
     STC_TRY(b.lanes->fork(0));
     return launch_conv_bwd_dw(a, b.lanes->stream(0));
@@ -772,6 +816,7 @@ static int bwd_candi(const BwdCtx& b, const float* Wc, float* dWc, float* dbc) {
   a.dW = dWc;
   a.Psave = b.sv + w.Pc;
   a.Wimg = (w.saved_total > w.Wimg_c && w.scratch_total > w.Wimg_dx) ? b.sc + w.Wimg_dx : nullptr;   // wide forward ran
+  if (det_mode()) a.det_ws = b.sc + w.det_dx;
   STC_TRY(launch_conv_bwd_dx(a, b.st));
   return launch_dw_beside(b, a);
 }
@@ -802,6 +847,7 @@ static int bwd_gates(const BwdCtx& b, const float* Wg, float* dWg, float* dbg) {
   a.dW = dWg;
   a.Psave = b.sv + w.Pg;
   a.Wimg = (w.Wimg_c > w.Wimg_g && w.scratch_total > w.Wimg_dx) ? b.sc + w.Wimg_dx : nullptr;   // wide forward ran
+  if (det_mode()) a.det_ws = b.sc + w.det_dx;
   if (b.lanes) STC_TRY(b.lanes->join(0));   // the candidate's dW reads dpre, which this dx overwrites
   STC_TRY(launch_conv_bwd_dx(a, b.st));
   STC_TRY(launch_dw_beside(b, a));
@@ -866,19 +912,24 @@ static int cell_bwd_impl(const StcDims* dp, const StcSupport* gs, const float* g
   //   side 2            hops of dXt
   STC_TRY(bwd_candi(b, Wc, dWc, dbc));
   // d(rH) through the spatial recurrence
+  float* const det_dgs = det_mode() ? b.sc + w.det_dgs : nullptr;   // (all outer products run on one lane)
   STC_TRY(adjoint_chain(d, *gs, CH, b.sv + w.Yr, (int64_t)d.N * CH, b.sv + w.Yr + Rh, b.sc + w.dYr, b.sc + w.dYr + Rh,
-                        dGs, st, &lanes, 1));
+                        dGs, st, &lanes, 1, det_dgs));
   STC_TRY(bwd_gates(b, Wg, dWg, dbg));
   if (!hoisted) {   // (hoisted: the x-part adjoints of terms k >= 1 sit in the caller's buffer; d_xt holds term 0 only)
     cudaStream_t sx = st;
-    if (lanes.active() && d.Ks > 1) {
+    // deterministic mode, learnable CSR support: both chains add their edge gradient into the same dGs in their hops,
+    // so the Xt-side chain stays on the caller's stream, ordered after the H-side additions
+    const bool csr_grad = dGs && gs->kind == STC_SUPPORT_CSR;
+    if (lanes.active() && d.Ks > 1 && !(det_mode() && csr_grad)) {
       STC_TRY(lanes.fork(2));
       sx = lanes.stream(2);
     }
-    STC_TRY(adjoint_chain(d, *gs, CD, xt, xt_batch_stride, b.sv + w.Yx, b.dYx0(), b.sc + w.dYx, dGs, sx, &lanes, 1));
+    STC_TRY(adjoint_chain(d, *gs, CD, xt, xt_batch_stride, b.sv + w.Yx, b.dYx0(), b.sc + w.dYx, dGs, sx, &lanes, 1, det_dgs));
   }
   if (!h_given)   // (given: the h-part adjoints of terms k >= 1 sit in dyh_terms_out, or are dropped when it is NULL)
-    STC_TRY(adjoint_chain(d, *gs, CH, h_prev, (int64_t)d.N * CH, b.sv + w.Yh, d_h_prev, b.sc + w.dYh, dGs, st, &lanes, 1));
+    STC_TRY(adjoint_chain(d, *gs, CH, h_prev, (int64_t)d.N * CH, b.sv + w.Yh, d_h_prev, b.sc + w.dYh, dGs, st, &lanes, 1,
+                          det_dgs));
   return lanes.join_all();
 }
 
@@ -910,8 +961,38 @@ int stc_support_outer(int32_t N, int32_t B, int32_t width, const float* a, int64
     set_error("stc_support_outer: NULL argument");
     return STC_ERR_BAD_ARG;
   }
+  if (det_mode()) {
+    set_error("stc_support_outer: deterministic mode needs the partial-slot workspace: use stc_support_outer_ws");
+    return STC_ERR_UNSUPPORTED;
+  }
   STC_TRY(check_arch());
   return launch_support_outer(N, B, width, a, a_batch_stride, b, coef, dGs, (cudaStream_t)stream);
+}
+
+size_t stc_support_outer_workspace_bytes(int32_t N, int32_t B, int32_t width) {
+  if (N <= 0 || B < 0 || width <= 0 || !det_mode()) return 0;
+  return (size_t)support_outer_det_floats(N, B, width) * sizeof(float);
+}
+
+int stc_support_outer_ws(int32_t N, int32_t B, int32_t width, const float* a, int64_t a_batch_stride, const float* b,
+                         float coef, float* dGs, void* ws, size_t ws_bytes, void* stream) {
+  reset_launch_count();
+  if (!a || !b || !dGs) {
+    set_error("stc_support_outer_ws: NULL argument");
+    return STC_ERR_BAD_ARG;
+  }
+  const size_t need = stc_support_outer_workspace_bytes(N, B, width);
+  if (ws_bytes < need || (need > 0 && ws == nullptr)) {
+    set_error("stc_support_outer_ws: workspace of %zu bytes, %zu needed", ws ? ws_bytes : (size_t)0, need);
+    return STC_ERR_WORKSPACE;
+  }
+  if ((reinterpret_cast<uintptr_t>(ws) & 15) != 0) {
+    set_error("stc_support_outer_ws: ws must be 16-byte aligned");
+    return STC_ERR_BAD_ARG;
+  }
+  STC_TRY(check_arch());
+  return launch_support_outer(N, B, width, a, a_batch_stride, b, coef, dGs, (cudaStream_t)stream,
+                              need > 0 ? (float*)ws : nullptr);
 }
 
 int stc_support_apply_edge_grad(const StcSupport* gs, int32_t N, int32_t B, int32_t width, const float* x,
@@ -1123,6 +1204,7 @@ int stc_cell_bwd_scratch_layout(const StcDims* dp, int64_t* offsets, int32_t n_o
   const WsLayout w = make_layout(*dp);
   const size_t v[STC_SCRATCH_REGIONS] = {w.dYr, w.dYx, w.dYh};
   for (int i = 0; i < STC_SCRATCH_REGIONS; ++i) offsets[i] = (int64_t)v[i];
+  if (n_offsets > STC_SCRATCH_DET) offsets[STC_SCRATCH_DET] = (int64_t)w.det_dw;
   return STC_OK;
 }
 

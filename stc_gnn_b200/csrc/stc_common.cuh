@@ -43,7 +43,7 @@ void reset_launch_count();
 enum KernelKind {
   KK_SUPPORT_DENSE = 0, KK_SUPPORT_CSR, KK_SUPPORT_OUTER, KK_CHEBY_SMALL, KK_CONV_FWD, KK_CONV_BWD_DX,
   KK_CONV_BWD_DW, KK_TC_CONV_FWD, KK_TC_CONV_BWD_DX, KK_TC_CONV_BWD_DW, KK_TC_SUPPORT, KK_TC_GEMM_TEST, KK_TC_OUTER, KK_TC_SUPPORT_BIG,
-  KK_SUPPORT_CSR_GRAD, KK_PAIR_SCORES_CSR, KK_EDGE_SOFTMAX, KK_PAIR_TOPK, KK_TC_SUPPORT_ADJ, KK_PAIR_TOPK_ROWS, KK_COUNT
+  KK_SUPPORT_CSR_GRAD, KK_PAIR_SCORES_CSR, KK_EDGE_SOFTMAX, KK_PAIR_TOPK, KK_TC_SUPPORT_ADJ, KK_PAIR_TOPK_ROWS, KK_DET_REDUCE, KK_COUNT
 };
 struct ScopedKernelTimer {  // declare right before a launch; the destructor records the stop event
   ScopedKernelTimer(int kind, cudaStream_t st, double alg_bytes);
@@ -82,13 +82,26 @@ __device__ __forceinline__ uint32_t fast_div(uint32_t n, const FastDiv f) {
 int device_sm_count();   // cached, current device
 int check_arch();        // STC_OK when the current device is compute capability 10.x
 
+// ---- deterministic mode (stc_deterministic_set) ----------------------------------------------------
+// On: every gradient that several CTAs add to is written as per-CTA partials into slots of a workspace (plain stores),
+// then launch_det_reduce sums the slots in slot order and adds the sum once into the destination.  Off: the atomics.
+bool det_mode();
+// dst[i] += sum_{s < n_slots} slots[s * slot_stride + i]  for i < n  (s ascending; one launch, stream-ordered)
+int launch_det_reduce(float* dst, const float* slots, int n_slots, long long n, long long slot_stride, cudaStream_t st);
+// slot counts the deterministic forms of the cross-CTA reductions use (upper bounds of their grids)
+int det_conv_slots();                                       // dW and dx kernels of one convolution
+long long support_outer_det_floats(int N, int B, int width);   // slots of one dense dGs product (0: nothing to reduce)
+
 // ---- workspace layout of one cell call (offsets in floats) -------------------------------------
 struct WsLayout {
   size_t R;  // B*N*C rows
   // `saved` buffer (written by forward, read by backward)
   size_t u, r, c, Yr, Yx, Yh, Q, Pg, Pc, Wimg_g, Wimg_c, saved_total;
   // backward `scratch` buffer
-  size_t dpre, dYx0, dYx, dYh, dYr, dQ, Wimg_dx, scratch_total;
+  size_t dpre, dYx0, dYx, dYh, dYr, dQ, Wimg_dx;
+  // deterministic mode only (empty otherwise): per-CTA partial slots of dW, of dbias / dQ, and of a dense dGs product
+  size_t det_dw, det_dx, det_dgs;
+  size_t scratch_total;
 };
 WsLayout make_layout(const StcDims& d);
 
@@ -110,7 +123,8 @@ int try_launch_support_tc_big(const float* G, int N, int B, int width, bool tran
                               const float* z, int64_t z_bs, float* y, float alpha, float beta, cudaStream_t st,
                               bool* handled);
 int try_launch_outer_tc(int N, int B, int width, const float* a, int64_t a_bs, const float* bmat, float coef, float* dG,
-                        cudaStream_t st, bool* handled);
+                        cudaStream_t st, bool* handled, float* det_ws = nullptr);
+int outer_tc_det_slots(int N, int B, int width);   // slots tc_outer uses in deterministic mode (0: it would not run)
 // one adjoint step of a dense support with N <= 112 in one kernel (rows of ybar are N * width floats apart):
 //   axpy_out -= x (when not NULL, its own pass first);  ybar += coef * Gs x;  dG += coef * a (x) x
 int try_launch_support_adj_tc(const float* G, int N, int B, int width, const float* x, int64_t x_bs, float* ybar,
@@ -127,8 +141,9 @@ int launch_support_csr_edge_grad(const StcSupport& gs, int N, int B, int width, 
                                  float axpy_coef, const float* a, int64_t a_bs, float coef, float* dvals,
                                  cudaStream_t st, const int32_t* row_list = nullptr, int n_list = 0);
 
+// det_ws: the slots of the deterministic form (support_outer_det_floats floats; required in deterministic mode)
 int launch_support_outer(int N, int B, int width, const float* a, int64_t a_bs, const float* bmat, float coef,
-                         float* dG, cudaStream_t st);
+                         float* dG, cudaStream_t st, float* det_ws = nullptr);
 
 // graph generator on a fixed CSR pattern (stc_pair_graph.cu): scores S[e = (n,m)] = <U_n,V_m> - <V_n,U_m> and the
 // softmax of relu(S) over each row's stored edges (bwd: dS from S, P, dP into `out`)
@@ -190,6 +205,9 @@ struct ConvArgs {
   const float* dYh_add;   // [Ks-1][R][h]
   float* dQ;          // [Kc][C][C] atomically accumulated, or null
   float* dW;           // atomically accumulated
+  // deterministic mode: per-CTA partial slots (det_conv_slots() slots; dW kernels: Ks*Kc*L*Hout floats each, dx
+  // kernels: Hout + (Kc-1)*C*C); null in the default mode
+  float* det_ws;
   // tuning switches (STC_OPT environment bit mask, default all on) and the optional phase trace (stc_debug_trace_set)
   int opt;
   long long* trace;    // [trace_tiles][TRACE_SLOTS] clock64 stamps of CTA 0's first tiles, or null
@@ -215,5 +233,8 @@ bool conv_tc_eligible(const ConvArgs& a);  // shape-only test shared by forward 
 bool conv_tc_dw_shape_ok(const ConvArgs& a);  // additionally: the tensor-core dW kernel tiles this shape
 int launch_conv_bwd_dx(const ConvArgs& a, cudaStream_t st);
 int launch_conv_bwd_dw(const ConvArgs& a, cudaStream_t st);
+// floats of the deterministic-mode slots of the general (FFMA) dx / dW kernels at this shape (0 if they do not tile it)
+size_t conv_dx_general_det_floats(const ConvArgs& a);
+size_t conv_dw_general_det_floats(const ConvArgs& a);
 
 }  // namespace stc

@@ -187,155 +187,16 @@ int launch_conv_fwd(const ConvArgs& a, cudaStream_t st) {
 // =================================================================================================
 // backward, part 1: pre-activation gradient, bias gradient, feature adjoints dY_k, categorical dQ
 // =================================================================================================
-template <int NI>
-__global__ void __launch_bounds__(CV_THREADS)
-conv_bwd_dx_kernel(const ConvArgs a, const ConvTile t, const int DP) {
-  extern __shared__ __align__(16) float smem[];
-  const int C = a.C, L = t.L, LP = t.LP, LP4 = t.LP4, Hout = a.Hout, h = a.h, Din = a.Din;
-  const bool mixed = a.Kc > 1;
-  const bool want_dQ = mixed && a.dQ != nullptr;
-  float* Ds = smem;                                   // [rowsP][DP]      pre-activation gradient
-  float* WsT = Ds + (size_t)t.rowsP * DP;             // [Hout][LP4]      W_{k,c}^T
-  float* DY = WsT + (size_t)Hout * LP4;               // [rowsP][LP]      adjoint of spatial term k
-  float* DF = DY + (size_t)t.rowsP * LP;              // [rowsP][LP]      dF_{k,c}, c > 0
-  float* Fin = DF + (mixed ? (size_t)t.rowsP * LP : 0);  // [rowsP][LP]   Y_k (only for dQ)
-  float* Qs = Fin + (want_dQ ? (size_t)t.rowsP * LP : 0);
-
-  const long long total_nodes = (long long)a.B * a.N;
-  const long long g0 = (long long)blockIdx.x * t.npt;
-  const int nodes_valid = (int)min((long long)t.npt, total_nodes - g0);
-  const int rows_valid = nodes_valid * C;
-  const long long row0 = g0 * C;
-  const long long R = total_nodes * C;
-  const FeatSrc fs = feat_src(a);
-  const int RG = t.rowsP / 4, CGL = LP4 / 4;
-
-  for (int i = threadIdx.x; i < (a.Kc - 1) * C * C; i += blockDim.x) Qs[i] = a.Q[C * C + i];
-
-  // ---- step 1: elementwise GRU adjoint -> Ds, dpre (global), direct dH terms ----
-  for (int idx = threadIdx.x; idx < t.rowsP * h; idx += blockDim.x) {
-    const int row = idx / h, j = idx - row * h;
-    const long long o = (row0 + row) * h + j;
-    if (row < rows_valid) {
-      const float dhn = a.dHn[o], uu = a.u[o], cc = a.c[o];
-      if (a.phase == 1) {
-        float g = dhn * uu * (1.f - cc * cc);
-        if (a.act == STC_ACT_RELU && !(cc > 0.f)) g = 0.f;
-        Ds[row * DP + j] = g;
-        a.dpre[(row0 + row) * a.dpre_ld + j] = g;
-      } else {
-        const float hp = a.Hprev[o], rr = a.r[o], drh = a.drH[o];
-        float gu = dhn * (cc - hp) * uu * (1.f - uu);
-        float gr = drh * hp * rr * (1.f - rr);
-        if (a.act == STC_ACT_RELU) {
-          if (!(uu > 0.5f)) gu = 0.f;
-          if (!(rr > 0.5f)) gr = 0.f;
-        }
-        Ds[row * DP + j] = gu;
-        Ds[row * DP + h + j] = gr;
-        a.dpre[(row0 + row) * a.dpre_ld + j] = gu;
-        a.dpre[(row0 + row) * a.dpre_ld + h + j] = gr;
-        a.dYh0[o] = dhn * (1.f - uu) + drh * rr;   // direct terms of dH; the conv adjoint is added below
-      }
-    } else {
-      Ds[row * DP + j] = 0.f;
-      if (a.phase == 0) Ds[row * DP + h + j] = 0.f;
-    }
-  }
-  __syncthreads();
-  if (a.dbias) {
-    for (int j = threadIdx.x; j < Hout; j += blockDim.x) {
-      float s = 0.f;
-      for (int row = 0; row < rows_valid; ++row) s += Ds[row * DP + j];
-      atomicAdd(&a.dbias[j], s);
-    }
-  }
-
-  // ---- step 2: per spatial term k, dY_k = sum_c unmix_c( Ds W_{k,c}^T ) ----
-  for (int k = 0; k < a.Ks; ++k) {
-    __syncthreads();
-    for (int idx = threadIdx.x; idx < t.rowsP * LP; idx += blockDim.x) DY[idx] = 0.f;
-    if (want_dQ) load_feat_tile(fs, k, g0, nodes_valid, t.rowsP, Fin, LP);
-    for (int c = 0; c < a.Kc; ++c) {
-      __syncthreads();
-      const float* Wblk = a.W + (size_t)(k * a.Kc + c) * L * Hout;
-      for (int idx = threadIdx.x; idx < Hout * LP4; idx += blockDim.x) {
-        int j = idx / LP4, l = idx - j * LP4;
-        WsT[idx] = (l < L) ? Wblk[l * Hout + j] : 0.f;
-      }
-      __syncthreads();
-      float acc[NI][4][4];
-#pragma unroll
-      for (int i = 0; i < NI; ++i)
-#pragma unroll
-        for (int x = 0; x < 4; ++x)
-#pragma unroll
-          for (int y = 0; y < 4; ++y) acc[i][x][y] = 0.f;
-      tile_gemm<NI>(acc, Ds, DP, WsT, LP4, Hout, RG, CGL);
-      float* dst = (c == 0) ? DY : DF;
-      const int items = RG * CGL;
-#pragma unroll
-      for (int i = 0; i < NI; ++i) {
-        const int it = threadIdx.x + i * CV_THREADS;
-        if (it >= items) break;
-        const int rg = it / CGL, lg = it - rg * CGL;
-#pragma unroll
-        for (int x = 0; x < 4; ++x)
-#pragma unroll
-          for (int y = 0; y < 4; ++y) {
-            const int l = lg * 4 + y;
-            if (l < L) {
-              float* p = dst + (rg * 4 + x) * LP + l;
-              if (c == 0) *p += acc[i][x][y]; else *p = acc[i][x][y];
-            }
-          }
-      }
-      if (c > 0) {
-        __syncthreads();
-        const float* Qc = Qs + (size_t)(c - 1) * C * C;
-        unmix_add_tile(DF, DY, Qc, rows_valid, C, L, LP);
-        if (want_dQ) {
-          // dQ_c[c'][d] += sum_{node,l} Y_k[(node,c')][l] * dF[(node,d)][l]
-          for (int pr = threadIdx.x; pr < C * C; pr += blockDim.x) {
-            const int cp = pr / C, d = pr - cp * C;
-            float s = 0.f;
-            for (int node = 0; node < nodes_valid; ++node) {
-              const float* y = Fin + (node * C + cp) * LP;
-              const float* f = DF + (node * C + d) * LP;
-              for (int l = 0; l < L; ++l) s = fmaf(y[l], f[l], s);
-            }
-            atomicAdd(&a.dQ[(size_t)c * C * C + pr], s);
-          }
-        }
-      }
-    }
-    __syncthreads();
-    // write DY: x-part then h-part
-    {
-      float* dx = (k == 0) ? a.dYx0 : a.dYx + (size_t)(k - 1) * R * Din;
-      if (dx) {
-        dx += row0 * Din;
-        // prior contents: the other convolution's x-part (accum_x), else a folded adjoint of the term (k >= 1)
-        const float* xprior = a.accum_x ? dx
-                              : (k >= 1 && a.dYx_add) ? a.dYx_add + (size_t)(k - 1) * R * Din + row0 * Din : nullptr;
-        for (int idx = threadIdx.x; idx < rows_valid * Din; idx += blockDim.x) {
-          int row = idx / Din, l = idx - row * Din;
-          float v = DY[row * LP + l];
-          dx[idx] = xprior ? xprior[idx] + v : v;
-        }
-      }
-      float* dh = (k == 0) ? a.dYh0 : a.dYh + (size_t)(k - 1) * R * h;
-      dh += row0 * h;
-      const float* hprior = (k == 0 && a.phase == 0) ? dh   // direct terms of dH
-                            : (k >= 1 && a.dYh_add) ? a.dYh_add + (size_t)(k - 1) * R * h + row0 * h : nullptr;
-      for (int idx = threadIdx.x; idx < rows_valid * h; idx += blockDim.x) {
-        int row = idx / h, l = idx - row * h;
-        float v = DY[row * LP + Din + l];
-        dh[idx] = hprior ? hprior[idx] + v : v;
-      }
-    }
-  }
-}
+#define STC_DX_KERNEL_NAME conv_bwd_dx_kernel
+#define STC_DX_DET 0
+#include "stc_conv_bwd_dx.cuh"
+#undef STC_DX_KERNEL_NAME
+#undef STC_DX_DET
+#define STC_DX_KERNEL_NAME gen_det_bwd_dx_kernel
+#define STC_DX_DET 1
+#include "stc_conv_bwd_dx.cuh"
+#undef STC_DX_KERNEL_NAME
+#undef STC_DX_DET
 
 static size_t conv_dx_smem(const ConvArgs& a, const ConvTile& t, int DP) {
   const bool mixed = a.Kc > 1;
@@ -345,14 +206,15 @@ static size_t conv_dx_smem(const ConvArgs& a, const ConvTile& t, int DP) {
   return f * sizeof(float);
 }
 
-int launch_conv_bwd_dx(const ConvArgs& a, cudaStream_t st) {
-  {
-    bool handled = false;
-    STC_TRY(try_launch_conv_bwd_dx_tc(a, st, &handled));
-    if (handled) return STC_OK;
-    STC_TRY(try_launch_conv_bwd_dx_big(a, st, &handled));
-    if (handled) return STC_OK;
-  }
+int det_reduce_dx(const ConvArgs& a, int grid, cudaStream_t st) {
+  const long long npairs = a.Kc > 1 ? (long long)(a.Kc - 1) * a.C * a.C : 0, stride = a.Hout + npairs;
+  if (a.dbias) STC_TRY(launch_det_reduce(a.dbias, a.det_ws, grid, a.Hout, stride, st));
+  if (a.dQ && npairs) STC_TRY(launch_det_reduce(a.dQ + (size_t)a.C * a.C, a.det_ws + a.Hout, grid, npairs, stride, st));
+  return STC_OK;
+}
+
+// tile of the general dx kernel (the largest that fits shared memory and the per-thread item budget)
+static int conv_dx_general_tile(const ConvArgs& a, ConvTile* tp, size_t* smemp, int* nip, int* DPp) {
   const int L = a.Din + a.h;
   const int CGL = ((L + 3) & ~3) / 4;
   const int HoutP = (a.Hout + 3) & ~3;
@@ -374,21 +236,58 @@ int launch_conv_bwd_dx(const ConvArgs& a, cudaStream_t st) {
     target = (t.npt / 2) * a.C;
     if (target < a.C) target = a.C;
   }
+  *tp = t; *smemp = smem; *nip = ni; *DPp = DP;
+  return STC_OK;
+}
+
+size_t conv_dx_general_det_floats(const ConvArgs& a0) {
+  ConvArgs a = a0;
+  a.dQ = reinterpret_cast<float*>(16);   // sized with the dT_c(Gc) pass (the smaller tile, the larger grid)
+  ConvTile t; size_t smem; int ni, DP;
+  if (a.B <= 0 || conv_dx_general_tile(a, &t, &smem, &ni, &DP) != STC_OK) return 0;
+  const long long grid = ceil_div((long long)a.B * a.N, t.npt);
+  return (size_t)grid * (a.Hout + (size_t)a.Ks * (a.Kc - 1) * a.C * a.C);
+}
+
+int launch_conv_bwd_dx(const ConvArgs& a, cudaStream_t st) {
+  {
+    bool handled = false;
+    STC_TRY(try_launch_conv_bwd_dx_tc(a, st, &handled));
+    if (handled) return STC_OK;
+    STC_TRY(try_launch_conv_bwd_dx_big(a, st, &handled));
+    if (handled) return STC_OK;
+  }
+  const int L = a.Din + a.h;
+  ConvTile t; size_t smem; int ni, DP;
+  STC_TRY(conv_dx_general_tile(a, &t, &smem, &ni, &DP));
   long long total_nodes = (long long)a.B * a.N;
   int grid = ceil_div(total_nodes, t.npt);
+  const bool det = a.det_ws != nullptr;
   // compulsory traffic per row: candidate reads dH',u,c (3h), gates reads dH',u,c,H,r,d(rH) (6h) and writes
   // the direct dH terms (h); both write dpre (Hout) and the Ks adjoint terms (Ks*L; the gates pass re-reads
   // the x-part it accumulates into); the spatial terms are re-read only when dGc is wanted.
   const double R = (double)total_nodes * a.C;
-  ScopedKernelTimer _t(KK_CONV_BWD_DX, st,
-                       4.0 * R * ((a.phase == 0 ? 7 * a.h + a.Ks * a.Din : 3 * a.h) + a.Hout + a.Ks * L +
-                                  ((a.dQ && a.Kc > 1) ? a.Ks * L : 0)) + 4.0 * a.Ks * a.Kc * L * a.Hout);
-  switch (ni) {
-    case 1: STC_TRY(set_smem(conv_bwd_dx_kernel<1>, smem)); conv_bwd_dx_kernel<1><<<grid, CV_THREADS, smem, st>>>(a, t, DP); break;
-    case 2: STC_TRY(set_smem(conv_bwd_dx_kernel<2>, smem)); conv_bwd_dx_kernel<2><<<grid, CV_THREADS, smem, st>>>(a, t, DP); break;
-    default: STC_TRY(set_smem(conv_bwd_dx_kernel<4>, smem)); conv_bwd_dx_kernel<4><<<grid, CV_THREADS, smem, st>>>(a, t, DP); break;
+  {
+    ScopedKernelTimer _t(KK_CONV_BWD_DX, st,
+                         4.0 * R * ((a.phase == 0 ? 7 * a.h + a.Ks * a.Din : 3 * a.h) + a.Hout + a.Ks * L +
+                                    ((a.dQ && a.Kc > 1) ? a.Ks * L : 0)) + 4.0 * a.Ks * a.Kc * L * a.Hout);
+#define STC_DX_LAUNCH(K, N) \
+  do { STC_TRY(set_smem(K<N>, smem)); K<N><<<grid, CV_THREADS, smem, st>>>(a, t, DP); } while (0)
+    switch (ni) {
+      case 1: if (det) STC_DX_LAUNCH(gen_det_bwd_dx_kernel, 1); else STC_DX_LAUNCH(conv_bwd_dx_kernel, 1); break;
+      case 2: if (det) STC_DX_LAUNCH(gen_det_bwd_dx_kernel, 2); else STC_DX_LAUNCH(conv_bwd_dx_kernel, 2); break;
+      default: if (det) STC_DX_LAUNCH(gen_det_bwd_dx_kernel, 4); else STC_DX_LAUNCH(conv_bwd_dx_kernel, 4); break;
+    }
+#undef STC_DX_LAUNCH
+    STC_LAUNCH_OK("conv_bwd_dx_kernel");
   }
-  STC_LAUNCH_OK("conv_bwd_dx_kernel");
+  if (!det) return STC_OK;
+  // slots [grid][Hout | Ks x (Kc-1) x C x C]: the bias over the CTAs, then dT_c(Gc) over the CTAs of each term k in turn
+  const long long npairs = (long long)(a.Kc - 1) * a.C * a.C, stride = a.Hout + a.Ks * npairs;
+  if (a.dbias) STC_TRY(launch_det_reduce(a.dbias, a.det_ws, grid, a.Hout, stride, st));
+  if (a.dQ && npairs)
+    for (int k = 0; k < a.Ks; ++k)
+      STC_TRY(launch_det_reduce(a.dQ + (size_t)a.C * a.C, a.det_ws + a.Hout + k * npairs, grid, npairs, stride, st));
   return STC_OK;
 }
 
@@ -399,9 +298,11 @@ int launch_conv_bwd_dx(const ConvArgs& a, cudaStream_t st) {
 // =================================================================================================
 constexpr int DW_SLAB = 64;
 
-template <int NI>
-__global__ void __launch_bounds__(CV_THREADS)
-conv_bwd_dw_kernel(const ConvArgs a, const ConvTile t, const int tiles_per_cta) {
+// DET (deterministic mode): row group g of row chunk blockIdx.x stores its partial into slot blockIdx.x * Gmax + g of
+// a.det_ws (Ks*Kc*L*Hout floats each; Gmax = the row-group count of the narrowest column slab; slot parts no group
+// writes were zeroed before the launch) instead of adding it with atomics.
+template <int NI, bool DET>
+__device__ __forceinline__ void conv_bwd_dw_body(const ConvArgs& a, const ConvTile& t, const int tiles_per_cta) {
   extern __shared__ __align__(16) float smem[];
   const int C = a.C, L = t.L, LP4 = t.LP4, Hout = a.Hout;
   const int blk = blockIdx.y, k = blk / a.Kc, c = blk - k * a.Kc;
@@ -483,6 +384,11 @@ conv_bwd_dw_kernel(const ConvArgs a, const ConvTile t, const int tiles_per_cta) 
   }
   if (active) {
     float* dWblk = a.dW + (size_t)blk * L * Hout;
+    if constexpr (DET) {
+      const int ncl = Hout - ((int)gridDim.z - 1) * DW_SLAB, ITl = LG * (((ncl + 3) & ~3) / 4);
+      const int Gmax = max(G, ITl < CV_THREADS ? CV_THREADS / ITl : 1);
+      dWblk = a.det_ws + ((size_t)blockIdx.x * Gmax + g) * a.Ks * a.Kc * L * Hout + (size_t)blk * L * Hout;
+    }
 #pragma unroll
     for (int i = 0; i < NI; ++i) {
       const int it = item0 + i * CV_THREADS;
@@ -495,21 +401,31 @@ conv_bwd_dw_kernel(const ConvArgs a, const ConvTile t, const int tiles_per_cta) 
 #pragma unroll
         for (int y = 0; y < 4; ++y) {
           const int j = cg * 4 + y;
-          if (j < ncol) atomicAdd(&dWblk[(size_t)l * Hout + col0 + j], acc[i][x][y]);
+          if (j >= ncol) continue;
+          if constexpr (DET) dWblk[(size_t)l * Hout + col0 + j] = acc[i][x][y];
+          else atomicAdd(&dWblk[(size_t)l * Hout + col0 + j], acc[i][x][y]);
         }
       }
     }
   }
 }
 
-int launch_conv_bwd_dw(const ConvArgs& a, cudaStream_t st) {
-  {
-    bool handled = false;
-    STC_TRY(try_launch_conv_bwd_dw_tc(a, st, &handled));
-    if (handled) return STC_OK;
-    STC_TRY(try_launch_conv_bwd_dw_big(a, st, &handled));
-    if (handled) return STC_OK;
-  }
+template <int NI>
+__global__ void __launch_bounds__(CV_THREADS)
+conv_bwd_dw_kernel(const ConvArgs a, const ConvTile t, const int tiles_per_cta) { conv_bwd_dw_body<NI, false>(a, t, tiles_per_cta); }
+// the deterministic-mode instantiation, under a name of its own (the convolution variant list names the default kernels)
+template <int NI>
+__global__ void __launch_bounds__(CV_THREADS)
+gen_det_bwd_dw_kernel(const ConvArgs a, const ConvTile t, const int tiles_per_cta) { conv_bwd_dw_body<NI, true>(a, t, tiles_per_cta); }
+
+// grid and tile of the general dW kernel; *slots = the deterministic form's slot count (row chunks x row groups of the
+// narrowest column slab)
+struct DwGeneralPlan {
+  ConvTile t;
+  size_t smem;
+  int ni, chunks, tiles_per_cta, slabs, slots;
+};
+static int conv_dw_general_plan(const ConvArgs& a, DwGeneralPlan* pl) {
   const int L = a.Din + a.h;
   const int LP4 = (L + 3) & ~3;
   int slabs = ceil_div(a.Hout, DW_SLAB);
@@ -539,19 +455,61 @@ int launch_conv_bwd_dw(const ConvArgs& a, cudaStream_t st) {
   long long want_chunks = (long long)device_sm_count() * 4 / (P * slabs);
   if (want_chunks < 1) want_chunks = 1;
   if (want_chunks > ntiles) want_chunks = ntiles;
-  int tiles_per_cta = ceil_div(ntiles, want_chunks);
-  int chunks = ceil_div(ntiles, tiles_per_cta);
-  dim3 grid(chunks, P, slabs);
-  // compulsory traffic per row: the Ks spatial terms once and dpre once; plus the dW block written
-  ScopedKernelTimer _t(KK_CONV_BWD_DW, st,
-                       4.0 * (double)total_nodes * a.C * (a.Ks * L + a.Hout) + 4.0 * P * L * a.Hout);
-  switch (ni) {
-    case 1: STC_TRY(set_smem(conv_bwd_dw_kernel<1>, smem)); conv_bwd_dw_kernel<1><<<grid, CV_THREADS, smem, st>>>(a, t, tiles_per_cta); break;
-    case 2: STC_TRY(set_smem(conv_bwd_dw_kernel<2>, smem)); conv_bwd_dw_kernel<2><<<grid, CV_THREADS, smem, st>>>(a, t, tiles_per_cta); break;
-    default: STC_TRY(set_smem(conv_bwd_dw_kernel<4>, smem)); conv_bwd_dw_kernel<4><<<grid, CV_THREADS, smem, st>>>(a, t, tiles_per_cta); break;
-  }
-  STC_LAUNCH_OK("conv_bwd_dw_kernel");
+  pl->t = t;
+  pl->smem = smem;
+  pl->ni = ni;
+  pl->tiles_per_cta = ceil_div(ntiles, want_chunks);
+  pl->chunks = ceil_div(ntiles, pl->tiles_per_cta);
+  pl->slabs = slabs;
+  const int ncl = a.Hout - (slabs - 1) * DW_SLAB, ITl = (LP4 / 4) * (((ncl + 3) & ~3) / 4);
+  const int ITf = (LP4 / 4) * (((ncol_max + 3) & ~3) / 4);
+  const int Gl = ITl < CV_THREADS ? CV_THREADS / ITl : 1, Gf = ITf < CV_THREADS ? CV_THREADS / ITf : 1;
+  pl->slots = pl->chunks * (Gl > Gf ? Gl : Gf);
   return STC_OK;
+}
+
+size_t conv_dw_general_det_floats(const ConvArgs& a) {
+  DwGeneralPlan pl;
+  if (a.B <= 0 || conv_dw_general_plan(a, &pl) != STC_OK) return 0;
+  return (size_t)pl.slots * a.Ks * a.Kc * (a.Din + a.h) * a.Hout;
+}
+
+int launch_conv_bwd_dw(const ConvArgs& a, cudaStream_t st) {
+  {
+    bool handled = false;
+    STC_TRY(try_launch_conv_bwd_dw_tc(a, st, &handled));
+    if (handled) return STC_OK;
+    STC_TRY(try_launch_conv_bwd_dw_big(a, st, &handled));
+    if (handled) return STC_OK;
+  }
+  const int L = a.Din + a.h;
+  DwGeneralPlan pl;
+  STC_TRY(conv_dw_general_plan(a, &pl));
+  const ConvTile& t = pl.t;
+  const size_t smem = pl.smem;
+  const int tiles_per_cta = pl.tiles_per_cta, P = a.Ks * a.Kc;
+  long long total_nodes = (long long)a.B * a.N;
+  dim3 grid(pl.chunks, P, pl.slabs);
+  const bool det = a.det_ws != nullptr;
+  const size_t slot = (size_t)P * L * a.Hout;
+  // (deterministic mode: a slot part that no row group of a narrower-than-widest slab writes must read as zero)
+  if (det) STC_CUDA_OK(cudaMemsetAsync(a.det_ws, 0, sizeof(float) * pl.slots * slot, st));
+  {
+    // compulsory traffic per row: the Ks spatial terms once and dpre once; plus the dW block written
+    ScopedKernelTimer _t(KK_CONV_BWD_DW, st,
+                         4.0 * (double)total_nodes * a.C * (a.Ks * L + a.Hout) + 4.0 * P * L * a.Hout);
+#define STC_DW_LAUNCH(K, N) \
+  do { STC_TRY(set_smem(K<N>, smem)); K<N><<<grid, CV_THREADS, smem, st>>>(a, t, tiles_per_cta); } while (0)
+    switch (pl.ni) {
+      case 1: if (det) STC_DW_LAUNCH(gen_det_bwd_dw_kernel, 1); else STC_DW_LAUNCH(conv_bwd_dw_kernel, 1); break;
+      case 2: if (det) STC_DW_LAUNCH(gen_det_bwd_dw_kernel, 2); else STC_DW_LAUNCH(conv_bwd_dw_kernel, 2); break;
+      default: if (det) STC_DW_LAUNCH(gen_det_bwd_dw_kernel, 4); else STC_DW_LAUNCH(conv_bwd_dw_kernel, 4); break;
+    }
+#undef STC_DW_LAUNCH
+    STC_LAUNCH_OK("conv_bwd_dw_kernel");
+  }
+  if (!det) return STC_OK;
+  return launch_det_reduce(a.dW, a.det_ws, pl.slots, (long long)slot, (long long)slot, st);
 }
 
 }  // namespace stc

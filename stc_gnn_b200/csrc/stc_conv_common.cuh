@@ -138,6 +138,10 @@ static inline int set_smem(K kernel, size_t smem) {
     if (tracing && trace_it < a.trace_tiles) a.trace[trace_it * TRACE_SLOTS + (slot)] = clock64();   \
   } while (0)
 
+// deterministic mode: after a dx kernel that stored its bias / dT_c(Gc) partials into `grid` slots of a.det_ws
+// ([Hout | (Kc-1)*C*C] floats each), their fixed-order sums are added into a.dbias and a.dQ[C*C..]
+int det_reduce_dx(const ConvArgs& a, int grid, cudaStream_t st);
+
 // tcgen05 path (stc_conv_tc.cu): returns STC_OK and sets *handled when it took the launch
 int try_launch_conv_fwd_tc(const ConvArgs& a, cudaStream_t st, bool* handled);
 int try_launch_conv_bwd_dx_tc(const ConvArgs& a, cudaStream_t st, bool* handled);

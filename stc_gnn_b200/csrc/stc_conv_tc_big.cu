@@ -556,8 +556,10 @@ __global__ void tc_big_dx_prep_kernel(const float* __restrict__ W, uint8_t* __re
 
 // (same role split as the forward kernel: warp 16 issues the MMAs and refills the weight ring, the 16 producer warps
 //  meet it only through mbarriers)
-__global__ void __launch_bounds__(BG_FWD_THREADS, 1)
-tc_conv_bwd_dx_big_kernel(const ConvArgs a, const BigDxPlan p, const uint8_t* __restrict__ img) {
+// DET (deterministic mode): the CTA's bias and dT_1(Gc) partials (one owner thread each) are stored into slot
+// blockIdx.x of a.det_ws ([Hout | C*C] floats) instead of being reduced with atomics.
+template <bool DET>
+__device__ __forceinline__ void tc_conv_bwd_dx_big_body(const ConvArgs& a, const BigDxPlan& p, const uint8_t* __restrict__ img) {
   extern __shared__ __align__(1024) uint8_t smem[];
   if ((smem_u32(smem) & 1023u) != 0u) __trap();
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
@@ -916,13 +918,21 @@ tc_conv_bwd_dx_big_kernel(const ConvArgs a, const BigDxPlan p, const uint8_t* __
       bg_producer_sync();    // the Ds tile is rewritten by the next tile's prologue
     }
   }
-  if (a.dbias && tid < Hout) atomicAdd(&a.dbias[tid], db_acc);
+  float* const slot = DET ? a.det_ws + (size_t)blockIdx.x * (Hout + C * C) : nullptr;
+  if (a.dbias && tid < Hout) grad_out<DET>(DET ? slot + tid : &a.dbias[tid], db_acc);
   if (want_dQ)
-    for (int i = tid; i < C * C; i += BG_THREADS) atomicAdd(&a.dQ[C * C + i], dQacc[i]);
+    for (int i = tid; i < C * C; i += BG_THREADS) grad_out<DET>(DET ? slot + Hout + i : &a.dQ[C * C + i], dQacc[i]);
   }   // producers
   __syncthreads();
   if (warp == 0) tmem_dealloc(tmem_base, 512u);
 }
+
+__global__ void __launch_bounds__(BG_FWD_THREADS, 1)
+tc_conv_bwd_dx_big_kernel(const ConvArgs a, const BigDxPlan p, const uint8_t* __restrict__ img) { tc_conv_bwd_dx_big_body<false>(a, p, img); }
+// the deterministic-mode instantiation, under a name of its own (the convolution variant list names the default
+// kernels)
+__global__ void __launch_bounds__(BG_FWD_THREADS, 1)
+tc_det_bwd_dx_big_kernel(const ConvArgs a, const BigDxPlan p, const uint8_t* __restrict__ img) { tc_conv_bwd_dx_big_body<true>(a, p, img); }
 
 static bool big_dx_shape_ok(const ConvArgs& a) {
   if (!conv_big_shape_ok(a.C, a.Din, a.h, a.Ks, a.Kc, a.Hout)) return false;
@@ -979,18 +989,26 @@ int try_launch_conv_bwd_dx_big(const ConvArgs& a, cudaStream_t st, bool* handled
         a.W, reinterpret_cast<uint8_t*>(a.Wimg), a.Din, a.h, a.Ks, a.Kc, a.Hout, p.KBL, p.KBLp, p.nkc);
     STC_LAUNCH_OK("tc_big_dx_prep_kernel");
   }
-  STC_TRY(set_smem(tc_conv_bwd_dx_big_kernel, p.smem_bytes));
+  const bool det = a.det_ws != nullptr;
+  auto kern = det ? tc_det_bwd_dx_big_kernel : tc_conv_bwd_dx_big_kernel;
+  STC_TRY(set_smem(kern, p.smem_bytes));
   int grid = device_sm_count();
   if (grid > p.ntiles) grid = p.ntiles;
+  if (det && grid > det_conv_slots()) {
+    set_error("tc_conv_bwd_dx_big: %d CTAs but %d partial slots", grid, det_conv_slots());
+    return STC_ERR_WORKSPACE;
+  }
   const int L = a.Din + a.h;
   const double R = (double)total_nodes * a.C;
-  ScopedKernelTimer _t(KK_TC_CONV_BWD_DX, st,
-                       4.0 * R * ((a.phase == 0 ? 6 * a.h + a.Ks * a.Din : 3 * a.h) + a.Hout + a.Ks * L +
-                                  (a.dQ ? a.Hout : 0)) + 4.0 * a.Ks * a.Kc * L * a.Hout);
-  tc_conv_bwd_dx_big_kernel<<<grid, BG_FWD_THREADS, p.smem_bytes, st>>>(a, p, reinterpret_cast<const uint8_t*>(a.Wimg));
-  STC_LAUNCH_OK("tc_conv_bwd_dx_big_kernel");
+  {
+    ScopedKernelTimer _t(KK_TC_CONV_BWD_DX, st,
+                         4.0 * R * ((a.phase == 0 ? 6 * a.h + a.Ks * a.Din : 3 * a.h) + a.Hout + a.Ks * L +
+                                    (a.dQ ? a.Hout : 0)) + 4.0 * a.Ks * a.Kc * L * a.Hout);
+    kern<<<grid, BG_FWD_THREADS, p.smem_bytes, st>>>(a, p, reinterpret_cast<const uint8_t*>(a.Wimg));
+    STC_LAUNCH_OK("tc_conv_bwd_dx_big_kernel");
+  }
   *handled = true;
-  return STC_OK;
+  return det ? det_reduce_dx(a, grid, st) : STC_OK;
 }
 
 // =================================================================================================
@@ -1016,8 +1034,10 @@ struct BigDwPlan {
   uint32_t off_img, off_bar, smem_bytes;
 };
 
-__global__ void __launch_bounds__(BG_THREADS, 1)
-tc_conv_bwd_dw_big_kernel(const ConvArgs a, const BigDwPlan p) {
+// DET (deterministic mode): row range `split` stores its partial dW into slot `split` of a.det_ws (Ks*Kc*L*Hout floats;
+// the Ks * NH CTAs of one range write the whole slot, zeros for an empty range) instead of reducing into a.dW.
+template <bool DET>
+__device__ __forceinline__ void tc_conv_bwd_dw_big_body(const ConvArgs& a, const BigDwPlan& p) {
   extern __shared__ __align__(1024) uint8_t smem[];
   if ((smem_u32(smem) & 1023u) != 0u) __trap();
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
@@ -1179,25 +1199,26 @@ tc_conv_bwd_dw_big_kernel(const ConvArgs a, const BigDwPlan p) {
     }
   }
   // ---- one atomicAdd per owned element: dW[((k*Kc + c)*L + l)*Hout + o] ----
-  if (nchunks > 0 && mrow < p.KBL) {
+  float* const dWo = DET ? a.det_ws + (size_t)split * a.Ks * a.Kc * L * Hout : a.dW;
+  if ((DET || nchunks > 0) && mrow < p.KBL) {
     const int l = mrow < h ? Din + mrow : (mrow - h < Din ? mrow - h : -1);
     if (l >= 0) {
-      const bool v4 = (Hout & 3) == 0 && (reinterpret_cast<uintptr_t>(a.dW) & 15) == 0;   // 16-byte vector reductions
+      const bool v4 = (Hout & 3) == 0 && (reinterpret_cast<uintptr_t>(dWo) & 15) == 0;   // 16-byte vector reductions
 #pragma unroll
       for (int i = 0; i < 4; ++i)
 #pragma unroll
         for (int j = 0; j < 8; j += 4) {
           const int n = nh * 128 + 32 * qtr + 8 * i + j;
           const int c = n / Hout, o = n - c * Hout;
-          float* dst = &a.dW[((size_t)(k * a.Kc + c) * L + l) * Hout + o];
+          float* dst = &dWo[((size_t)(k * a.Kc + c) * L + l) * Hout + o];
           if (v4 && n + 3 < p.N1) {
-            red_add_v4(dst, acc[i][j], acc[i][j + 1], acc[i][j + 2], acc[i][j + 3]);
+            grad_out_v4<DET>(dst, acc[i][j], acc[i][j + 1], acc[i][j + 2], acc[i][j + 3]);
           } else {
 #pragma unroll
             for (int e = 0; e < 4; ++e)
               if (n + e < p.N1) {
                 const int ce = (n + e) / Hout, oe = (n + e) - ce * Hout;
-                atomicAdd(&a.dW[((size_t)(k * a.Kc + ce) * L + l) * Hout + oe], acc[i][j + e]);
+                grad_out<DET>(&dWo[((size_t)(k * a.Kc + ce) * L + l) * Hout + oe], acc[i][j + e]);
               }
           }
         }
@@ -1206,6 +1227,13 @@ tc_conv_bwd_dw_big_kernel(const ConvArgs a, const BigDwPlan p) {
   __syncthreads();
   if (warp == 0) tmem_dealloc(tmem_base, 512u);
 }
+
+__global__ void __launch_bounds__(BG_THREADS, 1)
+tc_conv_bwd_dw_big_kernel(const ConvArgs a, const BigDwPlan p) { tc_conv_bwd_dw_big_body<false>(a, p); }
+// the deterministic-mode instantiation, under a name of its own (the convolution variant list names the default
+// kernels)
+__global__ void __launch_bounds__(BG_THREADS, 1)
+tc_det_bwd_dw_big_kernel(const ConvArgs a, const BigDwPlan p) { tc_conv_bwd_dw_big_body<true>(a, p); }
 
 bool conv_big_bwd_shape_ok(int C, int Din, int h, int Ks, int Kc, int Hout) {
   ConvArgs a;
@@ -1235,13 +1263,23 @@ int try_launch_conv_bwd_dw_big(const ConvArgs& a, cudaStream_t st, bool* handled
   p.off_img = (uint32_t)o; o += 2 * (size_t)p.img_bytes;
   p.off_bar = (uint32_t)o; o += 8 * 3 + 16;
   p.smem_bytes = (uint32_t)o;
-  STC_TRY(set_smem(tc_conv_bwd_dw_big_kernel, p.smem_bytes));
+  const bool det = a.det_ws != nullptr;
+  if (det && p.nsplit > det_conv_slots()) {
+    set_error("tc_conv_bwd_dw_big: %d row ranges but %d partial slots", p.nsplit, det_conv_slots());
+    return STC_ERR_WORKSPACE;
+  }
+  auto kern = det ? tc_det_bwd_dw_big_kernel : tc_conv_bwd_dw_big_kernel;
+  STC_TRY(set_smem(kern, p.smem_bytes));
   const int L = a.Din + a.h;
-  ScopedKernelTimer _t(KK_TC_CONV_BWD_DW, st, 4.0 * (double)R * (a.Ks * L + a.Kc * a.Hout));
-  tc_conv_bwd_dw_big_kernel<<<T * p.nsplit, BG_THREADS, p.smem_bytes, st>>>(a, p);
-  STC_LAUNCH_OK("tc_conv_bwd_dw_big_kernel");
+  {
+    ScopedKernelTimer _t(KK_TC_CONV_BWD_DW, st, 4.0 * (double)R * (a.Ks * L + a.Kc * a.Hout));
+    kern<<<T * p.nsplit, BG_THREADS, p.smem_bytes, st>>>(a, p);
+    STC_LAUNCH_OK("tc_conv_bwd_dw_big_kernel");
+  }
   *handled = true;
-  return STC_OK;
+  if (!det) return STC_OK;
+  const long long n = (long long)a.Ks * a.Kc * L * a.Hout;
+  return launch_det_reduce(a.dW, a.det_ws, p.nsplit, n, n, st);
 }
 
 }  // namespace stc

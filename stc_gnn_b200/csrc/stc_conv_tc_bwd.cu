@@ -114,9 +114,11 @@ __device__ __forceinline__ void dx_prefetch_tile(const ConvArgs& a, const TcDxPl
 // AT (implies FAST, Kc = 2): the A operand [Ds | Dm_1] goes from registers straight into TENSOR MEMORY (tcgen05.st) and
 //     the MMAs read it from there -- no A atoms in shared memory, no proxy fence, no MMA round trip between atoms
 //     (see tc_conv_fwd_at_kernel in stc_conv_tc.cu for the measurements behind this)
-template <bool FAST, bool AT>
-__global__ void __launch_bounds__(CV_THREADS, 2)
-tc_conv_bwd_dx_kernel(const ConvArgs a, const TcDxPlan p) {
+// DET (deterministic mode): the bias and dT_c(Gc) partials are summed inside the CTA in a fixed order (warp shuffles,
+// then per-warp / per-group partials in index order) and stored into slot blockIdx.x of a.det_ws
+// ([Hout | (Kc-1)*C*C] floats each) instead of being reduced with atomics.
+template <bool FAST, bool AT, bool DET>
+__device__ __forceinline__ void tc_conv_bwd_dx_body(const ConvArgs& a, const TcDxPlan& p) {
   extern __shared__ __align__(1024) uint8_t smem[];
   if ((smem_u32(smem) & 1023u) != 0u) __trap();
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
@@ -209,6 +211,7 @@ tc_conv_bwd_dx_kernel(const ConvArgs a, const TcDxPlan p) {
   float dq[DQ_C * DQ_C];
 #pragma unroll
   for (int i = 0; i < DQ_C * DQ_C; ++i) dq[i] = 0.f;
+  float dq_grp = 0.f;   // DET, node-group form: this thread's (group, pair) partial over all its tiles
   uint32_t mma_phase = 0, load_phase = 0;
   bool mma_pending = false;
   const bool tracing = a.trace != nullptr && blockIdx.x == 0 && tid == 0;
@@ -470,7 +473,8 @@ tc_conv_bwd_dx_kernel(const ConvArgs a, const TcDxPlan p) {
               s = fmaf(x.x, y.x, s); s = fmaf(x.y, y.y, s); s = fmaf(x.z, y.z, s); s = fmaf(x.w, y.w, s);
             }
           }
-          atomicAdd(&dQacc[pr], s);
+          if constexpr (DET) dq_grp += s;
+          else atomicAdd(&dQacc[pr], s);
         }
       } else {  // more pairs than threads (large C): each thread walks several pairs
         for (int pr = tid; pr < npairs; pr += CV_THREADS) {
@@ -644,48 +648,118 @@ tc_conv_bwd_dx_kernel(const ConvArgs a, const TcDxPlan p) {
     STC_TRACE(7);
     ++trace_it;
   }
-  if (a.dbias && !db_fast && tid < db_groups * Hout) atomicAdd(&a.dbias[db_col], db_acc);
-  __syncthreads();   // every tile is done: Dsm is free and serves as the reduction scratch
-  // End-of-kernel reductions.  Shared-memory float atomics are compare-and-swap loops: with every thread of the CTA
-  // adding into the same few addresses at once (the first version) the loops serialise -- ~100 us per launch, at any batch
-  // size (profiles/r3b_launches_b32.txt: 110 us per dx launch at B = 32 against 10 us for the forward).  Lanes that
-  // share an address are therefore summed with warp shuffles first; one lane per warp and address touches memory.
-  if (db_fast) {
-    for (int i = tid; i < Hout; i += CV_THREADS) Dsm[i] = 0.f;
-    __syncthreads();
-    const int cprw = h >> 2;                         // lanes l and l + cprw (mod 32) hold the same column chunk
-    float v[8] = {dbs0.x, dbs0.y, dbs0.z, dbs0.w, dbs1.x, dbs1.y, dbs1.z, dbs1.w};
-    for (int off = cprw; off < 32; off <<= 1) {
+  if constexpr (DET) {
+    __syncthreads();   // every tile is done: Dsm is free and holds the per-warp / per-group partials
+    const int npairs = (a.Kc - 1) * C * C;
+    float* slot = a.det_ws + (size_t)blockIdx.x * (Hout + npairs);
+    float* part = Dsm;
+    if (a.dbias) {
+      int nparts = db_groups;
+      if (db_fast) {
+        nparts = CV_THREADS / 32;
+        for (int i = tid; i < nparts * Hout; i += CV_THREADS) part[i] = 0.f;
+        __syncthreads();
+        const int cprw = h >> 2;
+        float v[8] = {dbs0.x, dbs0.y, dbs0.z, dbs0.w, dbs1.x, dbs1.y, dbs1.z, dbs1.w};
+        for (int off = cprw; off < 32; off <<= 1) {
 #pragma unroll
-      for (int i = 0; i < 8; ++i) v[i] += __shfl_xor_sync(0xffffffffu, v[i], off);
+          for (int i = 0; i < 8; ++i) v[i] += __shfl_xor_sync(0xffffffffu, v[i], off);
+        }
+        if (lane < cprw || cprw >= 32) {   // one writer per (warp, column)
+          float* w = part + warp * Hout + ((tid % cprw) << 2);
+          w[0] = v[0]; w[1] = v[1]; w[2] = v[2]; w[3] = v[3];
+          if (a.phase == 0) { w[h] = v[4]; w[h + 1] = v[5]; w[h + 2] = v[6]; w[h + 3] = v[7]; }
+        }
+      } else if (tid < db_groups * Hout) {
+        part[tid] = db_acc;   // (group db_grp, column db_col)
+      }
+      __syncthreads();
+      for (int i = tid; i < Hout; i += CV_THREADS) {
+        float s = 0.f;
+        for (int g = 0; g < nparts; ++g) s += part[g * Hout + i];
+        slot[i] = s;
+      }
+      __syncthreads();
     }
-    if (lane < cprw || cprw >= 32) {
-      const int j = (tid % cprw) << 2;
-      atomicAdd(&Dsm[j + 0], v[0]); atomicAdd(&Dsm[j + 1], v[1]); atomicAdd(&Dsm[j + 2], v[2]); atomicAdd(&Dsm[j + 3], v[3]);
-      if (a.phase == 0) {
-        atomicAdd(&Dsm[h + j + 0], v[4]); atomicAdd(&Dsm[h + j + 1], v[5]);
-        atomicAdd(&Dsm[h + j + 2], v[6]); atomicAdd(&Dsm[h + j + 3], v[7]);
+    if (want_dQ) {
+      const int groups = CV_THREADS / npairs;
+      int nparts = 0;
+      if (dq_fast) {
+        nparts = CV_THREADS / 32;
+#pragma unroll
+        for (int cp = 0; cp < DQ_C; ++cp)
+#pragma unroll
+          for (int d = 0; d < DQ_C; ++d) {
+            float s = dq[cp * DQ_C + d];
+#pragma unroll
+            for (int off = 16; off >= 1; off >>= 1) s += __shfl_xor_sync(0xffffffffu, s, off);
+            if (lane == 0 && cp < C && d < C) part[warp * npairs + cp * C + d] = s;
+          }
+      } else if (groups >= 1) {
+        nparts = groups;
+        if (tid < groups * npairs) part[tid] = dq_grp;   // (group tid / npairs, pair tid % npairs)
+      }
+      __syncthreads();
+      for (int i = tid; i < npairs; i += CV_THREADS) {
+        float s = 0.f;   // the large-C form: each pair has one owner thread, its sum is in dQacc
+        if (nparts == 0) s = dQacc[i];
+        for (int g = 0; g < nparts; ++g) s += part[g * npairs + i];
+        slot[Hout + i] = s;
       }
     }
-    __syncthreads();
-    for (int i = tid; i < Hout; i += CV_THREADS) atomicAdd(&a.dbias[i], Dsm[i]);
-  }
-  if (dq_fast) {   // CTA-uniform: every lane takes part in the shuffles (threads without a node slot hold zeros)
-#pragma unroll
-    for (int cp = 0; cp < DQ_C; ++cp)
-#pragma unroll
-      for (int d = 0; d < DQ_C; ++d) {
-        float s = dq[cp * DQ_C + d];
-#pragma unroll
-        for (int off = 16; off >= 1; off >>= 1) s += __shfl_xor_sync(0xffffffffu, s, off);
-        if (lane == 0 && cp < C && d < C) atomicAdd(&dQacc[cp * C + d], s);
+  } else {
+    if (a.dbias && !db_fast && tid < db_groups * Hout) atomicAdd(&a.dbias[db_col], db_acc);
+    __syncthreads();   // every tile is done: Dsm is free and serves as the reduction scratch
+    // End-of-kernel reductions.  Shared-memory float atomics are compare-and-swap loops: with every thread of the CTA
+    // adding into the same few addresses at once (the first version) the loops serialise -- ~100 us per launch, at any batch
+    // size (profiles/r3b_launches_b32.txt: 110 us per dx launch at B = 32 against 10 us for the forward).  Lanes that
+    // share an address are therefore summed with warp shuffles first; one lane per warp and address touches memory.
+    if (db_fast) {
+      for (int i = tid; i < Hout; i += CV_THREADS) Dsm[i] = 0.f;
+      __syncthreads();
+      const int cprw = h >> 2;                         // lanes l and l + cprw (mod 32) hold the same column chunk
+      float v[8] = {dbs0.x, dbs0.y, dbs0.z, dbs0.w, dbs1.x, dbs1.y, dbs1.z, dbs1.w};
+      for (int off = cprw; off < 32; off <<= 1) {
+  #pragma unroll
+        for (int i = 0; i < 8; ++i) v[i] += __shfl_xor_sync(0xffffffffu, v[i], off);
       }
+      if (lane < cprw || cprw >= 32) {
+        const int j = (tid % cprw) << 2;
+        atomicAdd(&Dsm[j + 0], v[0]); atomicAdd(&Dsm[j + 1], v[1]); atomicAdd(&Dsm[j + 2], v[2]); atomicAdd(&Dsm[j + 3], v[3]);
+        if (a.phase == 0) {
+          atomicAdd(&Dsm[h + j + 0], v[4]); atomicAdd(&Dsm[h + j + 1], v[5]);
+          atomicAdd(&Dsm[h + j + 2], v[6]); atomicAdd(&Dsm[h + j + 3], v[7]);
+        }
+      }
+      __syncthreads();
+      for (int i = tid; i < Hout; i += CV_THREADS) atomicAdd(&a.dbias[i], Dsm[i]);
+    }
+    if (dq_fast) {   // CTA-uniform: every lane takes part in the shuffles (threads without a node slot hold zeros)
+  #pragma unroll
+      for (int cp = 0; cp < DQ_C; ++cp)
+  #pragma unroll
+        for (int d = 0; d < DQ_C; ++d) {
+          float s = dq[cp * DQ_C + d];
+  #pragma unroll
+          for (int off = 16; off >= 1; off >>= 1) s += __shfl_xor_sync(0xffffffffu, s, off);
+          if (lane == 0 && cp < C && d < C) atomicAdd(&dQacc[cp * C + d], s);
+        }
+    }
+    __syncthreads();
+    if (want_dQ)
+      for (int i = tid; i < (a.Kc - 1) * C * C; i += CV_THREADS) atomicAdd(&a.dQ[C * C + i], dQacc[i]);
   }
-  __syncthreads();
-  if (want_dQ)
-    for (int i = tid; i < (a.Kc - 1) * C * C; i += CV_THREADS) atomicAdd(&a.dQ[C * C + i], dQacc[i]);
   if (warp == 0) tmem_dealloc(tmem_base, (uint32_t)p.tmem_cols);
 }
+
+template <bool FAST, bool AT>
+__global__ void __launch_bounds__(CV_THREADS, 2)
+tc_conv_bwd_dx_kernel(const ConvArgs a, const TcDxPlan p) { tc_conv_bwd_dx_body<FAST, AT, false>(a, p); }
+// the deterministic-mode instantiation, under a name of its own (the convolution variant list names the default
+// kernels)
+template <bool FAST, bool AT>
+__global__ void __launch_bounds__(CV_THREADS, 2)
+tc_det_bwd_dx_kernel(const ConvArgs a, const TcDxPlan p) { tc_conv_bwd_dx_body<FAST, AT, true>(a, p); }
 
 static bool aligned16b(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
 
@@ -732,8 +806,11 @@ int try_launch_conv_bwd_dx_tc(const ConvArgs& a, cudaStream_t st, bool* handled)
   }
   const bool fast = a.Ks == 2 && a.h == 16 && a.Din <= 16 && p.nmain == 1 && !(a.opt & OPT_GENERIC_EPILOGUE);
   const bool at = fast && a.Kc == 2 && p.Kdd <= 64 && (a.Hout == 16 || a.Hout == 32) && !(a.opt & OPT_SMEM_A);
-  auto kern = at ? tc_conv_bwd_dx_kernel<true, true>
-                 : (fast ? tc_conv_bwd_dx_kernel<true, false> : tc_conv_bwd_dx_kernel<false, false>);
+  const bool det = a.det_ws != nullptr;
+  auto kern = det ? (at ? tc_det_bwd_dx_kernel<true, true>
+                        : (fast ? tc_det_bwd_dx_kernel<true, false> : tc_det_bwd_dx_kernel<false, false>))
+                  : (at ? tc_conv_bwd_dx_kernel<true, true>
+                        : (fast ? tc_conv_bwd_dx_kernel<true, false> : tc_conv_bwd_dx_kernel<false, false>));
   if (at) p.tmem_cols = 256;   // 2 Npad accumulator columns + 64 A_hi + 64 A_lo
   STC_TRY(set_smem(kern, p.smem_bytes));
   int ctas_per_sm = (int)((228 * 1024) / (p.smem_bytes + 1024));
@@ -742,17 +819,23 @@ int try_launch_conv_bwd_dx_tc(const ConvArgs& a, cudaStream_t st, bool* handled)
   if (ctas_per_sm * p.tmem_cols > 512) ctas_per_sm = 512 / p.tmem_cols;
   int grid = device_sm_count() * ctas_per_sm;
   if (grid > p.ntiles) grid = p.ntiles;
+  if (det && grid > det_conv_slots()) {
+    set_error("tc_conv_bwd_dx: %d CTAs but %d partial slots", grid, det_conv_slots());
+    return STC_ERR_WORKSPACE;
+  }
   // compulsory traffic per row: candidate reads dH',u,c (3h), gates reads dH',u,c,H,r,d(rH) (6h); both write dpre
   // (Hout) and the Ks adjoint terms (Ks*L; the gates pass re-reads the x-part it accumulates into) and, for dGc,
   // read the saved partial outputs ((Kc-1)*Hout).
   const double R = (double)total_nodes * a.C;
-  ScopedKernelTimer _t(KK_TC_CONV_BWD_DX, st,
-                       4.0 * R * ((a.phase == 0 ? 6 * a.h + a.Ks * a.Din : 3 * a.h) + a.Hout + a.Ks * L +
-                                  ((a.dQ && a.Kc > 1) ? p.PW : 0)) + 4.0 * a.Ks * a.Kc * L * a.Hout);
-  kern<<<grid, CV_THREADS, p.smem_bytes, st>>>(a, p);
-  STC_LAUNCH_OK("tc_conv_bwd_dx_kernel");
+  {
+    ScopedKernelTimer _t(KK_TC_CONV_BWD_DX, st,
+                         4.0 * R * ((a.phase == 0 ? 6 * a.h + a.Ks * a.Din : 3 * a.h) + a.Hout + a.Ks * L +
+                                    ((a.dQ && a.Kc > 1) ? p.PW : 0)) + 4.0 * a.Ks * a.Kc * L * a.Hout);
+    kern<<<grid, CV_THREADS, p.smem_bytes, st>>>(a, p);
+    STC_LAUNCH_OK("tc_conv_bwd_dx_kernel");
+  }
   *handled = true;
-  return STC_OK;
+  return det ? det_reduce_dx(a, grid, st) : STC_OK;
 }
 
 }  // namespace stc

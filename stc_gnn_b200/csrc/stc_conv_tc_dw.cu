@@ -34,9 +34,10 @@ struct TcDwPlan {
   uint32_t off_a, off_b, off_bar, smem_bytes;
 };
 
-template <int NCH>  // 8-column accumulator chunks per thread
-__global__ void __launch_bounds__(CV_THREADS, 2)
-tc_conv_bwd_dw_kernel(const ConvArgs a, const TcDwPlan p) {
+// NCH: 8-column accumulator chunks per thread.  DET: CTA blockIdx.x stores its partial dW into slot blockIdx.x of
+// a.det_ws (Ks*Kc*L*Hout floats each; every CTA writes its whole slot) instead of reducing into a.dW.
+template <int NCH, bool DET>
+__device__ __forceinline__ void tc_conv_bwd_dw_body(const ConvArgs& a, const TcDwPlan& p) {
   extern __shared__ __align__(1024) uint8_t smem[];
   if ((smem_u32(smem) & 1023u) != 0u) __trap();
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
@@ -214,7 +215,8 @@ tc_conv_bwd_dw_kernel(const ConvArgs a, const TcDwPlan p) {
   }
 
   // ---- one (vector) atomic per owned element group ----
-  const bool dw_v4 = (Hout & 3) == 0 && (col0 & 3) == 0 && (reinterpret_cast<uintptr_t>(a.dW) & 15) == 0;
+  float* const dWo = DET ? a.det_ws + (size_t)blockIdx.x * a.Ks * a.Kc * L * Hout : a.dW;
+  const bool dw_v4 = (Hout & 3) == 0 && (col0 & 3) == 0 && (reinterpret_cast<uintptr_t>(dWo) & 15) == 0;
   if (own && mrow < p.M1) {
     const int k = mrow / p.KBL, kb = mrow - k * p.KBL;
     const int l = kb < h ? Din + kb : (kb - h < Din ? kb - h : -1);
@@ -226,15 +228,15 @@ tc_conv_bwd_dw_kernel(const ConvArgs a, const TcDwPlan p) {
         for (int j = 0; j < 8; j += 4) {
           const int n = col0 + i * 8 + j;
           const int c = n / Hout, o = n - c * Hout;
-          float* dst = &a.dW[((size_t)(k * a.Kc + c) * L + l) * Hout + o];
+          float* dst = &dWo[((size_t)(k * a.Kc + c) * L + l) * Hout + o];
           if (dw_v4 && n + 3 < p.N1) {
-            red_add_v4(dst, acc[i][j], acc[i][j + 1], acc[i][j + 2], acc[i][j + 3]);
+            grad_out_v4<DET>(dst, acc[i][j], acc[i][j + 1], acc[i][j + 2], acc[i][j + 3]);
           } else {
 #pragma unroll
             for (int e = 0; e < 4; ++e)
               if (n + e < p.N1) {
                 const int ce = (n + e) / Hout, oe = (n + e) - ce * Hout;
-                atomicAdd(&a.dW[((size_t)(k * a.Kc + ce) * L + l) * Hout + oe], acc[i][j + e]);
+                grad_out<DET>(&dWo[((size_t)(k * a.Kc + ce) * L + l) * Hout + oe], acc[i][j + e]);
               }
           }
         }
@@ -244,6 +246,15 @@ tc_conv_bwd_dw_kernel(const ConvArgs a, const TcDwPlan p) {
   __syncthreads();
   if (warp == 0) tmem_dealloc(tmem_base, (uint32_t)p.tmem_cols);
 }
+
+template <int NCH>
+__global__ void __launch_bounds__(CV_THREADS, 2)
+tc_conv_bwd_dw_kernel(const ConvArgs a, const TcDwPlan p) { tc_conv_bwd_dw_body<NCH, false>(a, p); }
+// the deterministic-mode instantiation, under a name of its own (the convolution variant list names the default
+// kernels)
+template <int NCH>
+__global__ void __launch_bounds__(CV_THREADS, 2)
+tc_det_bwd_dw_kernel(const ConvArgs a, const TcDwPlan p) { tc_conv_bwd_dw_body<NCH, true>(a, p); }
 
 // =================================================================================================
 // Pipelined variant (taken whenever every row piece is 16-byte aligned): the same product, but the operand tiles
@@ -261,9 +272,8 @@ struct TcDwPipePlan {
   uint32_t off_raw, off_img, img_bytes, off_bar, smem_bytes;
 };
 
-template <int NCH>
-__global__ void __launch_bounds__(DWP_THREADS, 1)
-tc_conv_bwd_dw_pipe_kernel(const ConvArgs a, const TcDwPipePlan p) {
+template <int NCH, bool DET>   // DET: as tc_conv_bwd_dw_body
+__device__ __forceinline__ void tc_conv_bwd_dw_pipe_body(const ConvArgs& a, const TcDwPipePlan& p) {
   extern __shared__ __align__(1024) uint8_t smem[];
   if ((smem_u32(smem) & 1023u) != 0u) __trap();
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
@@ -465,7 +475,8 @@ tc_conv_bwd_dw_pipe_kernel(const ConvArgs a, const TcDwPipePlan p) {
       }
     }
     // ---- one (vector) atomic per owned element group ----
-    const bool dw_v4 = (Hout & 3) == 0 && (col0 & 3) == 0 && (reinterpret_cast<uintptr_t>(a.dW) & 15) == 0;
+    float* const dWo = DET ? a.det_ws + (size_t)blockIdx.x * a.Ks * a.Kc * L * Hout : a.dW;
+    const bool dw_v4 = (Hout & 3) == 0 && (col0 & 3) == 0 && (reinterpret_cast<uintptr_t>(dWo) & 15) == 0;
     if (own && mrow < p.M1) {
       const int k = mrow / p.KBL, kb = mrow - k * p.KBL;
       const int l = kb < h ? Din + kb : (kb - h < Din ? kb - h : -1);
@@ -477,16 +488,16 @@ tc_conv_bwd_dw_pipe_kernel(const ConvArgs a, const TcDwPipePlan p) {
           for (int j = 0; j < 8; j += 4) {
             const int n = col0 + i * 8 + j;
             const int c = n / Hout, o = n - c * Hout;
-            float* dst = &a.dW[((size_t)(k * a.Kc + c) * L + l) * Hout + o];
+            float* dst = &dWo[((size_t)(k * a.Kc + c) * L + l) * Hout + o];
             // Hout % 4 == 0 and n % 4 == 0: the four columns stay inside one categorical block and one 16-byte slot
             if (dw_v4 && n + 3 < p.N1) {
-              red_add_v4(dst, acc[i][j], acc[i][j + 1], acc[i][j + 2], acc[i][j + 3]);
+              grad_out_v4<DET>(dst, acc[i][j], acc[i][j + 1], acc[i][j + 2], acc[i][j + 3]);
             } else {
 #pragma unroll
               for (int e = 0; e < 4; ++e)
                 if (n + e < p.N1) {
                   const int ce = (n + e) / Hout, oe = (n + e) - ce * Hout;
-                  atomicAdd(&a.dW[((size_t)(k * a.Kc + ce) * L + l) * Hout + oe], acc[i][j + e]);
+                  grad_out<DET>(&dWo[((size_t)(k * a.Kc + ce) * L + l) * Hout + oe], acc[i][j + e]);
                 }
             }
           }
@@ -499,7 +510,37 @@ tc_conv_bwd_dw_pipe_kernel(const ConvArgs a, const TcDwPipePlan p) {
   if (warp == 0) tmem_dealloc(tmem_base, (uint32_t)p.tmem_cols);
 }
 
+template <int NCH>
+__global__ void __launch_bounds__(DWP_THREADS, 1)
+tc_conv_bwd_dw_pipe_kernel(const ConvArgs a, const TcDwPipePlan p) { tc_conv_bwd_dw_pipe_body<NCH, false>(a, p); }
+// the deterministic-mode instantiation, under a name of its own (the convolution variant list names the default
+// kernels)
+template <int NCH>
+__global__ void __launch_bounds__(DWP_THREADS, 1)
+tc_det_bwd_dw_pipe_kernel(const ConvArgs a, const TcDwPipePlan p) { tc_conv_bwd_dw_pipe_body<NCH, true>(a, p); }
+
 static bool aligned16d(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
+
+// one dW launch (timed as tc_conv_bwd_dw); with a.det_ws (deterministic mode) the slot form, then the fixed-order sum of
+// its grid slots into a.dW
+template <typename Plan, typename K>
+static int launch_dw(K plain, K det, const ConvArgs& a, const Plan& p, int grid, int threads, double bytes, cudaStream_t st) {
+  const bool dm = a.det_ws != nullptr;
+  if (dm && grid > det_conv_slots()) {
+    set_error("tc_conv_bwd_dw: %d CTAs but %d partial slots", grid, det_conv_slots());
+    return STC_ERR_WORKSPACE;
+  }
+  K kern = dm ? det : plain;
+  STC_TRY(set_smem(kern, p.smem_bytes));
+  {
+    ScopedKernelTimer _t(KK_TC_CONV_BWD_DW, st, bytes);
+    kern<<<grid, threads, p.smem_bytes, st>>>(a, p);
+    STC_LAUNCH_OK("tc_conv_bwd_dw_kernel");
+  }
+  if (!dm) return STC_OK;
+  const long long n = (long long)a.Ks * a.Kc * (a.Din + a.h) * a.Hout;
+  return launch_det_reduce(a.dW, a.det_ws, grid, n, n, st);
+}
 
 // Pipelined dW kernel: every bulk copy must start 16-byte aligned and move a multiple of 16 bytes.
 static int try_launch_dw_pipe(const ConvArgs& a, cudaStream_t st, bool* piped) {
@@ -540,14 +581,12 @@ static int try_launch_dw_pipe(const ConvArgs& a, cudaStream_t st, bool* piped) {
   const int nch = (p.Npad / 2 + 7) / 8;
   long long grid = device_sm_count();
   if (grid > p.ntiles) grid = p.ntiles;
-  ScopedKernelTimer _t(KK_TC_CONV_BWD_DW, st,
-                       4.0 * (double)R * (a.Ks * L + a.Kc * a.Hout) + 4.0 * a.Ks * a.Kc * L * a.Hout);
+  const double bytes = 4.0 * (double)R * (a.Ks * L + a.Kc * a.Hout) + 4.0 * a.Ks * a.Kc * L * a.Hout;
   switch (nch) {
-    case 1: STC_TRY(set_smem(tc_conv_bwd_dw_pipe_kernel<1>, p.smem_bytes)); tc_conv_bwd_dw_pipe_kernel<1><<<(int)grid, DWP_THREADS, p.smem_bytes, st>>>(a, p); break;
-    case 2: STC_TRY(set_smem(tc_conv_bwd_dw_pipe_kernel<2>, p.smem_bytes)); tc_conv_bwd_dw_pipe_kernel<2><<<(int)grid, DWP_THREADS, p.smem_bytes, st>>>(a, p); break;
-    default: STC_TRY(set_smem(tc_conv_bwd_dw_pipe_kernel<4>, p.smem_bytes)); tc_conv_bwd_dw_pipe_kernel<4><<<(int)grid, DWP_THREADS, p.smem_bytes, st>>>(a, p); break;
+    case 1: STC_TRY(launch_dw(tc_conv_bwd_dw_pipe_kernel<1>, tc_det_bwd_dw_pipe_kernel<1>, a, p, (int)grid, DWP_THREADS, bytes, st)); break;
+    case 2: STC_TRY(launch_dw(tc_conv_bwd_dw_pipe_kernel<2>, tc_det_bwd_dw_pipe_kernel<2>, a, p, (int)grid, DWP_THREADS, bytes, st)); break;
+    default: STC_TRY(launch_dw(tc_conv_bwd_dw_pipe_kernel<4>, tc_det_bwd_dw_pipe_kernel<4>, a, p, (int)grid, DWP_THREADS, bytes, st)); break;
   }
-  STC_LAUNCH_OK("tc_conv_bwd_dw_pipe_kernel");
   *piped = true;
   return STC_OK;
 }
@@ -601,14 +640,12 @@ int try_launch_conv_bwd_dw_tc(const ConvArgs& a, cudaStream_t st, bool* handled)
   long long grid = (long long)device_sm_count() * ctas_per_sm;
   if (grid > p.ntiles) grid = p.ntiles;
   // compulsory traffic per row: the Ks spatial terms of [x|h] once and the (unmixed) pre-activation gradient once
-  ScopedKernelTimer _t(KK_TC_CONV_BWD_DW, st,
-                       4.0 * (double)R * (a.Ks * L + a.Kc * a.Hout) + 4.0 * a.Ks * a.Kc * L * a.Hout);
+  const double bytes = 4.0 * (double)R * (a.Ks * L + a.Kc * a.Hout) + 4.0 * a.Ks * a.Kc * L * a.Hout;
   switch (nch) {
-    case 1: STC_TRY(set_smem(tc_conv_bwd_dw_kernel<1>, p.smem_bytes)); tc_conv_bwd_dw_kernel<1><<<(int)grid, CV_THREADS, p.smem_bytes, st>>>(a, p); break;
-    case 2: STC_TRY(set_smem(tc_conv_bwd_dw_kernel<2>, p.smem_bytes)); tc_conv_bwd_dw_kernel<2><<<(int)grid, CV_THREADS, p.smem_bytes, st>>>(a, p); break;
-    default: STC_TRY(set_smem(tc_conv_bwd_dw_kernel<4>, p.smem_bytes)); tc_conv_bwd_dw_kernel<4><<<(int)grid, CV_THREADS, p.smem_bytes, st>>>(a, p); break;
+    case 1: STC_TRY(launch_dw(tc_conv_bwd_dw_kernel<1>, tc_det_bwd_dw_kernel<1>, a, p, (int)grid, CV_THREADS, bytes, st)); break;
+    case 2: STC_TRY(launch_dw(tc_conv_bwd_dw_kernel<2>, tc_det_bwd_dw_kernel<2>, a, p, (int)grid, CV_THREADS, bytes, st)); break;
+    default: STC_TRY(launch_dw(tc_conv_bwd_dw_kernel<4>, tc_det_bwd_dw_kernel<4>, a, p, (int)grid, CV_THREADS, bytes, st)); break;
   }
-  STC_LAUNCH_OK("tc_conv_bwd_dw_kernel");
   *handled = true;
   return STC_OK;
 }

@@ -249,6 +249,33 @@ support_csr_kernel(const int32_t* __restrict__ rowptr, const int32_t* __restrict
 
 static bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
 
+// Deterministic form of the edge-value gradient: one warp owns a row n and ALL of its edges' sums, over every sample and
+// feature in a fixed order (lane-strided partial sums, then a shuffle tree), so every dvals[e] has exactly one writer:
+//   dvals[e = (n, m)] += coef * sum_{b,j} a[b,n,j] * x[b,m,j]
+__global__ void __launch_bounds__(256)
+csr_edge_grad_det_kernel(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ col,
+                         const int32_t* __restrict__ row_list, int n_rows, int B, int W, const float* __restrict__ X,
+                         long long x_bs, const float* __restrict__ A, long long a_bs, float coef, float* dvals) {
+  const int lane = threadIdx.x & 31;
+  const long long warp0 = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const long long nwarps = ((long long)gridDim.x * blockDim.x) >> 5;
+  for (long long r = warp0; r < n_rows; r += nwarps) {
+    const int n = row_list ? row_list[r] : (int)r;
+    for (int e = rowptr[n]; e < rowptr[n + 1]; ++e) {
+      const long long m = col[e];
+      float dot = 0.f;
+      for (int b = 0; b < B; ++b) {
+        const float* ar = A + b * a_bs + (long long)n * W;
+        const float* xr = X + b * x_bs + m * W;
+        for (int j = lane; j < W; j += 32) dot = fmaf(ar[j], xr[j], dot);
+      }
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) dot += __shfl_xor_sync(0xffffffffu, dot, o);
+      if (lane == 0) dvals[e] += coef * dot;
+    }
+  }
+}
+
 // one CSR hop (rp, ci, va walk the rows of the operator applied); eg.dvals != nullptr selects the edge-gradient variant
 static int launch_csr(const int32_t* rp, const int32_t* ci, const float* va, long long nnz, int N, int B, int width,
                       const float* x, int64_t x_bs, const float* z, int64_t z_bs, float* y, float alpha, float beta,
@@ -369,6 +396,18 @@ int launch_support_csr_edge_grad(const StcSupport& gs, int N, int B, int width, 
     set_error("support_apply: beta != 0 needs z");
     return STC_ERR_BAD_ARG;
   }
+  if (det_mode()) {   // the plain hop (y bitwise that of stc_support_apply), then the one-writer edge gradient
+    STC_TRY(launch_csr(gs.rowptr, gs.col, gs.vals, gs.nnz, N, B, width, x, x_bs, z, z_bs, y, alpha, beta, axpy_out,
+                       axpy_coef, row_list, n_list, CsrEdgeGrad{nullptr, 0, 0.f, nullptr}, st));
+    const int rows = row_list ? n_list : N;
+    long long blocks = (rows + 7) / 8;
+    if (blocks > (long long)device_sm_count() * 16) blocks = (long long)device_sm_count() * 16;
+    ScopedKernelTimer _t(KK_SUPPORT_CSR_GRAD, st, 4.0 * (double)B * width * (rows + gs.nnz) + 8.0 * gs.nnz);
+    csr_edge_grad_det_kernel<<<(int)blocks, 256, 0, st>>>(gs.rowptr, gs.col, row_list, rows, B, width, x, x_bs, a, a_bs,
+                                                           coef, dvals);
+    STC_LAUNCH_OK("csr_edge_grad_det_kernel");
+    return STC_OK;
+  }
   return launch_csr(gs.rowptr, gs.col, gs.vals, gs.nnz, N, B, width, x, x_bs, z, z_bs, y, alpha, beta, axpy_out,
                     axpy_coef, row_list, n_list, CsrEdgeGrad{a, (long long)a_bs, coef, dvals}, st);
 }
@@ -427,6 +466,8 @@ int launch_halo_rows(bool pack, float* x_ext, long long x_bs, int W, int B, cons
 // ------------------------------------------------------------------------------------------------
 constexpr int SO_T = 64, SO_BK = 16, SO_THREADS = 256;
 
+// DET: batch slice z writes its partial into slot z of dG (N * N floats each) with plain stores
+template <bool DET>
 __global__ void __launch_bounds__(SO_THREADS)
 support_outer_kernel(int N, int B, int W, const float* __restrict__ A, long long a_bs,
                      const float* __restrict__ Bm, float coef, float* dG, int b_per_cta) {
@@ -474,17 +515,40 @@ support_outer_kernel(int N, int B, int W, const float* __restrict__ A, long long
 #pragma unroll
     for (int jj = 0; jj < 4; ++jj) {
       int m = m0 + tx * 4 + jj;
-      if (m < N) atomicAdd(&dG[(long long)n * N + m], coef * acc[i][jj]);
+      if (m >= N) continue;
+      if constexpr (DET) dG[((long long)blockIdx.z * N + n) * N + m] = coef * acc[i][jj];
+      else atomicAdd(&dG[(long long)n * N + m], coef * acc[i][jj]);
     }
   }
 }
 
+// batch slices of the FFMA form: as many as fill the device twice over
+static int outer_ffma_zsplit(int N, int B) {
+  const int tiles = ceil_div(N, SO_T);
+  int zsplit = device_sm_count() * 2 / (tiles * tiles);
+  if (zsplit < 1) zsplit = 1;
+  if (zsplit > B) zsplit = B;
+  return ceil_div(B, ceil_div(B, zsplit));
+}
+
+long long support_outer_det_floats(int N, int B, int width) {
+  if (B <= 0 || N <= 0 || width <= 0) return 0;
+  // the larger of the two forms' slot counts (operand alignment decides which one runs); one slice needs none
+  const int tc = outer_tc_det_slots(N, B, width), ffma = outer_ffma_zsplit(N, B);
+  const int slots = tc > ffma ? tc : ffma;
+  return slots > 1 ? (long long)slots * N * N : 0;
+}
+
 int launch_support_outer(int N, int B, int width, const float* a, int64_t a_bs, const float* bmat, float coef,
-                         float* dG, cudaStream_t st) {
+                         float* dG, cudaStream_t st, float* det_ws) {
   if (B <= 0 || N <= 0 || width <= 0) return STC_OK;
+  if (det_mode() && det_ws == nullptr && support_outer_det_floats(N, B, width) > 0) {
+    set_error("support outer product: the deterministic form needs its slot workspace");
+    return STC_ERR_WORKSPACE;
+  }
   {
     bool handled = false;
-    STC_TRY(try_launch_outer_tc(N, B, width, a, a_bs, bmat, coef, dG, st, &handled));
+    STC_TRY(try_launch_outer_tc(N, B, width, a, a_bs, bmat, coef, dG, st, &handled, det_ws));
     if (handled) return STC_OK;
   }
   int tiles = ceil_div(N, SO_T);
@@ -492,16 +556,44 @@ int launch_support_outer(int N, int B, int width, const float* a, int64_t a_bs, 
     set_error("dGs for N=%d is not tiled", N);
     return STC_ERR_UNSUPPORTED;
   }
-  int target = device_sm_count() * 2;
-  int zsplit = target / (tiles * tiles);
-  if (zsplit < 1) zsplit = 1;
-  if (zsplit > B) zsplit = B;
-  int b_per = ceil_div(B, zsplit);
-  zsplit = ceil_div(B, b_per);
+  const int zsplit = outer_ffma_zsplit(N, B);
+  const int b_per = ceil_div(B, zsplit);
   dim3 grid(tiles, tiles, zsplit);
-  ScopedKernelTimer _t(KK_SUPPORT_OUTER, st, 4.0 * B * N * width * 2 + 4.0 * N * N);
-  support_outer_kernel<<<grid, SO_THREADS, 0, st>>>(N, B, width, a, a_bs, bmat, coef, dG, b_per);
-  STC_LAUNCH_OK("support_outer_kernel");
+  const bool det = det_mode() && zsplit > 1;   // one slice: every element has a single writer already
+  {
+    ScopedKernelTimer _t(KK_SUPPORT_OUTER, st, 4.0 * B * N * width * 2 + 4.0 * N * N);
+    if (det)
+      support_outer_kernel<true><<<grid, SO_THREADS, 0, st>>>(N, B, width, a, a_bs, bmat, coef, det_ws, b_per);
+    else
+      support_outer_kernel<false><<<grid, SO_THREADS, 0, st>>>(N, B, width, a, a_bs, bmat, coef, dG, b_per);
+    STC_LAUNCH_OK("support_outer_kernel");
+  }
+  if (det) return launch_det_reduce(dG, det_ws, zsplit, (long long)N * N, (long long)N * N, st);
+  return STC_OK;
+}
+
+// ------------------------------------------------------------------------------------------------
+// deterministic mode: the fixed-order sum of per-CTA partial slots, added once into the destination.  One thread per
+// element walks the slots in ascending order (consecutive threads read consecutive floats of each slot).
+// ------------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(256)
+det_reduce_kernel(float* __restrict__ dst, const float* __restrict__ slots, int n_slots, long long n, long long stride) {
+  for (long long i = blockIdx.x * 256LL + threadIdx.x; i < n; i += (long long)gridDim.x * 256) {
+    // (unrolled so that eight slots' loads are in flight at once; the additions keep ascending slot order)
+    float s = 0.f;
+#pragma unroll 8
+    for (int k = 0; k < n_slots; ++k) s += __ldg(slots + (long long)k * stride + i);
+    dst[i] += s;
+  }
+}
+
+int launch_det_reduce(float* dst, const float* slots, int n_slots, long long n, long long slot_stride, cudaStream_t st) {
+  if (n <= 0 || n_slots <= 0) return STC_OK;
+  long long blocks = (n + 255) / 256;
+  if (blocks > (long long)device_sm_count() * 8) blocks = (long long)device_sm_count() * 8;
+  ScopedKernelTimer _t(KK_DET_REDUCE, st, 4.0 * n * (n_slots + 2));
+  det_reduce_kernel<<<(int)blocks, 256, 0, st>>>(dst, slots, n_slots, n, slot_stride);
+  STC_LAUNCH_OK("det_reduce_kernel");
   return STC_OK;
 }
 

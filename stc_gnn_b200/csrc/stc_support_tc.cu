@@ -340,7 +340,8 @@ struct TcOuterPlan {
 // [main | cross] used round-robin, drained into fp32 registers every `drain` atoms (bounded chains).
 // BLOCKS = false: the support fits one tile (n0 = m0 = 0, every row bound is N -- exactly the one-tile code);
 // BLOCKS = true: gridDim.y walks the 128 x 128 blocks of a larger support.
-template <bool BLOCKS>
+// DET: sample slice blockIdx.x stores its partial into slot blockIdx.x of dG (N * N floats each) instead of reducing
+template <bool BLOCKS, bool DET>
 __global__ void __launch_bounds__(TO_THREADS, 1)
 tc_outer_kernel(const float* __restrict__ A, long long a_bs, const float* __restrict__ Bm, float coef, float* dG,
                 const TcOuterPlan p) {
@@ -542,13 +543,20 @@ tc_outer_kernel(const float* __restrict__ A, long long a_bs, const float* __rest
 #pragma unroll
           for (int i = 0; i < 8; i += 4) {
             const int m = col0 + ch * 8 + i;
-            float* dst = &dG[(size_t)(n0 + nrow) * N + m0 + m];
+            float* dst = &dG[(DET ? (size_t)blockIdx.x * N * N : 0) + (size_t)(n0 + nrow) * N + m0 + m];
             if (v4 && m + 3 < rowsB) {
-              red_add_v4(dst, coef * acc[ch][i], coef * acc[ch][i + 1], coef * acc[ch][i + 2], coef * acc[ch][i + 3]);
+              if constexpr (DET)
+                *reinterpret_cast<float4*>(dst) =
+                    make_float4(coef * acc[ch][i], coef * acc[ch][i + 1], coef * acc[ch][i + 2], coef * acc[ch][i + 3]);
+              else
+                red_add_v4(dst, coef * acc[ch][i], coef * acc[ch][i + 1], coef * acc[ch][i + 2], coef * acc[ch][i + 3]);
             } else {
 #pragma unroll
               for (int e = 0; e < 4; ++e)
-                if (m + e < rowsB) atomicAdd(dst + e, coef * acc[ch][i + e]);
+                if (m + e < rowsB) {
+                  if constexpr (DET) dst[e] = coef * acc[ch][i + e];
+                  else atomicAdd(dst + e, coef * acc[ch][i + e]);
+                }
             }
           }
         }
@@ -560,23 +568,43 @@ tc_outer_kernel(const float* __restrict__ A, long long a_bs, const float* __rest
   if (warp == 0) tmem_dealloc(tmem_base, (uint32_t)p.tmem_cols);
 }
 
-int try_launch_outer_tc(int N, int B, int width, const float* a, int64_t a_bs, const float* bmat, float coef, float* dG,
-                        cudaStream_t st, bool* handled) {
-  *handled = false;
-  if (tc_support_disabled()) return STC_OK;
-  if (width % 4 != 0 || a_bs % 4 != 0 || !aligned16s(a) || !aligned16s(bmat) || N < 8) return STC_OK;
-  TcOuterPlan p;
-  p.N = N;
-  p.nblk = (N + 127) / 128;
-  if ((long long)p.nblk * p.nblk > 65535) return STC_OK;
+// whether tc_outer takes a product of this shape (operand alignment aside), and its CTAs along the samples
+static int outer_tc_grid(int N, int B, int width) {
+  if (tc_support_disabled() || width % 4 != 0 || N < 8) return 0;
+  const int nblk = (N + 127) / 128;
+  if ((long long)nblk * nblk > 65535) return 0;
   if (N > 128) {   // A/B switch for tools/bench_dense_support.py (shared with the N > 128 support kernel)
     static int big_off = -1;
     if (big_off < 0) {
       const char* e = getenv("STC_DISABLE_TC_SUPPORT_BIG");
       big_off = (e && e[0] && e[0] != '0') ? 1 : 0;
     }
-    if (big_off == 1) return STC_OK;
+    if (big_off == 1) return 0;
   }
+  // one tile: the CTAs split the samples.  N > 128: one CTA per 128 x 128 block of dGs and sample slice -- as few slices
+  // as still fill the device twice over (long K runs per CTA, one pass of vector reductions per CTA at the end)
+  const int nblocks = nblk * nblk;
+  int grid = device_sm_count();
+  if (nblocks > 1) grid = (2 * grid + nblocks - 1) / nblocks;
+  if (grid > B) grid = B;
+  return grid;
+}
+
+int outer_tc_det_slots(int N, int B, int width) {
+  const int g = B > 0 ? outer_tc_grid(N, B, width) : 0;
+  return g > 1 ? g : 0;
+}
+
+int try_launch_outer_tc(int N, int B, int width, const float* a, int64_t a_bs, const float* bmat, float coef, float* dG,
+                        cudaStream_t st, bool* handled, float* det_ws) {
+  *handled = false;
+  const int grid = outer_tc_grid(N, B, width);
+  if (grid == 0 || a_bs % 4 != 0 || !aligned16s(a) || !aligned16s(bmat)) return STC_OK;
+  // deterministic mode with one sample slice: every element already has a single writer, no slots needed
+  const bool det = det_mode() && grid > 1;
+  TcOuterPlan p;
+  p.N = N;
+  p.nblk = (N + 127) / 128;
   p.Npad = N > 128 ? 128 : (N + 15) & ~15;
   p.W = width;
   p.B = B;
@@ -598,18 +626,17 @@ int try_launch_outer_tc(int N, int B, int width, const float* a, int64_t a_bs, c
   p.off_bar = (TO_SH + TO_SL) * hsz;
   p.smem_bytes = p.off_bar + 8 * (2 * TO_SH + 1) + 16;
   if (p.smem_bytes > 227 * 1024) return STC_OK;
-  auto kern = p.nblk > 1 ? tc_outer_kernel<true> : tc_outer_kernel<false>;
+  auto kern = p.nblk > 1 ? (det ? tc_outer_kernel<true, true> : tc_outer_kernel<true, false>)
+                         : (det ? tc_outer_kernel<false, true> : tc_outer_kernel<false, false>);
   STC_TRY(set_smem(kern, p.smem_bytes));
-  // one tile: the CTAs split the samples.  N > 128: one CTA per 128 x 128 block of dGs and sample slice -- as few slices
-  // as still fill the device twice over (long K runs per CTA, one pass of vector reductions per CTA at the end)
   const int nblocks = p.nblk * p.nblk;
-  int grid = device_sm_count();
-  if (nblocks > 1) grid = (2 * grid + nblocks - 1) / nblocks;
-  if (grid > B) grid = B;
-  ScopedKernelTimer _t(KK_TC_OUTER, st, 4.0 * B * N * width * 2 + 4.0 * N * N);
-  kern<<<dim3(grid, nblocks), TO_THREADS, p.smem_bytes, st>>>(a, a_bs, bmat, coef, dG, p);
-  STC_LAUNCH_OK("tc_outer_kernel");
+  {
+    ScopedKernelTimer _t(KK_TC_OUTER, st, 4.0 * B * N * width * 2 + 4.0 * N * N);
+    kern<<<dim3(grid, nblocks), TO_THREADS, p.smem_bytes, st>>>(a, a_bs, bmat, coef, det ? det_ws : dG, p);
+    STC_LAUNCH_OK("tc_outer_kernel");
+  }
   *handled = true;
+  if (det) return launch_det_reduce(dG, det_ws, grid, (long long)N * N, (long long)N * N, st);
   return STC_OK;
 }
 
@@ -936,7 +963,8 @@ int try_launch_support_adj_tc(const float* G, int N, int B, int width, const flo
                               float* axpy_out, const float* a, int64_t a_bs, float coef, float* dG, cudaStream_t st,
                               bool* handled) {
   *handled = false;
-  if (tc_support_disabled() || B <= 0) return STC_OK;
+  // deterministic mode: the hop and the dGs product run as two launches (tc_outer's slot form)
+  if (tc_support_disabled() || B <= 0 || det_mode()) return STC_OK;
   if (N < 8 || N > TA_MAX_N || width % 4 != 0 || x_bs % 4 != 0 || a_bs % 4 != 0) return STC_OK;
   if (!aligned16s(x) || !aligned16s(ybar) || !aligned16s(a) || (axpy_out && !aligned16s(axpy_out))) return STC_OK;
   TcAdjPlan p;

@@ -284,6 +284,18 @@ __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_gr
 __device__ __forceinline__ void red_add_v4(float* p, float a, float b, float c, float d) {
   asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(p), "f"(a), "f"(b), "f"(c), "f"(d) : "memory");
 }
+// The end-of-kernel gradient output of one CTA: a vector reduction into the destination, or (DET, deterministic mode) a
+// plain store into the CTA's own partial slot, summed in slot order afterwards (launch_det_reduce).
+template <bool DET>
+__device__ __forceinline__ void grad_out_v4(float* p, float a, float b, float c, float d) {
+  if constexpr (DET) *reinterpret_cast<float4*>(p) = make_float4(a, b, c, d);
+  else red_add_v4(p, a, b, c, d);
+}
+template <bool DET>
+__device__ __forceinline__ void grad_out(float* p, float v) {
+  if constexpr (DET) *p = v;
+  else atomicAdd(p, v);
+}
 
 // ---- mbarrier --------------------------------------------------------------------------------------
 __device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {

@@ -770,6 +770,7 @@ class _PartitionedCell(torch.autograd.Function):
         stream = torch.cuda.current_stream().cuda_stream
         dHe = He.new_zeros(B, ne, C, h)          # halo rows carry no output gradient: they stay out of every dW
         dHe[:, :n] = dHn
+        _lib.sync_deterministic()   # the scratch holds the partial slots of the fixed-order reductions while it is on
         scratch = torch.empty(lib.stc_cell_bwd_scratch_bytes(dims) // 4, dtype=torch.float32, device=dev)
         lay = _lib.scratch_layout(dims)
         R = B * ne * C

@@ -55,8 +55,15 @@ class _XSideTerms(torch.autograd.Function):
                 piece.copy_(g.reshape(B, N, C * Din))
         dGs = torch.zeros(N, N, dtype=torch.float32, device=Xp.device)
         lib = _lib.load()
-        _lib.check(lib.stc_support_outer(N, B, Wp, Xp.data_ptr(), N * Wp, dYp.data_ptr(), 1.0, dGs.data_ptr(),
-                                         torch.cuda.current_stream().cuda_stream), "stc_support_outer")
+        stream = torch.cuda.current_stream().cuda_stream
+        if _lib.sync_deterministic():   # fixed-order form: per-slice partial slots in a workspace
+            ws = torch.empty(lib.stc_support_outer_workspace_bytes(N, B, Wp) // 4, dtype=torch.float32, device=Xp.device)
+            _lib.check(lib.stc_support_outer_ws(N, B, Wp, Xp.data_ptr(), N * Wp, dYp.data_ptr(), 1.0, dGs.data_ptr(),
+                                                ws.data_ptr() if ws.numel() else None, ws.numel() * 4, stream),
+                       "stc_support_outer_ws")
+        else:
+            _lib.check(lib.stc_support_outer(N, B, Wp, Xp.data_ptr(), N * Wp, dYp.data_ptr(), 1.0, dGs.data_ptr(), stream),
+                       "stc_support_outer")
         _lib.note_launches()
         return dGs, None
 

@@ -220,6 +220,7 @@ def support_apply_edge_grad(Gs: CsrSupport, X: torch.Tensor, A: torch.Tensor, dv
     if Y.shape != Xc.shape or not Y.is_contiguous():
         raise RuntimeError("support_apply_edge_grad: `out` must be a contiguous tensor of X's shape")
     zc = Z.contiguous() if Z is not None else None
+    _lib.sync_deterministic()   # the one-writer form of the edge gradient under torch.use_deterministic_algorithms
     common = (Gs.struct(), N, B, width, Xc.data_ptr(), N * width, zc.data_ptr() if zc is not None else None, N * width,
               Y.data_ptr(), float(alpha), float(beta), Ac.data_ptr(), a_bs, float(coef), dvals.data_ptr())
     stream = torch.cuda.current_stream().cuda_stream
