@@ -165,6 +165,30 @@ int stc_cell_bwd_x(const StcDims* d, const StcSupport* gs, const float* gc,
                    void* scratch, size_t scratch_bytes, const float* yx_terms, float* dyx_terms_out,
                    const float* dyx_fold, const float* yh_terms, float* dyh_terms_out, const float* dyh_fold,
                    void* stream);
+/* ---- forward-only calls (inference: no backward will follow) ----
+ * The same launches, in the same number and on the same side streams, as stc_cell_fwd_x / stc_cell_fwd_stage, and
+ * bitwise the same h_out, but on a smaller workspace `ws` that holds only what the forward itself reads back: u,
+ * r*H and its terms, the Xt- and H-side terms, the Gc terms and the wide-state weight images (same order and 256-byte
+ * alignment as `saved`).  r, c and the pre-mix partials P_1, which only the backward reads, are not stored.
+ *   stc_cell_fwd_only_bytes   size of `ws` (<= stc_cell_saved_bytes); a smaller ws_bytes returns STC_ERR_WORKSPACE.
+ *   stc_cell_fwd_only_layout  offsets in floats under the STC_SAVED_* indices; -1 for the absent regions
+ *                             (STC_SAVED_R, STC_SAVED_C, STC_SAVED_PG, STC_SAVED_PC).
+ *   stc_cell_fwd_only         stc_cell_fwd_x on `ws` (NULL yx_terms / yh_terms: the call computes that side's terms
+ *                             itself, as stc_cell_fwd does; the computed terms sit in regions STC_SAVED_YX / YH).
+ *   stc_cell_fwd_only_stage   stc_cell_fwd_stage on `ws` (the row-partitioned forward; the caller fills the
+ *                             spatial terms at the offsets of stc_cell_fwd_only_layout).
+ * A workspace filled by these calls cannot be handed to stc_cell_bwd. */
+size_t stc_cell_fwd_only_bytes(const StcDims* d);
+int stc_cell_fwd_only_layout(const StcDims* d, int64_t* offsets_floats, int32_t n_offsets);
+int stc_cell_fwd_only(const StcDims* d, const StcSupport* gs, const float* gc,
+                      const float* xt, int64_t xt_batch_stride, const float* h_prev,
+                      const float* Wg, const float* bg, const float* Wc, const float* bc,
+                      float* h_out, void* ws, size_t ws_bytes, const float* yx_terms, const float* yh_terms,
+                      void* stream);
+int stc_cell_fwd_only_stage(const StcDims* d, int32_t stage, const float* gc,
+                            const float* xt, int64_t xt_batch_stride, const float* h_prev,
+                            const float* Wg, const float* bg, const float* Wc, const float* bc,
+                            float* h_out, void* ws, size_t ws_bytes, void* stream);
 /* dGs[n][m] += coef * sum_{b,j} A[b][n][j] * Bm[b][m][j]  -- the gradient of the mode product Y = Gs^T X w.r.t. a dense
  * Gs [N][N] with A = X ([B][N][width], batch stride in elements) and Bm = dL/dY ([B][N][width] contiguous). */
 int stc_support_outer(int32_t N, int32_t B, int32_t width, const float* a, int64_t a_batch_stride, const float* b,

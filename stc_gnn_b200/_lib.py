@@ -27,6 +27,7 @@ EXPORTED = (
     "stc_pair_scores_csr_rows", "stc_pair_topk_workspace_bytes", "stc_pair_topk",
     "stc_pair_topk_rows_workspace_bytes", "stc_pair_topk_rows",
     "stc_deterministic_set", "stc_support_outer_workspace_bytes", "stc_support_outer_ws",
+    "stc_cell_fwd_only_bytes", "stc_cell_fwd_only_layout", "stc_cell_fwd_only", "stc_cell_fwd_only_stage",
 )
 STAGE_GATES, STAGE_CANDI = 0, 1
 SAVED_REGIONS = ("u", "r", "c", "Yr", "Yx", "Yh", "Q", "Pg", "Pc")
@@ -68,6 +69,12 @@ def load(build_if_missing: bool = True):
                                  c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]
     lib.stc_cell_fwd_x.restype = c_int
     lib.stc_cell_fwd_x.argtypes = lib.stc_cell_fwd.argtypes[:-1] + [c_void_p, c_void_p, c_void_p]
+    lib.stc_cell_fwd_only_bytes.restype = c_size_t
+    lib.stc_cell_fwd_only_bytes.argtypes = [POINTER(StcDims)]
+    lib.stc_cell_fwd_only_layout.restype = c_int
+    lib.stc_cell_fwd_only_layout.argtypes = [POINTER(StcDims), POINTER(c_int64), c_int32]
+    lib.stc_cell_fwd_only.restype = c_int
+    lib.stc_cell_fwd_only.argtypes = lib.stc_cell_fwd_x.argtypes
     lib.stc_support_outer.restype = c_int
     lib.stc_support_outer.argtypes = [c_int32, c_int32, c_int32, c_void_p, c_int64, c_void_p, c_float, c_void_p, c_void_p]
     lib.stc_support_outer_workspace_bytes.restype = c_size_t
@@ -107,6 +114,8 @@ def load(build_if_missing: bool = True):
     lib.stc_cell_fwd_stage.restype = c_int
     lib.stc_cell_fwd_stage.argtypes = [POINTER(StcDims), c_int32, c_void_p, c_void_p, c_int64, c_void_p, c_void_p,
                                        c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]
+    lib.stc_cell_fwd_only_stage.restype = c_int
+    lib.stc_cell_fwd_only_stage.argtypes = lib.stc_cell_fwd_stage.argtypes
     lib.stc_cell_bwd.restype = c_int
     lib.stc_cell_bwd.argtypes = [POINTER(StcDims), POINTER(StcSupport), c_void_p, c_void_p, c_int64, c_void_p,
                                  c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
@@ -148,11 +157,15 @@ def load(build_if_missing: bool = True):
     return lib
 
 
-def saved_layout(dims: StcDims) -> dict:
-    """{region name: offset in floats} of the `saved` buffer of one cell call."""
+def saved_layout(dims: StcDims, fwd_only: bool = False) -> dict:
+    """{region name: offset in floats} of the `saved` buffer of one cell call; with `fwd_only`, of the workspace of a
+    forward-only call (stc_cell_fwd_only_layout: -1 for the regions it does not have)."""
     lib = load()
     offs = (c_int64 * len(SAVED_REGIONS))()
-    check(lib.stc_cell_saved_layout(dims, offs, len(SAVED_REGIONS)), "stc_cell_saved_layout")
+    if fwd_only:
+        check(lib.stc_cell_fwd_only_layout(dims, offs, len(SAVED_REGIONS)), "stc_cell_fwd_only_layout")
+    else:
+        check(lib.stc_cell_saved_layout(dims, offs, len(SAVED_REGIONS)), "stc_cell_saved_layout")
     return {n: int(offs[i]) for i, n in enumerate(SAVED_REGIONS)}
 
 

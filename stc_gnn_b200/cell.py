@@ -8,6 +8,7 @@ libstc_b200.so per direction (include/stc_b200.h).  CUDA fp32 only -- anything e
 from __future__ import annotations
 
 import os
+from types import SimpleNamespace
 
 import torch
 from torch import nn
@@ -23,6 +24,12 @@ from .support import CsrSupport, dense_struct
 # `torch.autograd.grad(...)` w.r.t. these leaves needs the returned form: set STC_INPLACE_GRADS=0 or
 # `stc_gnn_b200.cell.INPLACE_LEAF_GRADS = False`.
 INPLACE_LEAF_GRADS = os.environ.get("STC_INPLACE_GRADS", "1") != "0"
+
+# A cell call that no gradient can be asked of (torch.no_grad / torch.inference_mode, or no tensor input requires grad)
+# runs the forward-only form (stc_cell_fwd_only): no autograd node, a workspace without the regions only the backward
+# reads (r, c, the P_1 partials), and bitwise the same output.  STC_FORWARD_ONLY=0 or
+# `stc_gnn_b200.cell.FORWARD_ONLY = False` keeps the training forward for such calls too (A/B runs).
+FORWARD_ONLY = os.environ.get("STC_FORWARD_ONLY", "1") != "0"
 
 _ACT_CODES = {None: _lib.ACT_NONE, nn.ReLU: _lib.ACT_RELU}
 _ACT_NAMES = {_lib.ACT_NONE: None, _lib.ACT_RELU: "relu"}
@@ -70,6 +77,23 @@ def _buffer_floats(lib, dims: _lib.StcDims, key):
     return hit
 
 
+def _fwd_only_floats(lib, dims: _lib.StcDims, key):
+    """Workspace size in floats of a forward-only cell call, cached per shape like _buffer_floats."""
+    key = ("fwd_only",) + key
+    hit = _SIZES.get(key)
+    if hit is None:
+        if len(_SIZES) > 256:
+            _SIZES.clear()
+        hit = _SIZES[key] = lib.stc_cell_fwd_only_bytes(dims) // 4
+    return hit
+
+
+def forward_only(*tensors) -> bool:
+    """True when a cell call over these tensor inputs takes the forward-only form: FORWARD_ONLY is on and autograd
+    cannot ask for a gradient (grad mode off, which includes inference mode, or no input requires grad)."""
+    return FORWARD_ONLY and not (torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in tensors))
+
+
 def _ptr(t):
     return t.data_ptr() if t is not None else None
 
@@ -77,17 +101,100 @@ def _ptr(t):
 _SAVED_OFFSETS = {}
 
 
-def _terms_view(saved, dims, key, side, shape):
-    """The spatial terms [Ks-1,B,N,C,w] a cell call computed for one side: a view of its `saved` buffer."""
-    offs = _SAVED_OFFSETS.get(key)
+def _terms_view(saved, dims, key, side, shape, fwd_only=False):
+    """The spatial terms [Ks-1,B,N,C,w] a cell call computed for one side: a view of its `saved` buffer (of its
+    forward-only workspace with `fwd_only`)."""
+    offs = _SAVED_OFFSETS.get((key, fwd_only))
     if offs is None:
         if len(_SAVED_OFFSETS) > 256:
             _SAVED_OFFSETS.clear()
-        offs = _SAVED_OFFSETS[key] = _lib.saved_layout(dims)
+        offs = _SAVED_OFFSETS[(key, fwd_only)] = _lib.saved_layout(dims, fwd_only)
     n = 1
     for s_ in shape:
         n *= s_
     return saved[offs["Yx" if side == "x" else "Yh"]:][:n].view(shape)
+
+
+def _run_forward(Gs, Gc, Xt, H, Wg, bg, Wc, bc, Yx, Ev, cfg, Yh, give, fwd_only):
+    """Argument checks and the forward launch of one cell step, shared by the training form (_CellFunction, which
+    fills `saved` for its backward) and the forward-only form (fwd_only: stc_cell_fwd_only on the smaller workspace).
+    Inputs as in _CellFunction; `give` the sides whose computed terms are returned.  Returns the contiguous operands the
+    launch read, the buffer it filled (`buf`), H' (`Hn`) and the given terms (`given`, views of `buf`)."""
+    lib = _lib.load()
+    Ks, Kc, act = cfg
+    B, N, C, Din = Xt.shape
+    h = H.shape[-1]
+    for name, t in (("Gc", Gc), ("Xt", Xt), ("Ht_1", H), ("gates.W", Wg), ("candi.W", Wc)):
+        if not t.is_cuda or t.dtype != torch.float32:
+            raise RuntimeError(f"STC_Cell (B200): {name} must be a float32 CUDA tensor, got {t.dtype} on {t.device}; "
+                               "there is no CPU fallback")
+    if H.shape != (B, N, C, h):
+        raise RuntimeError(f"Ht_1 shape {tuple(H.shape)} does not match Xt {tuple(Xt.shape)}")
+    rows = (Din + h) * Ks * Kc
+    if Wg.shape != (rows, 2 * h) or Wc.shape != (rows, h) or Gc.shape != (C, C):
+        raise RuntimeError(f"shape mismatch: gates.W {tuple(Wg.shape)} (want {(rows, 2 * h)}), candi.W "
+                           f"{tuple(Wc.shape)} (want {(rows, h)}), Gc {tuple(Gc.shape)} (want {(C, C)})")
+    for name, b_, n_ in (("gates.b", bg, 2 * h), ("candi.b", bc, h)):
+        if b_ is not None and (b_.shape != (n_,) or not b_.is_cuda or b_.dtype != torch.float32):
+            raise RuntimeError(f"{name} must be a float32 CUDA tensor of shape ({n_},)")
+    if (bg is None) != (bc is None):
+        raise RuntimeError("gates.b and candi.b must both be present or both absent")
+    csr = isinstance(Gs, CsrSupport)
+    gs_keep = None
+    if csr:
+        if Gs.N != N:
+            raise RuntimeError(f"CSR support has {Gs.N} nodes, Xt has {N}")
+        if Ev is not None and Ev is not Gs.vals:
+            raise RuntimeError("edge values passed to the cell must be the CsrSupport's own `vals`")
+        if Gs.learnable:   # the values may have changed since the last step (optimizer update, new with_values)
+            Gs.sync_t_vals()
+        gs_struct = Gs.struct()
+    else:
+        if not Gs.is_cuda or Gs.dtype != torch.float32 or Gs.shape != (N, N):
+            raise RuntimeError(f"Gs must be a float32 CUDA [N,N] tensor or a CsrSupport, got {tuple(Gs.shape)} {Gs.dtype}")
+        gs_keep = Gs.contiguous()
+        gs_struct = dense_struct(gs_keep)
+    Gc_c, H_c, Wg_c, Wc_c = Gc.contiguous(), H.contiguous(), Wg.contiguous(), Wc.contiguous()
+    bg_c = bg.contiguous() if bg is not None else None
+    bc_c = bc.contiguous() if bc is not None else None
+    # the encoder's [:, t] view keeps each sample's [N,C,Din] slab contiguous: pass the batch stride
+    Xt_c = Xt if (B == 0 or Xt[0].is_contiguous()) else Xt.contiguous()
+    xbs = Xt_c.stride(0) if B > 1 else N * C * Din
+    dims = _dims(B, N, C, Din, h, Ks, Kc, act, bg is not None)
+    size_key = (B, N, C, Din, h, Ks, Kc, act, bg is not None)
+    floats = _fwd_only_floats(lib, dims, size_key) if fwd_only else _buffer_floats(lib, dims, size_key)[0]
+    buf = torch.empty(floats, dtype=torch.float32, device=Xt.device)
+    Hn = torch.empty((B, N, C, h), dtype=torch.float32, device=Xt.device)
+    stream = torch.cuda.current_stream().cuda_stream
+
+    def supplied(Y, w, what):
+        if Y is None or Ks <= 1:
+            return None
+        if Y.shape != (Ks - 1, B, N, C, w) or not Y.is_cuda or Y.dtype != torch.float32:
+            raise RuntimeError(f"supplied {what} terms must be a float32 CUDA tensor of shape {(Ks - 1, B, N, C, w)}, "
+                               f"got {tuple(Y.shape)}")
+        return Y.contiguous()
+
+    Yx_c, Yh_c = supplied(Yx, Din, "Xt-side"), supplied(Yh, h, "H-side")
+    for side in give:
+        if side not in ("x", "h") or Ks <= 1 or (Yx_c if side == "x" else Yh_c) is not None:
+            raise RuntimeError(f"a cell can only give terms of a side it computes itself (give={give!r}, Ks={Ks})")
+    args = (dims, gs_struct, Gc_c.data_ptr(), Xt_c.data_ptr(), xbs, H_c.data_ptr(), Wg_c.data_ptr(), _ptr(bg_c),
+            Wc_c.data_ptr(), _ptr(bc_c), Hn.data_ptr(), buf.data_ptr(), buf.numel() * 4)
+    if B == 0:
+        status = 0
+    elif fwd_only:
+        status = lib.stc_cell_fwd_only(*args, _ptr(Yx_c), _ptr(Yh_c), stream)
+    elif Yx_c is not None or Yh_c is not None:
+        status = lib.stc_cell_fwd_x(*args, _ptr(Yx_c), _ptr(Yh_c), stream)
+    else:
+        status = lib.stc_cell_fwd(*args, stream)
+    _lib.check(status, "stc_cell_fwd_only" if fwd_only else "stc_cell_fwd")
+    _lib.note_launches()
+    given = tuple(_terms_view(buf, dims, size_key, side, (Ks - 1, B, N, C, Din if side == "x" else h), fwd_only)
+                  for side in give)
+    return SimpleNamespace(Hn=Hn, buf=buf, given=given, Gs=gs_keep, Gc=Gc_c, Xt=Xt_c, H=H_c, Wg=Wg_c, Wc=Wc_c, Yx=Yx_c,
+                           Yh=Yh_c, xbs=xbs, csr=csr, size_key=size_key, dims_tuple=(B, N, C, Din, h))
 
 
 class _CellFunction(torch.autograd.Function):
@@ -106,95 +213,27 @@ class _CellFunction(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, Gs, Gc, Xt, H, Wg, bg, Wc, bc, Yx, Ev, cfg, Yh=None, share=None):
-        lib = _lib.load()
-        Ks, Kc, act = cfg
-        B, N, C, Din = Xt.shape
-        h = H.shape[-1]
-        for name, t in (("Gc", Gc), ("Xt", Xt), ("Ht_1", H), ("gates.W", Wg), ("candi.W", Wc)):
-            if not t.is_cuda or t.dtype != torch.float32:
-                raise RuntimeError(f"STC_Cell (B200): {name} must be a float32 CUDA tensor, got {t.dtype} on {t.device}; "
-                                   "there is no CPU fallback")
-        if H.shape != (B, N, C, h):
-            raise RuntimeError(f"Ht_1 shape {tuple(H.shape)} does not match Xt {tuple(Xt.shape)}")
-        rows = (Din + h) * Ks * Kc
-        if Wg.shape != (rows, 2 * h) or Wc.shape != (rows, h) or Gc.shape != (C, C):
-            raise RuntimeError(f"shape mismatch: gates.W {tuple(Wg.shape)} (want {(rows, 2 * h)}), candi.W "
-                               f"{tuple(Wc.shape)} (want {(rows, h)}), Gc {tuple(Gc.shape)} (want {(C, C)})")
-        for name, b_, n_ in (("gates.b", bg, 2 * h), ("candi.b", bc, h)):
-            if b_ is not None and (b_.shape != (n_,) or not b_.is_cuda or b_.dtype != torch.float32):
-                raise RuntimeError(f"{name} must be a float32 CUDA tensor of shape ({n_},)")
-        if (bg is None) != (bc is None):
-            raise RuntimeError("gates.b and candi.b must both be present or both absent")
-        csr = isinstance(Gs, CsrSupport)
-        if csr:
-            if Gs.N != N:
-                raise RuntimeError(f"CSR support has {Gs.N} nodes, Xt has {N}")
-            if Ev is not None and Ev is not Gs.vals:
-                raise RuntimeError("edge values passed to the cell must be the CsrSupport's own `vals`")
-            if Gs.learnable:   # the values may have changed since the last step (optimizer update, new with_values)
-                Gs.sync_t_vals()
-            gs_struct = Gs.struct()
-        else:
-            if not Gs.is_cuda or Gs.dtype != torch.float32 or Gs.shape != (N, N):
-                raise RuntimeError(f"Gs must be a float32 CUDA [N,N] tensor or a CsrSupport, got {tuple(Gs.shape)} {Gs.dtype}")
-            gs_keep = Gs.contiguous()
-            gs_struct = dense_struct(gs_keep)
-        Gc_c, H_c, Wg_c, Wc_c = Gc.contiguous(), H.contiguous(), Wg.contiguous(), Wc.contiguous()
-        bg_c = bg.contiguous() if bg is not None else None
-        bc_c = bc.contiguous() if bc is not None else None
-        # the encoder's [:, t] view keeps each sample's [N,C,Din] slab contiguous: pass the batch stride
-        Xt_c = Xt if (B == 0 or Xt[0].is_contiguous()) else Xt.contiguous()
-        xbs = Xt_c.stride(0) if B > 1 else N * C * Din
-        dims = _dims(B, N, C, Din, h, Ks, Kc, act, bg is not None)
-        ctx.size_key = (B, N, C, Din, h, Ks, Kc, act, bg is not None)
-        saved = torch.empty(_buffer_floats(lib, dims, ctx.size_key)[0], dtype=torch.float32, device=Xt.device)
-        Hn = torch.empty((B, N, C, h), dtype=torch.float32, device=Xt.device)
-        stream = torch.cuda.current_stream().cuda_stream
         give, yx_shared = share if share is not None else ((), False)
-
-        def supplied(Y, w, what):
-            if Y is None or Ks <= 1:
-                return None
-            if Y.shape != (Ks - 1, B, N, C, w) or not Y.is_cuda or Y.dtype != torch.float32:
-                raise RuntimeError(f"supplied {what} terms must be a float32 CUDA tensor of shape {(Ks - 1, B, N, C, w)}, "
-                                   f"got {tuple(Y.shape)}")
-            return Y.contiguous()
-
-        Yx_c, Yh_c = supplied(Yx, Din, "Xt-side"), supplied(Yh, h, "H-side")
-        for side in give:
-            if side not in ("x", "h") or Ks <= 1 or (Yx_c if side == "x" else Yh_c) is not None:
-                raise RuntimeError(f"a cell can only give terms of a side it computes itself (give={give!r}, Ks={Ks})")
-        if B == 0:
-            status = 0
-        elif Yx_c is not None or Yh_c is not None:
-            status = lib.stc_cell_fwd_x(dims, gs_struct, Gc_c.data_ptr(), Xt_c.data_ptr(), xbs, H_c.data_ptr(),
-                                        Wg_c.data_ptr(), _ptr(bg_c), Wc_c.data_ptr(), _ptr(bc_c), Hn.data_ptr(),
-                                        saved.data_ptr(), saved.numel() * 4, _ptr(Yx_c), _ptr(Yh_c), stream)
-        else:
-            status = lib.stc_cell_fwd(dims, gs_struct, Gc_c.data_ptr(), Xt_c.data_ptr(), xbs, H_c.data_ptr(),
-                                      Wg_c.data_ptr(), _ptr(bg_c), Wc_c.data_ptr(), _ptr(bc_c), Hn.data_ptr(),
-                                      saved.data_ptr(), saved.numel() * 4, stream)
-        _lib.check(status, "stc_cell_fwd")
-        _lib.note_launches()
-        ctx.hoisted, ctx.h_given, ctx.yx_shared, ctx.give = Yx_c is not None, Yh_c is not None, bool(yx_shared), tuple(give)
-        ctx.cfg, ctx.dims_tuple, ctx.xbs, ctx.csr = cfg, (B, N, C, Din, h), xbs, csr
-        ctx.gs_obj = Gs if csr else None
+        f = _run_forward(Gs, Gc, Xt, H, Wg, bg, Wc, bc, Yx, Ev, cfg, Yh, give, fwd_only=False)
+        ctx.size_key = f.size_key
+        ctx.hoisted, ctx.h_given, ctx.yx_shared, ctx.give = f.Yx is not None, f.Yh is not None, bool(yx_shared), tuple(give)
+        ctx.cfg, ctx.dims_tuple, ctx.xbs, ctx.csr = cfg, f.dims_tuple, f.xbs, f.csr
+        ctx.gs_obj = Gs if f.csr else None
         ctx.has_bias = bg is not None
         # leaves whose gradient the backward adds into `.grad` directly (index = position among forward's inputs)
         ctx.sinks = {}
         if INPLACE_LEAF_GRADS:
-            for i, t in ((0, None if csr else Gs), (1, Gc), (4, Wg), (5, bg), (6, Wc), (7, bc), (9, Ev)):
+            for i, t in ((0, None if f.csr else Gs), (1, Gc), (4, Wg), (5, bg), (6, Wc), (7, bc), (9, Ev)):
                 if t is not None and ctx.needs_input_grad[i] and t.is_leaf and t.is_contiguous():
                     ctx.sinks[i] = t
         ctx.has_ev = Ev is not None
-        ctx.save_for_backward(*( [] if csr else [gs_keep] ), Gc_c, Xt_c, H_c, Wg_c, Wc_c, saved,
-                              *([Yx_c] if Yx_c is not None else []), *([Yh_c] if Yh_c is not None else []),
+        ctx.save_for_backward(*( [] if f.csr else [f.Gs] ), f.Gc, f.Xt, f.H, f.Wg, f.Wc, f.buf,
+                              *([f.Yx] if f.Yx is not None else []), *([f.Yh] if f.Yh is not None else []),
                               *([Ev] if Ev is not None else []))
         if not give:
-            return Hn
+            return f.Hn
         ctx.set_materialize_grads(False)   # no gradient for given terms: nothing to fold (rather than a zero tensor)
-        return (Hn,) + tuple(_terms_view(saved, dims, ctx.size_key, side, (Ks - 1, B, N, C, Din if side == "x" else h))
-                             for side in give)
+        return (f.Hn,) + f.given
 
     @staticmethod
     @torch.autograd.function.once_differentiable
@@ -276,10 +315,20 @@ class _CellFunction(torch.autograd.Function):
         return tuple(returned[:n_in])
 
 
+def _cell(Gs, Gc, Xt, H, Wg, bg, Wc, bc, Yx, Ev, cfg, Yh=None, share=None):
+    """One cell step (inputs as in _CellFunction): the training form when autograd may ask for a gradient, else the
+    forward-only form (see FORWARD_ONLY), which returns the same values without an autograd node."""
+    if not forward_only(Gs if isinstance(Gs, torch.Tensor) else None, Gc, Xt, H, Wg, bg, Wc, bc, Yx, Ev, Yh):
+        extra = () if Yh is None and share is None else (Yh, share)
+        return _CellFunction.apply(Gs, Gc, Xt, H, Wg, bg, Wc, bc, Yx, Ev, cfg, *extra)
+    give = share[0] if share is not None else ()
+    f = _run_forward(Gs, Gc, Xt, H, Wg, bg, Wc, bc, Yx, Ev, cfg, Yh, give, fwd_only=True)
+    return (f.Hn,) + f.given if give else f.Hn
+
+
 def stc_cell_forward(Gs, Gc, Xt, Ht_1, Wg, bg, Wc, bc, Ks: int, Kc: int, activation=None) -> torch.Tensor:
     """Functional form of the cell: H' = STC_Cell(Gs, Gc, Xt, Ht_1) with explicit weights (differentiable)."""
-    return _CellFunction.apply(Gs, Gc, Xt, Ht_1, Wg, bg, Wc, bc, None, _edge_values(Gs),
-                               (int(Ks), int(Kc), _activation_code(activation)))
+    return _cell(Gs, Gc, Xt, Ht_1, Wg, bg, Wc, bc, None, _edge_values(Gs), (int(Ks), int(Kc), _activation_code(activation)))
 
 
 def _edge_values(Gs):
@@ -314,9 +363,9 @@ class STC_Cell(nn.Module):
     def _shared_step(self, Gs, Gc, Xt, Ht_1, Yx=None, Yh=None, give=(), yx_shared=False):
         """One step of RecurrentStack with spatial terms shared between the two cells that read a hidden state
         (dense or CSR Gs): see _CellFunction.  Returns H' or, with `give`, (H', the terms of each side given)."""
-        return _CellFunction.apply(Gs, Gc, Xt, Ht_1, self.gates.W, getattr(self.gates, "b", None), self.candi.W,
-                                   getattr(self.candi, "b", None), Yx, _edge_values(Gs), (self.Ks, self.Kc, self._act),
-                                   Yh, (give, yx_shared))
+        return _cell(Gs, Gc, Xt, Ht_1, self.gates.W, getattr(self.gates, "b", None), self.candi.W,
+                     getattr(self.candi, "b", None), Yx, _edge_values(Gs), (self.Ks, self.Kc, self._act), Yh,
+                     (give, yx_shared))
 
     def forward(self, Gs, Gc: torch.Tensor, Xt: torch.Tensor, Ht_1: torch.Tensor, _Yx: torch.Tensor = None):
         """`_Yx` (not part of the reference's signature): the spatial terms of Xt, [Ks-1,B,N,C,Din], when the caller
@@ -331,8 +380,8 @@ class STC_Cell(nn.Module):
             return partitioned_cell_forward(Gs, Gc, Xt, Ht_1, self.gates.W, getattr(self.gates, "b", None), self.candi.W,
                                             getattr(self.candi, "b", None), self.Ks, self.Kc, _ACT_NAMES[self._act],
                                             reduce_params=getattr(Gs, "reduce_per_cell", True))
-        return _CellFunction.apply(Gs, Gc, Xt, Ht_1, self.gates.W, getattr(self.gates, "b", None), self.candi.W,
-                                   getattr(self.candi, "b", None), _Yx, _edge_values(Gs), (self.Ks, self.Kc, self._act))
+        return _cell(Gs, Gc, Xt, Ht_1, self.gates.W, getattr(self.gates, "b", None), self.candi.W,
+                     getattr(self.candi, "b", None), _Yx, _edge_values(Gs), (self.Ks, self.Kc, self._act))
 
 
 _CSR_CACHE = {}

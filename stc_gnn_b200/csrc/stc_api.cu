@@ -212,24 +212,25 @@ bool det_mode() { return g_det.load(std::memory_order_relaxed) != 0; }
 // every dW / dx kernel with a fixed-order form runs at most two CTAs per SM
 int det_conv_slots() { return 2 * device_sm_count(); }
 
-WsLayout make_layout(const StcDims& d) {
+WsLayout make_layout(const StcDims& d, bool fwd_only) {
   WsLayout w;
   const size_t A = 64;  // 256-byte alignment of every region
   w.R = (size_t)d.B * d.N * d.C;
   const size_t Rh = w.R * d.h, Rx = w.R * d.Din;
   const size_t km1 = d.Ks > 1 ? (size_t)(d.Ks - 1) : 0;
+  const size_t bwd = fwd_only ? 0 : 1;   // regions only the backward reads
   size_t o = 0;
   auto take = [&](size_t n) { size_t at = o; o = round_up(o + n, A); return at; };
   w.u = take(Rh);
-  w.r = take(Rh);
-  w.c = take(Rh);
+  w.r = take(bwd * Rh);
+  w.c = take(bwd * Rh);
   w.Yr = take((size_t)d.Ks * Rh);   // Yr[0] = r*H, then its spatial terms
   w.Yx = take(km1 * Rx);
   w.Yh = take(km1 * Rh);
   w.Q = take((size_t)d.Kc * d.C * d.C);
   const size_t kcm1 = d.Kc > 1 ? (size_t)(d.Kc - 1) : 0;
-  w.Pg = take(w.R * kcm1 * 2 * d.h);
-  w.Pc = take(w.R * kcm1 * d.h);
+  w.Pg = take(bwd * w.R * kcm1 * 2 * d.h);
+  w.Pc = take(bwd * w.R * kcm1 * d.h);
   {  // weight images of the wide-hidden-state forward: only for shapes the SF-class tensor-core kernels do not take
     ConvArgs t;
     memset(&t, 0, sizeof(t));
@@ -476,6 +477,7 @@ struct FwdCtx {
   Lanes* lanes = nullptr;   // set by stc_cell_fwd: the Xt-side terms and the Gc terms may run beside the H-side terms
   const float* yx_pre = nullptr;   // caller-supplied spatial terms of Xt ([Ks-1][B][N][C][Din]): skip the Xt-side hops
   const float* yh_pre = nullptr;   // caller-supplied spatial terms of H ([Ks-1][B][N][C][h]): skip the H-side hops
+  bool fwd_only = false;   // `ws` has the forward-only layout: r, c and the P_1 partials (backward-only) are not stored
 };
 
 // spatial Chebyshev terms of Xt and H:  Y_1 = Gs^T Y_0,  Y_k = 2 Gs^T Y_{k-1} - Y_{k-2}
@@ -525,9 +527,9 @@ static int fwd_gates(const FwdCtx& f, const float* Wg, const float* bg) {
   a.bias = d.has_bias ? bg : nullptr;
   a.Hprev = f.h_prev;
   a.u = ws + w.u;
-  a.r = ws + w.r;
+  a.r = f.fwd_only ? nullptr : ws + w.r;
   a.rH = ws + w.Yr;
-  a.Psave = ws + w.Pg;
+  a.Psave = f.fwd_only ? nullptr : ws + w.Pg;
   a.Wimg = (w.Wimg_c > w.Wimg_g) ? ws + w.Wimg_g : nullptr;   // region is empty when the shape is not eligible
   return launch_conv_fwd(a, f.st);
 }
@@ -563,16 +565,16 @@ static int fwd_candi(const FwdCtx& f, const float* Wc, const float* bc, float* h
   a.bias = d.has_bias ? bc : nullptr;
   a.Hprev = f.h_prev;
   a.u = ws + w.u;
-  a.c = ws + w.c;
+  a.c = f.fwd_only ? nullptr : ws + w.c;
   a.Hnew = h_out;
-  a.Psave = ws + w.Pc;
+  a.Psave = f.fwd_only ? nullptr : ws + w.Pc;
   a.Wimg = (w.saved_total > w.Wimg_c) ? ws + w.Wimg_c : nullptr;
   return launch_conv_fwd(a, f.st);
 }
 
 static int check_fwd_args(const StcDims* dp, const float* gc, const float* xt, const float* h_prev, const float* Wg,
                           const float* bg, const float* Wc, const float* bc, float* h_out, void* wsv, size_t ws_bytes,
-                          const char* who) {
+                          const char* who, bool fwd_only = false) {
   STC_TRY(check_dims(dp));
   if (!gc || !xt || !h_prev || !Wg || !Wc || !h_out || !wsv) {
     set_error("%s: NULL argument", who);
@@ -582,9 +584,13 @@ static int check_fwd_args(const StcDims* dp, const float* gc, const float* xt, c
     set_error("%s: has_bias set but bias pointer is NULL", who);
     return STC_ERR_BAD_ARG;
   }
-  const WsLayout w = make_layout(*dp);
+  const WsLayout w = make_layout(*dp, fwd_only);
   if (ws_bytes < w.saved_total * sizeof(float)) {
-    set_error("saved buffer too small: %zu < %zu bytes", ws_bytes, w.saved_total * sizeof(float));
+    if (fwd_only)
+      set_error("%s: workspace too small (STC_ERR_WORKSPACE): %zu < %zu bytes (stc_cell_fwd_only_bytes)", who, ws_bytes,
+                w.saved_total * sizeof(float));
+    else
+      set_error("saved buffer too small: %zu < %zu bytes", ws_bytes, w.saved_total * sizeof(float));
     return STC_ERR_WORKSPACE;
   }
   return STC_OK;
@@ -593,9 +599,9 @@ static int check_fwd_args(const StcDims* dp, const float* gc, const float* xt, c
 static int cell_fwd_impl(const StcDims* dp, const StcSupport* gs, const float* gc, const float* xt,
                          int64_t xt_batch_stride, const float* h_prev, const float* Wg, const float* bg, const float* Wc,
                          const float* bc, float* h_out, void* wsv, size_t ws_bytes, const float* yx_terms,
-                         const float* yh_terms, void* stream, const char* who) {
+                         const float* yh_terms, void* stream, const char* who, bool fwd_only = false) {
   reset_launch_count();
-  STC_TRY(check_fwd_args(dp, gc, xt, h_prev, Wg, bg, Wc, bc, h_out, wsv, ws_bytes, who));
+  STC_TRY(check_fwd_args(dp, gc, xt, h_prev, Wg, bg, Wc, bc, h_out, wsv, ws_bytes, who, fwd_only));
   if (!gs) {
     set_error("%s: NULL support", who);
     return STC_ERR_BAD_ARG;
@@ -603,10 +609,11 @@ static int cell_fwd_impl(const StcDims* dp, const StcSupport* gs, const float* g
   const StcDims& d = *dp;
   if (d.B == 0) return STC_OK;
   STC_TRY(check_arch());
-  const WsLayout w = make_layout(d);
+  const WsLayout w = make_layout(d, fwd_only);
   Lanes lanes((cudaStream_t)stream, d);
   FwdCtx f{d, w, gs, gc, xt, xt_batch_stride, h_prev, (float*)wsv, (cudaStream_t)stream};
   f.lanes = &lanes;
+  f.fwd_only = fwd_only;
   f.yx_pre = d.Ks > 1 ? yx_terms : nullptr;
   f.yh_pre = d.Ks > 1 ? yh_terms : nullptr;
   STC_TRY(fwd_terms_xh(f));
@@ -643,21 +650,64 @@ int stc_cell_saved_layout(const StcDims* dp, int64_t* offsets, int32_t n_offsets
   return STC_OK;
 }
 
-int stc_cell_fwd_stage(const StcDims* dp, int32_t stage, const float* gc, const float* xt, int64_t xt_batch_stride,
-                       const float* h_prev, const float* Wg, const float* bg, const float* Wc, const float* bc,
-                       float* h_out, void* wsv, size_t ws_bytes, void* stream) {
+static int cell_fwd_stage_impl(const StcDims* dp, int32_t stage, const float* gc, const float* xt,
+                               int64_t xt_batch_stride, const float* h_prev, const float* Wg, const float* bg,
+                               const float* Wc, const float* bc, float* h_out, void* wsv, size_t ws_bytes, void* stream,
+                               const char* who, bool fwd_only) {
   reset_launch_count();
-  STC_TRY(check_fwd_args(dp, gc, xt, h_prev, Wg, bg, Wc, bc, h_out, wsv, ws_bytes, "stc_cell_fwd_stage"));
+  STC_TRY(check_fwd_args(dp, gc, xt, h_prev, Wg, bg, Wc, bc, h_out, wsv, ws_bytes, who, fwd_only));
   if (stage != STC_STAGE_GATES && stage != STC_STAGE_CANDI) {
-    set_error("stc_cell_fwd_stage: bad stage %d", stage);
+    set_error("%s: bad stage %d", who, stage);
     return STC_ERR_BAD_ARG;
   }
   const StcDims& d = *dp;
   if (d.B == 0) return STC_OK;
   STC_TRY(check_arch());
-  const WsLayout w = make_layout(d);
-  const FwdCtx f{d, w, nullptr, gc, xt, xt_batch_stride, h_prev, (float*)wsv, (cudaStream_t)stream};
+  const WsLayout w = make_layout(d, fwd_only);
+  FwdCtx f{d, w, nullptr, gc, xt, xt_batch_stride, h_prev, (float*)wsv, (cudaStream_t)stream};
+  f.fwd_only = fwd_only;
   return stage == STC_STAGE_GATES ? fwd_gates(f, Wg, bg) : fwd_candi(f, Wc, bc, h_out);
+}
+
+int stc_cell_fwd_stage(const StcDims* dp, int32_t stage, const float* gc, const float* xt, int64_t xt_batch_stride,
+                       const float* h_prev, const float* Wg, const float* bg, const float* Wc, const float* bc,
+                       float* h_out, void* wsv, size_t ws_bytes, void* stream) {
+  return cell_fwd_stage_impl(dp, stage, gc, xt, xt_batch_stride, h_prev, Wg, bg, Wc, bc, h_out, wsv, ws_bytes, stream,
+                             "stc_cell_fwd_stage", false);
+}
+
+// ---- forward-only calls: the same launches on the smaller workspace of make_layout(d, true) ----
+size_t stc_cell_fwd_only_bytes(const StcDims* d) {
+  if (check_dims(d) != STC_OK) return 0;
+  return make_layout(*d, true).saved_total * sizeof(float);
+}
+
+int stc_cell_fwd_only_layout(const StcDims* dp, int64_t* offsets, int32_t n_offsets) {
+  STC_TRY(check_dims(dp));
+  if (!offsets || n_offsets < STC_SAVED_REGIONS) {
+    set_error("stc_cell_fwd_only_layout: need room for %d offsets", (int)STC_SAVED_REGIONS);
+    return STC_ERR_BAD_ARG;
+  }
+  const WsLayout w = make_layout(*dp, true);
+  const int64_t v[STC_SAVED_REGIONS] = {(int64_t)w.u, -1, -1, (int64_t)w.Yr, (int64_t)w.Yx, (int64_t)w.Yh,
+                                        (int64_t)w.Q, -1, -1};
+  for (int i = 0; i < STC_SAVED_REGIONS; ++i) offsets[i] = v[i];
+  return STC_OK;
+}
+
+int stc_cell_fwd_only(const StcDims* dp, const StcSupport* gs, const float* gc, const float* xt,
+                      int64_t xt_batch_stride, const float* h_prev, const float* Wg, const float* bg, const float* Wc,
+                      const float* bc, float* h_out, void* wsv, size_t ws_bytes, const float* yx_terms,
+                      const float* yh_terms, void* stream) {
+  return cell_fwd_impl(dp, gs, gc, xt, xt_batch_stride, h_prev, Wg, bg, Wc, bc, h_out, wsv, ws_bytes, yx_terms, yh_terms,
+                       stream, "stc_cell_fwd_only", true);
+}
+
+int stc_cell_fwd_only_stage(const StcDims* dp, int32_t stage, const float* gc, const float* xt, int64_t xt_batch_stride,
+                            const float* h_prev, const float* Wg, const float* bg, const float* Wc, const float* bc,
+                            float* h_out, void* wsv, size_t ws_bytes, void* stream) {
+  return cell_fwd_stage_impl(dp, stage, gc, xt, xt_batch_stride, h_prev, Wg, bg, Wc, bc, h_out, wsv, ws_bytes, stream,
+                             "stc_cell_fwd_only_stage", true);
 }
 
 // reverse of the feature-side recurrence Y_k = 2 A^T Y_{k-1} - Y_{k-2} (Y_1 = A^T Y_0) for one operand:

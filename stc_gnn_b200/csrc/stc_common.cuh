@@ -103,7 +103,9 @@ struct WsLayout {
   size_t det_dw, det_dx, det_dgs;
   size_t scratch_total;
 };
-WsLayout make_layout(const StcDims& d);
+// fwd_only: the forward-only workspace (stc_cell_fwd_only): r, c, Pg and Pc are empty, every other region is laid out
+// in the same order; the scratch part is unchanged
+WsLayout make_layout(const StcDims& d, bool fwd_only = false);
 
 // ---- launchers implemented in the kernel TUs -----------------------------------------------------
 int launch_support_apply(const StcSupport& gs, int N, int B, int width, bool transpose, const float* x,
@@ -213,6 +215,12 @@ struct ConvArgs {
   long long* trace;    // [trace_tiles][TRACE_SLOTS] clock64 stamps of CTA 0's first tiles, or null
   int trace_tiles;
 };
+// compulsory state traffic per row of a forward convolution beside its Ks spatial terms, in floats (the timers'
+// algorithmic bytes): gates write u, r*H and r; the candidate reads u and H, writes H' and c.  A forward-only call
+// (r / c null) stores neither r nor c.
+static inline int conv_fwd_state_floats(const ConvArgs& a) {
+  return a.phase == 0 ? (a.r ? 3 : 2) * a.h : (a.c ? 4 : 3) * a.h;
+}
 enum { OPT_L2_PREFETCH = 1, OPT_GENERIC_EPILOGUE = 4 /* diagnostic: force the general epilogues */,
        OPT_SMEM_A = 8 /* diagnostic: convolutions with the A operand staged in shared memory */,
        OPT_WIDE_DX_FFMA = 32 /* diagnostic: wide-state backward dx on the general path */ };

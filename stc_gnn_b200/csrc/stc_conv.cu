@@ -41,6 +41,48 @@ __device__ __forceinline__ void tile_gemm(float (&acc)[NI][4][4], const float* _
 // =================================================================================================
 // forward: out = sum_{k,c} F_{k,c} W_{k,c} + b ; gates: u,r = sigmoid, rH = r*H ; candi: c = tanh, H' blend
 // =================================================================================================
+// forward epilogue: bias, activation and the GRU non-linearities of the accumulator items this thread owns
+template <int NI, bool SAVE>
+__device__ __forceinline__ void conv_fwd_epilogue(const ConvArgs& a, const float (&acc)[NI][4][4], long long row0,
+                                                  int rows_valid, int items, int CG) {
+  const int Hout = a.Hout, h = a.h;
+#pragma unroll
+  for (int i = 0; i < NI; ++i) {
+    const int it = threadIdx.x + i * CV_THREADS;
+    if (it >= items) break;
+    const int rg = it / CG, cg = it - rg * CG;
+#pragma unroll
+    for (int x = 0; x < 4; ++x) {
+      const int row = rg * 4 + x;
+      if (row >= rows_valid) continue;
+      const long long gr = row0 + row;
+#pragma unroll
+      for (int y = 0; y < 4; ++y) {
+        const int col = cg * 4 + y;
+        if (col >= Hout) continue;
+        float pre = acc[i][x][y] + (a.bias ? a.bias[col] : 0.f);
+        if (a.act == STC_ACT_RELU) pre = fmaxf(pre, 0.f);
+        if (a.phase == 0) {
+          float s = sigmoidf_acc(pre);
+          if (col < h) {
+            a.u[gr * h + col] = s;
+          } else {
+            const long long o = gr * h + (col - h);
+            if (SAVE) a.r[o] = s;
+            a.rH[o] = s * a.Hprev[o];
+          }
+        } else {
+          const long long o = gr * h + col;
+          float cc = tanhf(pre);
+          float uu = a.u[o], hp = a.Hprev[o];
+          if (SAVE) a.c[o] = cc;
+          a.Hnew[o] = fmaf(uu, cc - hp, hp);  // (1-u)*H + u*c
+        }
+      }
+    }
+  }
+}
+
 template <int NI>
 __global__ void __launch_bounds__(CV_THREADS)
 conv_fwd_kernel(const ConvArgs a, const ConvTile t) {
@@ -89,44 +131,12 @@ conv_fwd_kernel(const ConvArgs a, const ConvTile t) {
     }
   }
 
-  // epilogue
-  const long long row0 = g0 * C;
-  const int items = RG * CG;
-#pragma unroll
-  for (int i = 0; i < NI; ++i) {
-    const int it = threadIdx.x + i * CV_THREADS;
-    if (it >= items) break;
-    const int rg = it / CG, cg = it - rg * CG;
-#pragma unroll
-    for (int x = 0; x < 4; ++x) {
-      const int row = rg * 4 + x;
-      if (row >= rows_valid) continue;
-      const long long gr = row0 + row;
-#pragma unroll
-      for (int y = 0; y < 4; ++y) {
-        const int col = cg * 4 + y;
-        if (col >= Hout) continue;
-        float pre = acc[i][x][y] + (a.bias ? a.bias[col] : 0.f);
-        if (a.act == STC_ACT_RELU) pre = fmaxf(pre, 0.f);
-        if (a.phase == 0) {
-          float s = sigmoidf_acc(pre);
-          if (col < h) {
-            a.u[gr * h + col] = s;
-          } else {
-            const long long o = gr * h + (col - h);
-            a.r[o] = s;
-            a.rH[o] = s * a.Hprev[o];
-          }
-        } else {
-          const long long o = gr * h + col;
-          float cc = tanhf(pre);
-          float uu = a.u[o], hp = a.Hprev[o];
-          a.c[o] = cc;
-          a.Hnew[o] = fmaf(uu, cc - hp, hp);  // (1-u)*H + u*c
-        }
-      }
-    }
-  }
+  // SAVE = false (a forward-only call, r / c null): only the backward reads r and c.  The test is taken once, outside
+  // the unrolled epilogue, so that the training form keeps its code.
+  if ((a.phase == 0 ? a.r : a.c) != nullptr)
+    conv_fwd_epilogue<NI, true>(a, acc, g0 * C, rows_valid, RG * CG, CG);
+  else
+    conv_fwd_epilogue<NI, false>(a, acc, g0 * C, rows_valid, RG * CG, CG);
 }
 
 static size_t conv_fwd_smem(const ConvArgs& a, const ConvTile& t) {
@@ -170,11 +180,10 @@ int launch_conv_fwd(const ConvArgs& a, cudaStream_t st) {
   STC_TRY(pick_rows_fwd(a, &t, &smem, &ni));
   long long total_nodes = (long long)a.B * a.N;
   int grid = ceil_div(total_nodes, t.npt);
-  // compulsory traffic per row: the Ks spatial terms of [x|h] once, then gates: write u, r, r*H;
-  // candidate: read u, H, write c, H'.  Plus the weights.
+  // compulsory traffic per row: the Ks spatial terms of [x|h] once, then the state traffic (conv_fwd_state_floats).
+  // Plus the weights.
   const double R = (double)total_nodes * a.C;
-  ScopedKernelTimer _t(KK_CONV_FWD, st,
-                       4.0 * R * (a.Ks * t.L + (a.phase == 0 ? 3 * a.h : 4 * a.h)) + 4.0 * a.Ks * a.Kc * t.L * a.Hout);
+  ScopedKernelTimer _t(KK_CONV_FWD, st, 4.0 * R * (a.Ks * t.L + conv_fwd_state_floats(a)) + 4.0 * a.Ks * a.Kc * t.L * a.Hout);
   switch (ni) {
     case 1: STC_TRY(set_smem(conv_fwd_kernel<1>, smem)); conv_fwd_kernel<1><<<grid, CV_THREADS, smem, st>>>(a, t); break;
     case 2: STC_TRY(set_smem(conv_fwd_kernel<2>, smem)); conv_fwd_kernel<2><<<grid, CV_THREADS, smem, st>>>(a, t); break;

@@ -224,9 +224,11 @@ __device__ __forceinline__ void tc_fwd_epilogue_fast(const ConvArgs& a, const Tc
         const int ch = col - h;
         const float4 h0 = *reinterpret_cast<const float4*>(stage_e + erow * h + ch);
         const float4 h1 = *reinterpret_cast<const float4*>(stage_e + erow * h + ch + 4);
-        float* dr = a.r + gr * h + ch;
-        *reinterpret_cast<float4*>(dr) = make_float4(v[g][0], v[g][1], v[g][2], v[g][3]);
-        *reinterpret_cast<float4*>(dr + 4) = make_float4(v[g][4], v[g][5], v[g][6], v[g][7]);
+        if (a.r) {   // null in a forward-only call: only the backward reads r
+          float* dr = a.r + gr * h + ch;
+          *reinterpret_cast<float4*>(dr) = make_float4(v[g][0], v[g][1], v[g][2], v[g][3]);
+          *reinterpret_cast<float4*>(dr + 4) = make_float4(v[g][4], v[g][5], v[g][6], v[g][7]);
+        }
         float* drh = a.rH + gr * h + ch;
         *reinterpret_cast<float4*>(drh) = make_float4(v[g][0] * h0.x, v[g][1] * h0.y, v[g][2] * h0.z, v[g][3] * h0.w);
         *reinterpret_cast<float4*>(drh + 4) = make_float4(v[g][4] * h1.x, v[g][5] * h1.y, v[g][6] * h1.z, v[g][7] * h1.w);
@@ -249,8 +251,10 @@ __device__ __forceinline__ void tc_fwd_epilogue_fast(const ConvArgs& a, const Tc
         cc[i] = tanhf_fast(v[g][i]);
         hn[i] = fmaf(uu[i], cc[i] - hp[i], hp[i]);
       }
-      *reinterpret_cast<float4*>(a.c + o) = make_float4(cc[0], cc[1], cc[2], cc[3]);
-      *reinterpret_cast<float4*>(a.c + o + 4) = make_float4(cc[4], cc[5], cc[6], cc[7]);
+      if (a.c) {   // null in a forward-only call: only the backward reads c
+        *reinterpret_cast<float4*>(a.c + o) = make_float4(cc[0], cc[1], cc[2], cc[3]);
+        *reinterpret_cast<float4*>(a.c + o + 4) = make_float4(cc[4], cc[5], cc[6], cc[7]);
+      }
       *reinterpret_cast<float4*>(a.Hnew + o) = make_float4(hn[0], hn[1], hn[2], hn[3]);
       *reinterpret_cast<float4*>(a.Hnew + o + 4) = make_float4(hn[4], hn[5], hn[6], hn[7]);
     }
@@ -514,9 +518,11 @@ tc_conv_fwd_kernel(const ConvArgs a, const TcFwdPlan p) {
             const long long o = gr * h + (c0 - h);
             const float4 h0 = *reinterpret_cast<const float4*>(stage_e + erow * h + (c0 - h));
             const float4 h1 = *reinterpret_cast<const float4*>(stage_e + erow * h + (c0 - h) + 4);
-            float4* dr = reinterpret_cast<float4*>(a.r + o);
-            dr[0] = make_float4(v[0], v[1], v[2], v[3]);
-            dr[1] = make_float4(v[4], v[5], v[6], v[7]);
+            if (a.r) {
+              float4* dr = reinterpret_cast<float4*>(a.r + o);
+              dr[0] = make_float4(v[0], v[1], v[2], v[3]);
+              dr[1] = make_float4(v[4], v[5], v[6], v[7]);
+            }
             float4* drh = reinterpret_cast<float4*>(a.rH + o);
             drh[0] = make_float4(v[0] * h0.x, v[1] * h0.y, v[2] * h0.z, v[3] * h0.w);
             drh[1] = make_float4(v[4] * h1.x, v[5] * h1.y, v[6] * h1.z, v[7] * h1.w);
@@ -533,9 +539,11 @@ tc_conv_fwd_kernel(const ConvArgs a, const TcFwdPlan p) {
             cc[i] = tanhf_fast(v[i]);
             hn[i] = fmaf(uu[i], cc[i] - hp[i], hp[i]);
           }
-          float4* dc = reinterpret_cast<float4*>(a.c + o);
-          dc[0] = make_float4(cc[0], cc[1], cc[2], cc[3]);
-          dc[1] = make_float4(cc[4], cc[5], cc[6], cc[7]);
+          if (a.c) {
+            float4* dc = reinterpret_cast<float4*>(a.c + o);
+            dc[0] = make_float4(cc[0], cc[1], cc[2], cc[3]);
+            dc[1] = make_float4(cc[4], cc[5], cc[6], cc[7]);
+          }
           float4* dh = reinterpret_cast<float4*>(a.Hnew + o);
           dh[0] = make_float4(hn[0], hn[1], hn[2], hn[3]);
           dh[1] = make_float4(hn[4], hn[5], hn[6], hn[7]);
@@ -648,9 +656,11 @@ __device__ __forceinline__ void tc_fwd_epilogue_regs(const ConvArgs& a, const Tc
         *reinterpret_cast<float4*>(dst + 4) = make_float4(v[g][4], v[g][5], v[g][6], v[g][7]);
       } else {
         const int ch = col - h;   // == cb
-        float* dr = a.r + gr * h + ch;
-        *reinterpret_cast<float4*>(dr) = make_float4(v[g][0], v[g][1], v[g][2], v[g][3]);
-        *reinterpret_cast<float4*>(dr + 4) = make_float4(v[g][4], v[g][5], v[g][6], v[g][7]);
+        if (a.r) {
+          float* dr = a.r + gr * h + ch;
+          *reinterpret_cast<float4*>(dr) = make_float4(v[g][0], v[g][1], v[g][2], v[g][3]);
+          *reinterpret_cast<float4*>(dr + 4) = make_float4(v[g][4], v[g][5], v[g][6], v[g][7]);
+        }
         float* drh = a.rH + gr * h + ch;
         *reinterpret_cast<float4*>(drh) = make_float4(v[g][0] * hpv[0], v[g][1] * hpv[1], v[g][2] * hpv[2], v[g][3] * hpv[3]);
         *reinterpret_cast<float4*>(drh + 4) = make_float4(v[g][4] * hpv[4], v[g][5] * hpv[5], v[g][6] * hpv[6], v[g][7] * hpv[7]);
@@ -665,8 +675,10 @@ __device__ __forceinline__ void tc_fwd_epilogue_regs(const ConvArgs& a, const Tc
       cc[i] = tanhf_fast(v[0][i]);
       hn[i] = fmaf(uuv[i], cc[i] - hpv[i], hpv[i]);
     }
-    *reinterpret_cast<float4*>(a.c + o) = make_float4(cc[0], cc[1], cc[2], cc[3]);
-    *reinterpret_cast<float4*>(a.c + o + 4) = make_float4(cc[4], cc[5], cc[6], cc[7]);
+    if (a.c) {
+      *reinterpret_cast<float4*>(a.c + o) = make_float4(cc[0], cc[1], cc[2], cc[3]);
+      *reinterpret_cast<float4*>(a.c + o + 4) = make_float4(cc[4], cc[5], cc[6], cc[7]);
+    }
     *reinterpret_cast<float4*>(a.Hnew + o) = make_float4(hn[0], hn[1], hn[2], hn[3]);
     *reinterpret_cast<float4*>(a.Hnew + o + 4) = make_float4(hn[4], hn[5], hn[6], hn[7]);
   }
@@ -951,8 +963,7 @@ int try_launch_conv_fwd_tc(const ConvArgs& a, cudaStream_t st, bool* handled) {
   int grid = device_sm_count() * ctas_per_sm;
   if (grid > p.ntiles) grid = p.ntiles;
   const double R = (double)total_nodes * a.C;
-  ScopedKernelTimer _t(KK_TC_CONV_FWD, st,
-                       4.0 * R * (a.Ks * L + (a.phase == 0 ? 3 * a.h : 4 * a.h)) + 4.0 * P * L * a.Hout);
+  ScopedKernelTimer _t(KK_TC_CONV_FWD, st, 4.0 * R * (a.Ks * L + conv_fwd_state_floats(a)) + 4.0 * P * L * a.Hout);
   kern<<<grid, CV_THREADS, p.smem_bytes, st>>>(a, p);
   STC_LAUNCH_OK("tc_conv_fwd_kernel");
   *handled = true;

@@ -391,9 +391,11 @@ tc_conv_fwd_big_kernel(const ConvArgs a, const BigPlan p, const uint8_t* __restr
             const long long o = gr * h + (c0 - h);
             const float4 h0 = *reinterpret_cast<const float4*>(a.Hprev + o);
             const float4 h1 = *reinterpret_cast<const float4*>(a.Hprev + o + 4);
-            float4* dr = reinterpret_cast<float4*>(a.r + o);
-            dr[0] = make_float4(v[0], v[1], v[2], v[3]);
-            dr[1] = make_float4(v[4], v[5], v[6], v[7]);
+            if (a.r) {   // null in a forward-only call: only the backward reads r
+              float4* dr = reinterpret_cast<float4*>(a.r + o);
+              dr[0] = make_float4(v[0], v[1], v[2], v[3]);
+              dr[1] = make_float4(v[4], v[5], v[6], v[7]);
+            }
             float4* drh = reinterpret_cast<float4*>(a.rH + o);
             drh[0] = make_float4(v[0] * h0.x, v[1] * h0.y, v[2] * h0.z, v[3] * h0.w);
             drh[1] = make_float4(v[4] * h1.x, v[5] * h1.y, v[6] * h1.z, v[7] * h1.w);
@@ -410,9 +412,11 @@ tc_conv_fwd_big_kernel(const ConvArgs a, const BigPlan p, const uint8_t* __restr
             cc[i] = tanhf_fast(v[i]);
             hn[i] = fmaf(uu[i], cc[i] - hp[i], hp[i]);
           }
-          float4* dc = reinterpret_cast<float4*>(a.c + o);
-          dc[0] = make_float4(cc[0], cc[1], cc[2], cc[3]);
-          dc[1] = make_float4(cc[4], cc[5], cc[6], cc[7]);
+          if (a.c) {   // likewise c
+            float4* dc = reinterpret_cast<float4*>(a.c + o);
+            dc[0] = make_float4(cc[0], cc[1], cc[2], cc[3]);
+            dc[1] = make_float4(cc[4], cc[5], cc[6], cc[7]);
+          }
           float4* dh = reinterpret_cast<float4*>(a.Hnew + o);
           dh[0] = make_float4(hn[0], hn[1], hn[2], hn[3]);
           dh[1] = make_float4(hn[4], hn[5], hn[6], hn[7]);
@@ -504,8 +508,7 @@ int try_launch_conv_fwd_big(const ConvArgs& a, cudaStream_t st, bool* handled) {
   if (grid > p.ntiles) grid = p.ntiles;
   const int L = a.Din + a.h, P = a.Ks * a.Kc;
   const double R = (double)total_nodes * a.C;
-  ScopedKernelTimer _t(KK_TC_CONV_FWD, st,
-                       4.0 * R * (a.Ks * L + (a.phase == 0 ? 3 * a.h : 4 * a.h)) + 4.0 * P * L * a.Hout);
+  ScopedKernelTimer _t(KK_TC_CONV_FWD, st, 4.0 * R * (a.Ks * L + conv_fwd_state_floats(a)) + 4.0 * P * L * a.Hout);
   tc_conv_fwd_big_kernel<<<grid, BG_FWD_THREADS, p.smem_bytes, st>>>(a, p, reinterpret_cast<const uint8_t*>(a.Wimg));
   STC_LAUNCH_OK("tc_conv_fwd_big_kernel");
   *handled = true;

@@ -689,70 +689,80 @@ def gather_edges(ps: PartitionedSupport, x_loc: torch.Tensor) -> torch.Tensor:
     return _GatherEdges.apply(x_loc, ps)
 
 
+def _partitioned_forward(Gc, Xt, Ht_1, Wg, bg, Wc, bc, cfg, fwd_only):
+    """The forward of one STC cell on this rank's node block: the node-local stages (`stc_cell_fwd_stage`, or
+    `stc_cell_fwd_only_stage` on the smaller forward-only workspace with `fwd_only`) with the spatial hops in between.
+    Returns (the local block of H', (Gc, Xe, He, Wg, Wc, buffer) as the stages read them, dims, buffer layout)."""
+    from . import _lib
+    from .cell import _activation_code, _ptr
+    ps, Ks, Kc, activation, reduce_params = cfg
+    lib = _lib.load()
+    ps.sync_values(Xt.device)        # learnable: the values as they are now (e.g. after an optimizer step)
+    B, n, C, Din = Xt.shape
+    h = Ht_1.shape[-1]
+    # Everything lives in the EXTENDED node set [local | halo]: the node-local stages simply run over
+    # nloc + nhalo nodes (the halo rows, ~1 % at k = 8, are recomputed garbage that the next exchange overwrites),
+    # so the spatial terms are written straight into the `saved` regions the stages read -- no slicing, no compaction.
+    ne = ps.fwd.next
+    Gc = Gc.detach().contiguous()
+    Wg, Wc = Wg.detach().contiguous(), Wc.detach().contiguous()
+    bg = bg.detach().contiguous() if bg is not None else None
+    bc = bc.detach().contiguous() if bc is not None else None
+    Xe = Xt.new_zeros(B, ne, C, Din)
+    Xe[:, :n] = Xt.detach()
+    He = Ht_1.new_zeros(B, ne, C, h)
+    He[:, :n] = Ht_1.detach()
+    dims = _lib.StcDims(B, ne, C, Din, h, Ks, Kc, _activation_code(activation), 1 if bg is not None else 0)
+    lay = _lib.saved_layout(dims, fwd_only)
+    nbytes = lib.stc_cell_fwd_only_bytes(dims) if fwd_only else lib.stc_cell_saved_bytes(dims)
+    saved = torch.empty(nbytes // 4, dtype=torch.float32, device=Xt.device)
+    Hn = torch.empty_like(He)
+    R = B * ne * C
+    stream = torch.cuda.current_stream().cuda_stream
+    run_stage, what = ((lib.stc_cell_fwd_only_stage, "stc_cell_fwd_only_stage") if fwd_only else
+                       (lib.stc_cell_fwd_stage, "stc_cell_fwd_stage"))
+
+    def region(name, k, width):
+        o = lay[name] + k * R * width
+        return saved[o:o + R * width].view(B, ne, C, width)
+
+    def stage(which):
+        _lib.check(run_stage(dims, which, Gc.data_ptr(), Xe.data_ptr(), ne * C * Din, He.data_ptr(), Wg.data_ptr(),
+                             _ptr(bg), Wc.data_ptr(), _ptr(bc), Hn.data_ptr(), saved.data_ptr(), saved.numel() * 4,
+                             stream), what)
+        _lib.note_launches()
+
+    def chain(term0, name, width, first):
+        """Y_1 = Gs^T Y_0, Y_k = 2 Gs^T Y_{k-1} - Y_{k-2} into regions `name`[first ...]."""
+        prev2, prev = None, term0
+        for k in range(1, Ks):
+            out = region(name, first + k - 1, width)
+            if k == 1:
+                ps.hop_ext(prev, out)
+            else:
+                ps.hop_ext(prev, out, Z_ext=prev2, alpha=2.0, beta=-1.0)
+            prev2, prev = prev, out
+
+    chain(Xe, "Yx", Din, 0)
+    chain(He, "Yh", h, 0)
+    stage(_lib.STAGE_GATES)
+    chain(region("Yr", 0, h), "Yr", h, 1)
+    stage(_lib.STAGE_CANDI)
+    return Hn[:, :n].contiguous(), (Gc, Xe, He, Wg, Wc, saved), dims, lay
+
+
 class _PartitionedCell(torch.autograd.Function):
     """One STC cell on this rank's node block; forward and backward are the C-ABI stages of include/stc_b200.h with
     the spatial hops (halo exchange + `stc_support_apply`) in between."""
 
     @staticmethod
     def forward(ctx, Gc, Xt, Ht_1, Wg, bg, Wc, bc, Ev, cfg):
-        from . import _lib
-        from .cell import _activation_code, _ptr
-        ps, Ks, Kc, activation, reduce_params = cfg
-        lib = _lib.load()
-        ps.sync_values(Xt.device)        # learnable: the values as they are now (e.g. after an optimizer step)
-        B, n, C, Din = Xt.shape
-        h = Ht_1.shape[-1]
-        # Everything lives in the EXTENDED node set [local | halo]: the node-local stages simply run over
-        # nloc + nhalo nodes (the halo rows, ~1 % at k = 8, are recomputed garbage that the next exchange overwrites),
-        # so the spatial terms are written straight into the `saved` regions the stages read -- no slicing, no compaction.
-        ne = ps.fwd.next
-        Gc = Gc.detach().contiguous()
-        Wg, Wc = Wg.detach().contiguous(), Wc.detach().contiguous()
-        bg = bg.detach().contiguous() if bg is not None else None
-        bc = bc.detach().contiguous() if bc is not None else None
-        Xe = Xt.new_zeros(B, ne, C, Din)
-        Xe[:, :n] = Xt.detach()
-        He = Ht_1.new_zeros(B, ne, C, h)
-        He[:, :n] = Ht_1.detach()
-        dims = _lib.StcDims(B, ne, C, Din, h, Ks, Kc, _activation_code(activation), 1 if bg is not None else 0)
-        lay = _lib.saved_layout(dims)
-        saved = torch.empty(lib.stc_cell_saved_bytes(dims) // 4, dtype=torch.float32, device=Xt.device)
-        Hn = torch.empty_like(He)
-        R = B * ne * C
-        stream = torch.cuda.current_stream().cuda_stream
-
-        def region(name, k, width):
-            o = lay[name] + k * R * width
-            return saved[o:o + R * width].view(B, ne, C, width)
-
-        def stage(which):
-            _lib.check(lib.stc_cell_fwd_stage(dims, which, Gc.data_ptr(), Xe.data_ptr(), ne * C * Din, He.data_ptr(),
-                                              Wg.data_ptr(), _ptr(bg), Wc.data_ptr(), _ptr(bc), Hn.data_ptr(),
-                                              saved.data_ptr(), saved.numel() * 4, stream), "stc_cell_fwd_stage")
-            _lib.note_launches()
-
-        def chain(term0, name, width, first):
-            """Y_1 = Gs^T Y_0, Y_k = 2 Gs^T Y_{k-1} - Y_{k-2} into regions `name`[first ...]."""
-            prev2, prev = None, term0
-            for k in range(1, Ks):
-                out = region(name, first + k - 1, width)
-                if k == 1:
-                    ps.hop_ext(prev, out)
-                else:
-                    ps.hop_ext(prev, out, Z_ext=prev2, alpha=2.0, beta=-1.0)
-                prev2, prev = prev, out
-
-        chain(Xe, "Yx", Din, 0)
-        chain(He, "Yh", h, 0)
-        stage(_lib.STAGE_GATES)
-        chain(region("Yr", 0, h), "Yr", h, 1)
-        stage(_lib.STAGE_CANDI)
-        ctx.cfg, ctx.dims, ctx.lay = cfg, dims, lay
+        Hn, ctx.keep, ctx.dims, ctx.lay = _partitioned_forward(Gc, Xt, Ht_1, Wg, bg, Wc, bc, cfg, fwd_only=False)
+        ctx.cfg = cfg
         ctx.has_bias = bg is not None
-        ctx.keep = (Gc, Xe, He, Wg, Wc, saved)
         # saved only so that autograd refuses a backward after an in-place change of the values
         ctx.save_for_backward(*([Ev] if Ev is not None else []))
-        return Hn[:, :n].contiguous()
+        return Hn
 
     @staticmethod
     @torch.autograd.function.once_differentiable
@@ -851,4 +861,8 @@ def partitioned_cell_forward(ps: PartitionedSupport, Gc: torch.Tensor, Xt: torch
         raise RuntimeError("partitioned cell: gates.b and candi.b must both be given or both be None")
     if B == 0:   # empty batch (the same on every rank: the batch is replicated, the nodes are split): nothing to exchange
         return Ht_1.new_zeros(0, n, C, h)
-    return _PartitionedCell.apply(Gc, Xt, Ht_1, Wg, bg, Wc, bc, ps.vals, (ps, Ks, Kc, activation, reduce_params))
+    cfg = (ps, Ks, Kc, activation, reduce_params)
+    from .cell import forward_only
+    if forward_only(Gc, Xt, Ht_1, Wg, bg, Wc, bc, ps.vals):   # no gradient can be asked for: no backward state
+        return _partitioned_forward(Gc, Xt, Ht_1, Wg, bg, Wc, bc, cfg, fwd_only=True)[0]
+    return _PartitionedCell.apply(Gc, Xt, Ht_1, Wg, bg, Wc, bc, ps.vals, cfg)
