@@ -41,7 +41,7 @@ typedef enum {
 } StcStatus;
 
 enum { STC_ACT_NONE = 0, STC_ACT_RELU = 1 };          /* BDG_Dif(activation=...), STC_GNN.py:13,46 */
-enum { STC_SUPPORT_DENSE = 0, STC_SUPPORT_CSR = 1 };
+enum { STC_SUPPORT_DENSE = 0, STC_SUPPORT_CSR = 1, STC_SUPPORT_CSR_PER_SAMPLE = 2 };
 
 /* Static shape of one cell call.  Mirrors STC_Cell.__init__ (STC_GNN.py:52-58) plus the batch. */
 typedef struct {
@@ -64,7 +64,13 @@ typedef struct {
  *          Column indices are int32; nnz < 2^31.
  *          The edge values may be learned: stc_cell_bwd then returns their gradient in Gs-CSR order (the order of
  *          `vals`, [nnz]) through its dGs argument; the sparsity pattern itself is fixed.  An edge stored with the
- *          value 0 is still an edge and gets a gradient. */
+ *          value 0 is still an edge and gets a gradient.
+ *   CSR per sample (STC_SUPPORT_CSR_PER_SAMPLE): the CSR fields, one pattern for the whole batch, but vals and t_vals
+ *          are [B][nnz] (sample b's values at b * nnz, B the call's batch): sample b is hopped with its own values in
+ *          every Chebyshev term, forward and adjoint.  Its edge gradient (dGs, dvals) is [B][nnz], row b that of
+ *          sample b's values; nothing is summed over the batch.  Taken by stc_cell_fwd / _fwd_x / _fwd_only,
+ *          stc_cell_bwd / _bwd_x, stc_support_apply and stc_support_apply_edge_grad; the row-list calls
+ *          (stc_support_apply_rows, stc_support_apply_rows_edge_grad) return STC_ERR_UNSUPPORTED. */
 typedef struct {
   int32_t kind;
   int64_t nnz;
@@ -121,7 +127,8 @@ int stc_cell_fwd_stage(const StcDims* d, int32_t stage, const float* gc,
  *   d_h_prev  [B][N][C][h]
  *   dWg,dbg,dWc,dbc  same shapes as the parameters (dbg/dbc NULL when has_bias == 0)
  *   dGs       dense support: [N][N];  CSR support: [nnz], the gradient w.r.t. the edge values `vals` (Gs-CSR
- *             order), computed inside the adjoint hops (stc_support_apply_edge_grad);  NULL: no support gradient
+ *             order), computed inside the adjoint hops (stc_support_apply_edge_grad);  per-sample CSR support:
+ *             [B][nnz];  NULL: no support gradient
  *   dGc       [C][C] or NULL
  *   accumulate_params != 0: parameter/support gradients are ADDED to the buffers' contents
  *   (lets a time loop accumulate dW over steps); == 0: they are overwritten.
@@ -200,7 +207,8 @@ int stc_support_outer(int32_t N, int32_t B, int32_t width, const float* a, int64
 size_t stc_support_outer_workspace_bytes(int32_t N, int32_t B, int32_t width);
 int stc_support_outer_ws(int32_t N, int32_t B, int32_t width, const float* a, int64_t a_batch_stride, const float* b,
                          float coef, float* dGs, void* ws, size_t ws_bytes, void* stream);
-/* The same gradient for a CSR support, sampled at its edges and fused into the adjoint hop (CSR only):
+/* The same gradient for a CSR support, sampled at its edges and fused into the adjoint hop (CSR only; for a per-sample
+ * support dvals is [B][nnz] and sample b's sums go to row b):
  *   y = alpha * Gs x + beta * z                                    (exactly what stc_support_apply, transpose = 0, writes)
  *   dvals[e] += coef * sum_{b,j} a[b][row(e)][j] * x[b][col(e)][j] (e walks Gs's CSR: rowptr / col / vals order)
  * x, z, y as in stc_support_apply; a [B][N][width] with its own batch stride (elements); dvals [nnz] is only added
@@ -242,6 +250,18 @@ int stc_pair_scores_csr_rows(const StcSupport* gs, int32_t N, int64_t width, int
 int stc_edge_softmax_fwd(const StcSupport* gs, int32_t N, const float* scores, float* p, void* stream);
 int stc_edge_softmax_bwd(const StcSupport* gs, int32_t N, const float* scores, const float* p, const float* dp,
                          float* dscores, void* stream);
+/* The same three per sample, over B samples at once on one pattern (the per-sample generator, one graph per input
+ * window; gs may be of either CSR kind, only rowptr / col are read):
+ *   stc_pair_scores_csr_batched   u, v [B][N][width] sample-major; scores [B][nnz], sample b bitwise what
+ *                                 stc_pair_scores_csr writes for u + b * N * width, v + b * N * width alone.
+ *   stc_edge_softmax_fwd_batched  / _bwd_batched: scores, p, dp, dscores [B][nnz]; row n of sample b normalised over
+ *                                 its own stored edges, each sample bitwise the unbatched call on its [nnz] slice.
+ * B == 0 launches nothing; B must be at most 65,535. */
+int stc_pair_scores_csr_batched(const StcSupport* gs, int32_t N, int32_t B, int64_t width, const float* u,
+                                const float* v, float* scores, void* stream);
+int stc_edge_softmax_fwd_batched(const StcSupport* gs, int32_t N, int32_t B, const float* scores, float* p, void* stream);
+int stc_edge_softmax_bwd_batched(const StcSupport* gs, int32_t N, int32_t B, const float* scores, const float* p,
+                                 const float* dp, float* dscores, void* stream);
 
 /* Top-k pair scores of the graph generator over ALL candidate columns (no pattern):
  *   S[n][m] = <u[n], v[m]> - <v[n], u[m]>  (3xTF32, S[n][n] = 0 exactly), u, v [N][width] row-major, width % 4 == 0,

@@ -12,7 +12,7 @@ LIB_PATH = os.path.join(HERE, "libstc_b200.so")
 
 ABI_VERSION = 7
 ACT_NONE, ACT_RELU = 0, 1
-SUPPORT_DENSE, SUPPORT_CSR = 0, 1
+SUPPORT_DENSE, SUPPORT_CSR, SUPPORT_CSR_PER_SAMPLE = 0, 1, 2
 
 # every symbol include/stc_b200.h declares (tests check the built library exports all of them)
 EXPORTED = (
@@ -28,6 +28,7 @@ EXPORTED = (
     "stc_pair_topk_rows_workspace_bytes", "stc_pair_topk_rows",
     "stc_deterministic_set", "stc_support_outer_workspace_bytes", "stc_support_outer_ws",
     "stc_cell_fwd_only_bytes", "stc_cell_fwd_only_layout", "stc_cell_fwd_only", "stc_cell_fwd_only_stage",
+    "stc_pair_scores_csr_batched", "stc_edge_softmax_fwd_batched", "stc_edge_softmax_bwd_batched",
 )
 STAGE_GATES, STAGE_CANDI = 0, 1
 SAVED_REGIONS = ("u", "r", "c", "Yr", "Yx", "Yh", "Q", "Pg", "Pc")
@@ -109,6 +110,14 @@ def load(build_if_missing: bool = True):
     lib.stc_edge_softmax_fwd.argtypes = [POINTER(StcSupport), c_int32, c_void_p, c_void_p, c_void_p]
     lib.stc_edge_softmax_bwd.restype = c_int
     lib.stc_edge_softmax_bwd.argtypes = [POINTER(StcSupport), c_int32, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]
+    lib.stc_pair_scores_csr_batched.restype = c_int
+    lib.stc_pair_scores_csr_batched.argtypes = [POINTER(StcSupport), c_int32, c_int32, c_int64, c_void_p, c_void_p,
+                                                c_void_p, c_void_p]
+    lib.stc_edge_softmax_fwd_batched.restype = c_int
+    lib.stc_edge_softmax_fwd_batched.argtypes = [POINTER(StcSupport), c_int32, c_int32, c_void_p, c_void_p, c_void_p]
+    lib.stc_edge_softmax_bwd_batched.restype = c_int
+    lib.stc_edge_softmax_bwd_batched.argtypes = [POINTER(StcSupport), c_int32, c_int32, c_void_p, c_void_p, c_void_p,
+                                                 c_void_p, c_void_p]
     lib.stc_cell_saved_layout.restype = c_int
     lib.stc_cell_saved_layout.argtypes = [POINTER(StcDims), POINTER(c_int64), c_int32]
     lib.stc_cell_fwd_stage.restype = c_int

@@ -144,10 +144,12 @@ def _run_forward(Gs, Gc, Xt, H, Wg, bg, Wc, bc, Yx, Ev, cfg, Yh, give, fwd_only)
     if csr:
         if Gs.N != N:
             raise RuntimeError(f"CSR support has {Gs.N} nodes, Xt has {N}")
+        if Gs.batch is not None and Gs.batch != B:
+            raise RuntimeError(f"per-sample CSR support has values for B = {Gs.batch} samples, Xt has B = {B}")
         if Ev is not None and Ev is not Gs.vals:
             raise RuntimeError("edge values passed to the cell must be the CsrSupport's own `vals`")
-        if Gs.learnable:   # the values may have changed since the last step (optimizer update, new with_values)
-            Gs.sync_t_vals()
+        if Gs.learnable or Gs.batch is not None:   # the values may have changed since the last step (optimizer update,
+            Gs.sync_t_vals()                       # new with_values, an in-place write)
         gs_struct = Gs.struct()
     else:
         if not Gs.is_cuda or Gs.dtype != torch.float32 or Gs.shape != (N, N):
@@ -287,8 +289,8 @@ class _CellFunction(torch.autograd.Function):
 
         dWg, dWc = target(4, (P * L, 2 * h)), target(6, (P * L, h))
         dbg, dbc = target(5, (2 * h,), ctx.has_bias), target(7, (h,), ctx.has_bias)
-        # a CSR support's gradient is that of its edge values: [nnz] in Gs-CSR order
-        dGs = target(9, (Gs.nnz,), need[9]) if ctx.csr else target(0, (N, N), need[0])
+        # a CSR support's gradient is that of its edge values: [nnz] in Gs-CSR order ([B, nnz] per sample)
+        dGs = target(9, tuple(Gs.vals.shape), need[9]) if ctx.csr else target(0, (N, N), need[0])
         dGc = target(1, (C, C), need[1])
         returned[2], returned[3], returned[8], returned[11] = dXt, dH, dYx, dYh
         if B == 0:  # empty batch: every parameter gradient is zero (the targets are zeroed or untouched), nothing to launch

@@ -421,6 +421,10 @@ int stc_support_apply_rows(const StcSupport* gs, int32_t N, int32_t B, int32_t w
     set_error("stc_support_apply_rows: NULL argument");
     return STC_ERR_BAD_ARG;
   }
+  if (gs->kind == STC_SUPPORT_CSR_PER_SAMPLE) {
+    set_error("stc_support_apply_rows: a per-sample CSR support (STC_SUPPORT_CSR_PER_SAMPLE) takes no row list");
+    return STC_ERR_UNSUPPORTED;
+  }
   if (n_rows < 0 || n_rows > N) {
     set_error("stc_support_apply_rows: n_rows %d outside [0, N = %d]", n_rows, N);
     return STC_ERR_BAD_ARG;
@@ -726,7 +730,7 @@ static int adjoint_chain(const StcDims& d, const StcSupport& gs, int width, cons
     float* yb_km1 = k == 1 ? ybar0 : ybark + (size_t)(k - 2) * Rw;
     float* axpy = nullptr;
     if (k >= 2) axpy = k == 2 ? ybar0 : ybark + (size_t)(k - 3) * Rw;
-    if (dGs && gs.kind == STC_SUPPORT_CSR) {
+    if (dGs && is_csr_kind(gs.kind)) {
       const float* yprev = k == 1 ? y0 : yk + (size_t)(k - 2) * Rw;
       const int64_t yprev_bs = k == 1 ? y0_bs : nbs;
       STC_TRY(launch_support_csr_edge_grad(gs, d.N, d.B, width, yb_k, nbs, yb_km1, nbs, yb_km1, coef, 1.f, axpy, -1.f,
@@ -920,7 +924,7 @@ static int cell_bwd_impl(const StcDims* dp, const StcSupport* gs, const float* g
     set_error("%s: NULL argument", who);
     return STC_ERR_BAD_ARG;
   }
-  if (dGs && gs->kind == STC_SUPPORT_CSR && (!gs->rowptr || !gs->col || !gs->vals || gs->nnz < 0)) {
+  if (dGs && is_csr_kind(gs->kind) && (!gs->rowptr || !gs->col || !gs->vals || gs->nnz < 0)) {
     set_error("%s: the edge-value gradient of a CSR support needs its rowptr/col/vals and nnz", who);
     return STC_ERR_BAD_ARG;
   }
@@ -949,7 +953,10 @@ static int cell_bwd_impl(const StcDims* dp, const StcSupport* gs, const float* g
     b.dyx_fold = dyx_fold;
     b.dyh_fold = dyh_fold;
   }
-  const size_t dGs_floats = gs->kind == STC_SUPPORT_CSR ? (size_t)gs->nnz : (size_t)d.N * d.N;
+  // a per-sample CSR support's gradient is [B][nnz]: one row per sample
+  const size_t dGs_floats = gs->kind == STC_SUPPORT_CSR_PER_SAMPLE ? (size_t)d.B * gs->nnz
+                            : gs->kind == STC_SUPPORT_CSR           ? (size_t)gs->nnz
+                                                                    : (size_t)d.N * d.N;
   STC_TRY(bwd_begin(b, dWg, dbg, dWc, dbc, dGs, dGs_floats, accumulate_params));
   if (d.B == 0) return STC_OK;
   const size_t Rh = w.R * d.h;
@@ -970,7 +977,7 @@ static int cell_bwd_impl(const StcDims* dp, const StcSupport* gs, const float* g
     cudaStream_t sx = st;
     // deterministic mode, learnable CSR support: both chains add their edge gradient into the same dGs in their hops,
     // so the Xt-side chain stays on the caller's stream, ordered after the H-side additions
-    const bool csr_grad = dGs && gs->kind == STC_SUPPORT_CSR;
+    const bool csr_grad = dGs && is_csr_kind(gs->kind);
     if (lanes.active() && d.Ks > 1 && !(det_mode() && csr_grad)) {
       STC_TRY(lanes.fork(2));
       sx = lanes.stream(2);
@@ -1054,7 +1061,7 @@ int stc_support_apply_edge_grad(const StcSupport* gs, int32_t N, int32_t B, int3
     set_error("stc_support_apply_edge_grad: NULL argument");
     return STC_ERR_BAD_ARG;
   }
-  if (gs->kind != STC_SUPPORT_CSR) {
+  if (!is_csr_kind(gs->kind)) {
     set_error("stc_support_apply_edge_grad: CSR supports only (a dense support's gradient is stc_support_outer)");
     return STC_ERR_UNSUPPORTED;
   }
@@ -1072,6 +1079,10 @@ int stc_support_apply_rows_edge_grad(const StcSupport* gs, int32_t N, int32_t B,
     set_error("stc_support_apply_rows_edge_grad: NULL argument");
     return STC_ERR_BAD_ARG;
   }
+  if (gs->kind == STC_SUPPORT_CSR_PER_SAMPLE) {
+    set_error("stc_support_apply_rows_edge_grad: a per-sample CSR support (STC_SUPPORT_CSR_PER_SAMPLE) takes no row list");
+    return STC_ERR_UNSUPPORTED;
+  }
   if (gs->kind != STC_SUPPORT_CSR) {
     set_error("stc_support_apply_rows_edge_grad: CSR supports only");
     return STC_ERR_UNSUPPORTED;
@@ -1085,12 +1096,12 @@ int stc_support_apply_rows_edge_grad(const StcSupport* gs, int32_t N, int32_t B,
                                       0.f, a, a_batch_stride, coef, dvals, (cudaStream_t)stream, rows, n_rows);
 }
 
-static int check_pattern(const StcSupport* gs, int32_t N, const char* who) {
+static int check_pattern(const StcSupport* gs, int32_t N, const char* who, bool any_csr = false) {
   if (!gs) {
     set_error("%s: NULL pattern", who);
     return STC_ERR_BAD_ARG;
   }
-  if (gs->kind != STC_SUPPORT_CSR) {
+  if (any_csr ? !is_csr_kind(gs->kind) : gs->kind != STC_SUPPORT_CSR) {
     set_error("%s: the pattern must be a CSR support (kind %d)", who, gs->kind);
     return STC_ERR_UNSUPPORTED;
   }
@@ -1168,6 +1179,59 @@ int stc_edge_softmax_bwd(const StcSupport* gs, int32_t N, const float* scores, c
   }
   STC_TRY(check_arch());
   return launch_edge_softmax(true, gs->rowptr, gs->nnz, N, scores, p, dp, dscores, (cudaStream_t)stream);
+}
+
+static int check_batch(int32_t B, const char* who) {
+  if (B < 0 || B > 65535) {
+    set_error("%s: B = %d outside [0, 65535]", who, B);
+    return STC_ERR_BAD_ARG;
+  }
+  return STC_OK;
+}
+
+int stc_pair_scores_csr_batched(const StcSupport* gs, int32_t N, int32_t B, int64_t width, const float* u,
+                                const float* v, float* scores, void* stream) {
+  reset_launch_count();
+  STC_TRY(check_pattern(gs, N, "stc_pair_scores_csr_batched", true));
+  STC_TRY(check_batch(B, "stc_pair_scores_csr_batched"));
+  if (B == 0) return STC_OK;
+  if (!u || !v || !scores) {
+    set_error("stc_pair_scores_csr_batched: NULL argument");
+    return STC_ERR_BAD_ARG;
+  }
+  if (width <= 0) {
+    set_error("stc_pair_scores_csr_batched: width = %lld must be positive", (long long)width);
+    return STC_ERR_BAD_ARG;
+  }
+  STC_TRY(check_arch());
+  return launch_pair_scores_csr_batched(gs->rowptr, gs->col, gs->nnz, N, B, width, u, v, scores, (cudaStream_t)stream);
+}
+
+int stc_edge_softmax_fwd_batched(const StcSupport* gs, int32_t N, int32_t B, const float* scores, float* p, void* stream) {
+  reset_launch_count();
+  STC_TRY(check_pattern(gs, N, "stc_edge_softmax_fwd_batched", true));
+  STC_TRY(check_batch(B, "stc_edge_softmax_fwd_batched"));
+  if (B == 0) return STC_OK;
+  if (!scores || !p) {
+    set_error("stc_edge_softmax_fwd_batched: NULL argument");
+    return STC_ERR_BAD_ARG;
+  }
+  STC_TRY(check_arch());
+  return launch_edge_softmax(false, gs->rowptr, gs->nnz, N, scores, nullptr, nullptr, p, (cudaStream_t)stream, B);
+}
+
+int stc_edge_softmax_bwd_batched(const StcSupport* gs, int32_t N, int32_t B, const float* scores, const float* p,
+                                 const float* dp, float* dscores, void* stream) {
+  reset_launch_count();
+  STC_TRY(check_pattern(gs, N, "stc_edge_softmax_bwd_batched", true));
+  STC_TRY(check_batch(B, "stc_edge_softmax_bwd_batched"));
+  if (B == 0) return STC_OK;
+  if (!scores || !p || !dp || !dscores) {
+    set_error("stc_edge_softmax_bwd_batched: NULL argument");
+    return STC_ERR_BAD_ARG;
+  }
+  STC_TRY(check_arch());
+  return launch_edge_softmax(true, gs->rowptr, gs->nnz, N, scores, p, dp, dscores, (cudaStream_t)stream, B);
 }
 
 static int check_topk_shape(int32_t N, int64_t width, int32_t k, const char* who) {

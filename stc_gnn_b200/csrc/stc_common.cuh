@@ -56,6 +56,10 @@ struct ScopedKernelTimer {  // declare right before a launch; the destructor rec
 
 static inline size_t round_up(size_t x, size_t m) { return (x + m - 1) / m * m; }
 static inline int ceil_div(long long a, long long b) { return (int)((a + b - 1) / b); }
+// batch stride in floats of a CSR support's vals / t_vals (and of its edge gradient): nnz for per-sample values, 0 when
+// every sample shares them
+static inline long long csr_vals_stride(const StcSupport& gs) { return gs.kind == STC_SUPPORT_CSR_PER_SAMPLE ? gs.nnz : 0; }
+static inline bool is_csr_kind(int kind) { return kind == STC_SUPPORT_CSR || kind == STC_SUPPORT_CSR_PER_SAMPLE; }
 
 // exact division of a 32-bit unsigned by a launch-invariant divisor: multiply-high + one correction step
 // (M = floor((2^(32+s) - 1) / d), s = floor(log2 d): the estimate is q or q - 1 for every n < 2^32)
@@ -155,8 +159,12 @@ int launch_pair_scores_csr(const int32_t* rowptr, const int32_t* col, long long 
 int launch_pair_scores_csr_rows(const int32_t* rowptr, const int32_t* col, long long nnz, int N, long long width,
                                 long long ld, const float* u, const float* v, float* scores, const int32_t* rows,
                                 int n_rows, cudaStream_t st);
+// the same per sample over B samples: u, v [B][N][width], scores [B][nnz]
+int launch_pair_scores_csr_batched(const int32_t* rowptr, const int32_t* col, long long nnz, int N, int B,
+                                   long long width, const float* u, const float* v, float* scores, cudaStream_t st);
+// B > 1: the B * N rows of [B][nnz] buffers (sample b at b * nnz)
 int launch_edge_softmax(bool bwd, const int32_t* rowptr, long long nnz, int N, const float* s, const float* p,
-                        const float* dp, float* out, cudaStream_t st);
+                        const float* dp, float* out, cudaStream_t st, int B = 1);
 // top-k pair scores of the rows [row0, row0 + n_rows) over all N columns (stc_pair_topk.cu); arguments checked by the
 // caller (1 <= k <= min(N, 32), width % 4 == 0, 0 <= row0, row0 + n_rows <= N, u / v 16-byte aligned, ws of
 // pair_topk_ws_bytes); n_rows == 0 launches nothing and needs no workspace

@@ -35,13 +35,18 @@ constexpr int PS_E = 4;   // edges of one group (8 spills at VEC = 4; the grid a
 // ROWS: only the n_rows rows listed in `rows` are scored (the other entries of `scores` are not touched), and U / V
 // have the row stride ld >= W, so that U and V can share one extended buffer [U | V] (the row-partitioned generator,
 // stc_gnn_b200/sparse_mgp.py).  A listed row's arithmetic is the plain kernel's, so its scores are bitwise the same.
+// blockIdx.y is the sample of a batched launch (the per-sample generator): U, V of sample s start s * s_bs floats in,
+// its scores s * nnz floats in; the arithmetic of each sample is that of the plain kernel on that sample alone.
 template <int VEC, bool ROWS>
 __global__ void __launch_bounds__(256)
 pair_scores_csr_kernel(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ col, int N, long long W,
                        const float* __restrict__ U, const float* __restrict__ V, float* __restrict__ scores,
-                       long long ld, const int32_t* __restrict__ rows, int n_rows) {
+                       long long ld, const int32_t* __restrict__ rows, int n_rows, long long s_bs, long long nnz) {
   constexpr long long CHUNK = 32LL * VEC * PS_U;
   const long long LD = ROWS ? ld : W;
+  U += blockIdx.y * s_bs;
+  V += blockIdx.y * s_bs;
+  scores += blockIdx.y * nnz;
   const int lane = threadIdx.x & 31;
   const long long warp0 = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const long long nwarps = ((long long)gridDim.x * blockDim.x) >> 5;
@@ -120,9 +125,26 @@ int launch_pair_scores_csr(const int32_t* rowptr, const int32_t* col, long long 
   // are L2 hits of rows other warps have just read.
   ScopedKernelTimer _t(KK_PAIR_SCORES_CSR, st,
                        4.0 * 2 * N * width + 4.0 * 2 * width * nnz + 8.0 * nnz + 4.0 * (N + 1) + 4.0 * nnz);
-  if (vec) pair_scores_csr_kernel<4, false><<<grid, 256, 0, st>>>(rowptr, col, N, width, u, v, scores, width, nullptr, 0);
-  else pair_scores_csr_kernel<1, false><<<grid, 256, 0, st>>>(rowptr, col, N, width, u, v, scores, width, nullptr, 0);
+  if (vec) pair_scores_csr_kernel<4, false><<<grid, 256, 0, st>>>(rowptr, col, N, width, u, v, scores, width, nullptr, 0, 0, 0);
+  else pair_scores_csr_kernel<1, false><<<grid, 256, 0, st>>>(rowptr, col, N, width, u, v, scores, width, nullptr, 0, 0, 0);
   STC_LAUNCH_OK("pair_scores_csr_kernel");
+  return STC_OK;
+}
+
+int launch_pair_scores_csr_batched(const int32_t* rowptr, const int32_t* col, long long nnz, int N, int B,
+                                   long long width, const float* u, const float* v, float* scores, cudaStream_t st) {
+  if (B <= 0) return STC_OK;
+  // each sample's rows start N * width floats after the previous sample's, so the vector form is taken exactly when the
+  // unbatched call on sample 0 takes it and every sample then starts 16-byte aligned
+  const bool vec = (width % 4 == 0) && aligned16(u) && aligned16(v);
+  const dim3 grid(csr_warp_grid(N, 8), B);
+  const long long s_bs = (long long)N * width;
+  // the unbatched count, per sample (the pattern itself is read once)
+  ScopedKernelTimer _t(KK_PAIR_SCORES_CSR, st,
+                       (double)B * (4.0 * 2 * N * width + 4.0 * 2 * width * nnz + 4.0 * nnz) + 8.0 * nnz + 4.0 * (N + 1));
+  if (vec) pair_scores_csr_kernel<4, false><<<grid, 256, 0, st>>>(rowptr, col, N, width, u, v, scores, width, nullptr, 0, s_bs, nnz);
+  else pair_scores_csr_kernel<1, false><<<grid, 256, 0, st>>>(rowptr, col, N, width, u, v, scores, width, nullptr, 0, s_bs, nnz);
+  STC_LAUNCH_OK("pair_scores_csr_kernel<batched>");
   return STC_OK;
 }
 
@@ -137,15 +159,16 @@ int launch_pair_scores_csr_rows(const int32_t* rowptr, const int32_t* col, long 
   const double er = (double)nnz * n_rows / N;
   ScopedKernelTimer _t(KK_PAIR_SCORES_CSR, st,
                        4.0 * 2 * n_rows * width + 4.0 * 2 * width * er + 4.0 * er + 8.0 * n_rows + 4.0 * er + 4.0 * n_rows);
-  if (vec) pair_scores_csr_kernel<4, true><<<grid, 256, 0, st>>>(rowptr, col, N, width, u, v, scores, ld, rows, n_rows);
-  else pair_scores_csr_kernel<1, true><<<grid, 256, 0, st>>>(rowptr, col, N, width, u, v, scores, ld, rows, n_rows);
+  if (vec) pair_scores_csr_kernel<4, true><<<grid, 256, 0, st>>>(rowptr, col, N, width, u, v, scores, ld, rows, n_rows, 0, 0);
+  else pair_scores_csr_kernel<1, true><<<grid, 256, 0, st>>>(rowptr, col, N, width, u, v, scores, ld, rows, n_rows, 0, 0);
   STC_LAUNCH_OK("pair_scores_csr_kernel<rows>");
   return STC_OK;
 }
 
 // ------------------------------------------------------------------------------------------------
 // softmax over the stored edges of each row: one warp per row, lanes stride over the row's edges, row sums through an
-// xor-shuffle tree (fixed order).  An empty row writes nothing.
+// xor-shuffle tree (fixed order).  An empty row writes nothing.  The rows are the B * N rows of [B][nnz] buffers (row
+// b * N + n is row n of sample b, whose entries start b * nnz in); B = 1 is the unbatched softmax.
 // ------------------------------------------------------------------------------------------------
 __device__ __forceinline__ float warp_sum(float s) {
 #pragma unroll
@@ -155,39 +178,42 @@ __device__ __forceinline__ float warp_sum(float s) {
 
 template <bool BWD>
 __global__ void __launch_bounds__(256)
-edge_softmax_kernel(const int32_t* __restrict__ rowptr, int N, const float* __restrict__ S,
+edge_softmax_kernel(const int32_t* __restrict__ rowptr, int N, long long rows, long long nnz, const float* __restrict__ S,
                     const float* __restrict__ P, const float* __restrict__ dP, float* __restrict__ out) {
   const int lane = threadIdx.x & 31;
   const long long warp0 = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const long long nwarps = ((long long)gridDim.x * blockDim.x) >> 5;
-  for (long long n = warp0; n < N; n += nwarps) {
-    const int e0 = rowptr[n], e1 = rowptr[n + 1];
+  for (long long r = warp0; r < rows; r += nwarps) {
+    const long long b = r / N, n = r - b * N;
+    const long long e0 = rowptr[n] + b * nnz, e1 = rowptr[n + 1] + b * nnz;
     if (e0 >= e1) continue;
     if (BWD) {   // dS = [S > 0] * P * (dP - sum_row P dP)
       float dot = 0.f;
-      for (int e = e0 + lane; e < e1; e += 32) dot = fmaf(P[e], dP[e], dot);
+      for (long long e = e0 + lane; e < e1; e += 32) dot = fmaf(P[e], dP[e], dot);
       dot = warp_sum(dot);
-      for (int e = e0 + lane; e < e1; e += 32) out[e] = S[e] > 0.f ? P[e] * (dP[e] - dot) : 0.f;
+      for (long long e = e0 + lane; e < e1; e += 32) out[e] = S[e] > 0.f ? P[e] * (dP[e] - dot) : 0.f;
     } else {     // P = exp(relu(S) - max) / sum, the max subtracted as torch.softmax does
       float mx = 0.f;   // relu(S) >= 0
-      for (int e = e0 + lane; e < e1; e += 32) mx = fmaxf(mx, S[e]);
+      for (long long e = e0 + lane; e < e1; e += 32) mx = fmaxf(mx, S[e]);
 #pragma unroll
       for (int o = 16; o > 0; o >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
       float sum = 0.f;
-      for (int e = e0 + lane; e < e1; e += 32) sum += expf(fmaxf(S[e], 0.f) - mx);
+      for (long long e = e0 + lane; e < e1; e += 32) sum += expf(fmaxf(S[e], 0.f) - mx);
       const float inv = 1.f / warp_sum(sum);
-      for (int e = e0 + lane; e < e1; e += 32) out[e] = expf(fmaxf(S[e], 0.f) - mx) * inv;
+      for (long long e = e0 + lane; e < e1; e += 32) out[e] = expf(fmaxf(S[e], 0.f) - mx) * inv;
     }
   }
 }
 
 int launch_edge_softmax(bool bwd, const int32_t* rowptr, long long nnz, int N, const float* s, const float* p,
-                        const float* dp, float* out, cudaStream_t st) {
-  const int grid = csr_warp_grid(N, 8);
-  // compulsory: the pattern's rowptr, then S in / P out (forward) or S, P, dP in / dS out (backward)
-  ScopedKernelTimer _t(KK_EDGE_SOFTMAX, st, 4.0 * (N + 1) + (bwd ? 16.0 : 8.0) * nnz);
-  if (bwd) edge_softmax_kernel<true><<<grid, 256, 0, st>>>(rowptr, N, s, p, dp, out);
-  else edge_softmax_kernel<false><<<grid, 256, 0, st>>>(rowptr, N, s, nullptr, nullptr, out);
+                        const float* dp, float* out, cudaStream_t st, int B) {
+  if (B <= 0) return STC_OK;
+  const long long rows = (long long)B * N;
+  const int grid = csr_warp_grid(rows, 8);
+  // compulsory: the pattern's rowptr, then S in / P out (forward) or S, P, dP in / dS out (backward), per sample
+  ScopedKernelTimer _t(KK_EDGE_SOFTMAX, st, 4.0 * (N + 1) + (bwd ? 16.0 : 8.0) * nnz * B);
+  if (bwd) edge_softmax_kernel<true><<<grid, 256, 0, st>>>(rowptr, N, rows, nnz, s, p, dp, out);
+  else edge_softmax_kernel<false><<<grid, 256, 0, st>>>(rowptr, N, rows, nnz, s, nullptr, nullptr, out);
   STC_LAUNCH_OK("edge_softmax_kernel");
   return STC_OK;
 }

@@ -5,6 +5,8 @@
 //  support_csr_kernel    same operator for a CSR support (one warp per (batch, node) row slab).  GRAD = true: the
 //                        adjoint hop with the gradient of the edge values fused in (learnable CSR supports),
 //                        dvals[e = (n,m)] += coef * sum_{b,j} A[b,n,j] * X[b,m,j]; Y is computed exactly as without it.
+//                        PS = true: per-sample values (vals [B][nnz]); sample b is hopped with vals + b * nnz and,
+//                        with GRAD, its edge gradient goes to dvals + b * nnz (no sum over the batch).
 //  support_outer_kernel  dGs[n',m] += coef * sum_{b,j} A[b,n',j] * Bm[b,m,j]  (gradient of the spatial
 //                        mode product w.r.t. the support; reference gets it from autograd of :37).
 //  cheby_small_*         matrix-space Chebyshev terms of the small C x C categorical support and their
@@ -137,16 +139,16 @@ struct CsrEdgeGrad {
   const float* a;   // [B][N][W], batch stride a_bs (elements)
   long long a_bs;
   float coef;
-  float* dvals;     // [nnz], in the order of the walked CSR (rowptr / col)
+  float* dvals;     // [nnz] ([B][nnz] per-sample), in the order of the walked CSR (rowptr / col)
 };
 
-template <int VEC, bool GRAD>
+template <int VEC, bool GRAD, bool PS = false>
 __global__ void __launch_bounds__(256)
 support_csr_kernel(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ col,
                    const float* __restrict__ vals, int N, long long rows_total, const float* __restrict__ X,
                    long long x_bs, const float* Z, long long z_bs, float* Y, int W, float alpha, float beta,
                    float* axpy_out, float axpy_coef, const int32_t* __restrict__ row_list, int n_list,
-                   CsrEdgeGrad eg) {
+                   CsrEdgeGrad eg, long long v_bs) {
   // row_list != nullptr: only the n_list output nodes it names are computed (rows_total = B * n_list); the other
   // rows of Y are not touched (the row-partitioned path computes interior rows while the halo exchange is in flight);
   // with GRAD only the edges of the listed rows get a gradient, and A is read at the listed rows only
@@ -161,6 +163,8 @@ support_csr_kernel(const int32_t* __restrict__ rowptr, const int32_t* __restrict
     const int m = row_list ? row_list[mi] : mi;
     const int e0 = rowptr[m], e1 = rowptr[m + 1];
     const float* xb = X + b * x_bs;
+    const float* vb = PS ? vals + b * v_bs : vals;   // (v_bs = nnz: the values and their gradient of sample b)
+    float* dvb = (GRAD && PS) ? eg.dvals + b * v_bs : eg.dvals;
     for (int j0 = 0; j0 < W; j0 += 32 * VEC * U) {
       float acc[U][VEC];
 #pragma unroll
@@ -186,7 +190,7 @@ support_csr_kernel(const int32_t* __restrict__ rowptr, const int32_t* __restrict
         }
       }
       for (int e = e0; e < e1; ++e) {
-        const float g = vals[e];
+        const float g = vb[e];
         const float* xr = xb + (long long)col[e] * W;
         float dot = 0.f;
 #pragma unroll
@@ -216,7 +220,7 @@ support_csr_kernel(const int32_t* __restrict__ rowptr, const int32_t* __restrict
         if (GRAD) {
 #pragma unroll
           for (int o = 16; o > 0; o >>= 1) dot += __shfl_xor_sync(0xffffffffu, dot, o);
-          if (lane == 0) atomicAdd(eg.dvals + e, eg.coef * dot);
+          if (lane == 0) atomicAdd(dvb + e, eg.coef * dot);
         }
       }
 #pragma unroll
@@ -252,35 +256,42 @@ static bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 
 // Deterministic form of the edge-value gradient: one warp owns a row n and ALL of its edges' sums, over every sample and
 // feature in a fixed order (lane-strided partial sums, then a shuffle tree), so every dvals[e] has exactly one writer:
 //   dvals[e = (n, m)] += coef * sum_{b,j} a[b,n,j] * x[b,m,j]
+// PS: per-sample values; one warp per (b, n) and one writer per (b, e) of dvals [B][nnz] (no row list), each sample's
+// sums in the order the B = 1 call takes them:  dvals[b][e] += coef * sum_j a[b,n,j] * x[b,m,j]
+template <bool PS = false>
 __global__ void __launch_bounds__(256)
 csr_edge_grad_det_kernel(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ col,
                          const int32_t* __restrict__ row_list, int n_rows, int B, int W, const float* __restrict__ X,
-                         long long x_bs, const float* __restrict__ A, long long a_bs, float coef, float* dvals) {
+                         long long x_bs, const float* __restrict__ A, long long a_bs, float coef, float* dvals,
+                         long long v_bs) {
   const int lane = threadIdx.x & 31;
   const long long warp0 = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const long long nwarps = ((long long)gridDim.x * blockDim.x) >> 5;
-  for (long long r = warp0; r < n_rows; r += nwarps) {
-    const int n = row_list ? row_list[r] : (int)r;
+  for (long long r = warp0; r < (PS ? (long long)B * n_rows : n_rows); r += nwarps) {
+    const int bs = PS ? (int)(r / n_rows) : 0;
+    const int n = PS ? (int)(r - (long long)bs * n_rows) : (row_list ? row_list[r] : (int)r);
+    float* dv = PS ? dvals + bs * v_bs : dvals;
     for (int e = rowptr[n]; e < rowptr[n + 1]; ++e) {
       const long long m = col[e];
       float dot = 0.f;
-      for (int b = 0; b < B; ++b) {
+      for (int b = PS ? bs : 0; b < (PS ? bs + 1 : B); ++b) {
         const float* ar = A + b * a_bs + (long long)n * W;
         const float* xr = X + b * x_bs + m * W;
         for (int j = lane; j < W; j += 32) dot = fmaf(ar[j], xr[j], dot);
       }
 #pragma unroll
       for (int o = 16; o > 0; o >>= 1) dot += __shfl_xor_sync(0xffffffffu, dot, o);
-      if (lane == 0) dvals[e] += coef * dot;
+      if (lane == 0) dv[e] += coef * dot;
     }
   }
 }
 
-// one CSR hop (rp, ci, va walk the rows of the operator applied); eg.dvals != nullptr selects the edge-gradient variant
+// one CSR hop (rp, ci, va walk the rows of the operator applied); eg.dvals != nullptr selects the edge-gradient variant;
+// v_bs: the batch stride of va (and of eg.dvals) in floats, 0 for values shared by every sample, nnz for per-sample ones
 static int launch_csr(const int32_t* rp, const int32_t* ci, const float* va, long long nnz, int N, int B, int width,
                       const float* x, int64_t x_bs, const float* z, int64_t z_bs, float* y, float alpha, float beta,
                       float* axpy_out, float axpy_coef, const int32_t* row_list, int n_list, const CsrEdgeGrad& eg,
-                      cudaStream_t st) {
+                      cudaStream_t st, long long v_bs = 0) {
   const bool grad = eg.dvals != nullptr;
   long long rows_total = (long long)B * (row_list ? n_list : N);
   bool vec = (width % 4 == 0) && (x_bs % 4 == 0) && (z == nullptr || z_bs % 4 == 0) && aligned16(x) &&
@@ -291,19 +302,31 @@ static int launch_csr(const int32_t* rp, const int32_t* ci, const float* va, lon
   int grid = (int)(want < (long long)device_sm_count() * 16 ? want : (long long)device_sm_count() * 16);
   if (grid < 1) grid = 1;
   // compulsory traffic of the hop; the edge-gradient variant also reads the row's own slab of A and updates dvals
-  const double hop = 4.0 * rows_total * width * (2 + (beta != 0.f ? 1 : 0) + (axpy_out ? 2 : 0)) + 8.0 * nnz + 4.0 * (N + 1);
-  ScopedKernelTimer _t(grad ? KK_SUPPORT_CSR_GRAD : KK_SUPPORT_CSR, st, grad ? hop + 4.0 * rows_total * width + 4.0 * nnz : hop);
+  // (per-sample values: B value vectors and B gradient vectors, one pattern)
+  const double vals_bytes = 4.0 * nnz * (v_bs ? B : 1);
+  const double hop = 4.0 * rows_total * width * (2 + (beta != 0.f ? 1 : 0) + (axpy_out ? 2 : 0)) + 4.0 * nnz +
+                     vals_bytes + 4.0 * (N + 1);
+  ScopedKernelTimer _t(grad ? KK_SUPPORT_CSR_GRAD : KK_SUPPORT_CSR, st, grad ? hop + 4.0 * rows_total * width + vals_bytes : hop);
   const dim3 blk(warps_per_block * 32);
-#define STC_CSR_LAUNCH(V, G)                                                                                        \
-  support_csr_kernel<V, G><<<grid, blk, 0, st>>>(rp, ci, va, N, rows_total, x, x_bs, z, z_bs, y, width, alpha, beta, \
-                                                 axpy_out, axpy_coef, row_list, n_list, eg)
-  if (grad) {
-    if (vec) STC_CSR_LAUNCH(4, true);
-    else STC_CSR_LAUNCH(1, true);
+#define STC_CSR_LAUNCH(V, G, P)                                                                                         \
+  support_csr_kernel<V, G, P><<<grid, blk, 0, st>>>(rp, ci, va, N, rows_total, x, x_bs, z, z_bs, y, width, alpha, beta, \
+                                                    axpy_out, axpy_coef, row_list, n_list, eg, v_bs)
+  if (v_bs) {
+    if (grad) {
+      if (vec) STC_CSR_LAUNCH(4, true, true);
+      else STC_CSR_LAUNCH(1, true, true);
+    } else {
+      if (vec) STC_CSR_LAUNCH(4, false, true);
+      else STC_CSR_LAUNCH(1, false, true);
+    }
+    STC_LAUNCH_OK("support_csr_kernel<per-sample>");
+  } else if (grad) {
+    if (vec) STC_CSR_LAUNCH(4, true, false);
+    else STC_CSR_LAUNCH(1, true, false);
     STC_LAUNCH_OK("support_csr_kernel<grad>");
   } else {
-    if (vec) STC_CSR_LAUNCH(4, false);
-    else STC_CSR_LAUNCH(1, false);
+    if (vec) STC_CSR_LAUNCH(4, false, false);
+    else STC_CSR_LAUNCH(1, false, false);
     STC_LAUNCH_OK("support_csr_kernel");
   }
 #undef STC_CSR_LAUNCH
@@ -315,6 +338,11 @@ int launch_support_apply(const StcSupport& gs, int N, int B, int width, bool tra
                          float* axpy_out, float axpy_coef, cudaStream_t st, const int32_t* row_list, int n_list) {
   if (B <= 0 || N <= 0 || width <= 0) return STC_OK;
   if (row_list) {
+    if (gs.kind == STC_SUPPORT_CSR_PER_SAMPLE) {
+      set_error("support_apply: a row list is not supported for a per-sample CSR support (STC_SUPPORT_CSR_PER_SAMPLE); "
+                "the row-partitioned path shares one set of edge values over the batch");
+      return STC_ERR_UNSUPPORTED;
+    }
     if (n_list <= 0) return STC_OK;
     if (gs.kind != STC_SUPPORT_CSR) {
       set_error("support_apply: a row list is only supported for a CSR support");
@@ -363,7 +391,7 @@ int launch_support_apply(const StcSupport& gs, int N, int B, int width, bool tra
     STC_LAUNCH_OK("support_dense_kernel");
     return STC_OK;
   }
-  if (gs.kind != STC_SUPPORT_CSR) {
+  if (gs.kind != STC_SUPPORT_CSR && gs.kind != STC_SUPPORT_CSR_PER_SAMPLE) {
     set_error("unknown support kind %d", gs.kind);
     return STC_ERR_BAD_ARG;
   }
@@ -375,7 +403,7 @@ int launch_support_apply(const StcSupport& gs, int N, int B, int width, bool tra
     return STC_ERR_BAD_ARG;
   }
   return launch_csr(rp, ci, va, gs.nnz, N, B, width, x, x_bs, z, z_bs, y, alpha, beta, axpy_out, axpy_coef, row_list,
-                    n_list, CsrEdgeGrad{nullptr, 0, 0.f, nullptr}, st);
+                    n_list, CsrEdgeGrad{nullptr, 0, 0.f, nullptr}, st, csr_vals_stride(gs));
 }
 
 int launch_support_csr_edge_grad(const StcSupport& gs, int N, int B, int width, const float* x, int64_t x_bs,
@@ -383,11 +411,17 @@ int launch_support_csr_edge_grad(const StcSupport& gs, int N, int B, int width, 
                                  float axpy_coef, const float* a, int64_t a_bs, float coef, float* dvals,
                                  cudaStream_t st, const int32_t* row_list, int n_list) {
   if (B <= 0 || N <= 0 || width <= 0) return STC_OK;
+  if (row_list && gs.kind == STC_SUPPORT_CSR_PER_SAMPLE) {
+    set_error("support edge gradient: a row list is not supported for a per-sample CSR support "
+              "(STC_SUPPORT_CSR_PER_SAMPLE)");
+    return STC_ERR_UNSUPPORTED;
+  }
   if (row_list && n_list <= 0) return STC_OK;
-  if (gs.kind != STC_SUPPORT_CSR || !gs.rowptr || !gs.col || !gs.vals) {
+  if ((gs.kind != STC_SUPPORT_CSR && gs.kind != STC_SUPPORT_CSR_PER_SAMPLE) || !gs.rowptr || !gs.col || !gs.vals) {
     set_error("support edge gradient: needs a CSR support with rowptr/col/vals");
     return STC_ERR_BAD_ARG;
   }
+  const long long v_bs = csr_vals_stride(gs);
   if (!a || !dvals) {
     set_error("support edge gradient: NULL a or dvals");
     return STC_ERR_BAD_ARG;
@@ -398,18 +432,24 @@ int launch_support_csr_edge_grad(const StcSupport& gs, int N, int B, int width, 
   }
   if (det_mode()) {   // the plain hop (y bitwise that of stc_support_apply), then the one-writer edge gradient
     STC_TRY(launch_csr(gs.rowptr, gs.col, gs.vals, gs.nnz, N, B, width, x, x_bs, z, z_bs, y, alpha, beta, axpy_out,
-                       axpy_coef, row_list, n_list, CsrEdgeGrad{nullptr, 0, 0.f, nullptr}, st));
+                       axpy_coef, row_list, n_list, CsrEdgeGrad{nullptr, 0, 0.f, nullptr}, st, v_bs));
     const int rows = row_list ? n_list : N;
-    long long blocks = (rows + 7) / 8;
+    const long long warps = v_bs ? (long long)B * rows : rows;
+    long long blocks = (warps + 7) / 8;
     if (blocks > (long long)device_sm_count() * 16) blocks = (long long)device_sm_count() * 16;
-    ScopedKernelTimer _t(KK_SUPPORT_CSR_GRAD, st, 4.0 * (double)B * width * (rows + gs.nnz) + 8.0 * gs.nnz);
-    csr_edge_grad_det_kernel<<<(int)blocks, 256, 0, st>>>(gs.rowptr, gs.col, row_list, rows, B, width, x, x_bs, a, a_bs,
-                                                           coef, dvals);
+    ScopedKernelTimer _t(KK_SUPPORT_CSR_GRAD, st,
+                         4.0 * (double)B * width * (rows + gs.nnz) + 4.0 * gs.nnz + 4.0 * gs.nnz * (v_bs ? B : 1));
+    if (v_bs)
+      csr_edge_grad_det_kernel<true><<<(int)blocks, 256, 0, st>>>(gs.rowptr, gs.col, nullptr, rows, B, width, x, x_bs, a,
+                                                                  a_bs, coef, dvals, v_bs);
+    else
+      csr_edge_grad_det_kernel<false><<<(int)blocks, 256, 0, st>>>(gs.rowptr, gs.col, row_list, rows, B, width, x, x_bs, a,
+                                                                   a_bs, coef, dvals, 0);
     STC_LAUNCH_OK("csr_edge_grad_det_kernel");
     return STC_OK;
   }
   return launch_csr(gs.rowptr, gs.col, gs.vals, gs.nnz, N, B, width, x, x_bs, z, z_bs, y, alpha, beta, axpy_out,
-                    axpy_coef, row_list, n_list, CsrEdgeGrad{a, (long long)a_bs, coef, dvals}, st);
+                    axpy_coef, row_list, n_list, CsrEdgeGrad{a, (long long)a_bs, coef, dvals}, st, v_bs);
 }
 
 // ------------------------------------------------------------------------------------------------

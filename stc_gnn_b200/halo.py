@@ -234,6 +234,9 @@ class PartitionedSupport:
     @classmethod
     def from_csr_support(cls, cs, rank: int, world: int, group=None) -> "PartitionedSupport":
         """The partition of a `CsrSupport`; a learnable one shares its `vals` (the same tensor, not a copy)."""
+        if getattr(cs, "batch", None) is not None:
+            raise RuntimeError("PartitionedSupport.from_csr_support: per-sample edge values [B, nnz] are not supported "
+                               "on the row-partitioned graph (one set of values is shared by the batch)")
         return cls(cs.rowptr, cs.col, cs.vals, cs.N, rank, world, group)
 
     @classmethod
@@ -252,6 +255,9 @@ class PartitionedSupport:
         return self.vals is not None
 
     def _check_values(self, vals: torch.Tensor) -> torch.Tensor:
+        if vals.dim() == 2:
+            raise RuntimeError(f"PartitionedSupport: per-sample edge values {tuple(vals.shape)} are not supported on the "
+                               f"row-partitioned graph; give one [nnz] vector (nnz = {self.nnz}) shared by the batch")
         if vals.dim() != 1 or vals.numel() != self.nnz:
             raise RuntimeError(f"PartitionedSupport: edge values must be a [nnz] vector in Gs-CSR order "
                                f"(nnz = {self.nnz}), got shape {tuple(vals.shape)}")

@@ -50,6 +50,17 @@ all-gathers the [N, k] selection and partitions it on the device (`RowPartition.
 copy), then forms P exactly as on a fixed partitioned pattern.  Scores of unrelated nodes pick neighbours anywhere in
 the graph, so the halo of a selected pattern can approach every remote node: each hop then moves close to an
 all-gather.
+
+Per sample (`gen(X_seq, pattern, per_sample=True)`): the scores are not summed over the batch, so each input window gets
+its own graph on the shared pattern, independent of which other windows share its batch:
+
+    S_b[e] = sum_{t,h} U[b,t,n,h] V[b,t,m,h] - V[b,t,n,h] U[b,t,m,h]      P[b, e] = softmax of relu(S_b) over row n
+
+U, V are laid out [B, N, T*hg]; stc_pair_scores_csr_batched and stc_edge_softmax_*_batched run every sample in one
+launch, each bitwise the unbatched kernel on that sample alone, so P[b] is bitwise `gen(X_seq[b:b+1], pattern).vals`.
+The result is a per-sample `CsrSupport` (values [B, nnz]); the backward is the same four hops, per sample.  Nothing
+is communicated: under batch data-parallelism each rank generates its own samples' graphs, and the Wu / Wv gradients
+are the shard's partial sums for `dp.GradBucket`.
 """
 from __future__ import annotations
 
@@ -76,15 +87,23 @@ def _check_pattern(pattern, N: int, who: str) -> None:
 
 
 class _PairScores(torch.autograd.Function):
-    """S[e] = <U_n, V_m> - <V_n, U_m> at the pattern's stored edges; U, V [N, width]."""
+    """S[e] = <U_n, V_m> - <V_n, U_m> at the pattern's stored edges; U, V [N, width] -> S [nnz], or per sample
+    U, V [B, N, width] -> S [B, nnz]."""
 
     @staticmethod
     def forward(ctx, U, V, pattern):
         lib = _lib.load()
-        N, width = U.shape
-        S = torch.empty(pattern.nnz, dtype=torch.float32, device=U.device)
-        _lib.check(lib.stc_pair_scores_csr(pattern.struct(), N, width, U.data_ptr(), V.data_ptr(), S.data_ptr(),
-                                           torch.cuda.current_stream().cuda_stream), "stc_pair_scores_csr")
+        stream = torch.cuda.current_stream().cuda_stream
+        if U.dim() == 3:
+            B, N, width = U.shape
+            S = torch.empty(B, pattern.nnz, dtype=torch.float32, device=U.device)
+            _lib.check(lib.stc_pair_scores_csr_batched(pattern.struct(), N, B, width, U.data_ptr(), V.data_ptr(),
+                                                       S.data_ptr(), stream), "stc_pair_scores_csr_batched")
+        else:
+            N, width = U.shape
+            S = torch.empty(pattern.nnz, dtype=torch.float32, device=U.device)
+            _lib.check(lib.stc_pair_scores_csr(pattern.struct(), N, width, U.data_ptr(), V.data_ptr(), S.data_ptr(),
+                                               stream), "stc_pair_scores_csr")
         ctx.save_for_backward(U, V)
         ctx.pattern = pattern
         return S
@@ -94,9 +113,11 @@ class _PairScores(torch.autograd.Function):
         U, V = ctx.saved_tensors
         D = ctx.pattern.with_values(dS.detach())
 
-        def skew(A, sign):   # sign * (D - D^T) A, as [N, width]
-            Y = support_apply(D, A[None], transpose=False, alpha=sign)
-            return support_apply(D, A[None], transpose=True, alpha=-sign, beta=1.0, Z=Y, out=Y)[0]
+        def skew(A, sign):   # sign * (D - D^T) A, as [N, width] (per sample: [B, N, width], D carrying dS[b])
+            X = A if A.dim() == 3 else A[None]
+            Y = support_apply(D, X, transpose=False, alpha=sign)
+            Y = support_apply(D, X, transpose=True, alpha=-sign, beta=1.0, Z=Y, out=Y)
+            return Y if A.dim() == 3 else Y[0]
 
         dU = skew(V, 1.0) if ctx.needs_input_grad[0] else None
         dV = skew(U, -1.0) if ctx.needs_input_grad[1] else None
@@ -104,14 +125,19 @@ class _PairScores(torch.autograd.Function):
 
 
 class _EdgeSoftmax(torch.autograd.Function):
-    """P = softmax of relu(S) over each row's stored edges."""
+    """P = softmax of relu(S) over each row's stored edges (S [nnz], or [B, nnz]: each sample's rows on their own)."""
 
     @staticmethod
     def forward(ctx, S, pattern):
         lib = _lib.load()
         P = torch.empty_like(S)
-        _lib.check(lib.stc_edge_softmax_fwd(pattern.struct(), pattern.N, S.data_ptr(), P.data_ptr(),
-                                            torch.cuda.current_stream().cuda_stream), "stc_edge_softmax_fwd")
+        stream = torch.cuda.current_stream().cuda_stream
+        if S.dim() == 2:
+            _lib.check(lib.stc_edge_softmax_fwd_batched(pattern.struct(), pattern.N, S.shape[0], S.data_ptr(),
+                                                        P.data_ptr(), stream), "stc_edge_softmax_fwd_batched")
+        else:
+            _lib.check(lib.stc_edge_softmax_fwd(pattern.struct(), pattern.N, S.data_ptr(), P.data_ptr(), stream),
+                       "stc_edge_softmax_fwd")
         ctx.save_for_backward(S, P)
         ctx.pattern = pattern
         return P
@@ -121,9 +147,14 @@ class _EdgeSoftmax(torch.autograd.Function):
         S, P = ctx.saved_tensors
         dPc = dP.contiguous()
         dS = torch.empty_like(S)
-        _lib.check(_lib.load().stc_edge_softmax_bwd(ctx.pattern.struct(), ctx.pattern.N, S.data_ptr(), P.data_ptr(),
-                                                    dPc.data_ptr(), dS.data_ptr(),
-                                                    torch.cuda.current_stream().cuda_stream), "stc_edge_softmax_bwd")
+        stream = torch.cuda.current_stream().cuda_stream
+        if S.dim() == 2:
+            _lib.check(_lib.load().stc_edge_softmax_bwd_batched(ctx.pattern.struct(), ctx.pattern.N, S.shape[0],
+                                                                S.data_ptr(), P.data_ptr(), dPc.data_ptr(), dS.data_ptr(),
+                                                                stream), "stc_edge_softmax_bwd_batched")
+        else:
+            _lib.check(_lib.load().stc_edge_softmax_bwd(ctx.pattern.struct(), ctx.pattern.N, S.data_ptr(), P.data_ptr(),
+                                                        dPc.data_ptr(), dS.data_ptr(), stream), "stc_edge_softmax_bwd")
         return dS, None
 
 
@@ -137,18 +168,28 @@ def pair_softmax_csr(U: torch.Tensor, V: torch.Tensor, pattern: CsrSupport, grou
     columns) the partial scores are summed over the ranks before the softmax (`mgp.sum_forward`) and the gradient
     arriving at P is all-reduced (`mgp.reduce_grad`), as `mgp.mgp_forward_dp` does for the dense generator: every rank
     gets the global-batch P, and the gradients of what produced U, V are this shard's partial sums for the caller's
-    `dp.GradBucket` (`average`: the bucket is averaged).  [nnz] floats are communicated each way."""
+    `dp.GradBucket` (`average`: the bucket is averaged).  [nnz] floats are communicated each way.
+
+    Per sample: U, V [B, N, width] (sample-major) give P [B, nnz], row b the softmax of sample b's own scores, bitwise
+    what U[b], V[b] alone give.  Nothing is summed over the batch, so no process group is taken."""
     for name, t in (("U", U), ("V", V)):
-        if not t.is_cuda or t.dtype != torch.float32 or t.dim() != 2:
-            raise RuntimeError(f"pair_softmax_csr: {name} must be a [N, width] float32 CUDA tensor (there is no CPU "
-                               f"path), got {tuple(t.shape)} {t.dtype} on {t.device}")
+        if not t.is_cuda or t.dtype != torch.float32 or t.dim() not in (2, 3):
+            raise RuntimeError(f"pair_softmax_csr: {name} must be a [N, width] or [B, N, width] float32 CUDA tensor "
+                               f"(there is no CPU path), got {tuple(t.shape)} {t.dtype} on {t.device}")
     if U.shape != V.shape or U.device != V.device:
         raise RuntimeError(f"pair_softmax_csr: U {tuple(U.shape)} on {U.device} and V {tuple(V.shape)} on {V.device} "
                            f"must match")
-    _check_pattern(pattern, U.shape[0], "pair_softmax_csr")
+    if U.dim() == 3 and (group is not None or average):
+        raise RuntimeError("pair_softmax_csr: per-sample scores ([B, N, width]) are not summed over the batch, so there "
+                           "is nothing to reduce over a process group (group= / average=)")
+    _check_pattern(pattern, U.shape[-2], "pair_softmax_csr")
+    if isinstance(pattern, PartitionedSupport) and U.dim() == 3:
+        raise RuntimeError("pair_softmax_csr: per-sample scores are not supported on a row-partitioned pattern")
     if pattern.device != U.device:
         raise RuntimeError(f"pair_softmax_csr: the pattern lives on {pattern.device}, U on {U.device}")
     S = _PairScores.apply(U.contiguous(), V.contiguous(), pattern)
+    if U.dim() == 3:   # (sum_forward / reduce_grad with group=None would reduce over the default group)
+        return _EdgeSoftmax.apply(S, pattern)
     S = mgp.sum_forward(S, group, average)
     return mgp.reduce_grad(_EdgeSoftmax.apply(S, pattern), group, average)
 
@@ -339,7 +380,7 @@ class SparseGraphGenerator(nn.Module):
             nn.init.xavier_normal_(p)
 
     def forward(self, X_seq: torch.Tensor, pattern=None, group=None, average: bool = False, k: int = None,
-                partition: halo.RowPartition = None):
+                partition: halo.RowPartition = None, per_sample: bool = False):
         """X_seq [B, T, N, C] float32 CUDA -> `pattern.with_values(P)`.  Under torch.no_grad() the values do not require
         grad and the cell treats the support as constant.  `group` / `average`: batch data-parallel, as in
         `pair_softmax_csr` (X_seq is this rank's shard).
@@ -361,9 +402,25 @@ class SparseGraphGenerator(nn.Module):
         (`pair_topk(..., rows=(start, nloc))`), the [N, k] selection is all-gathered and partitioned on the device
         (`partition.support`), and P is formed on it exactly as on a fixed partitioned pattern (gradients, the Wu / Wv
         reduction by `partition.reduce_per_cell`, the no-grad path).  The result is a `PartitionedSupport`; every rank
-        runs the forward and the backward."""
+        runs the forward and the backward.
+
+        `per_sample=True`: one graph per input window (module docstring).  Returns `pattern.with_values(P)` with P
+        [B, nnz], a per-sample `CsrSupport`; P[b] is bitwise `forward(X_seq[b:b+1], pattern).vals`.  Takes a fixed
+        `CsrSupport` pattern only: not `k=`, `partition=`, a `PartitionedSupport`, nor `group=` / `average=`."""
         Wu, Wv = self.params_S["Wu"], self.params_S["Wv"]
         partitioned = isinstance(pattern, PartitionedSupport)
+        if per_sample:
+            if k is not None or partition is not None:
+                raise RuntimeError("SparseGraphGenerator: per_sample=True takes a fixed pattern: per-sample top-k "
+                                   "(k= / partition=) would give every sample its own pattern, which is not supported")
+            if partitioned:
+                raise RuntimeError("SparseGraphGenerator: per_sample=True is not supported on a row-partitioned pattern "
+                                   "(halo.PartitionedSupport): its edge values are shared by the batch")
+            if group is not None or average:
+                raise RuntimeError("SparseGraphGenerator: per_sample=True sums nothing over the batch, so batch "
+                                   "data-parallelism needs no communication in the generator: drop group= / average= "
+                                   "(each rank generates its own samples' graphs; reduce the Wu / Wv gradients with "
+                                   "dp.GradBucket as for every other parameter)")
         if partition is not None:
             if not isinstance(partition, halo.RowPartition):
                 raise RuntimeError(f"SparseGraphGenerator: partition must be a halo.RowPartition, got "
@@ -412,6 +469,11 @@ class SparseGraphGenerator(nn.Module):
         rows_split = pattern if partitioned else partition
         if rows_split is not None and rows_split.reduce_per_cell and rows_split.world > 1:
             Wu, Wv = mgp.reduce_grad(Wu, rows_split.group), mgp.reduce_grad(Wv, rows_split.group)
+        if per_sample:   # sample-major [B, N, T*hg]: sample b's rows are exactly the B = 1 generator's U, V
+            Xb = X_seq.permute(0, 2, 1, 3).reshape(B, N, T, C)
+            U = torch.tanh(self.alpha * (Xb @ Wu)).reshape(B, N, -1)
+            V = torch.tanh(self.alpha * (Xb @ Wv)).reshape(B, N, -1)
+            return pattern.with_values(pair_softmax_csr(U, V, pattern))
         Xn = X_seq.permute(2, 0, 1, 3).reshape(N, B * T, C)       # node-major copy of the small input
         U = torch.tanh(self.alpha * (Xn @ Wu)).reshape(N, -1)      # [N, B*T*hg], contiguous
         V = torch.tanh(self.alpha * (Xn @ Wv)).reshape(N, -1)

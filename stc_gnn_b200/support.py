@@ -19,6 +19,11 @@ class CsrSupport:
     ``t_perm`` maps Gs-CSR order to Gs^T-CSR order (``t_vals = vals[t_perm]``); the cell re-gathers ``t_vals`` before
     each forward, so an in-place update of ``vals`` is seen by the next step.  ``with_values(v)`` gives a support
     that shares the structure and the permutation with new values (values recomputed every step).
+
+    Per-sample values: ``vals`` of shape [B, nnz] (constant or learnable) gives one graph per input window on the shared
+    pattern.  Sample b of a cell call is hopped with ``vals[b]`` (the call's batch must be B, `batch`), and the edge
+    gradient is [B, nnz], row b that of ``vals[b]``.  ``t_vals = vals[:, t_perm]`` is re-gathered before each forward.
+    The row-partitioned graph, the row-list hops and dense supports take no per-sample values.
     """
 
     def __init__(self, rowptr: torch.Tensor, col: torch.Tensor, vals: torch.Tensor, num_nodes: int):
@@ -31,6 +36,15 @@ class CsrSupport:
         self.nnz = int(self.vals.numel())
         self.device = self.vals.device
         self.t_perm, self._t_struct = None, None
+        if self.vals.dim() == 2:   # per-sample values [B, nnz] on one pattern
+            self.nnz = int(self.col.numel())
+            if self.vals.shape[1] != self.nnz or self.nnz != int(self.rowptr[-1].item()):
+                raise RuntimeError(f"CsrSupport: per-sample values must be [B, nnz] in the order of `col` "
+                                   f"(nnz = {self.col.numel()}), got shape {tuple(self.vals.shape)}")
+            self.t_rowptr, self.t_col, self.t_perm = self._transpose_structure()
+            self.t_vals = torch.empty_like(self.vals, requires_grad=False)
+            self.sync_t_vals()
+            return
         if self.vals.requires_grad:
             if self.vals.dim() != 1 or self.nnz != self.col.numel() or self.nnz != int(self.rowptr[-1].item()):
                 raise RuntimeError(f"CsrSupport: learnable values must be a [nnz] vector in the order of `col` "
@@ -65,23 +79,29 @@ class CsrSupport:
         """True when the edge values require grad (the cell then returns / accumulates their gradient)."""
         return self.vals.requires_grad
 
+    @property
+    def batch(self):
+        """B of per-sample values [B, nnz] (one graph per sample of a cell call's batch); None for shared values."""
+        return self.vals.shape[0] if self.vals.dim() == 2 else None
+
     def sync_t_vals(self) -> None:
-        """t_vals = vals[t_perm] into the persistent Gs^T buffer, on the current stream (a CUDA-graph capture
+        """t_vals = vals[..., t_perm] into the persistent Gs^T buffer, on the current stream (a CUDA-graph capture
         records the gather, so a replay sees the values as they are then)."""
         if self.t_perm is not None:
-            torch.index_select(self.vals.detach(), 0, self.t_perm, out=self.t_vals)
+            torch.index_select(self.vals.detach(), self.vals.dim() - 1, self.t_perm, out=self.t_vals)
 
     def with_values(self, vals: torch.Tensor) -> "CsrSupport":
-        """A support with this one's pattern (and Gs^T permutation) and new edge values [nnz] (Gs-CSR order)."""
+        """A support with this one's pattern (and Gs^T permutation) and new edge values (Gs-CSR order): [nnz] shared by
+        every sample, or [B, nnz] per sample."""
         v = vals.to(torch.float32).contiguous()
-        if v.device != self.device or v.shape != (self.nnz,):
-            raise RuntimeError(f"CsrSupport.with_values: values must be a [{self.nnz}] vector on {self.device}, got "
-                               f"{tuple(v.shape)} on {v.device}")
+        if v.device != self.device or v.dim() not in (1, 2) or v.shape[-1] != self.nnz:
+            raise RuntimeError(f"CsrSupport.with_values: values must be [{self.nnz}] or [B, {self.nnz}] on {self.device}, "
+                               f"got {tuple(v.shape)} on {v.device}")
         out = CsrSupport.__new__(CsrSupport)
         out.N, out.rowptr, out.col, out.vals, out.nnz, out.device = self.N, self.rowptr, self.col, v, self.nnz, self.device
         out._t_struct = self._transpose_structure()
         out.t_rowptr, out.t_col, out.t_perm = out._t_struct
-        out.t_vals = torch.empty(self.nnz, dtype=torch.float32, device=self.device)
+        out.t_vals = torch.empty(v.shape, dtype=torch.float32, device=self.device)
         out.sync_t_vals()
         return out
 
@@ -110,11 +130,14 @@ class CsrSupport:
         return cls(s.crow_indices(), s.col_indices(), s.values(), G.shape[0])
 
     def to_dense(self) -> torch.Tensor:
+        """Gs [N, N] ([B, N, N] for per-sample values)."""
+        if self.batch is not None:
+            return torch.stack([self.with_values(v).to_dense() for v in self.vals])
         return torch.sparse_csr_tensor(self.rowptr.long(), self.col.long(), self.vals, size=(self.N, self.N)).to_dense()
 
     def struct(self) -> _lib.StcSupport:
         s = _lib.StcSupport()
-        s.kind = _lib.SUPPORT_CSR
+        s.kind = _lib.SUPPORT_CSR if self.batch is None else _lib.SUPPORT_CSR_PER_SAMPLE
         s.nnz = self.nnz
         s.vals, s.rowptr, s.col = self.vals.data_ptr(), self.rowptr.data_ptr(), self.col.data_ptr()
         s.t_vals, s.t_rowptr, s.t_col = self.t_vals.data_ptr(), self.t_rowptr.data_ptr(), self.t_col.data_ptr()
@@ -137,6 +160,12 @@ def k_regular_structure(cols: torch.Tensor):
     t_rowptr = torch.zeros(N + 1, dtype=torch.int64, device=dev)
     t_rowptr[1:] = torch.cumsum(counts, 0)
     return rowptr, col, t_rowptr.to(torch.int32).contiguous(), row[t_perm].to(torch.int32).contiguous(), t_perm
+
+
+def _check_batch(Gs: CsrSupport, B: int, who: str) -> None:
+    if Gs.batch is not None and Gs.batch != B:
+        raise RuntimeError(f"{who}: the per-sample CsrSupport has values for B = {Gs.batch} samples, the input has "
+                           f"B = {B}")
 
 
 def dense_struct(G: torch.Tensor) -> _lib.StcSupport:
@@ -165,6 +194,9 @@ def support_apply(Gs, X: torch.Tensor, transpose: bool = True, alpha: float = 1.
     else:
         Y = torch.empty_like(Xc)
     if isinstance(Gs, CsrSupport):
+        _check_batch(Gs, B, "support_apply")
+        if rows is not None and Gs.batch is not None:
+            raise RuntimeError("support_apply: `rows` is not supported for a per-sample CsrSupport (values [B, nnz])")
         if transpose:
             Gs.sync_t_vals()
         st = Gs.struct()
@@ -207,9 +239,14 @@ def support_apply_edge_grad(Gs: CsrSupport, X: torch.Tensor, A: torch.Tensor, dv
     for name, t in (("X", X), ("A", A), ("dvals", dvals)):
         if not t.is_cuda or t.dtype != torch.float32:
             raise RuntimeError(f"support_apply_edge_grad: {name} must be a float32 CUDA tensor")
-    if dvals.shape != (Gs.nnz,) or not dvals.is_contiguous():
-        raise RuntimeError(f"support_apply_edge_grad: dvals must be a contiguous [{Gs.nnz}] tensor")
     B, N = X.shape[0], X.shape[1]
+    _check_batch(Gs, B, "support_apply_edge_grad")
+    want = (Gs.nnz,) if Gs.batch is None else (B, Gs.nnz)
+    if dvals.shape != want or not dvals.is_contiguous():
+        raise RuntimeError(f"support_apply_edge_grad: dvals must be a contiguous {list(want)} tensor")
+    if rows is not None and Gs.batch is not None:
+        raise RuntimeError("support_apply_edge_grad: `rows` is not supported for a per-sample CsrSupport "
+                           "(values [B, nnz])")
     Xc = X.contiguous()
     width = Xc[0, 0].numel() if Xc.numel() else 0
     if A.shape != X.shape:
